@@ -3,6 +3,7 @@
 trajectory x agent x step evaluations / s; p50 per-planning-step latency).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c-sweep|c-lat]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the dense metric core over the whole synthetic sweep bundle
 (C-sweep: 1,000,000 trajectories x 256 phantom agents x 50 steps, all seven metrics), split by
@@ -333,6 +334,20 @@ def run_ours(args):
     evals_total = N_total * A * (T - 1)
     ms, launches, clocks, kern_ms = timed(step_resident, args.steps, args.warmup, sample_clocks=True, per_step_events=True)
     value = evals_total * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # what the last timed step returned, taken before the e2e calls below write into the same buffers, so that two
+        # builds can be compared output for output.  flags (u32 bit masks) go to float64, which holds every value
+        # exactly; C-sweep writes 4 + 40 + 8 MB.  The files hold finite numbers only, and the summary's special values
+        # map without loss: +inf (min_dce / wttc when there is none) becomes the float32 maximum, which no real value
+        # reaches, and NaN (the two BE columns of a trajectory flagged FO_F_BE_RANGE, as flags.npy records) becomes 0
+        if gatherer is not None:
+            gatherer.current_result()
+            valid, summary, flags = gatherer.assembled()          # global trajectory order
+        else:
+            valid, summary, flags = out.valid, out.summary, out.flags
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t, dtype in (("valid", valid, np.float32), ("summary", summary, np.float32), ("flags", flags, np.float64)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), np.nan_to_num(t.cpu().numpy().astype(dtype)))
     e2e_how = ""
     if world == 1:
         # the reference-facing C-ABI call with HOST buffers: fo_metric_bundle_host copies the bundle and the raw
@@ -839,7 +854,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--no-stages", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result arrays of the last timed step as DIR/<name>.npy (same arguments, same inputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     _quiet_stdout()
     if args.impl == "reference":
         run_reference(args)

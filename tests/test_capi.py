@@ -72,10 +72,13 @@ def test_hot_kernels_stay_inside_the_instruction_cache_budget():
     import shutil
     import subprocess
     import pytest
+    from torch.utils.cpp_extension import CUDA_HOME
     from frenetix_occlusion_b200 import _lib as L
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
-    sass = subprocess.run(["cuobjdump", "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
+    # the toolkit that built the library has it, whether or not its bin/ is on PATH
+    cuobjdump = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
+    if not cuobjdump:
+        pytest.skip("cuobjdump not found (no CUDA toolkit)")
+    sass = subprocess.run([cuobjdump, "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
     sizes, name = {}, None
     for line in sass.splitlines():
         m = re.search(r"Function : (\S+)", line)
@@ -86,7 +89,7 @@ def test_hot_kernels_stay_inside_the_instruction_cache_budget():
     # cold helpers that live in the kernel's text section but not in its hot set: the float64 re-rounding of
     # np.round(d, 3) ties runs for a fraction of a per cent of the exact distance evaluations
     cold = {}
-    elf = subprocess.run(["cuobjdump", "-elf", L.LIB_PATH], capture_output=True, text=True).stdout
+    elf = subprocess.run([cuobjdump, "-elf", L.LIB_PATH], capture_output=True, text=True).stdout
     for line in elf.splitlines():
         m = re.match(r"\s*0x[0-9a-f]+\s+0x[0-9a-f]+\s+(0x[0-9a-f]+)\s+.*\$(_ZN\S+?)\$(_ZN\S+)", line)
         if m and ("obb_round_mm_f64" in m.group(3) or "sincos_f64_of_f32" in m.group(3)):

@@ -62,6 +62,16 @@ class FoMetricArgs(C.Structure):
                 ("n_peers", C.c_int32), ("reserved_", C.c_int32), ("peer_delta", C.c_int64 * FO_MAX_PEERS)]
 
 
+class FoBatchProblem(C.Structure):
+    _fields_ = [("traj_begin", C.c_int64), ("n_traj", C.c_int32), ("n_agents", C.c_int32), ("t_stride", C.c_int32),
+                ("reserved_", C.c_int32), ("table_offset", C.c_int64)]
+
+
+class FoMetricBatchArgs(C.Structure):
+    _fields_ = [("common", FoMetricArgs), ("n_problems", C.c_int32), ("reserved_", C.c_int32),
+                ("problems", C.POINTER(FoBatchProblem)), ("arena_bytes", C.c_size_t)]
+
+
 class FoPeerHandle(C.Structure):
     _fields_ = [("bytes", C.c_uint8 * 64)]
 
@@ -150,6 +160,10 @@ _PROTOS = {
     "fo_metric_bundle_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(FoAgentsRaw),
                                         C.POINTER(FoMetricArgs), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_void_p]),
+    "fo_agent_batch_layout": (C.c_size_t, [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fo_agents_pack_batch": (C.c_int, [C.POINTER(FoAgentsRaw), C.c_int32, C.POINTER(FoBatchProblem),
+                                       C.POINTER(FoVehicle), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "fo_metric_batch": (C.c_int, [C.POINTER(FoMetricBatchArgs), C.c_void_p]),
     "fo_visibility_raycast": (C.c_int, [C.POINTER(FoVisibilityArgs), C.c_void_p]),
     "fo_visibility_stats": (C.c_int, [C.POINTER(FoVisibilityArgs), C.c_void_p, C.c_void_p]),
     "fo_visibility_points": (C.c_int, [C.POINTER(FoPointQueryArgs), C.c_void_p]),

@@ -30,8 +30,23 @@ __device__ __forceinline__ int protection_model(int kind) {  // harm_model.py:15
   }
 }
 
-// Slot order: stable sort by harm model.  One CTA; A is a few hundred at most, so the O(A^2) rank count is free.
-__global__ void fo_agents_order_kernel(const int32_t* __restrict__ kind, int A, int Ap, int32_t* orig, int32_t* slot) {
+// One problem of a packing launch: its agents are rows [a_begin, a_begin + A) of the raw arrays (row stride
+// raw.t_stride), its table (stride Tp) starts table_off bytes into the arena.  fo_agents_pack is the one-problem case.
+struct PackProblem {
+  int a_begin, A, Tp, pad_;
+  long long table_off;
+};
+
+// Slot order: stable sort by harm model.  One CTA per problem; A is a few hundred at most, so the O(A^2) rank count is free.
+__global__ void fo_agents_order_kernel(const int32_t* __restrict__ kind_all, PackProblem one, const PackProblem* many,
+                                       unsigned char* arena) {
+  const PackProblem pp = many ? many[blockIdx.x] : one;
+  const int A = pp.A;
+  const AgentTableView v = agent_table_view(arena + pp.table_off, A, pp.Tp);
+  const int Ap = v.Ap;
+  int32_t* orig = const_cast<int32_t*>(v.orig);
+  int32_t* slot = const_cast<int32_t*>(v.slot);
+  const int32_t* kind = kind_all + pp.a_begin;
   for (int a = threadIdx.x; a < Ap; a += blockDim.x) {
     if (a >= A) { orig[a] = -1; slot[a] = a; continue; }      // padding slots keep their place behind the real ones
 #ifdef FO_NO_SORT
@@ -48,71 +63,151 @@ __global__ void fo_agents_order_kernel(const int32_t* __restrict__ kind, int A, 
   }
 }
 
-__global__ void fo_agents_pack_kernel(FoAgentsRaw raw, float m_ego, float4* s0, float4* s1, float2* s2, AgentParams* prm,
-                                      float4* t0, float* tv, float* tpsi, float4* aw, float* avw,
-                                      const int32_t* __restrict__ orig, const int32_t* __restrict__ slot, int Ap) {
+// one thread per (agent slot, state) of a problem; blockIdx.y strides over the problems
+__global__ void fo_agents_pack_kernel(FoAgentsRaw raw, float m_ego, PackProblem one, const PackProblem* many, int P,
+                                      unsigned char* arena) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  const int A = raw.n_agents, Tp = raw.t_stride;
-  const int nW = agent_windows(Tp);
-  if (idx < Ap * nW) {                       // window boxes for the summary kernel's filter (slot order)
-    const int sl = idx / nW, wi = idx - sl * nW;
-    float xl = 1e30f, xh = -1e30f, yl = 1e30f, yh = -1e30f, vm = 0.0f;
-    if (sl < A) {
-      const int a = orig[sl];
-      const int nS = min(raw.n_states[a], Tp);
-      const int lo = wi * kWinSteps;
-      for (int i = max(lo - 1, 0); i < min(lo + kWinSteps, nS); ++i) {
-        const float x = raw.x[a * Tp + i], y = raw.y[a * Tp + i];
-        xl = fminf(xl, x); xh = fmaxf(xh, x); yl = fminf(yl, y); yh = fmaxf(yh, y);
-        if (i >= lo) vm = fmaxf(vm, fabsf(raw.v[a * Tp + i]));
+  const int S = raw.t_stride;
+  for (int p = blockIdx.y; p < P; p += gridDim.y) {
+    const PackProblem pp = many ? many[p] : one;
+    const int A = pp.A, Tp = pp.Tp;
+    const AgentTableView v = agent_table_view(arena + pp.table_off, A, Tp);
+    const int Ap = v.Ap;
+    float4* s0 = const_cast<float4*>(v.s0);
+    float4* s1 = const_cast<float4*>(v.s1);
+    float2* s2 = const_cast<float2*>(v.s2);
+    float4* t0 = const_cast<float4*>(v.t0);
+    float* tv = const_cast<float*>(v.tv);
+    float* tpsi = const_cast<float*>(v.tpsi);
+    const int32_t* orig = v.orig;
+    const int32_t* slot = v.slot;
+    const size_t r0 = (size_t)pp.a_begin * S;     // raw element of (agent 0, state 0) of this problem
+    const int nW = agent_windows(Tp);
+    if (idx < Ap * nW) {                       // window boxes for the summary kernel's filter (slot order)
+      const int sl = idx / nW, wi = idx - sl * nW;
+      float xl = 1e30f, xh = -1e30f, yl = 1e30f, yh = -1e30f, vm = 0.0f;
+      if (sl < A) {
+        const int a = orig[sl];
+        const int nS = min(raw.n_states[pp.a_begin + a], Tp);
+        const int lo = wi * kWinSteps;
+        for (int i = max(lo - 1, 0); i < min(lo + kWinSteps, nS); ++i) {
+          const size_t r = r0 + (size_t)a * S + i;
+          const float x = raw.x[r], y = raw.y[r];
+          xl = fminf(xl, x); xh = fmaxf(xh, x); yl = fminf(yl, y); yh = fmaxf(yh, y);
+          if (i >= lo) vm = fmaxf(vm, fabsf(raw.v[r]));
+        }
       }
+      const_cast<float4*>(v.aw)[(size_t)wi * Ap + sl] = make_float4(xl, xh, yl, yh);
+      const_cast<float*>(v.avw)[(size_t)wi * Ap + sl] = vm;
     }
-    aw[(size_t)wi * Ap + sl] = make_float4(xl, xh, yl, yh);
-    avw[(size_t)wi * Ap + sl] = vm;
-  }
-  if (idx >= A * Tp && idx < Ap * Tp) {      // padding slots of the time-major copies
-    const int sl = idx / Tp, i = idx - sl * Tp;
-    t0[(size_t)i * Ap + sl] = make_float4(0, 0, 1, 0);
-    tv[(size_t)i * Ap + sl] = 0.0f;
-    tpsi[(size_t)i * Ap + sl] = 0.0f;
-  }
-  if (idx < A * Tp) {
-    const int a = idx / Tp, i = idx - a * Tp;
-    const int sl = slot[a];
-    float4 o0 = make_float4(0, 0, 1, 0), o1 = make_float4(0, 0, 0, 0);
-    float2 o2 = make_float2(1, 1);
-    if (i < raw.n_states[a]) {
-      float yaw = raw.yaw[idx];
-      float sn, cs;
-      sincosf(yaw, &sn, &cs);
-      const int ip = i > 0 ? idx - 1 : idx;   // state i-1 (CP pairs ego step i with agent position / covariance i-1)
-      float vx = raw.var_x[ip], vy = raw.var_y[ip];
-      if (vx == 0.0f && vy == 0.0f) { vx = 0.1f; vy = 0.1f; }  // collision_probability.py:85-87
-      o0 = make_float4(raw.x[idx], raw.y[idx], cs, sn);
-      o1 = make_float4(yaw, raw.v[idx], raw.x[ip], raw.y[ip]);
-      o2 = make_float2(rsqrtf(2.0f * vx), rsqrtf(2.0f * vy));
+    if (idx >= A * Tp && idx < Ap * Tp) {      // padding slots of the time-major copies
+      const int sl = idx / Tp, i = idx - sl * Tp;
+      t0[(size_t)i * Ap + sl] = make_float4(0, 0, 1, 0);
+      tv[(size_t)i * Ap + sl] = 0.0f;
+      tpsi[(size_t)i * Ap + sl] = 0.0f;
     }
-    const size_t am = (size_t)sl * Tp + i, tm = (size_t)i * Ap + sl;
-    s0[am] = o0;
-    s1[am] = o1;
-    s2[am] = o2;
-    t0[tm] = o0;
-    tv[tm] = o1.y;
-    tpsi[tm] = o1.x;
+    if (idx < A * Tp) {
+      const int a = idx / Tp, i = idx - a * Tp;
+      const int sl = slot[a];
+      const size_t r = r0 + (size_t)a * S + i;
+      float4 o0 = make_float4(0, 0, 1, 0), o1 = make_float4(0, 0, 0, 0);
+      float2 o2 = make_float2(1, 1);
+      if (i < raw.n_states[pp.a_begin + a]) {
+        float yaw = raw.yaw[r];
+        float sn, cs;
+        sincosf(yaw, &sn, &cs);
+        const size_t ip = i > 0 ? r - 1 : r;   // state i-1 (CP pairs ego step i with agent position / covariance i-1)
+        float vx = raw.var_x[ip], vy = raw.var_y[ip];
+        if (vx == 0.0f && vy == 0.0f) { vx = 0.1f; vy = 0.1f; }  // collision_probability.py:85-87
+        o0 = make_float4(raw.x[r], raw.y[r], cs, sn);
+        o1 = make_float4(yaw, raw.v[r], raw.x[ip], raw.y[ip]);
+        o2 = make_float2(rsqrtf(2.0f * vx), rsqrtf(2.0f * vy));
+      }
+      const size_t am = (size_t)sl * Tp + i, tm = (size_t)i * Ap + sl;
+      s0[am] = o0;
+      s1[am] = o1;
+      s2[am] = o2;
+      t0[tm] = o0;
+      tv[tm] = o1.y;
+      tpsi[tm] = o1.x;
+    }
+    if (idx < A) {
+      const int g = pp.a_begin + idx;
+      AgentParams q;
+      q.n_states = raw.n_states[g];
+      q.model = protection_model(raw.kind[g]);
+      q.hl = 0.5f * raw.length[g];
+      q.hw = 0.5f * raw.width[g];
+      q.hlb = 0.5f * raw.buf_length[g];
+      float mo = obstacle_mass(raw.kind[g], raw.buf_length[g] * raw.buf_width[g]);  // harm_model.py:73,78
+      q.ke = mo / (m_ego + mo);
+      q.ko = m_ego / (m_ego + mo);
+      q.pad = sqrtf(q.hl * q.hl + q.hw * q.hw);   // circumradius of the unbuffered rectangle (distance lower bound)
+      const_cast<AgentParams*>(v.prm)[slot[idx]] = q;
+    }
   }
-  if (idx < A) {
-    AgentParams p;
-    p.n_states = raw.n_states[idx];
-    p.model = protection_model(raw.kind[idx]);
-    p.hl = 0.5f * raw.length[idx];
-    p.hw = 0.5f * raw.width[idx];
-    p.hlb = 0.5f * raw.buf_length[idx];
-    float mo = obstacle_mass(raw.kind[idx], raw.buf_length[idx] * raw.buf_width[idx]);  // harm_model.py:73,78
-    p.ke = mo / (m_ego + mo);
-    p.ko = m_ego / (m_ego + mo);
-    p.pad = sqrtf(p.hl * p.hl + p.hw * p.hw);   // circumradius of the unbuffered rectangle (distance lower bound)
-    prm[slot[idx]] = p;
+}
+static void launch_pack(const FoAgentsRaw& raw, float m_ego, const PackProblem& one, const PackProblem* many, int P,
+                        int max_cells, unsigned char* arena, cudaStream_t st) {
+  fo_agents_order_kernel<<<P, 256, 0, st>>>(raw.kind, one, many, arena);
+  const dim3 grid((max_cells + 255) / 256, P < 65535 ? P : 65535);
+  fo_agents_pack_kernel<<<grid, 256, 0, st>>>(raw, m_ego, one, many, P, arena);
+}
+
+// Staging of the per-problem descriptors of the batch entry points, per calling thread and device: a ring of slots, each
+// a page-locked host buffer and a device buffer.  A slot is refilled only after the event recorded behind its last use
+// (the upload from the host buffer and the launches that read the device copy) has completed.
+constexpr int kStageRing = 4, kStageMaxDev = 64;
+struct StageSlot {
+  unsigned char* host = nullptr;
+  unsigned char* dev = nullptr;
+  size_t bytes = 0;
+  cudaEvent_t done = nullptr;
+};
+struct StageRing {
+  StageSlot slot[kStageRing];
+  int next = 0;
+};
+static thread_local StageRing g_stage[kStageMaxDev];
+
+static int stage_acquire(size_t bytes, StageSlot** out) {
+  int dev = 0;
+  FO_CUDA_TRY(cudaGetDevice(&dev));
+  if (dev < 0 || dev >= kStageMaxDev) { set_error("batch staging: device ordinal %d out of range", dev); return FO_ERR_UNSUPPORTED; }
+  StageRing& ring = g_stage[dev];
+  StageSlot& s = ring.slot[ring.next];
+  ring.next = (ring.next + 1) % kStageRing;
+  if (!s.done) FO_CUDA_TRY(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+  FO_CUDA_TRY(cudaEventSynchronize(s.done));
+  if (bytes > s.bytes) {
+    if (s.host) FO_CUDA_TRY(cudaFreeHost(s.host));
+    if (s.dev) FO_CUDA_TRY(cudaFree(s.dev));
+    s.host = s.dev = nullptr;
+    s.bytes = 0;
+    const size_t want = bytes + bytes / 4 > 4096 ? bytes + bytes / 4 : 4096;
+    FO_CUDA_TRY(cudaMallocHost(&s.host, want));
+    FO_CUDA_TRY(cudaMalloc(&s.dev, want));
+    s.bytes = want;
   }
+  *out = &s;
+  return FO_OK;
+}
+
+static int stage_upload(StageSlot* s, size_t bytes, cudaStream_t st) {
+  FO_CUDA_TRY(cudaMemcpyAsync(s->dev, s->host, bytes, cudaMemcpyHostToDevice, st));
+  return FO_OK;
+}
+
+// Checks the table of one problem against the arena (A > 0): stride range, 16-byte alignment, bounds.
+static int check_table(const char* fn, int p, int A, int Tp, int64_t off, size_t arena_bytes) {
+  if (Tp < 1) { set_error("%s: problem %d has agents but t_stride %d", fn, p, Tp); return FO_ERR_INVALID_ARG; }
+  if (Tp > FO_MAX_STATES) { set_error("%s: problem %d t_stride %d > FO_MAX_STATES", fn, p, Tp); return FO_ERR_UNSUPPORTED; }
+  if (off < 0 || (off & 15) || (size_t)off > arena_bytes || arena_bytes - (size_t)off < agent_table_bytes(A, Tp)) {
+    set_error("%s: table of problem %d (offset %lld, %zu bytes) misaligned or outside the arena (%zu bytes)", fn, p,
+              (long long)off, agent_table_bytes(A, Tp), arena_bytes);
+    return FO_ERR_INVALID_ARG;
+  }
+  return FO_OK;
 }
 
 }  // namespace fo
@@ -139,16 +234,81 @@ extern "C" int fo_agents_pack(const FoAgentsRaw* raw, const FoVehicle* vehicle, 
     fo::set_error("fo_agents_pack: NULL array in FoAgentsRaw");
     return FO_ERR_INVALID_ARG;
   }
-  fo::AgentTableView v = fo::agent_table_view(table_dev, A, Tp);
-  const int total = v.Ap * Tp;
-  fo::fo_agents_order_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(raw->kind, A, v.Ap, const_cast<int32_t*>(v.orig),
-                                                                  const_cast<int32_t*>(v.slot));
-  fo::fo_agents_pack_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
-      *raw, vehicle->mass, const_cast<float4*>(v.s0), const_cast<float4*>(v.s1), const_cast<float2*>(v.s2),
-      const_cast<fo::AgentParams*>(v.prm), const_cast<float4*>(v.t0), const_cast<float*>(v.tv),
-      const_cast<float*>(v.tpsi), const_cast<float4*>(v.aw), const_cast<float*>(v.avw), v.orig, v.slot, v.Ap);
+  const fo::PackProblem one{0, A, Tp, 0, 0};
+  fo::launch_pack(*raw, vehicle->mass, one, nullptr, 1, fo::agent_pad(A) * Tp, (unsigned char*)table_dev, (cudaStream_t)stream);
   fo::count_launch(2);
   FO_CUDA_TRY(cudaGetLastError());
+  return FO_OK;
+}
+
+extern "C" size_t fo_agent_batch_layout(int32_t n_problems, const int32_t* n_agents, const int32_t* t_stride,
+                                        int64_t* table_offset) {
+  if (n_problems < 0 || (n_problems > 0 && (!n_agents || !t_stride || !table_offset))) {
+    fo::set_error("fo_agent_batch_layout: bad argument");
+    return 0;
+  }
+  size_t off = 0;
+  for (int p = 0; p < n_problems; ++p) {
+    const int A = n_agents[p], Tp = t_stride[p];
+    if (A < 0 || Tp < 0 || Tp > FO_MAX_STATES) {
+      fo::set_error("fo_agent_batch_layout: problem %d: n_agents %d / t_stride %d out of range", p, A, Tp);
+      return 0;
+    }
+    table_offset[p] = (int64_t)off;
+    if (A > 0 && Tp > 0) off += (fo::agent_table_bytes(A, Tp) + 15) & ~(size_t)15;
+  }
+  return off;
+}
+
+extern "C" int fo_agents_pack_batch(const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
+                                    const FoVehicle* vehicle, void* arena_dev, size_t arena_bytes, void* stream) {
+  const char* fn = "fo_agents_pack_batch";
+  if (!raw || !vehicle || n_problems < 0 || (n_problems > 0 && !problems)) { fo::set_error("%s: bad argument", fn); return FO_ERR_INVALID_ARG; }
+  if (raw->n_agents < 0 || raw->t_stride < 0) { fo::set_error("%s: negative size", fn); return FO_ERR_INVALID_ARG; }
+  if (reinterpret_cast<uintptr_t>(arena_dev) & 15) { fo::set_error("%s: arena must be 16-byte aligned", fn); return FO_ERR_INVALID_ARG; }
+  long long total = 0;
+  int n_packed = 0, max_cells = 0;
+  for (int p = 0; p < n_problems; ++p) {
+    const FoBatchProblem& q = problems[p];
+    if (q.n_agents < 0) { fo::set_error("%s: problem %d has %d agents", fn, p, q.n_agents); return FO_ERR_INVALID_ARG; }
+    total += q.n_agents;
+    if (q.n_agents == 0) continue;
+    const int rc = fo::check_table(fn, p, q.n_agents, q.t_stride, q.table_offset, arena_dev ? arena_bytes : 0);
+    if (rc != FO_OK) return rc;
+    if (q.t_stride > raw->t_stride) { fo::set_error("%s: problem %d t_stride %d > raw row stride %d", fn, p, q.t_stride, raw->t_stride); return FO_ERR_INVALID_ARG; }
+    ++n_packed;
+    const int cells = fo::agent_pad(q.n_agents) * q.t_stride;
+    if (cells > max_cells) max_cells = cells;
+  }
+  if (total != raw->n_agents) {
+    fo::set_error("%s: the problems hold %lld agents, raw->n_agents is %d", fn, total, raw->n_agents);
+    return FO_ERR_INVALID_ARG;
+  }
+  if (n_packed == 0) return FO_OK;
+  if (!raw->x || !raw->y || !raw->yaw || !raw->v || !raw->var_x || !raw->var_y || !raw->n_states || !raw->kind ||
+      !raw->length || !raw->width || !raw->buf_length || !raw->buf_width) {
+    fo::set_error("%s: NULL array in FoAgentsRaw", fn);
+    return FO_ERR_INVALID_ARG;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const size_t bytes = (size_t)n_packed * sizeof(fo::PackProblem);
+  fo::StageSlot* slot = nullptr;
+  int rc = fo::stage_acquire(bytes, &slot);
+  if (rc != FO_OK) return rc;
+  fo::PackProblem* pp = reinterpret_cast<fo::PackProblem*>(slot->host);
+  int a_begin = 0, j = 0;
+  for (int p = 0; p < n_problems; ++p) {
+    const FoBatchProblem& q = problems[p];
+    if (q.n_agents > 0) pp[j++] = fo::PackProblem{a_begin, q.n_agents, q.t_stride, 0, (long long)q.table_offset};
+    a_begin += q.n_agents;
+  }
+  rc = fo::stage_upload(slot, bytes, st);
+  if (rc != FO_OK) return rc;
+  fo::launch_pack(*raw, vehicle->mass, fo::PackProblem{}, reinterpret_cast<const fo::PackProblem*>(slot->dev), n_packed,
+                  max_cells, (unsigned char*)arena_dev, st);
+  fo::count_launch(2);
+  FO_CUDA_TRY(cudaGetLastError());
+  FO_CUDA_TRY(cudaEventRecord(slot->done, st));
   return FO_OK;
 }
 
@@ -167,6 +327,38 @@ static int num_sms_of_current_device(int* out) {
   *out = n;
   return FO_OK;
 }
+// Kernel arguments of a validated FoMetricArgs: inputs, vehicle / harm constants and the threshold clauses in kernel units.
+static void fill_kargs(const FoMetricArgs* a, fo::MetricKArgs& k) {
+  k.ego = a->ego; k.N = a->n_traj; k.T = a->n_states; k.A = a->n_agents; k.Tp = a->t_stride;
+  k.tab = fo::agent_table_view(a->agent_table, a->n_agents, a->t_stride);
+  k.hEx = 0.5f * a->vehicle.length; k.hEy = 0.5f * a->vehicle.width;
+  k.wb = a->vehicle.wb_rear_axle; k.a_max = a->vehicle.a_max;
+  k.L3 = a->vehicle.length / 3.0f; k.L6 = a->vehicle.length / 6.0f; k.W2 = a->vehicle.width / 2.0f;
+  k.hc = a->harm; k.dt = (float)a->dt; k.dtd = a->dt;
+  k.mmask = a->metric_mask; k.tmask = a->threshold_mask;
+  k.thr_harm = a->thr_harm; k.thr_risk = a->thr_risk; k.thr_be = a->thr_be; k.thr_cp = a->thr_cp;
+  k.thr_ttc = a->thr_ttc; k.thr_dce = a->thr_dce;
+  {
+    // smallest r with r / 1000.0 >= thr_dce (the reference compares np.round(d, 3) = r / 1000.0 in float64)
+    long long c = (long long)ceil(a->thr_dce * 1000.0);
+    if (!(a->thr_dce > 0.0)) c = 0;
+    if (c > 0xffffff) c = 0xffffff;
+    while (c > 0 && (double)(c - 1) / 1000.0 >= a->thr_dce) --c;
+    while (c < 0xffffff && (double)c / 1000.0 < a->thr_dce) ++c;
+    k.thr_dce_mm = (uint32_t)c;
+    // smallest step with np.round(step * dt, 3) >= thr_ttc
+    uint32_t q = 0;
+    while (q < (uint32_t)FO_MAX_STATES + 1u && rint((double)q * a->dt * 1000.0) / 1000.0 < a->thr_ttc) ++q;
+    k.thr_ttc_col = q;
+  }
+  k.valid = a->valid; k.summary = a->summary; k.flags = a->flags; k.pair = a->pair; k.step = a->step;
+  k.stats = nullptr;
+  { const char* e = getenv("FO_EXACT_DCE"); k.exact_dce = e && e[0] == '1'; }
+  k.claim = nullptr;
+  k.n_peers = 0;
+  for (int p = 0; p < FO_MAX_PEERS; ++p) k.peer_delta[p] = 0;
+}
+
 static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, void* stream);
 
 extern "C" int fo_metric_bundle(const FoMetricArgs* a, void* stream) { return metric_bundle_impl(a, nullptr, stream); }
@@ -198,32 +390,8 @@ static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, 
   int g_num_sms = 0;
   { const int rc = num_sms_of_current_device(&g_num_sms); if (rc != FO_OK) return rc; }
   fo::MetricKArgs k;
-  k.ego = a->ego; k.N = a->n_traj; k.T = a->n_states; k.A = a->n_agents; k.Tp = a->t_stride;
-  k.tab = fo::agent_table_view(a->agent_table, a->n_agents, a->t_stride);
-  k.hEx = 0.5f * a->vehicle.length; k.hEy = 0.5f * a->vehicle.width;
-  k.wb = a->vehicle.wb_rear_axle; k.a_max = a->vehicle.a_max;
-  k.L3 = a->vehicle.length / 3.0f; k.L6 = a->vehicle.length / 6.0f; k.W2 = a->vehicle.width / 2.0f;
-  k.hc = a->harm; k.dt = (float)a->dt; k.dtd = a->dt;
-  k.mmask = a->metric_mask; k.tmask = a->threshold_mask;
-  k.thr_harm = a->thr_harm; k.thr_risk = a->thr_risk; k.thr_be = a->thr_be; k.thr_cp = a->thr_cp;
-  k.thr_ttc = a->thr_ttc; k.thr_dce = a->thr_dce;
-  {
-    // smallest r with r / 1000.0 >= thr_dce (the reference compares np.round(d, 3) = r / 1000.0 in float64)
-    long long c = (long long)ceil(a->thr_dce * 1000.0);
-    if (!(a->thr_dce > 0.0)) c = 0;
-    if (c > 0xffffff) c = 0xffffff;
-    while (c > 0 && (double)(c - 1) / 1000.0 >= a->thr_dce) --c;
-    while (c < 0xffffff && (double)c / 1000.0 < a->thr_dce) ++c;
-    k.thr_dce_mm = (uint32_t)c;
-    // smallest step with np.round(step * dt, 3) >= thr_ttc
-    uint32_t q = 0;
-    while (q < (uint32_t)FO_MAX_STATES + 1u && rint((double)q * a->dt * 1000.0) / 1000.0 < a->thr_ttc) ++q;
-    k.thr_ttc_col = q;
-  }
-  k.valid = a->valid; k.summary = a->summary; k.flags = a->flags; k.pair = a->pair; k.step = a->step;
+  fill_kargs(a, k);
   k.stats = stats;
-  { const char* e = getenv("FO_EXACT_DCE"); k.exact_dce = e && e[0] == '1'; }
-  k.claim = nullptr;
   if (a->summary && (reinterpret_cast<uintptr_t>(a->summary) & 7u)) { fo::set_error("fo_metric_bundle: summary must be 8-byte aligned"); return FO_ERR_INVALID_ARG; }
   if (a->n_peers < 0 || a->n_peers > FO_MAX_PEERS) { fo::set_error("fo_metric_bundle: n_peers %d outside [0, %d]", a->n_peers, FO_MAX_PEERS); return FO_ERR_INVALID_ARG; }
   if (a->n_peers > 0 && (a->pair || a->step || stats)) { fo::set_error("fo_metric_bundle: peer stores exist on the summary path only"); return FO_ERR_UNSUPPORTED; }
@@ -233,4 +401,111 @@ static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, 
   cudaStream_t st = (cudaStream_t)stream;
   if (k.pair || k.step) return fo::launch_metric_detail(k, g_num_sms, st);
   return fo::launch_metric_sweep(k, g_num_sms, st);
+}
+
+extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
+  const char* fn = "fo_metric_batch";
+  if (!b) { fo::set_error("%s: NULL args", fn); return FO_ERR_INVALID_ARG; }
+  const FoMetricArgs& c = b->common;
+  const int P = b->n_problems;
+  if (P < 0 || c.n_traj < 0 || (P > 0 && !b->problems)) { fo::set_error("%s: bad problem list", fn); return FO_ERR_INVALID_ARG; }
+  if (c.pair || c.step || c.n_peers != 0) {
+    fo::set_error("%s: batches have summary outputs only (no pair / step, no peer stores)", fn);
+    return FO_ERR_UNSUPPORTED;
+  }
+  if (c.n_states < 1 || c.n_states > FO_MAX_STATES) {
+    fo::set_error("%s: n_states %d outside [1, %d]", fn, c.n_states, FO_MAX_STATES);
+    return FO_ERR_UNSUPPORTED;
+  }
+  if ((c.metric_mask & FO_M_BE) && !(c.metric_mask & FO_M_TTC)) {
+    fo::set_error("%s: 'be' needs 'ttc' (reference raises KeyError, be.py:39)", fn);
+    return FO_ERR_INVALID_ARG;
+  }
+  if (reinterpret_cast<uintptr_t>(c.agent_table) & 15) { fo::set_error("%s: arena must be 16-byte aligned", fn); return FO_ERR_INVALID_ARG; }
+  // problems in order, their rows contiguous and together exactly [0, n_traj); tables inside the arena
+  long long next_row = 0;
+  int n_run = 0, a_min = 1 << 30;
+  for (int p = 0; p < P; ++p) {
+    const FoBatchProblem& q = b->problems[p];
+    if (q.n_traj < 0 || q.n_agents < 0) { fo::set_error("%s: problem %d: negative size", fn, p); return FO_ERR_INVALID_ARG; }
+    if (q.traj_begin != next_row) {
+      fo::set_error("%s: problem %d starts at row %lld, expected %lld (rows are contiguous, in problem order)", fn, p,
+                    (long long)q.traj_begin, next_row);
+      return FO_ERR_INVALID_ARG;
+    }
+    next_row += q.n_traj;
+    if (next_row > c.n_traj) { fo::set_error("%s: problem %d ends at row %lld > n_traj %d", fn, p, next_row, c.n_traj); return FO_ERR_INVALID_ARG; }
+    if (q.n_agents > 0) {
+      const int rc = fo::check_table(fn, p, q.n_agents, q.t_stride, q.table_offset, c.agent_table ? b->arena_bytes : 0);
+      if (rc != FO_OK) return rc;
+    }
+    if (q.n_traj > 0) {
+      ++n_run;
+      if (q.n_agents < a_min) a_min = q.n_agents;
+    }
+  }
+  if (next_row != c.n_traj) { fo::set_error("%s: the problems cover %lld of %d rows", fn, next_row, c.n_traj); return FO_ERR_INVALID_ARG; }
+  if (c.n_traj == 0) return FO_OK;
+  if (!c.ego || !c.valid) { fo::set_error("%s: ego/valid must not be NULL", fn); return FO_ERR_INVALID_ARG; }
+  if (c.summary && (reinterpret_cast<uintptr_t>(c.summary) & 7u)) { fo::set_error("%s: summary must be 8-byte aligned", fn); return FO_ERR_INVALID_ARG; }
+
+  int num_sms = 0;
+  { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
+  // one team size for the whole batch, as fo_metric_bundle picks it; with W = 1 problems with >= 17 agents run the
+  // window-filter shape, the others the team shape with their own lane grouping
+  const int W = fo::pick_team_warps(c.n_traj, c.n_states, a_min, num_sms);
+  int n_uni = 0;
+  for (int p = 0; p < P; ++p) {
+    const FoBatchProblem& q = b->problems[p];
+    if (q.n_traj > 0 && W == 1 && fo::lane_group_log2(q.n_agents) == 5) ++n_uni;
+  }
+  const int n_team = n_run - n_uni;
+  // staged: first[] of both classes, then their descriptors (16-byte aligned)
+  const size_t first_bytes = ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15;
+  const size_t bytes = first_bytes + (size_t)n_run * sizeof(fo::BatchProb);
+  fo::StageSlot* slot = nullptr;
+  int rc = fo::stage_acquire(bytes, &slot);
+  if (rc != FO_OK) return rc;
+  int* first = reinterpret_cast<int*>(slot->host);
+  fo::BatchProb* prob = reinterpret_cast<fo::BatchProb*>(slot->host + first_bytes);
+  const unsigned char* arena = reinterpret_cast<const unsigned char*>(c.agent_table);
+  int iu = 0, it = n_uni, nu = 0, nt = 0;       // uni class first, team class after it
+  for (int p = 0; p < P; ++p) {
+    const FoBatchProblem& q = b->problems[p];
+    if (q.n_traj == 0) continue;
+    const int lg = fo::lane_group_log2(q.n_agents);
+    const bool uni = W == 1 && lg == 5;
+    int& i = uni ? iu : it;
+    int& n = uni ? nu : nt;
+    fo::BatchProb& d = prob[i];
+    const int Tp = q.n_agents > 0 ? q.t_stride : 1;
+    const fo::AgentTableView v = fo::agent_table_view(arena + (q.n_agents > 0 ? q.table_offset : 0), q.n_agents, Tp);
+    d.t0 = v.t0; d.tv = v.tv; d.aw = v.aw; d.avw = v.avw; d.s0 = v.s0; d.s1 = v.s1; d.s2 = v.s2; d.prm = v.prm;
+    d.first = n; d.row0 = (int)q.traj_begin; d.A = q.n_agents; d.Tp = Tp; d.Ap = v.Ap; d.lg = lg;
+    first[i] = n;
+    n += q.n_traj;
+    ++i;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = fo::stage_upload(slot, bytes, st);
+  if (rc != FO_OK) return rc;
+  fo::MetricKArgs k;
+  FoMetricArgs ca = c;
+  ca.n_agents = 0;                           // per problem
+  ca.agent_table = nullptr;
+  fill_kargs(&ca, k);
+  const int* first_dev = reinterpret_cast<const int*>(slot->dev);
+  const fo::BatchProb* prob_dev = reinterpret_cast<const fo::BatchProb*>(slot->dev + first_bytes);
+  if (n_uni > 0) {
+    k.N = nu;
+    rc = fo::launch_metric_batch(k, num_sms, W, true, fo::BatchView{first_dev, prob_dev, n_uni}, st);
+    if (rc != FO_OK) return rc;
+  }
+  if (n_team > 0) {
+    k.N = nt;
+    rc = fo::launch_metric_batch(k, num_sms, W, false, fo::BatchView{first_dev + n_uni, prob_dev + n_uni, n_team}, st);
+    if (rc != FO_OK) return rc;
+  }
+  FO_CUDA_TRY(cudaEventRecord(slot->done, st));
+  return FO_OK;
 }

@@ -460,5 +460,34 @@ struct EgoState {
 unsigned int* claim_slot(cudaStream_t st);
 int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st);
 int launch_metric_sweep(const MetricKArgs& k, int num_sms, cudaStream_t st);
+// Batch of independent problems (fo_metric_batch): the trajectories of one launch belong to problems with their own
+// agent tables.  A launch sees the problems of one shape class; `first` numbers their trajectories consecutively.  The
+// table pointers are resolved on the host (agent_table_view of the problem's table in the arena): the kernel loads them
+// and does no address arithmetic of its own per trajectory.
+struct __align__(16) BatchProb {
+  const float4* t0;
+  const float* tv;
+  const float4* aw;
+  const float* avw;
+  const float4* s0;
+  const float4* s1;
+  const float2* s2;
+  const AgentParams* prm;
+  int first;            // index of the problem's first trajectory within the launch
+  int row0;             // its row in ego / valid / summary / flags
+  int A, Tp, Ap;        // agents, table stride, agents padded to 32
+  int lg;               // log2 of the agents held by one warp (team shape)
+};
+static_assert(sizeof(BatchProb) == 96, "six 16-byte loads");
+struct BatchView {
+  const int* first;     // [P] BatchProb::first, strictly increasing (problems without trajectories are left out)
+  const BatchProb* prob;
+  int P;
+};
+// summary kernel over one shape class of a batch (uni: the one-warp window-filter shape, W == 1); k.N = the class's
+// trajectory count
+int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st);
+int lane_group_log2(int A);                                  // team shape: a warp holds 1 << lg agents
+int pick_team_warps(int N, int T, int A, int num_sms);       // team size W (FO_TEAM_WARPS overrides)
 
 }  // namespace fo

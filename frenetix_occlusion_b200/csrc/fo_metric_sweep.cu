@@ -164,9 +164,9 @@ __device__ __forceinline__ void sw_harm_logits(const MetricKArgs& k, int model, 
 // collision (r <= 1) or lie below the minimum found since (r <= rmin); when no lane holds such an entry the float64
 // code is not entered at all -- in a dense sweep the minimum is 0 after the first collision and the 6 kB stay out of the
 // instruction cache.
-static __device__ __noinline__ uint32_t sw_drain_ties(const MetricKArgs& k, const float4* egoA, const float2* egoB,
-                                                      uint32_t* colfirst, const uint32_t* src, int cnt, int a0, int lane,
-                                                      uint32_t rmin) {
+__device__ __forceinline__ uint32_t drain_ties_body(const MetricKArgs& k, const AgentTableView& tab, const int& Tp,
+                                                    const float4* egoA, const float2* egoB, uint32_t* colfirst,
+                                                    const uint32_t* src, int cnt, int a0, int lane, uint32_t rmin) {
   uint32_t r = 0xffffffu;
   uint32_t item = 0u;
   bool keep = false;
@@ -179,14 +179,38 @@ static __device__ __noinline__ uint32_t sw_drain_ties(const MetricKArgs& k, cons
   if (keep) {
     const int ial = (int)((item >> 8) & 0xffu), ii = (int)(item & 0xffu);
     const int a = a0 + ial;
-    const float4 s0 = __ldg(&k.tab.t0[(size_t)ii * k.tab.Ap + a]);
-    const int4 pa = __ldg(reinterpret_cast<const int4*>(k.tab.prm + a));
+    const float4 s0 = __ldg(&tab.t0[(size_t)ii * tab.Ap + a]);
+    const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + a));
     const float4 EA = egoA[ii];
     r = obb_round_mm_f64(EA.x, EA.y, egoB[ii].x, k.wb, k.hEx, k.hEy, s0.x, s0.y,
-                         __ldg(&k.tab.s1[(size_t)a * k.Tp + ii]).x, __int_as_float(pa.z), __int_as_float(pa.w));
+                         __ldg(&tab.s1[(size_t)a * Tp + ii]).x, __int_as_float(pa.z), __int_as_float(pa.w));
     if (r == 0u) atomicMin(&colfirst[ial], (uint32_t)ii);
   }
   return __reduce_min_sync(kFull, r);
+}
+static __device__ __noinline__ uint32_t sw_drain_ties(const MetricKArgs& k, const float4* egoA, const float2* egoB,
+                                                      uint32_t* colfirst, const uint32_t* src, int cnt, int a0, int lane,
+                                                      uint32_t rmin) {
+  return drain_ties_body(k, k.tab, k.Tp, egoA, egoB, colfirst, src, cnt, a0, lane, rmin);
+}
+// batched kernel: the agent table is the trajectory's problem's, passed in registers
+static __device__ __noinline__ uint32_t sw_drain_ties_batch(const MetricKArgs& k, const float4* t0, const AgentParams* prm,
+                                                            const float4* s1, int Ap, int Tp, const float4* egoA,
+                                                            const float2* egoB, uint32_t* colfirst, const uint32_t* src,
+                                                            int cnt, int a0, int lane, uint32_t rmin) {
+  AgentTableView tab;
+  tab.t0 = t0; tab.prm = prm; tab.s1 = s1; tab.Ap = Ap;
+  return drain_ties_body(k, tab, Tp, egoA, egoB, colfirst, src, cnt, a0, lane, rmin);
+}
+
+// problem of trajectory n: the last p with first[p] <= n
+__device__ __forceinline__ int batch_find(const BatchView& b, int n) {
+  int lo = 0, hi = b.P - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(b.first + mid) <= n) lo = mid; else hi = mid - 1;
+  }
+  return lo;
 }
 
 struct SweepShape {
@@ -196,13 +220,15 @@ struct SweepShape {
 // ---------------------------------------------------------------------------------------------
 // UNI: one warp per trajectory and 32 agents per warp pass (the throughput shape): window filter + lane = (agent, window)
 // items, no pooled leftovers (see the header comment).
-template <uint32_t MASK, bool STATS, bool UNI, bool TIES>
-__global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
-fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape) {
+// BATCH: every trajectory takes its agent table, agent count and lane grouping from its problem (bv); otherwise from k.
+// tid / block_dim are read in the __global__ function, where the compiler knows their range from the launch bounds.
+template <uint32_t MASK, bool STATS, bool UNI, bool TIES, bool BATCH>
+__device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShape shape, const BatchView& bv,
+                                           const int tid, const int block_dim) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   // the one-warp shape is launched with 32 threads: warp index, team size and lane are compile-time facts there (the
   // queue addresses become immediates instead of being re-derived from %tid wherever registers are short)
-  const int tid = threadIdx.x, nthr = UNI ? 32 : blockDim.x;
+  const int nthr = UNI ? 32 : block_dim;
   const int lane = UNI ? tid : (tid & 31), wib = UNI ? 0 : (tid >> 5), W = UNI ? 1 : (nthr >> 5);
   const int T = k.T;
   const SweepSmem w = sweep_smem(smem_raw, T, UNI ? 1 : W, UNI, TIES);
@@ -215,10 +241,10 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
   const unsigned lt_mask = (1u << lane) - 1u;
   const float rE = sqrtf(k.hEx * k.hEx + k.hEy * k.hEy);   // ego circumradius
   const float cmax = fmaxf(0.0f, fmaxf(k.hc.rs_side, k.hc.rs_rear));
-  const int Ap = k.tab.Ap;
+  int Ap = k.tab.Ap;
   const auto soff = [&](const void* q) { return (uint32_t)(reinterpret_cast<const unsigned char*>(q) - smem_raw); };
   const BeView bev{soff(w.egoA), soff(w.egoB), soff(w.dist), soff(w.inv), soff(w.seg)};
-  const BeConst bek = be_const(k);
+  BeConst bek = be_const(k);                       // batched: the table and its stride are set per trajectory
   // lane -> (agent within the lane group, time slice); every (warp, slice) owns a contiguous range of steps
   const int lg = shape.lg_agents;
   const int group = 1 << lg;                      // agents per warp pass
@@ -230,14 +256,47 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
   unsigned long long st_dense = 0, st_obb = 0, st_lr = 0, st_cp = 0, st_be = 0, st_probe = 0, st_win = 0, st_wkeep = 0;
 
   // Trajectories are claimed from a device counter (their cost varies several-fold with the number of near agents and
-  // braking pairs); the claim for the next one is issued here and read at the bottom, so its latency is hidden.
-  __shared__ int s_next;
+  // braking pairs); the claim for the next one is issued here and read at the bottom, so its latency is hidden.  A batch
+  // looks up the problem of the claimed trajectory in the same place.
+  __shared__ int s_claim[BATCH ? 2 : 1];               // next trajectory (and, batched, its problem)
+  int& s_next = s_claim[0];
+  int p = BATCH ? batch_find(bv, blockIdx.x) : 0;
   for (int n = blockIdx.x; n < k.N;) {
+    AgentTableView btab;
+    int row = n, bA = 0, bTp = 0, b_group = 1, b_la = 0, b_slo = 0, b_shi = 0;
+    if constexpr (BATCH) {
+      const BatchProb bp = bv.prob[p];
+      row = bp.row0 + (n - bp.first);
+      bA = bp.A; bTp = bp.Tp;
+      btab.t0 = bp.t0; btab.tv = bp.tv; btab.aw = bp.aw; btab.avw = bp.avw;
+      btab.s0 = bp.s0; btab.s1 = bp.s1; btab.s2 = bp.s2; btab.prm = bp.prm;
+      btab.Ap = Ap = bp.Ap;
+      bek.s0 = bp.s0;                                // BE bisections read the agent-major states
+      bek.Tp = bTp;
+      b_group = 1 << bp.lg;                          // lane map of the problem's lane grouping, as above
+      b_la = lane & (b_group - 1);
+      const int bL = (T + W * (32 >> bp.lg) - 1) / (W * (32 >> bp.lg));
+      b_slo = (wib * (32 >> bp.lg) + (lane >> bp.lg)) * bL;
+      b_shi = min(T, b_slo + bL);
+    }
+    // references into the kernel parameters when not batched: their uses stay constant-bank operands
+    const AgentTableView& tab = BATCH ? btab : k.tab;
+    const int& A = BATCH ? bA : k.A;
+    const int& Tp = BATCH ? bTp : k.Tp;
+    const auto drain_ties = [&](const uint32_t* src, int cnt, int a0, int lane, uint32_t rmin) {
+      if constexpr (BATCH)
+        return sw_drain_ties_batch(k, tab.t0, tab.prm, tab.s1, Ap, Tp, w.egoA, w.egoB, w.colfirst, src, cnt, a0, lane, rmin);
+      else
+        return sw_drain_ties(k, w.egoA, w.egoB, w.colfirst, src, cnt, a0, lane, rmin);
+    };
     // ---- stage the ego trajectory (whole team) ---------------------------------------------------
-    const float* eg = k.ego + (size_t)n * T * 5;
+    const float* eg = k.ego + (size_t)row * T * 5;
     __syncthreads();                                   // previous trajectory fully consumed
     if (tid < 8) w.scal[tid] = 0u;
-    if (tid == 0) s_next = k.claim ? (int)(gridDim.x + atomicAdd(k.claim, 1u)) : n + (int)gridDim.x;
+    if (tid == 0) {
+      s_next = k.claim ? (int)(gridDim.x + atomicAdd(k.claim, 1u)) : n + (int)gridDim.x;
+      if constexpr (BATCH) s_claim[1] = s_next < k.N ? batch_find(bv, s_next) : 0;
+    }
     __syncthreads();
     {
       float amin = 0.0f;
@@ -278,8 +337,8 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
     uint32_t flags = 0;
     bool be_ready = false;
 
-    for (int a0 = 0; a0 < k.A; a0 += kSwTile) {
-      const int nAt = min(kSwTile, k.A - a0);
+    for (int a0 = 0; a0 < A; a0 += kSwTile) {
+      const int nAt = min(kSwTile, A - a0);
       for (int j = tid; j < nAt; j += nthr) { w.pairkey[j] = 0ull; w.colfirst[j] = 0xffffffffu; }
       __syncthreads();                                 // ego staged, pair arrays cleared
       int qn = 0, qc = 0, qt = 0;
@@ -318,12 +377,12 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
         if (lane < cnt) {
           const int ial = (int)((item >> 8) & 0xffffu), ii = (int)(item & 0xffu);
           const int a = a0 + ial;
-          const float4 s0 = __ldg(&k.tab.t0[(size_t)ii * Ap + a]);
+          const float4 s0 = __ldg(&tab.t0[(size_t)ii * Ap + a]);
           const float4 EA = w.egoA[ii];
           const float c = fmaf(EA.z, s0.z, EA.w * s0.w), s = fmaf(s0.w, EA.z, -s0.z * EA.w);
           const float dxr = s0.x - EA.x, dyr = s0.y - EA.y;
           if (item & 0x40000000u) {            // exact oriented-box distance, np.round(d, 3) (dce.py:75-79)
-            const int4 pa = __ldg(reinterpret_cast<const int4*>(k.tab.prm + a));
+            const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + a));
             const float dx = dxr - k.wb * EA.z, dy = dyr - k.wb * EA.w;
             const float rx = fmaf(dx, EA.z, dy * EA.w), ry = fmaf(dy, EA.z, -dx * EA.w);
             const float d = sqrtf(obb_d2(rx, ry, c, s, k.hEx, k.hEy, __int_as_float(pa.z), __int_as_float(pa.w)));
@@ -340,8 +399,8 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
             if (STATS) ++st_obb;
           }
           if (item & 0x80000000u) {            // LR4S logits with the impact-angle class (protected agents)
-            const int4 pb = __ldg(reinterpret_cast<const int4*>(k.tab.prm + a) + 1);
-            const float4 s1 = __ldg(&k.tab.s1[(size_t)a * k.Tp + ii]);
+            const int4 pb = __ldg(reinterpret_cast<const int4*>(tab.prm + a) + 1);
+            const float4 s1 = __ldg(&tab.s1[(size_t)a * Tp + ii]);
             const float2 EB = w.egoB[ii];
             const float dv2 = fmaxf(fmaf(EB.y, EB.y, s1.y * s1.y) - 2.0f * EB.y * s1.y * c, 0.0f);
             const float dv = dv2 * rsqrtf(fmaxf(dv2, 1e-30f));
@@ -359,7 +418,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
             if (tie) q_tie[qt + __popc(tb & lt_mask)] = (item & 0xffffu) | (min(r - 1u, 0xffffu) << 16);   // r was bumped above
             qt += __popc(tb);
             __syncwarp();
-            if (qt >= 32) { qt -= 32; rmin = min(rmin, sw_drain_ties(k, w.egoA, w.egoB, w.colfirst, q_tie + qt, 32, a0, lane, rmin)); }
+            if (qt >= 32) { qt -= 32; rmin = min(rmin, drain_ties(q_tie + qt, 32, a0, lane, rmin)); }
           }
         }
         zb_e = fmaxf(zb_e, warp_max_signed(acc_ze));
@@ -374,18 +433,18 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
         if (lane < cnt) {
           const int ial = (int)(item >> 8), ii = (int)(item & 0xffu), t = ii - 1;
           const int a = a0 + ial;
-          const AgentParams P = load_params(k.tab.prm + a);
-          const size_t idx = (size_t)a * k.Tp + ii;
-          const float4 s0i = __ldg(&k.tab.s0[idx]);
-          const float4 s1i = __ldg(&k.tab.s1[idx]);
-          const float2 s2i = __ldg(&k.tab.s2[idx]);
+          const AgentParams P = load_params(tab.prm + a);
+          const size_t idx = (size_t)a * Tp + ii;
+          const float4 s0i = __ldg(&tab.s0[idx]);
+          const float4 s1i = __ldg(&tab.s1[idx]);
+          const float2 s2i = __ldg(&tab.s2[idx]);
           const float4 Ei = w.egoA[ii];
           const float cp = cp_gauss_boxes(s1i.z - Ei.x, s1i.w - Ei.y, P.hlb * s0i.z, P.hlb * s0i.w, k.L3 * Ei.z,
                                           k.L3 * Ei.w, s2i, k.L6, k.W2);
           acc_cp = fmaxf(acc_cp, cp);
           if (do_hr) {                       // risk[t] = harm[t] * cp[t], cp[t] = CP of step t+1 (hr.py:78-79)
-            const float4 s0t = __ldg(&k.tab.s0[idx - 1]);
-            const float4 s1t = __ldg(&k.tab.s1[idx - 1]);
+            const float4 s0t = __ldg(&tab.s0[idx - 1]);
+            const float4 s1t = __ldg(&tab.s1[idx - 1]);
             const float4 Et = w.egoA[t];
             const float2 EtB = w.egoB[t];
             const float ct = fmaf(Et.z, s0t.z, Et.w * s0t.w);
@@ -409,7 +468,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
         const int a = a0 + al;
         AgentParams P;
         P.n_states = 0; P.model = 2; P.hl = P.hw = P.hlb = P.ke = P.ko = P.pad = 0.0f;
-        if (alive) P = load_params(k.tab.prm + a);
+        if (alive) P = load_params(tab.prm + a);
         const int nS = min(P.n_states, i_hi);             // this lane evaluates steps [i_lo, nS)
         const int nH = min(nS, T - 1);                    // harm is evaluated at steps < min(T-1, n_states)
         const int n_it = flush ? 1 : (int)__reduce_max_sync(kFull, (unsigned)max(nS - i_lo, 0));
@@ -431,7 +490,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
         // one 32-bit element offset into both time-major arrays (base pointers are kernel arguments: uniform registers)
         uint32_t toff = (uint32_t)(i_lo * Ap + a);
         float pxp = 0.0f, pyp = 0.0f;                      // position at i-1 (collision_probability.py:52)
-        if (do_cp && i_lo >= 1 && i_lo < nS) { const float4 sp = __ldg(k.tab.t0 + (toff - (uint32_t)Ap)); pxp = sp.x; pyp = sp.y; }
+        if (do_cp && i_lo >= 1 && i_lo < nS) { const float4 sp = __ldg(tab.t0 + (toff - (uint32_t)Ap)); pxp = sp.x; pyp = sp.y; }
         float acc_dv2 = -1.0f;                             // unprotected agents: max_t logit = ks sqrt(max_t dv^2) + kc
         int i = i_lo;
 #pragma unroll kSwUnroll
@@ -439,7 +498,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
           const bool live = i < nS;
           float4 s0 = make_float4(0.0f, 0.0f, 1.0f, 0.0f);
           float va = 0.0f;
-          if (live) { s0 = __ldg(k.tab.t0 + toff); va = __ldg(k.tab.tv + toff); }
+          if (live) { s0 = __ldg(tab.t0 + toff); va = __ldg(tab.tv + toff); }
           const int ie = min(i, T - 1);
           const float4 EA = w.egoA[ie];
           const float ve = w.egoB[ie].y;
@@ -501,8 +560,8 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
         int sub = 0, wi = 0, qw = 0, f_nS = 0, f_nH = 0, f_nW = 0;
         float f_reach2 = 0.0f, f_thr2 = -1.0f;
         // cursors into the window tables; re-derived whenever the per-agent state is (they do not live across run_group)
-        const float4* awp = k.tab.aw;
-        const float* avp = k.tab.avw;
+        const float4* awp = tab.aw;
+        const float* avp = tab.avw;
         const float4* ewp = w.ew;
         const float* evp = w.evw;
         bool more = nAt > 0, stale = true, flushed = false;
@@ -512,7 +571,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
             if (stale) {
               AgentParams P;
               P.n_states = 0; P.model = 2; P.hl = P.hw = P.hlb = P.ke = P.ko = P.pad = 0.0f;
-              if (al < nAt) P = load_params(k.tab.prm + a0 + al);
+              if (al < nAt) P = load_params(tab.prm + a0 + al);
               f_nS = min(P.n_states, T);
               f_nH = min(f_nS, T - 1);
               f_nW = (int)__reduce_max_sync(kFull, (unsigned)((f_nS + kWinSteps - 1) / kWinSteps));
@@ -536,8 +595,8 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
                 t2 = (tm > 0.0f) ? tm * tm * 0.99999f : -1.0f;
               }
               f_thr2 = t2;
-              awp = k.tab.aw + (size_t)wi * Ap + a0 + al;
-              avp = k.tab.avw + (size_t)wi * Ap + a0 + al;
+              awp = tab.aw + (size_t)wi * Ap + a0 + al;
+              avp = tab.avw + (size_t)wi * Ap + a0 + al;
               ewp = w.ew + wi;
               evp = w.evw + wi;
               stale = false;
@@ -573,11 +632,15 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
           stale = true;
         }
       } else {
-        for (int sub = 0; sub < nAt; sub += group) run_group(sub + la, sub + la < nAt, s_lo, s_hi, false);
+        if constexpr (BATCH) {
+          for (int sub = 0; sub < nAt; sub += b_group) run_group(sub + b_la, sub + b_la < nAt, b_slo, b_shi, false);
+        } else {
+          for (int sub = 0; sub < nAt; sub += group) run_group(sub + la, sub + la < nAt, s_lo, s_hi, false);
+        }
       }
       // ---- pool what is left in the per-warp queues across the team and drain it cooperatively --------------
       is_m1 = false;
-      if (TIES && UNI && qt > 0) { rmin = min(rmin, sw_drain_ties(k, w.egoA, w.egoB, w.colfirst, q_tie, qt, a0, lane, rmin)); qt = 0; }
+      if (TIES && UNI && qt > 0) { rmin = min(rmin, drain_ties(q_tie, qt, a0, lane, rmin)); qt = 0; }
       if (!UNI) {
         unsigned base_n = 0, base_c = 0;
         if (lane == 0) {
@@ -592,7 +655,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
         const int tot_n = (int)w.scal[2], tot_c = (int)w.scal[3];
         for (int c = wib * 32; c < tot_n; c += 32 * W) drain_near(w.pool_near + c, min(32, tot_n - c));
         for (int c = wib * 32; c < tot_c; c += 32 * W) drain_cp(w.pool_cp + c, min(32, tot_c - c));
-        while (TIES && qt > 0) { const int c = min(qt, 32); qt -= c; rmin = min(rmin, sw_drain_ties(k, w.egoA, w.egoB, w.colfirst, q_tie + qt, c, a0, lane, rmin)); }
+        while (TIES && qt > 0) { const int c = min(qt, 32); qt -= c; rmin = min(rmin, drain_ties(q_tie + qt, c, a0, lane, rmin)); }
       }
       __syncthreads();                                 // pairkey / colfirst of the tile complete
       if (tid == 0) { w.scal[2] = 0u; w.scal[3] = 0u; }
@@ -604,10 +667,10 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
         if (key != 0ull) {
           const int t = (int)(0xffffu - (unsigned)((key >> 16) & 0xffffu));
           const int a = a0 + j;
-          const AgentParams P = load_params(k.tab.prm + a);
-          const size_t idx = (size_t)a * k.Tp + t;
-          const float4 s0t = __ldg(&k.tab.s0[idx]);
-          const float4 s1t = __ldg(&k.tab.s1[idx]);
+          const AgentParams P = load_params(tab.prm + a);
+          const size_t idx = (size_t)a * Tp + t;
+          const float4 s0t = __ldg(&tab.s0[idx]);
+          const float4 s1t = __ldg(&tab.s1[idx]);
           const float4 Et = w.egoA[t];
           const float2 EtB = w.egoB[t];
           const float ct = fmaf(Et.z, s0t.z, Et.w * s0t.w);
@@ -634,7 +697,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
           // (be_bisect), and a range error makes every further one moot (the outputs are NaN, the trajectory invalid)
           for (int q = wib; q < n_be && !(flags & FO_F_BE_RANGE); q += W) {   // bisections dealt round-robin to the warps
             const int a = a0 + (int)w.be_list[q];
-            const int4 pa = __ldg(reinterpret_cast<const int4*>(k.tab.prm + a));
+            const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + a));
 #ifdef FO_BE_NO_FLOOR
             const float be_floor = -1.0f;
 #else
@@ -679,7 +742,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
         btn = fmaxf(btn, r[9]); rcd = fmaxf(rcd, r[10]);
       }
       const float eh = sw_sigmoid(ze), oh = sw_sigmoid(zo);   // logistic is monotone: max harm = logistic(max logit)
-      const bool has_agents = k.A > 0 && mm != 0;
+      const bool has_agents = A > 0 && mm != 0;
       const bool has_col = col != 0xffffffffu;
       bool ok = true;
       if (has_agents) {
@@ -699,10 +762,10 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
 #pragma unroll 1
       for (int p = -1; p < k.n_peers; ++p) {
         const long long dl = p < 0 ? 0ll : k.peer_delta[p];
-        reinterpret_cast<uint8_t*>(reinterpret_cast<char*>(k.valid) + dl)[n] = ok ? 1 : 0;
-        if (k.flags) reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(k.flags) + dl)[n] = fl;
+        reinterpret_cast<uint8_t*>(reinterpret_cast<char*>(k.valid) + dl)[row] = ok ? 1 : 0;
+        if (k.flags) reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(k.flags) + dl)[row] = fl;
         if (k.summary) {
-          float2* sm = reinterpret_cast<float2*>(reinterpret_cast<char*>(k.summary) + dl) + (size_t)n * (FO_SUMMARY_K / 2);
+          float2* sm = reinterpret_cast<float2*>(reinterpret_cast<char*>(k.summary) + dl) + (size_t)row * (FO_SUMMARY_K / 2);
           sm[0] = make_float2(er, orr);
           sm[1] = make_float2(do_hr ? eh : 0.0f, do_hr ? oh : 0.0f);
           sm[2] = make_float2(cpm, hwc_all);
@@ -712,6 +775,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
       }
     }
     n = s_next;
+    if constexpr (BATCH) p = s_claim[1];
   }
   if (STATS && k.stats) {
     auto wsum = [&](unsigned long long v) {
@@ -729,23 +793,46 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
   }
 }
 
+template <uint32_t MASK, bool STATS, bool UNI, bool TIES>
+__global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
+fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape) {
+  sweep_body<MASK, STATS, UNI, TIES, false>(k, shape, BatchView{}, threadIdx.x, blockDim.x);
+}
+
+// One shape class of a batch of independent problems (fo_metric_batch): k.N is the class's trajectory count, k.tab / k.A
+// / k.Tp and shape.lg_agents are unused -- every trajectory takes them from its problem.
+template <uint32_t MASK, bool UNI, bool TIES>
+__global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
+fo_metric_batch_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape, const __grid_constant__ BatchView bv) {
+  sweep_body<MASK, false, UNI, TIES, true>(k, shape, bv, threadIdx.x, blockDim.x);
+}
+
 // Team shape.  lg_agents: a warp holds min(32, next power of two >= A) agents, the remaining lanes are time slices.
 // W: as many warps per trajectory as keeps the whole bundle resident in one wave (the latency of a bundle is its
 // slowest trajectory), as long as every (warp, slice) still owns at least 4 steps.
-static void pick_shape(const MetricKArgs& k, int num_sms, int& W, SweepShape& shape) {
+int lane_group_log2(int A) {
   int lg = 0;
-  while ((1 << lg) < k.A && lg < 5) ++lg;
-  shape.lg_agents = lg;
-  const int slices_per_warp = 32 >> lg;
+  while ((1 << lg) < A && lg < 5) ++lg;
+  return lg;
+}
+
+// A batch takes N = its total trajectory count and A = the fewest agents of any problem (the most time slices per warp).
+int pick_team_warps(int N, int T, int A, int num_sms) {
+  const int slices_per_warp = 32 >> lane_group_log2(A);
   const int warp_slots = num_sms * 8 * FO_SW_MINB;               // registers per thread are capped for FO_SW_MINB 256-thread CTAs per SM
-  int w = warp_slots / (k.N > 0 ? k.N : 1);
-  const int max_w = k.T / (4 * slices_per_warp);
+  int w = warp_slots / (N > 0 ? N : 1);
+  const int max_w = T / (4 * slices_per_warp);
   if (w > max_w) w = max_w;
   if (w > kSwMaxWarps) w = kSwMaxWarps;
   if (w < 1) w = 1;
   const char* forced = getenv("FO_TEAM_WARPS");                  // measurement / test switch (DESIGN.md)
   if (forced) { int f = atoi(forced); if (f >= 1 && f <= kSwMaxWarps) w = f; }
-  W = w;
+  return w;
+}
+
+static void pick_shape(const MetricKArgs& k, int num_sms, int& W, SweepShape& shape) {
+  shape.lg_agents = lane_group_log2(k.A);
+  W = pick_team_warps(k.N, k.T, k.A, num_sms);
 }
 
 // Claim counters: one 4-byte slot per launch, zeroed in-stream before the kernel.  Eager launches rotate through a ring
@@ -779,41 +866,22 @@ unsigned int* claim_slot(cudaStream_t st) {
   return pool[dev] + s;
 }
 
-template <uint32_t MASK, bool STATS, bool UNI, bool TIES>
-static int launch_sweep_shape(const MetricKArgs& k, int num_sms, int W, const SweepShape& shape, cudaStream_t st);
-
-template <uint32_t MASK, bool STATS>
-static int launch_sweep_inst(const MetricKArgs& k, int num_sms, cudaStream_t st) {
-  int W = 1;
-  SweepShape shape;
-  pick_shape(k, num_sms, W, shape);
-  // Float64 re-rounding of np.round(d, 3) ties is compiled into the variants that run when a clause of the validity mask
-  // hangs on a rounded distance (dce / ttc / be thresholds armed, or the caller asked for it): there the mask is the
-  // float64 reference's.  With those thresholds null (the deployment default, occlusion.yaml:20-28) only the last
-  // digit of the reported min_dce could differ, and the kernel without the tie path is a quarter faster (DESIGN.md 5.1).
-  const bool ties = (k.tmask & (FO_T_DCE | FO_T_TTC | FO_T_BE)) != 0 || k.exact_dce;
-  const bool uni = W == 1 && shape.lg_agents == 5;
-  if (uni) return ties ? launch_sweep_shape<MASK, STATS, true, true>(k, num_sms, W, shape, st)
-                       : launch_sweep_shape<MASK, STATS, true, false>(k, num_sms, W, shape, st);
-  return ties ? launch_sweep_shape<MASK, STATS, false, true>(k, num_sms, W, shape, st)
-              : launch_sweep_shape<MASK, STATS, false, false>(k, num_sms, W, shape, st);
-}
-
-template <uint32_t MASK, bool STATS, bool UNI, bool TIES>
-static int launch_sweep_shape(const MetricKArgs& k, int num_sms, int W, const SweepShape& shape, cudaStream_t st) {
-  const size_t smem = sweep_smem_bytes(k.T, W, UNI, TIES);
+// Persistent launch of one summary-kernel instantiation: as many teams as fit on the device, claiming trajectories.
+template <auto KERNEL, class... Extra>
+static int launch_team_kernel(const MetricKArgs& k, int num_sms, int W, bool uni, bool ties, cudaStream_t st,
+                              const SweepShape& shape, const Extra&... extra) {
+  const size_t smem = sweep_smem_bytes(k.T, W, uni, ties);
   // the opt-in shared-memory size is a per-device function attribute: remember what each device has been given
   static std::atomic<size_t> configured[kMaxDev];
   int dev = 0;
   FO_CUDA_TRY(cudaGetDevice(&dev));
   const bool tracked = dev >= 0 && dev < kMaxDev;
   if (!tracked || smem > configured[dev].load(std::memory_order_acquire)) {
-    FO_CUDA_TRY(cudaFuncSetAttribute(fo_metric_sweep_kernel<MASK, STATS, UNI, TIES>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)smem));
+    FO_CUDA_TRY(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (tracked) configured[dev].store(smem, std::memory_order_release);
   }
   int per_sm = 1;
-  FO_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fo_metric_sweep_kernel<MASK, STATS, UNI, TIES>, W * 32, smem));
+  FO_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, KERNEL, W * 32, smem));
   if (per_sm < 1) per_sm = 1;
   const int full = num_sms * per_sm;
   const int grid = k.N < full ? k.N : full;       // persistent: teams claim trajectories
@@ -821,19 +889,55 @@ static int launch_sweep_shape(const MetricKArgs& k, int num_sms, int W, const Sw
   const char* fixed = getenv("FO_STATIC_STRIDE");          // A/B switch: teams stride over trajectories instead
   kk.claim = (k.N > grid && !(fixed && fixed[0] == '1')) ? claim_slot(st) : nullptr;
   if (kk.claim) FO_CUDA_TRY(cudaMemsetAsync(kk.claim, 0, sizeof(unsigned int), st));
-  fo_metric_sweep_kernel<MASK, STATS, UNI, TIES><<<grid, W * 32, smem, st>>>(kk, shape);
+  KERNEL<<<grid, W * 32, smem, st>>>(kk, shape, extra...);
   count_launch();
   FO_CUDA_TRY(cudaGetLastError());
   return FO_OK;
 }
 
+// Float64 re-rounding of np.round(d, 3) ties is compiled into the variants that run when a clause of the validity mask
+// hangs on a rounded distance (dce / ttc / be thresholds armed, or the caller asked for it): there the mask is the
+// float64 reference's.  With those thresholds null (the deployment default, occlusion.yaml:20-28) only the last
+// digit of the reported min_dce could differ, and the kernel without the tie path is a quarter faster (DESIGN.md 5.1).
+static bool needs_ties(const MetricKArgs& k) { return (k.tmask & (FO_T_DCE | FO_T_TTC | FO_T_BE)) != 0 || k.exact_dce; }
+
+template <uint32_t MASK, bool STATS>
+static int launch_sweep_inst(const MetricKArgs& k, int num_sms, cudaStream_t st) {
+  int W = 1;
+  SweepShape shape;
+  pick_shape(k, num_sms, W, shape);
+  const bool ties = needs_ties(k);
+  const bool uni = W == 1 && shape.lg_agents == 5;
+  if (uni) return ties ? launch_team_kernel<fo_metric_sweep_kernel<MASK, STATS, true, true>>(k, num_sms, W, uni, ties, st, shape)
+                       : launch_team_kernel<fo_metric_sweep_kernel<MASK, STATS, true, false>>(k, num_sms, W, uni, ties, st, shape);
+  return ties ? launch_team_kernel<fo_metric_sweep_kernel<MASK, STATS, false, true>>(k, num_sms, W, uni, ties, st, shape)
+              : launch_team_kernel<fo_metric_sweep_kernel<MASK, STATS, false, false>>(k, num_sms, W, uni, ties, st, shape);
+}
+
+constexpr uint32_t kAllMetrics = FO_M_CP | FO_M_DCE | FO_M_TTC | FO_M_HR | FO_M_BE | FO_M_TTCE | FO_M_WTTC;
+constexpr uint32_t kDefaultMetrics = kAllMetrics & ~FO_M_BE;   // occlusion.yaml:12-18
+
 int launch_metric_sweep(const MetricKArgs& k, int num_sms, cudaStream_t st) {
-  constexpr uint32_t kAll = FO_M_CP | FO_M_DCE | FO_M_TTC | FO_M_HR | FO_M_BE | FO_M_TTCE | FO_M_WTTC;
-  constexpr uint32_t kDefault = kAll & ~FO_M_BE;   // occlusion.yaml:12-18
   if (k.stats) return launch_sweep_inst<0u, true>(k, num_sms, st);
-  if (k.mmask == kAll) return launch_sweep_inst<kAll, false>(k, num_sms, st);
-  if (k.mmask == kDefault) return launch_sweep_inst<kDefault, false>(k, num_sms, st);
+  if (k.mmask == kAllMetrics) return launch_sweep_inst<kAllMetrics, false>(k, num_sms, st);
+  if (k.mmask == kDefaultMetrics) return launch_sweep_inst<kDefaultMetrics, false>(k, num_sms, st);
   return launch_sweep_inst<0u, false>(k, num_sms, st);
+}
+
+template <uint32_t MASK>
+static int launch_batch_inst(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st) {
+  const SweepShape shape{0};
+  const bool ties = needs_ties(k);
+  if (uni) return ties ? launch_team_kernel<fo_metric_batch_kernel<MASK, true, true>>(k, num_sms, W, uni, ties, st, shape, bv)
+                       : launch_team_kernel<fo_metric_batch_kernel<MASK, true, false>>(k, num_sms, W, uni, ties, st, shape, bv);
+  return ties ? launch_team_kernel<fo_metric_batch_kernel<MASK, false, true>>(k, num_sms, W, uni, ties, st, shape, bv)
+              : launch_team_kernel<fo_metric_batch_kernel<MASK, false, false>>(k, num_sms, W, uni, ties, st, shape, bv);
+}
+
+int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st) {
+  if (k.mmask == kAllMetrics) return launch_batch_inst<kAllMetrics>(k, num_sms, W, uni, bv, st);
+  if (k.mmask == kDefaultMetrics) return launch_batch_inst<kDefaultMetrics>(k, num_sms, W, uni, bv, st);
+  return launch_batch_inst<0u>(k, num_sms, W, uni, bv, st);
 }
 
 }  // namespace fo

@@ -138,6 +138,21 @@ class BundleResult:
     peer_delta: Optional[Sequence[int]] = None   # byte offsets to the peer-mapped copies of valid / summary / flags (parallel.py)
 
 
+@dataclass
+class BatchResult:
+    """Results of a batch of independent problems: rows ``offsets[p]:offsets[p+1]`` belong to problem p."""
+    valid: torch.Tensor                # uint8 [N_total]
+    summary: torch.Tensor              # float32 [N_total, FO_SUMMARY_K]
+    flags: torch.Tensor                # int32 [N_total]
+    offsets: np.ndarray                # int64 [P + 1]
+
+    def split(self) -> list:
+        """Per-problem ``BundleResult`` views of the batch tensors (no copies)."""
+        o = [int(x) for x in self.offsets]
+        return [BundleResult(self.valid[o[p]:o[p + 1]], self.summary[o[p]:o[p + 1]], self.flags[o[p]:o[p + 1]])
+                for p in range(len(o) - 1)]
+
+
 class MetricEngine:
     """Owns the device-side agent table and launches ``fo_metric_bundle``."""
 
@@ -170,6 +185,9 @@ class MetricEngine:
         self._raw_dev = None
         self.n_agents = 0
         self.t_stride = 0
+        self._batch = None
+        self._staging = None          # page-locked staging of assess_batch's host bundles
+        self._staging_done = None
 
     # ------------------------------------------------------------------------------------------
     def _stream(self):
@@ -208,22 +226,26 @@ class MetricEngine:
             self._raw_dev = (d_fl, d_pa, d_ia)  # keep alive until the stream work is done
 
     # ------------------------------------------------------------------------------------------
-    def to_device_bundle(self, ego) -> torch.Tensor:
-        """[N, T, 5] -> contiguous float32 CUDA tensor (origin-shifted when given as host float64)."""
+    def to_device_bundle(self, ego, origin=None) -> torch.Tensor:
+        """[N, T, 5] -> contiguous float32 CUDA tensor (origin-shifted when given as host float64).  ``origin``: (x, y)
+        for every trajectory, or an [N, 2] array of one origin per trajectory; default the agents' origin."""
+        origin = self.origin if origin is None else np.asarray(origin, dtype=np.float64)
+        per_row = origin.ndim == 2
         if isinstance(ego, torch.Tensor) and ego.is_cuda:
             t = ego
-            if np.any(self.origin != 0.0):
+            if np.any(origin != 0.0):
                 # device tensors are in the caller's frame: shift them like the agents (float64 offset vector)
-                off = torch.tensor([self.origin[0], self.origin[1], 0.0, 0.0, 0.0], dtype=torch.float64, device=t.device)
-                t = (t.to(torch.float64) - off).to(torch.float32)
+                off = np.zeros((origin.shape[0], 1, 5) if per_row else (5,))
+                off[..., 0], off[..., 1] = (origin[:, None, 0], origin[:, None, 1]) if per_row else (origin[0], origin[1])
+                t = (t.to(torch.float64) - torch.from_numpy(off).to(t.device)).to(torch.float32)
             if t.dtype != torch.float32 or not t.is_contiguous():
                 t = t.to(torch.float32).contiguous()
             return t
         arr = np.array(ego, dtype=np.float64, copy=True)
         if arr.ndim == 2:
             arr = arr[None]
-        arr[..., 0] -= self.origin[0]
-        arr[..., 1] -= self.origin[1]
+        arr[..., 0] -= origin[:, None, 0] if per_row else origin[0]
+        arr[..., 1] -= origin[:, None, 1] if per_row else origin[1]
         host = torch.from_numpy(arr.astype(np.float32))
         if host.numel() >= (1 << 18):          # page-locking only pays for bundles of a megabyte and more
             return host.pin_memory().to(self.device, non_blocking=True)
@@ -313,3 +335,135 @@ class MetricEngine:
             with torch.cuda.graph(g):
                 self.assess(ego_dev, out=out)
         return g, out
+
+    # ---- batches of independent problems ------------------------------------------------------------------------
+    def set_agent_batch(self, agent_sets: Sequence[AgentSet], origins=None):
+        """Upload + pack the phantom predictions of P independent problems (``fo_agents_pack_batch``): one float64
+        origin shift per problem, one host-to-device copy of all of them, one pack call.  ``origins``: [P, 2] or None
+        (no shift).  Problem p's table equals what ``set_agents(agent_sets[p], origins[p])`` packs."""
+        P = len(agent_sets)
+        org = np.zeros((P, 2)) if origins is None else np.asarray(origins, dtype=np.float64).reshape(P, 2)
+        n_agents = np.array([a.n_agents if a.t_stride > 0 else 0 for a in agent_sets], dtype=np.int32)
+        t_stride = np.array([a.t_stride if n else 0 for a, n in zip(agent_sets, n_agents)], dtype=np.int32)
+        if np.any(t_stride > L.FO_MAX_STATES):
+            raise ValueError(f"predictions longer than {L.FO_MAX_STATES} states are not supported")
+        offsets = np.zeros(P, dtype=np.int64)
+        arena_bytes = L.lib.fo_agent_batch_layout(P, n_agents.ctypes.data, t_stride.ctypes.data, offsets.ctypes.data)
+        problems = (L.FoBatchProblem * max(P, 1))()
+        for p in range(P):
+            problems[p].n_agents, problems[p].t_stride, problems[p].table_offset = int(n_agents[p]), int(t_stride[p]), int(offsets[p])
+        A, S = int(n_agents.sum()), int(t_stride.max(initial=0))
+        dev = self.device
+        self._batch = {"problems": problems, "P": P, "origins": org, "agents": list(agent_sets), "arena": None,
+                       "arena_bytes": arena_bytes}
+        if A == 0:
+            return
+        # one host buffer: 6 float rows [A, S] (x, y shifted per problem), 4 float columns [A], 2 int32 columns [A]
+        buf = np.zeros(6 * A * S + 6 * A, dtype=np.float32)
+        fl = buf[:6 * A * S].reshape(6, A, S)
+        pa = buf[6 * A * S:6 * A * S + 4 * A].reshape(4, A)
+        ia = buf[6 * A * S + 4 * A:].view(np.int32).reshape(2, A)
+        a0 = 0
+        for p, ag in enumerate(agent_sets):
+            n, tp = int(n_agents[p]), int(t_stride[p])
+            if n == 0:
+                continue
+            rows = slice(a0, a0 + n)
+            fl[0, rows, :tp] = ag.x - org[p, 0]
+            fl[1, rows, :tp] = ag.y - org[p, 1]
+            fl[2, rows, :tp], fl[3, rows, :tp], fl[4, rows, :tp], fl[5, rows, :tp] = ag.yaw, ag.v, ag.var_x, ag.var_y
+            pa[:, rows] = (ag.length, ag.width, ag.buf_length, ag.buf_width)
+            ia[:, rows] = (ag.n_states, ag.kind)
+            a0 += n
+        with torch.cuda.device(dev):
+            host = torch.from_numpy(buf)
+            d_buf = host.pin_memory().to(dev, non_blocking=True) if buf.nbytes >= (1 << 20) else host.to(dev)
+            ptr, f4 = d_buf.data_ptr(), 4
+            raw = L.FoAgentsRaw()
+            raw.n_agents, raw.t_stride = A, S
+            raw.x, raw.y, raw.yaw, raw.v, raw.var_x, raw.var_y = [ptr + f4 * i * A * S for i in range(6)]
+            base = ptr + f4 * 6 * A * S
+            raw.length, raw.width, raw.buf_length, raw.buf_width = [base + f4 * i * A for i in range(4)]
+            raw.n_states, raw.kind = base + f4 * 4 * A, base + f4 * 5 * A
+            arena = torch.empty(max(arena_bytes, 16), dtype=torch.uint8, device=dev)
+            L.check(L.lib.fo_agents_pack_batch(C.byref(raw), P, problems, C.byref(self.vehicle),
+                                               C.c_void_p(arena.data_ptr()), arena_bytes, self._stream()),
+                    "fo_agents_pack_batch")
+        self._batch["arena"] = arena
+        self._batch["raw_dev"] = d_buf           # keep alive until the stream work is done
+
+    def _stage_host_batch(self, parts, origins, offsets, T) -> torch.Tensor:
+        """Host bundles of a batch -> one float32 device tensor: each problem shifted by its origin in float64 and
+        written straight into a page-locked staging buffer kept by the engine (grown on demand; before it is refilled
+        the copy out of it is waited for), then one asynchronous upload."""
+        n = int(offsets[-1]) * T * 5
+        if self._staging is None or self._staging.numel() < n:
+            self._staging = torch.empty(n + n // 4, dtype=torch.float32).pin_memory()
+            self._staging_done = None
+        if self._staging_done is not None:
+            self._staging_done.synchronize()
+        view = self._staging.numpy()[:n].reshape(-1, T, 5)
+        for p, e in enumerate(parts):
+            lo, hi = int(offsets[p]), int(offsets[p + 1])
+            if hi == lo:
+                continue
+            e = e.reshape(-1, T, 5)
+            view[lo:hi] = e                              # same values as to_device_bundle: float64 shift, then float32
+            view[lo:hi, :, 0] = e[..., 0] - origins[p, 0]
+            view[lo:hi, :, 1] = e[..., 1] - origins[p, 1]
+        t = self._staging[:n].view(-1, T, 5).to(self.device, non_blocking=True)
+        self._staging_done = torch.cuda.Event()
+        self._staging_done.record(torch.cuda.current_stream(self.device))
+        return t
+
+    def assess_batch(self, egos: Sequence) -> BatchResult:
+        """Summary pass over every problem of the batch set by ``set_agent_batch`` in one ``fo_metric_batch`` call.
+        ``egos[p]``: problem p's [N_p, T, 5] bundle (host array or CUDA tensor, in the caller's frame: it is shifted by
+        the problem's origin).  Asynchronous on the current stream."""
+        b = self._batch
+        if b is None:
+            raise RuntimeError("assess_batch() needs set_agent_batch() first")
+        P = b["P"]
+        if len(egos) != P:
+            raise ValueError(f"{len(egos)} bundles for {P} problems")
+        on_dev = [isinstance(e, torch.Tensor) and e.is_cuda for e in egos]
+        if any(on_dev) and not all(on_dev):
+            raise ValueError("bundles of one batch are either all CUDA tensors or all host arrays")
+        if all(on_dev) and P:
+            parts = [e if e.ndim == 3 else e[None] for e in egos]
+        else:
+            parts = [np.asarray(e.cpu() if isinstance(e, torch.Tensor) else e, dtype=np.float64) for e in egos]
+            parts = [e if e.ndim == 3 else e[None] for e in parts]
+        shapes = {tuple(e.shape[1:]) for e in parts if e.shape[0] > 0}
+        if len(shapes) > 1 or any(s[1] != 5 for s in shapes):
+            raise ValueError(f"every bundle must be [N_p, T, 5] with one T for the batch, got {sorted(shapes)}")
+        T = shapes.pop()[0] if shapes else max([int(e.shape[1]) for e in parts], default=1)
+        if T > L.FO_MAX_STATES:
+            raise ValueError(f"trajectories longer than {L.FO_MAX_STATES} states are not supported")
+        counts = np.array([int(e.shape[0]) for e in parts], dtype=np.int64)
+        offsets = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+        N = int(offsets[-1])
+        dev = self.device
+        row_origin = np.repeat(b["origins"], counts, axis=0)
+        with torch.cuda.device(dev):
+            if N and all(on_dev):
+                t = self.to_device_bundle(torch.cat([e.reshape(-1, T, 5) for e in parts]), origin=row_origin)
+            elif N:
+                t = self._stage_host_batch(parts, b["origins"], offsets, T)
+            else:
+                t = torch.empty((0, T, 5), dtype=torch.float32, device=dev)
+            out = BundleResult(torch.empty(N, dtype=torch.uint8, device=dev),
+                               torch.empty((N, L.FO_SUMMARY_K), dtype=torch.float32, device=dev),
+                               torch.empty(N, dtype=torch.int32, device=dev))
+            problems = b["problems"]
+            for p in range(P):
+                problems[p].traj_begin, problems[p].n_traj = int(offsets[p]), int(counts[p])
+            a = L.FoMetricBatchArgs()
+            a.common = self._args(t, out)
+            a.common.agent_table = b["arena"].data_ptr() if b["arena"] is not None else None
+            a.common.n_agents, a.common.t_stride = 0, 1
+            a.n_problems, a.problems, a.arena_bytes = P, problems, b["arena_bytes"]
+            L.check(L.lib.fo_metric_batch(C.byref(a), self._stream()), "fo_metric_batch")
+        res = BatchResult(out.valid, out.summary, out.flags, offsets)
+        res._keepalive = (t, b["arena"])
+        return res

@@ -172,6 +172,51 @@ int fo_metric_bundle_host(const float *ego_host, int32_t n_traj, int32_t n_state
                           uint8_t *out_valid, float *out_summary, uint32_t *out_flags, float *out_pair,
                           float *out_step);
 
+/* ---- batches of independent planning problems --------------------------------------------------------
+ * P problems (one ego each: the vehicles of a multi-agent simulation, the scenes of a re-simulation) assessed by
+ * ONE pack call and ONE metric call.  Replaces a loop of Metric.evaluate_metrics / assess_bundle calls, one
+ * set_agents + fo_metric_bundle per problem.  Problem p has its own phantom agents (A_p may be 0) and trajectories
+ * (N_p may be 0); T, the vehicle, dt, metrics, thresholds and harm coefficients are shared.  Problem p's results
+ * equal those fo_metric_bundle gives for it alone under FO_TEAM_WARPS set to the batch's team size. */
+typedef struct FoBatchProblem {
+  int64_t traj_begin;      /* first row of the problem in ego / valid / summary / flags: rows are contiguous, in problem
+                              order, and the problems together cover [0, n_traj) */
+  int32_t n_traj;          /* N_p */
+  int32_t n_agents;        /* A_p */
+  int32_t t_stride;        /* stride of the problem's packed table (>= its longest prediction, <= FO_MAX_STATES) */
+  int32_t reserved_;
+  int64_t table_offset;    /* byte offset of the problem's packed table in the arena (16-byte aligned) */
+} FoBatchProblem;
+
+/* Arena layout of P packed tables: table_offset_host[p] receives the offset of problem p's table, every table starts
+ * 16-byte aligned and takes fo_agent_table_bytes(A_p, t_stride_p) bytes, problems without agents take none.  Returns
+ * the arena size (0 and an error message for malformed input).  Host only. */
+size_t fo_agent_batch_layout(int32_t n_problems, const int32_t *n_agents_host, const int32_t *t_stride_host,
+                             int64_t *table_offset_host);
+
+/* fo_agents_pack for P problems in two launches: `raw` (device arrays) holds the agents of all problems concatenated in
+ * problem order -- raw->n_agents = sum A_p, row stride raw->t_stride >= every t_stride_p.  Problem p's table is
+ * byte-identical to what fo_agents_pack writes for its agents alone with t_stride_p.  `problems_host`: n_agents,
+ * t_stride and table_offset are read (HOST memory). */
+int fo_agents_pack_batch(const FoAgentsRaw *raw, int32_t n_problems, const FoBatchProblem *problems_host,
+                         const FoVehicle *vehicle, void *arena_dev, size_t arena_bytes, void *stream);
+
+typedef struct FoMetricBatchArgs {
+  FoMetricArgs common;     /* ego [n_traj, T, 5] of all problems, n_traj = sum N_p; agent_table = the arena;
+                              n_agents / t_stride are ignored (per problem); pair / step must be NULL, n_peers 0 */
+  int32_t n_problems;
+  int32_t reserved_;
+  const FoBatchProblem *problems;   /* HOST [n_problems]: validated before any device work */
+  size_t arena_bytes;
+} FoMetricBatchArgs;
+
+/* fo_metric_bundle's summary path over a batch: valid / summary / flags of every row.  One team size W for the batch,
+ * chosen as fo_metric_bundle chooses it for n_traj trajectories and the problem with the fewest agents; with W = 1 the
+ * problems with >= 17 agents run the one-warp window-filter shape (one launch) and the others the team shape (a second
+ * launch).  The per-problem descriptors are staged through library-owned page-locked and device buffers (per calling
+ * thread and device).  Not capturable in a CUDA graph. */
+int fo_metric_batch(const FoMetricBatchArgs *args, void *stream);
+
 
 /* ---- stage 1: sensor visibility by ray casting ----------------------------------------------------
  * Replaces SensorModel.calc_visible_and_occluded_area (sensor_model.py:41-193): the reference clips

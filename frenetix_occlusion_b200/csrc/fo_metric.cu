@@ -403,13 +403,20 @@ static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, 
   return fo::launch_metric_sweep(k, g_num_sms, st);
 }
 
-extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
-  const char* fn = "fo_metric_batch";
+// Host-side checks of the batch entry points, before any device work: the outputs each one accepts, row order and
+// contiguity, rows inside n_traj, tables inside the arena, alignment, stride and T limits, 'be' needs 'ttc'.  On success
+// *n_run = the problems with trajectories and *a_min = the fewest agents among them.
+static int check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, int* n_run, int* a_min) {
   if (!b) { fo::set_error("%s: NULL args", fn); return FO_ERR_INVALID_ARG; }
   const FoMetricArgs& c = b->common;
   const int P = b->n_problems;
   if (P < 0 || c.n_traj < 0 || (P > 0 && !b->problems)) { fo::set_error("%s: bad problem list", fn); return FO_ERR_INVALID_ARG; }
-  if (c.pair || c.step || c.n_peers != 0) {
+  if (detail) {
+    if (!c.pair && !c.step) { fo::set_error("%s: pair or step is required (summary outputs only: fo_metric_batch)", fn); return FO_ERR_INVALID_ARG; }
+    if (c.n_peers != 0) { fo::set_error("%s: peer stores exist on the summary path only", fn); return FO_ERR_UNSUPPORTED; }
+    if (reinterpret_cast<uintptr_t>(c.pair) & 15u) { fo::set_error("%s: pair must be 16-byte aligned", fn); return FO_ERR_INVALID_ARG; }
+    if (reinterpret_cast<uintptr_t>(c.step) & 3u) { fo::set_error("%s: step must be 4-byte aligned", fn); return FO_ERR_INVALID_ARG; }
+  } else if (c.pair || c.step || c.n_peers != 0) {
     fo::set_error("%s: batches have summary outputs only (no pair / step, no peer stores)", fn);
     return FO_ERR_UNSUPPORTED;
   }
@@ -424,7 +431,8 @@ extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
   if (reinterpret_cast<uintptr_t>(c.agent_table) & 15) { fo::set_error("%s: arena must be 16-byte aligned", fn); return FO_ERR_INVALID_ARG; }
   // problems in order, their rows contiguous and together exactly [0, n_traj); tables inside the arena
   long long next_row = 0;
-  int n_run = 0, a_min = 1 << 30;
+  *n_run = 0;
+  *a_min = 1 << 30;
   for (int p = 0; p < P; ++p) {
     const FoBatchProblem& q = b->problems[p];
     if (q.n_traj < 0 || q.n_agents < 0) { fo::set_error("%s: problem %d: negative size", fn, p); return FO_ERR_INVALID_ARG; }
@@ -440,15 +448,26 @@ extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
       if (rc != FO_OK) return rc;
     }
     if (q.n_traj > 0) {
-      ++n_run;
-      if (q.n_agents < a_min) a_min = q.n_agents;
+      ++*n_run;
+      if (q.n_agents < *a_min) *a_min = q.n_agents;
     }
   }
   if (next_row != c.n_traj) { fo::set_error("%s: the problems cover %lld of %d rows", fn, next_row, c.n_traj); return FO_ERR_INVALID_ARG; }
   if (c.n_traj == 0) return FO_OK;
   if (!c.ego || !c.valid) { fo::set_error("%s: ego/valid must not be NULL", fn); return FO_ERR_INVALID_ARG; }
   if (c.summary && (reinterpret_cast<uintptr_t>(c.summary) & 7u)) { fo::set_error("%s: summary must be 8-byte aligned", fn); return FO_ERR_INVALID_ARG; }
+  return FO_OK;
+}
 
+extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
+  const char* fn = "fo_metric_batch";
+  int n_run = 0, a_min = 0;
+  {
+    const int rc = check_batch(fn, b, false, &n_run, &a_min);
+    if (rc != FO_OK || b->common.n_traj == 0) return rc;
+  }
+  const FoMetricArgs& c = b->common;
+  const int P = b->n_problems;
   int num_sms = 0;
   { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
   // one team size for the whole batch, as fo_metric_bundle picks it; with W = 1 problems with >= 17 agents run the
@@ -506,6 +525,58 @@ extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
     rc = fo::launch_metric_batch(k, num_sms, W, false, fo::BatchView{first_dev + n_uni, prob_dev + n_uni, n_team}, st);
     if (rc != FO_OK) return rc;
   }
+  FO_CUDA_TRY(cudaEventRecord(slot->done, st));
+  return FO_OK;
+}
+
+extern "C" int fo_metric_batch_detail(const FoMetricBatchArgs* b, void* stream) {
+  int n_run = 0, a_min = 0;
+  {
+    const int rc = check_batch("fo_metric_batch_detail", b, true, &n_run, &a_min);
+    if (rc != FO_OK || b->common.n_traj == 0) return rc;
+  }
+  const FoMetricArgs& c = b->common;
+  const int P = b->n_problems, Tm1 = c.n_states - 1;
+  int num_sms = 0;
+  { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
+  // staged: the problems' first rows, then their descriptors (16-byte aligned)
+  const size_t first_bytes = ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15;
+  const size_t bytes = first_bytes + (size_t)n_run * sizeof(fo::DetailProb);
+  fo::StageSlot* slot = nullptr;
+  int rc = fo::stage_acquire(bytes, &slot);
+  if (rc != FO_OK) return rc;
+  int* first = reinterpret_cast<int*>(slot->host);
+  fo::DetailProb* prob = reinterpret_cast<fo::DetailProb*>(slot->host + first_bytes);
+  const unsigned char* arena = reinterpret_cast<const unsigned char*>(c.agent_table);
+  long long pairs = 0;                           // sum of N_q A_q over the problems before p: the offset of p's blocks
+  int i = 0;
+  for (int p = 0; p < P; ++p) {
+    const FoBatchProblem& q = b->problems[p];
+    if (q.n_traj == 0) continue;
+    const int Tp = q.n_agents > 0 ? q.t_stride : 1;
+    const fo::AgentTableView v = fo::agent_table_view(arena + (q.n_agents > 0 ? q.table_offset : 0), q.n_agents, Tp);
+    fo::DetailProb& d = prob[i];
+    d.t0 = v.t0; d.tv = v.tv; d.s0 = v.s0; d.s1 = v.s1; d.s2 = v.s2; d.prm = v.prm; d.orig = v.orig; d.tpsi = v.tpsi;
+    d.pair = c.pair ? c.pair + (size_t)pairs * FO_PAIR_K : nullptr;
+    d.step = c.step ? c.step + (size_t)pairs * Tm1 * FO_STEP_K : nullptr;
+    d.row0 = (int)q.traj_begin; d.A = q.n_agents; d.Tp = Tp; d.Ap = v.Ap;
+    first[i++] = d.row0;
+    pairs += (long long)q.n_traj * q.n_agents;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = fo::stage_upload(slot, bytes, st);
+  if (rc != FO_OK) return rc;
+  fo::MetricKArgs k;
+  FoMetricArgs ca = c;
+  ca.n_agents = 0;                           // per problem
+  ca.agent_table = nullptr;
+  ca.pair = ca.step = nullptr;
+  fill_kargs(&ca, k);
+  rc = fo::launch_metric_batch_detail(k, num_sms,
+                                      fo::DetailView{reinterpret_cast<const int*>(slot->dev),
+                                                     reinterpret_cast<const fo::DetailProb*>(slot->dev + first_bytes), n_run},
+                                      st);
+  if (rc != FO_OK) return rc;
   FO_CUDA_TRY(cudaEventRecord(slot->done, st));
   return FO_OK;
 }

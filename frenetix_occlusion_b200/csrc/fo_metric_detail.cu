@@ -102,31 +102,44 @@ __device__ __forceinline__ void dt_harm(const FoHarmCoeffs& hc, int model, const
 // np.round(d, 3) next to a x.xxx5 boundary (dce.py:79): queued candidates are re-rounded from a float64 evaluation, up to
 // 32 at a time and out of line.  A candidate matters only while its float32 rounding is within two units of its pair's
 // running minimum (the float32 value is off by at most one unit); by the time the queue is drained most are not.
-static __device__ __noinline__ void dt_drain_ties(const MetricKArgs& k, const float4* egoA, const float2* egoB,
-                                                  uint32_t* dkey, const uint2* src, int cnt, int a0, int lane) {
+__device__ __forceinline__ void dt_drain_ties_body(const MetricKArgs& k, const float4* t0, const AgentParams* prm,
+                                                   const float* tpsi, int Ap, const float4* egoA, const float2* egoB,
+                                                   uint32_t* dkey, const uint2* src, int cnt, int a0, int lane) {
   if (lane < cnt) {
     const uint2 it = src[lane];
     const int ial = (int)(it.x >> 8), ii = (int)(it.x & 0xffu);
     if (it.y <= (dkey[ial] >> 8) + 2u) {
       const int as = a0 + ial;
-      const float4 s0 = __ldg(&k.tab.t0[(size_t)ii * k.tab.Ap + as]);
-      const int4 pa = __ldg(reinterpret_cast<const int4*>(k.tab.prm + as));
+      const float4 s0 = __ldg(&t0[(size_t)ii * Ap + as]);
+      const int4 pa = __ldg(reinterpret_cast<const int4*>(prm + as));
       const float4 EA = egoA[ii];
       const uint32_t r = obb_round_mm_f64(EA.x, EA.y, egoB[ii].x, k.wb, k.hEx, k.hEy, s0.x, s0.y,
-                                          __ldg(&k.tab.tpsi[(size_t)ii * k.tab.Ap + as]), __int_as_float(pa.z),
+                                          __ldg(&tpsi[(size_t)ii * Ap + as]), __int_as_float(pa.z),
                                           __int_as_float(pa.w));
       atomicMin(&dkey[ial], (r << 8) | (uint32_t)ii);
     }
   }
   __syncwarp();
 }
+static __device__ __noinline__ void dt_drain_ties(const MetricKArgs& k, const float4* egoA, const float2* egoB,
+                                                  uint32_t* dkey, const uint2* src, int cnt, int a0, int lane) {
+  dt_drain_ties_body(k, k.tab.t0, k.tab.prm, k.tab.tpsi, k.tab.Ap, egoA, egoB, dkey, src, cnt, a0, lane);
+}
+// batched kernel: the agent table is the trajectory's problem's, passed in registers
+static __device__ __noinline__ void dt_drain_ties_batch(const MetricKArgs& k, const float4* t0, const AgentParams* prm,
+                                                        const float* tpsi, int Ap, const float4* egoA, const float2* egoB,
+                                                        uint32_t* dkey, const uint2* src, int cnt, int a0, int lane) {
+  dt_drain_ties_body(k, t0, prm, tpsi, Ap, egoA, egoB, dkey, src, cnt, a0, lane);
+}
 
-// MASK != 0: the activated metrics are a compile-time constant (all seven / the default six); 0 = read k.mmask
-template <uint32_t MASK>
-__global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_kernel(const __grid_constant__ MetricKArgs k) {
+// MASK != 0: the activated metrics are a compile-time constant (all seven / the default six); 0 = read k.mmask.
+// BATCH: every trajectory takes its agent table, agent count and pair / step blocks from its problem (bv); otherwise
+// from k, whose fields then stay kernel-parameter operands.
+template <uint32_t MASK, bool BATCH>
+__device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailView& bv) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const int T = k.T, Ap = k.tab.Ap, Tm1 = T - 1;
+  const int T = k.T, Tm1 = T - 1, Apk = k.tab.Ap;
   // ---- shared memory of this warp -----------------------------------------------------------------------------
   unsigned char* const wbase = smem_raw + (size_t)wib * detail_warp_bytes(T);
   float* const stage = reinterpret_cast<float*>(wbase);                          // [32][kDtRow] (cp, ego_harm, obst_harm)
@@ -143,22 +156,53 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
   float* const dist = reinterpret_cast<float*>(egoB + T);                        // [T] cumulative chord length (BE)
   const auto soff = [&](const void* q) { return (uint32_t)(reinterpret_cast<const unsigned char*>(q) - smem_raw); };
   const BeView bev{soff(egoA), soff(egoB), soff(dist), soff(inv), 0u};
-  const BeConst bek = be_const(k);
+  const BeConst bek = be_const(k);                // batched: the table and its stride are set per bisection
+  // batched: the warp's copy of its problem's descriptor, behind the per-warp regions (read where used, not held in
+  // registers across the trajectory)
+  DetailProb* const sdp = reinterpret_cast<DetailProb*>(smem_raw + kDtWarps * detail_warp_bytes(T)) + wib;
 
   const uint32_t mm = MASK ? MASK : k.mmask;
   const bool do_cp = mm & FO_M_CP, do_dce = mm & FO_M_DCE, do_hr = mm & FO_M_HR, do_be = mm & FO_M_BE,
              do_ttc = mm & FO_M_TTC;
   const unsigned lt_mask = (1u << lane) - 1u;
   const float rE = sqrtf(k.hEx * k.hEx + k.hEy * k.hEy);
-  const bool rows8 = (Tm1 & 1) == 0 && (reinterpret_cast<uintptr_t>(k.step) & 7u) == 0;   // row segments 8-byte aligned
-  const size_t traj_step = (size_t)k.A * (size_t)Tm1 * FO_STEP_K;
+  bool rows8 = (Tm1 & 1) == 0 && (reinterpret_cast<uintptr_t>(k.step) & 7u) == 0;   // row segments 8-byte aligned
+  size_t traj_step = (size_t)k.A * (size_t)Tm1 * FO_STEP_K;
   float* const srow_lane = stage + lane * kDtRow;
 
-  // warp = trajectory: the first one by global warp index, every further one from the device counter
+  // warp = trajectory: the first one by global warp index, every further one from the device counter.  A batch looks up
+  // the problem of the next trajectory together with its claim.
   const int gw = blockIdx.x * kDtWarps + wib, n_gw = gridDim.x * kDtWarps;
+  int p = BATCH ? find_problem(bv.first, bv.P, gw) : 0;
   for (int n = gw; n < k.N;) {
-    int n_next = 0;
-    if (lane == 0) n_next = k.claim ? (int)(n_gw + atomicAdd(k.claim, 1u)) : n + n_gw;
+    int n_next = 0, p_next = 0;
+    if (lane == 0) {
+      n_next = k.claim ? (int)(n_gw + atomicAdd(k.claim, 1u)) : n + n_gw;
+      if constexpr (BATCH) p_next = n_next < k.N ? find_problem(bv.first, bv.P, n_next) : 0;
+    }
+    int nb = n;                                        // the trajectory's index in its pair / step block
+    if constexpr (BATCH) {
+      if (lane < (int)(sizeof(DetailProb) / 16))
+        reinterpret_cast<int4*>(sdp)[lane] = __ldg(reinterpret_cast<const int4*>(bv.prob + p) + lane);
+      __syncwarp();
+      nb = n - sdp->row0;
+      rows8 = (Tm1 & 1) == 0 && (reinterpret_cast<uintptr_t>(sdp->step) & 7u) == 0;
+      traj_step = (size_t)sdp->A * (size_t)Tm1 * FO_STEP_K;
+    }
+    // references into the kernel parameters when not batched (their uses stay constant-bank operands), into the
+    // descriptor's shared-memory copy when batched
+    const auto& tab = [&]() -> const auto& { if constexpr (BATCH) return *sdp; else return k.tab; }();
+    const int& A = BATCH ? sdp->A : k.A;
+    const int& Tp = BATCH ? sdp->Tp : k.Tp;
+    const int& Ap = BATCH ? sdp->Ap : Apk;
+    float* const& pair = BATCH ? sdp->pair : k.pair;
+    float* const& step = BATCH ? sdp->step : k.step;
+    const auto drain_ties = [&](const uint2* src, int cnt, int a0) {
+      if constexpr (BATCH)
+        dt_drain_ties_batch(k, tab.t0, tab.prm, tab.tpsi, Ap, egoA, egoB, dkey, src, cnt, a0, lane);
+      else
+        dt_drain_ties(k, egoA, egoB, dkey, src, cnt, a0, lane);
+    };
     // ---- stage the ego trajectory (this warp only) ---------------------------------------------------------------
     const float* eg = k.ego + (size_t)n * T * 5;
     float amin = 0.0f;
@@ -178,20 +222,20 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
       const float am = __uint_as_float(__reduce_max_sync(kFull, __float_as_uint(fabsf(amin))));   // |min(min a, 0)|, be.py:68 (amin <= 0)
       be_lo0 = rintf(am * 100.0f) / 100.0f;
     }
-    float* const step_n = k.step ? k.step + (size_t)n * traj_step : nullptr;
+    float* const step_n = step ? step + (size_t)nb * traj_step : nullptr;
 
     // per-lane accumulators over the tiles (reduced once per trajectory)
     float acc_er = 0.0f, acc_or = 0.0f, acc_eh = 0.0f, acc_oh = 0.0f, acc_cp = 0.0f, acc_hwc = 0.0f;
     float acc_btn = 0.0f, acc_rcd = 0.0f;
     uint32_t acc_rmin = 0xffffffu, acc_col = 0xffffffffu, flags = 0u;
 
-    for (int a0 = 0; a0 < k.A; a0 += 32) {
+    for (int a0 = 0; a0 < A; a0 += 32) {
       const int a = a0 + lane;                           // slot (always inside the padded tables)
-      const bool alive = a < k.A;
+      const bool alive = a < A;
       AgentParams P;
       P.n_states = 0; P.model = 2; P.hl = P.hw = P.hlb = P.ke = P.ko = P.pad = 0.0f;
       int ao = 0;
-      if (alive) { P = load_params(k.tab.prm + a); ao = __ldg(k.tab.orig + a); }
+      if (alive) { P = load_params(tab.prm + a); ao = __ldg(tab.orig + a); }
       const int nA = min(T, P.n_states);                 // DCE / CP range (dce.py:87-88, collision_probability.py:73)
       const int nH = min(Tm1, P.n_states);               // harm range (harm_model.py:67)
       const uint32_t rowoff = alive ? (uint32_t)ao * (uint32_t)(Tm1 * FO_STEP_K) : 0xffffffffu;
@@ -202,7 +246,7 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
       int i_star = -1;                                   // step of the smallest centre distance
       if (do_dce) {
         const int nAmax = (int)__reduce_max_sync(kFull, (unsigned)nA);
-        const float4* t0p = k.tab.t0 + a;
+        const float4* t0p = tab.t0 + a;
 #pragma unroll 2
         for (int i = 0; i < nAmax; ++i, t0p += Ap) {
           if (i < nA) {
@@ -240,8 +284,8 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
         if (lane < cnt) {
           const int ial = (int)(item >> 8), ii = (int)(item & 0xffu);
           const int as = a0 + ial;
-          const float4 s0 = __ldg(&k.tab.t0[(size_t)ii * Ap + as]);
-          const int4 pa = __ldg(reinterpret_cast<const int4*>(k.tab.prm + as));
+          const float4 s0 = __ldg(&tab.t0[(size_t)ii * Ap + as]);
+          const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + as));
           const float4 EA = egoA[ii];
           const float c = fmaf(EA.z, s0.z, EA.w * s0.w), s = fmaf(s0.w, EA.z, -s0.z * EA.w);
           const float dx = (s0.x - EA.x) - k.wb * EA.z, dy = (s0.y - EA.y) - k.wb * EA.w;
@@ -260,7 +304,7 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
             if (tie) q_tie[qt + __popc(tb & lt_mask)] = make_uint2(item, r32);
             qt += __popc(tb);
             __syncwarp();
-            if (qt >= 32) { qt -= 32; dt_drain_ties(k, egoA, egoB, dkey, q_tie + qt, 32, a0, lane); }
+            if (qt >= 32) { qt -= 32; drain_ties(q_tie + qt, 32, a0); }
           }
         }
         __syncwarp();
@@ -274,11 +318,11 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
         const uint32_t ro = __shfl_sync(kFull, rowoff, ial);
         if (lane < cnt) {
           const int as = a0 + ial;
-          const AgentParams Q = load_params(k.tab.prm + as);
-          const size_t idx = (size_t)as * k.Tp + ii;
-          const float4 s0i = __ldg(&k.tab.s0[idx]);
-          const float4 s1i = __ldg(&k.tab.s1[idx]);
-          const float2 s2i = __ldg(&k.tab.s2[idx]);
+          const AgentParams Q = load_params(tab.prm + as);
+          const size_t idx = (size_t)as * Tp + ii;
+          const float4 s0i = __ldg(&tab.s0[idx]);
+          const float4 s1i = __ldg(&tab.s1[idx]);
+          const float2 s2i = __ldg(&tab.s2[idx]);
           const float4 Ei = egoA[ii];
           const float cp = cp_gauss_boxes<false>(s1i.z - Ei.x, s1i.w - Ei.y, Q.hlb * s0i.z, Q.hlb * s0i.w, k.L3 * Ei.z,
                                           k.L3 * Ei.w, s2i, k.L6, k.W2);
@@ -295,8 +339,8 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
               he = staged ? srow[1] : __ldcg(grow + 1);
               ho = staged ? srow[2] : __ldcg(grow + 2);
             } else {                           // no step array to read back from: same arithmetic as the step loop
-              const float4 s0t = __ldg(&k.tab.s0[idx - 1]);
-              const float4 s1t = __ldg(&k.tab.s1[idx - 1]);
+              const float4 s0t = __ldg(&tab.s0[idx - 1]);
+              const float4 s1t = __ldg(&tab.s1[idx - 1]);
               const float4 Et = egoA[t];
               const float2 EtB = egoB[t];
               dt_harm(k.hc, Q.model, harm_lin(k.hc, Q.model, Q.ke, Q.ko), EtB.y, s1t.y, fmaf(Et.z, s0t.z, Et.w * s0t.w),
@@ -359,7 +403,7 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
         const bool liveA = i < nA;
         float4 s0 = make_float4(0.0f, 0.0f, 1.0f, 0.0f);
         float va = 0.0f;
-        if (liveA) { s0 = __ldg(k.tab.t0 + toff); va = __ldg(k.tab.tv + toff); }
+        if (liveA) { s0 = __ldg(tab.t0 + toff); va = __ldg(tab.tv + toff); }
         const int ie = last ? Tm1 : i;
         const float4 EA = egoA[ie];
         const float2 EB = egoB[ie];
@@ -380,7 +424,7 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
           // harm at state t = i (same index both sides), harm_model.py:81-105; NaN where the agent has no state
           float he = CUDART_NAN_F, ho = CUDART_NAN_F;
           if (do_hr && i < nH) {
-            const float psi = (P.model == 1) ? __ldg(k.tab.tpsi + toff) : 0.0f;
+            const float psi = (P.model == 1) ? __ldg(tab.tpsi + toff) : 0.0f;
             dt_harm(k.hc, P.model, hl, EB.y, va, c, dxr, dyr, EB.x, psi, he, ho);
             eh_m = fmaxf(eh_m, he);
             oh_m = fmaxf(oh_m, ho);
@@ -411,7 +455,7 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
         }
       }
       __syncwarp();
-      while (qt > 0) { const int cn = min(qt, 32); qt -= cn; dt_drain_ties(k, egoA, egoB, dkey, q_tie + qt, cn, a0, lane); }
+      while (qt > 0) { const int cn = min(qt, 32); qt -= cn; drain_ties(q_tie + qt, cn, a0); }
 
       // ---- per-pair results ---------------------------------------------------------------------------------------
       const unsigned long long ck = ckey[lane], ok = okey[lane];
@@ -426,9 +470,9 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
         if (step_n) {
           hwc = __ldcg(step_n + rowoff + 3 * cp_arg + 2);
         } else {
-          const size_t idx = (size_t)a * k.Tp + cp_arg;
-          const float4 s0t = __ldg(&k.tab.s0[idx]);
-          const float4 s1t = __ldg(&k.tab.s1[idx]);
+          const size_t idx = (size_t)a * Tp + cp_arg;
+          const float4 s0t = __ldg(&tab.s0[idx]);
+          const float4 s1t = __ldg(&tab.s1[idx]);
           const float4 Et = egoA[cp_arg];
           const float2 EtB = egoB[cp_arg];
           float he;
@@ -456,15 +500,17 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
           todo &= todo - 1;
           const int ns_s = __shfl_sync(kFull, P.n_states, src);
           const float hl_s = __shfl_sync(kFull, P.hl, src), hw_s = __shfl_sync(kFull, P.hw, src);
-          const float r = be_bisect<false>(bek, bev, a0 + src, ns_s, hl_s, hw_s, be_lo0, lane, -1.0f).x;
+          BeConst bk = bek;
+          if constexpr (BATCH) { bk.s0 = tab.s0; bk.Tp = Tp; }   // BE bisections read the problem's agent-major states
+          const float r = be_bisect<false>(bk, bev, a0 + src, ns_s, hl_s, hw_s, be_lo0, lane, -1.0f).x;
           if (r != r) flags |= FO_F_BE_RANGE;            // NaN: the re-timed path overruns the planned one
           if (lane == src) { rcd = r; btn = __fdividef(r, k.a_max); }
         }
         acc_rcd = fmaxf(acc_rcd, rcd);     // fmaxf ignores NaN
         acc_btn = fmaxf(acc_btn, btn);
       }
-      if (k.pair && alive) {
-        float4* pr = reinterpret_cast<float4*>(k.pair + ((size_t)n * k.A + ao) * FO_PAIR_K);
+      if (pair && alive) {
+        float4* pr = reinterpret_cast<float4*>(pair + ((size_t)nb * A + ao) * FO_PAIR_K);
         pr[0] = make_float4(has_d ? mm_to_m(kmin >> 8) : CUDART_INF_F, has_d ? (float)t_col : 0.0f, er_m, or_m);
         pr[1] = make_float4((float)or_arg, hwc, eh_m, oh_m);
         pr[2] = make_float4(cpmax, rcd, btn, (float)cp_arg);
@@ -479,7 +525,7 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
       const uint32_t rmin = __reduce_min_sync(kFull, acc_rmin), col = __reduce_min_sync(kFull, acc_col);
       const uint32_t fl = __reduce_or_sync(kFull, flags);
       if (lane == 0) {
-        const bool has_agents = k.A > 0 && mm != 0;
+        const bool has_agents = A > 0 && mm != 0;
         const bool has_col = col != 0xffffffffu;
         bool ok = true;
         if (has_agents) {
@@ -504,24 +550,40 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
       }
     }
     n = __shfl_sync(kFull, n_next, 0);
+    if constexpr (BATCH) p = __shfl_sync(kFull, p_next, 0);
     __syncwarp();                                      // the ego arrays are rewritten by the next trajectory
   }
 }
 
 template <uint32_t MASK>
-static int launch_detail_inst(const MetricKArgs& k, int num_sms, cudaStream_t st) {
-  const size_t smem = (size_t)kDtWarps * detail_warp_bytes(k.T);
+__global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_kernel(const __grid_constant__ MetricKArgs k) {
+  detail_body<MASK, false>(k, DetailView{});
+}
+
+// A batch of independent problems (fo_metric_batch_detail): k.N = all rows of the batch, k.tab / k.A / k.Tp / k.pair /
+// k.step are unused -- every trajectory takes them from its problem.
+template <uint32_t MASK>
+__global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB)
+fo_metric_batch_detail_kernel(const __grid_constant__ MetricKArgs k, const __grid_constant__ DetailView bv) {
+  detail_body<MASK, true>(k, bv);
+}
+
+// Persistent launch of one detail-kernel instantiation: as many CTAs as fit on the device, warps claiming trajectories.
+template <auto KERNEL, class... Extra>
+static int launch_detail_kernel(const MetricKArgs& k, int num_sms, size_t smem_extra, cudaStream_t st,
+                                const Extra&... extra) {
+  const size_t smem = (size_t)kDtWarps * detail_warp_bytes(k.T) + smem_extra;
   constexpr int kMaxDev = 64;
   static std::atomic<size_t> configured[kMaxDev];
   int dev = 0;
   FO_CUDA_TRY(cudaGetDevice(&dev));
   const bool tracked = dev >= 0 && dev < kMaxDev;
   if (!tracked || smem > configured[dev].load(std::memory_order_acquire)) {
-    FO_CUDA_TRY(cudaFuncSetAttribute(fo_metric_detail_kernel<MASK>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    FO_CUDA_TRY(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     if (tracked) configured[dev].store(smem, std::memory_order_release);
   }
   int per_sm = 1;
-  FO_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fo_metric_detail_kernel<MASK>, kDtWarps * 32, smem));
+  FO_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, KERNEL, kDtWarps * 32, smem));
   if (per_sm < 1) per_sm = 1;
   const int full = num_sms * per_sm;
   const int need = (k.N + kDtWarps - 1) / kDtWarps;
@@ -529,11 +591,14 @@ static int launch_detail_inst(const MetricKArgs& k, int num_sms, cudaStream_t st
   MetricKArgs kk = k;
   kk.claim = (k.N > grid * kDtWarps) ? claim_slot(st) : nullptr;     // trajectories differ several-fold in cost
   if (kk.claim) FO_CUDA_TRY(cudaMemsetAsync(kk.claim, 0, sizeof(unsigned int), st));
-  fo_metric_detail_kernel<MASK><<<grid, kDtWarps * 32, smem, st>>>(kk);
+  KERNEL<<<grid, kDtWarps * 32, smem, st>>>(kk, extra...);
   count_launch();
   FO_CUDA_TRY(cudaGetLastError());
   return FO_OK;
 }
+
+constexpr uint32_t kDtAll = FO_M_CP | FO_M_DCE | FO_M_TTC | FO_M_HR | FO_M_BE | FO_M_TTCE | FO_M_WTTC;
+constexpr uint32_t kDtDefault = kDtAll & ~FO_M_BE;   // occlusion.yaml:12-18
 
 int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st) {
   if (k.pair && (reinterpret_cast<uintptr_t>(k.pair) & 15u)) {
@@ -544,11 +609,17 @@ int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st) {
     set_error("fo_metric_bundle: step must be 4-byte aligned");
     return FO_ERR_INVALID_ARG;
   }
-  constexpr uint32_t kAll = FO_M_CP | FO_M_DCE | FO_M_TTC | FO_M_HR | FO_M_BE | FO_M_TTCE | FO_M_WTTC;
-  constexpr uint32_t kDefault = kAll & ~FO_M_BE;   // occlusion.yaml:12-18
-  if (k.mmask == kAll) return launch_detail_inst<kAll>(k, num_sms, st);
-  if (k.mmask == kDefault) return launch_detail_inst<kDefault>(k, num_sms, st);
-  return launch_detail_inst<0u>(k, num_sms, st);
+  if (k.mmask == kDtAll) return launch_detail_kernel<fo_metric_detail_kernel<kDtAll>>(k, num_sms, 0, st);
+  if (k.mmask == kDtDefault) return launch_detail_kernel<fo_metric_detail_kernel<kDtDefault>>(k, num_sms, 0, st);
+  return launch_detail_kernel<fo_metric_detail_kernel<0u>>(k, num_sms, 0, st);
+}
+
+// k.N = the batch's rows; the caller has validated the descriptors and the alignment of every pair / step block
+int launch_metric_batch_detail(const MetricKArgs& k, int num_sms, const DetailView& bv, cudaStream_t st) {
+  constexpr size_t x = kDtWarps * sizeof(DetailProb);   // the warps' descriptor copies
+  if (k.mmask == kDtAll) return launch_detail_kernel<fo_metric_batch_detail_kernel<kDtAll>>(k, num_sms, x, st, bv);
+  if (k.mmask == kDtDefault) return launch_detail_kernel<fo_metric_batch_detail_kernel<kDtDefault>>(k, num_sms, x, st, bv);
+  return launch_detail_kernel<fo_metric_batch_detail_kernel<0u>>(k, num_sms, x, st, bv);
 }
 
 }  // namespace fo

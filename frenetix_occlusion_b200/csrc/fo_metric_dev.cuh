@@ -484,6 +484,39 @@ struct BatchView {
   const BatchProb* prob;
   int P;
 };
+// the last p in [0, P) with first[p] <= n (first strictly increasing, first[0] <= n)
+__device__ __forceinline__ int find_problem(const int* first, int P, int n) {
+  int lo = 0, hi = P - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(first + mid) <= n) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+// Batch of independent problems with detail outputs (fo_metric_batch_detail): one launch over all rows [0, n_traj).
+// Besides the table pointers the detail kernel and its helpers read, a descriptor holds the base of the problem's pair /
+// step block (NULL when that output is not requested); all resolved on the host.
+struct __align__(16) DetailProb {
+  const float4* t0;
+  const float* tv;
+  const float4* s0;
+  const float4* s1;
+  const float2* s2;
+  const AgentParams* prm;
+  const int32_t* orig;
+  const float* tpsi;
+  float* pair;          // [N_p, A_p, FO_PAIR_K]
+  float* step;          // [N_p, A_p, T-1, FO_STEP_K]
+  int row0;             // the problem's first row in ego / valid / summary / flags
+  int A, Tp, Ap;        // agents, table stride, agents padded to 32
+};
+static_assert(sizeof(DetailProb) == 96, "six 16-byte loads");
+struct DetailView {
+  const int* first;     // [P] DetailProb::row0, strictly increasing (problems without trajectories are left out)
+  const DetailProb* prob;
+  int P;
+};
+int launch_metric_batch_detail(const MetricKArgs& k, int num_sms, const DetailView& bv, cudaStream_t st);
 // summary kernel over one shape class of a batch (uni: the one-warp window-filter shape, W == 1); k.N = the class's
 // trajectory count
 int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st);

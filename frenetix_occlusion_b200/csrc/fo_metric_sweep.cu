@@ -204,14 +204,7 @@ static __device__ __noinline__ uint32_t sw_drain_ties_batch(const MetricKArgs& k
 }
 
 // problem of trajectory n: the last p with first[p] <= n
-__device__ __forceinline__ int batch_find(const BatchView& b, int n) {
-  int lo = 0, hi = b.P - 1;
-  while (lo < hi) {
-    const int mid = (lo + hi + 1) >> 1;
-    if (__ldg(b.first + mid) <= n) lo = mid; else hi = mid - 1;
-  }
-  return lo;
-}
+__device__ __forceinline__ int batch_find(const BatchView& b, int n) { return find_problem(b.first, b.P, n); }
 
 struct SweepShape {
   int lg_agents;   // log2 of the agents held by one warp (0..5); a warp has 32 >> lg_agents time slices

@@ -140,17 +140,32 @@ class BundleResult:
 
 @dataclass
 class BatchResult:
-    """Results of a batch of independent problems: rows ``offsets[p]:offsets[p+1]`` belong to problem p."""
+    """Results of a batch of independent problems: rows ``offsets[p]:offsets[p+1]`` belong to problem p.  The detail
+    outputs are flat: problem p's [N_p, A_p, ...] blocks sit back to back in problem order (``fo_metric_batch_detail``)."""
     valid: torch.Tensor                # uint8 [N_total]
     summary: torch.Tensor              # float32 [N_total, FO_SUMMARY_K]
     flags: torch.Tensor                # int32 [N_total]
     offsets: np.ndarray                # int64 [P + 1]
+    pair: Optional[torch.Tensor] = None     # float32 [sum_p N_p A_p FO_PAIR_K]
+    step: Optional[torch.Tensor] = None     # float32 [sum_p N_p A_p (T-1) FO_STEP_K]
+    n_agents: Optional[np.ndarray] = None   # A_p, with pair / step
+    n_states: int = 0                       # T, with pair / step
 
     def split(self) -> list:
-        """Per-problem ``BundleResult`` views of the batch tensors (no copies)."""
+        """Per-problem ``BundleResult`` views of the batch tensors (no copies): pair [N_p, A_p, FO_PAIR_K] and step
+        [N_p, A_p, T-1, FO_STEP_K] where the batch has them."""
         o = [int(x) for x in self.offsets]
-        return [BundleResult(self.valid[o[p]:o[p + 1]], self.summary[o[p]:o[p + 1]], self.flags[o[p]:o[p + 1]])
-                for p in range(len(o) - 1)]
+        out, q, tm1 = [], 0, max(self.n_states - 1, 0)
+        for p in range(len(o) - 1):
+            r = BundleResult(self.valid[o[p]:o[p + 1]], self.summary[o[p]:o[p + 1]], self.flags[o[p]:o[p + 1]])
+            n, a = o[p + 1] - o[p], int(self.n_agents[p]) if self.n_agents is not None else 0
+            if self.pair is not None:
+                r.pair = self.pair[q * L.FO_PAIR_K:(q + n * a) * L.FO_PAIR_K].view(n, a, L.FO_PAIR_K)
+            if self.step is not None:
+                r.step = self.step[q * tm1 * L.FO_STEP_K:(q + n * a) * tm1 * L.FO_STEP_K].view(n, a, tm1, L.FO_STEP_K)
+            q += n * a
+            out.append(r)
+        return out
 
 
 class MetricEngine:
@@ -185,6 +200,7 @@ class MetricEngine:
         self._raw_dev = None
         self.n_agents = 0
         self.t_stride = 0
+        self._pack_pending = False    # agents adopted without their table (_adopt_agents): packed by the next launch
         self._batch = None
         self._staging = None          # page-locked staging of assess_batch's host bundles
         self._staging_done = None
@@ -196,16 +212,31 @@ class MetricEngine:
     def set_agents(self, agents: AgentSet, origin=None):
         """Upload + pack the phantom predictions (once per planning cycle).  ``origin`` (x, y) is
         subtracted in float64 from agent and ego positions before the cast to float32."""
+        self._adopt_agents(agents, origin)
+        self._pack_agents()
+
+    def _adopt_agents(self, agents: AgentSet, origin=None):
+        """The host side of ``set_agents``: the engine takes ``agents`` and ``origin`` as its own, and the next launch
+        that needs their table packs it (for results computed elsewhere, e.g. by ``batch.prefetch_interfaces``)."""
         self.agents = agents
         self.origin = np.zeros(2) if origin is None else np.asarray(origin, dtype=np.float64)
         A, Tp = agents.n_agents, agents.t_stride
         self.n_agents, self.t_stride = A, Tp
+        self._table = None
+        self._pack_pending = False
         if A == 0 or Tp == 0:
-            self._table = None
             self.n_agents = 0
             return
         if Tp > L.FO_MAX_STATES:
             raise ValueError(f"predictions longer than {L.FO_MAX_STATES} states are not supported")
+        self._pack_pending = True
+
+    def _pack_agents(self):
+        """Upload + pack the adopted agents' table, if it is not packed yet."""
+        if not self._pack_pending:
+            return
+        self._pack_pending = False
+        agents, A, Tp = self.agents, self.n_agents, self.t_stride
         fl = np.stack([agents.x - self.origin[0], agents.y - self.origin[1], agents.yaw, agents.v,
                        agents.var_x, agents.var_y]).astype(np.float32)
         pa = np.stack([agents.length, agents.width, agents.buf_length, agents.buf_width]).astype(np.float32)
@@ -277,6 +308,7 @@ class MetricEngine:
         t = self.to_device_bundle(ego)
         N = int(t.shape[0])
         dev = self.device
+        self._pack_agents()
         with torch.cuda.device(dev):
             out = BundleResult(torch.empty(N, dtype=torch.uint8, device=dev),
                                torch.empty((N, L.FO_SUMMARY_K), dtype=torch.float32, device=dev),
@@ -299,6 +331,7 @@ class MetricEngine:
             raise ValueError(f"trajectories longer than {L.FO_MAX_STATES} states are not supported")
         A = self.n_agents
         dev = self.device
+        self._pack_agents()
         with torch.cuda.device(dev):
             if out is None:
                 out = BundleResult(torch.empty(N, dtype=torch.uint8, device=dev),
@@ -355,7 +388,7 @@ class MetricEngine:
         A, S = int(n_agents.sum()), int(t_stride.max(initial=0))
         dev = self.device
         self._batch = {"problems": problems, "P": P, "origins": org, "agents": list(agent_sets), "arena": None,
-                       "arena_bytes": arena_bytes}
+                       "arena_bytes": arena_bytes, "n_agents": n_agents}
         if A == 0:
             return
         # one host buffer: 6 float rows [A, S] (x, y shifted per problem), 4 float columns [A], 2 int32 columns [A]
@@ -416,10 +449,14 @@ class MetricEngine:
         self._staging_done.record(torch.cuda.current_stream(self.device))
         return t
 
-    def assess_batch(self, egos: Sequence) -> BatchResult:
-        """Summary pass over every problem of the batch set by ``set_agent_batch`` in one ``fo_metric_batch`` call.
-        ``egos[p]``: problem p's [N_p, T, 5] bundle (host array or CUDA tensor, in the caller's frame: it is shifted by
-        the problem's origin).  Asynchronous on the current stream."""
+    def assess_batch(self, egos: Sequence, want_pair: bool = False, want_step: bool = False,
+                     out: Optional[BatchResult] = None) -> BatchResult:
+        """One pass over every problem of the batch set by ``set_agent_batch`` in one metric call.  ``egos[p]``: problem
+        p's [N_p, T, 5] bundle (host array or CUDA tensor, in the caller's frame: it is shifted by the problem's origin).
+        Without detail outputs this is ``fo_metric_batch``; with ``want_pair`` / ``want_step`` it is
+        ``fo_metric_batch_detail``, and ``split()`` gives problem p what ``set_agents`` + ``assess(want_pair,
+        want_step)`` gives it alone.  ``out``: preallocated outputs of the batch's sizes (valid / summary / flags, and
+        the flat pair / step where wanted).  Asynchronous on the current stream."""
         b = self._batch
         if b is None:
             raise RuntimeError("assess_batch() needs set_agent_batch() first")
@@ -445,6 +482,7 @@ class MetricEngine:
         N = int(offsets[-1])
         dev = self.device
         row_origin = np.repeat(b["origins"], counts, axis=0)
+        n_pairs = int(np.dot(counts, b["n_agents"].astype(np.int64))) if P else 0
         with torch.cuda.device(dev):
             if N and all(on_dev):
                 t = self.to_device_bundle(torch.cat([e.reshape(-1, T, 5) for e in parts]), origin=row_origin)
@@ -452,18 +490,34 @@ class MetricEngine:
                 t = self._stage_host_batch(parts, b["origins"], offsets, T)
             else:
                 t = torch.empty((0, T, 5), dtype=torch.float32, device=dev)
-            out = BundleResult(torch.empty(N, dtype=torch.uint8, device=dev),
-                               torch.empty((N, L.FO_SUMMARY_K), dtype=torch.float32, device=dev),
-                               torch.empty(N, dtype=torch.int32, device=dev))
+            if out is None:
+                out = BatchResult(torch.empty(N, dtype=torch.uint8, device=dev),
+                                  torch.empty((N, L.FO_SUMMARY_K), dtype=torch.float32, device=dev),
+                                  torch.empty(N, dtype=torch.int32, device=dev), offsets)
+                if want_pair:
+                    out.pair = torch.empty(n_pairs * L.FO_PAIR_K, dtype=torch.float32, device=dev)
+                if want_step:
+                    out.step = torch.empty(n_pairs * max(T - 1, 0) * L.FO_STEP_K, dtype=torch.float32, device=dev)
+            out.offsets, out.n_agents, out.n_states = offsets, b["n_agents"], T
+            if not want_pair:
+                out.pair = None
+            if not want_step:
+                out.step = None
             problems = b["problems"]
             for p in range(P):
                 problems[p].traj_begin, problems[p].n_traj = int(offsets[p]), int(counts[p])
             a = L.FoMetricBatchArgs()
-            a.common = self._args(t, out)
+            a.common = self._args(t, BundleResult(out.valid, out.summary, out.flags))
             a.common.agent_table = b["arena"].data_ptr() if b["arena"] is not None else None
             a.common.n_agents, a.common.t_stride = 0, 1
             a.n_problems, a.problems, a.arena_bytes = P, problems, b["arena_bytes"]
-            L.check(L.lib.fo_metric_batch(C.byref(a), self._stream()), "fo_metric_batch")
-        res = BatchResult(out.valid, out.summary, out.flags, offsets)
-        res._keepalive = (t, b["arena"])
-        return res
+            # a problem without agents or a horizon of one state has no detail to write: as in assess, the summary
+            # path runs when no detail buffer is left
+            a.common.pair = out.pair.data_ptr() if (out.pair is not None and out.pair.numel()) else None
+            a.common.step = out.step.data_ptr() if (out.step is not None and out.step.numel()) else None
+            if a.common.pair or a.common.step:
+                L.check(L.lib.fo_metric_batch_detail(C.byref(a), self._stream()), "fo_metric_batch_detail")
+            else:
+                L.check(L.lib.fo_metric_batch(C.byref(a), self._stream()), "fo_metric_batch")
+        out._keepalive = (t, b["arena"])
+        return out

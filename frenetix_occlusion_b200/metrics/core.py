@@ -99,7 +99,19 @@ class MetricCore:
                 "summary": r.summary.cpu().numpy().astype(np.float64),
                 "pair": r.pair.cpu().numpy().astype(np.float64), "step": r.step.cpu().numpy().astype(np.float64),
                 "ego": ego}
-        self._prefetch_host = host
+        return self.install_prefetch(trajectories, host)
+
+    def install_prefetch(self, trajectories, host, agents=None, origin=None):
+        """Serve the per-trajectory calls for ``trajectories`` (row k of ``host`` belongs to ``trajectories[k]``) from
+        the host results ``host``: valid [N], flags [N], summary [N, K], pair [N, A, FO_PAIR_K], step [N, A, T-1,
+        FO_STEP_K] and the stacked ego [N, T, 5].  ``agents`` / ``origin``: the agent set the results were computed for,
+        when they were computed outside this core (``batch.prefetch_interfaces``).  It becomes the core's agent set for
+        the current predictions without a pack of its own; a trajectory that misses the prefetch packs it first."""
+        if agents is not None:
+            self.engine._adopt_agents(agents, origin=origin)
+            self._fingerprint = self._agents_fingerprint()
+            self._cache = self._cache_ego = None
+        self._prefetch_host = host if trajectories else None
         self._prefetched = {id(t): (t, k) for k, t in enumerate(trajectories)}
         return len(trajectories)
 

@@ -203,7 +203,8 @@ int fo_agents_pack_batch(const FoAgentsRaw *raw, int32_t n_problems, const FoBat
 
 typedef struct FoMetricBatchArgs {
   FoMetricArgs common;     /* ego [n_traj, T, 5] of all problems, n_traj = sum N_p; agent_table = the arena;
-                              n_agents / t_stride are ignored (per problem); pair / step must be NULL, n_peers 0 */
+                              n_agents / t_stride are ignored (per problem); n_peers 0; pair / step must be NULL for
+                              fo_metric_batch (see fo_metric_batch_detail) */
   int32_t n_problems;
   int32_t reserved_;
   const FoBatchProblem *problems;   /* HOST [n_problems]: validated before any device work */
@@ -216,6 +217,18 @@ typedef struct FoMetricBatchArgs {
  * launch).  The per-problem descriptors are staged through library-owned page-locked and device buffers (per calling
  * thread and device).  Not capturable in a CUDA graph. */
 int fo_metric_batch(const FoMetricBatchArgs *args, void *stream);
+
+/* fo_metric_bundle's detail path over a batch, in one launch: valid / summary / flags of every row and the pair / step
+ * arrays of every problem.  Same arguments as fo_metric_batch, except that common.pair and / or common.step must be
+ * non-NULL (both NULL: FO_ERR_INVALID_ARG) and n_peers must be 0 (else FO_ERR_UNSUPPORTED).  Problem p's blocks sit back
+ * to back, in problem order:
+ *   pair: [N_p, A_p, FO_PAIR_K]          at float offset  FO_PAIR_K * sum_{q<p} N_q A_q
+ *   step: [N_p, A_p, T-1, FO_STEP_K]     at float offset  FO_STEP_K * (T-1) * sum_{q<p} N_q A_q
+ * pair must be 16-byte aligned (then so is every block) and step 4-byte aligned (every block is 8-byte aligned when T-1
+ * is even and step is).  Problem p's five outputs equal, bit for bit, what fo_metric_bundle gives for it alone with the
+ * same detail buffers requested; a problem without agents gets what fo_metric_bundle gives it without detail buffers.
+ * The descriptors are validated and staged as in fo_metric_batch.  Not capturable in a CUDA graph. */
+int fo_metric_batch_detail(const FoMetricBatchArgs *args, void *stream);
 
 
 /* ---- stage 1: sensor visibility by ray casting ----------------------------------------------------

@@ -21,9 +21,8 @@ from .engine import AgentSet, BatchResult, BundleResult, MetricEngine
 def _config(fi) -> dict:
     """What the batched call shares across problems, read from an interface's metric engine."""
     eng = fi.metrics._core.engine
-    v, h = eng.vehicle, eng.harm
+    h = eng.harm
     return {"device": torch.device(eng.device), "dt": eng.dt,
-            "vehicle": tuple(getattr(v, f) for f, _ in v._fields_),
             "metrics": eng.metric_mask,
             "thresholds": (eng.threshold_mask, tuple(sorted(eng.thresholds.items(), key=lambda kv: kv[0]))),
             "harm": tuple(getattr(h, f) for f, _ in h._fields_)}
@@ -38,8 +37,8 @@ def _bundle_array(bundle):
 
 
 def _batch_engine(interfaces, egos) -> MetricEngine:
-    """An engine with the configuration the interfaces share; ``ValueError`` when they or their trajectory lengths
-    differ."""
+    """An engine with the configuration the interfaces share (the ego vehicle is per problem: ``_vehicles``);
+    ``ValueError`` when they or their trajectory lengths differ."""
     cfgs = [_config(fi) for fi in interfaces]
     for i, c in enumerate(cfgs[1:], 1):
         diff = [k for k in c if c[k] != cfgs[0][k]]
@@ -49,9 +48,13 @@ def _batch_engine(interfaces, egos) -> MetricEngine:
     if len(lengths) > 1:
         raise ValueError(f"trajectory lengths differ across interfaces: {sorted(lengths)}")
     eng0 = interfaces[0].metrics._core.engine
-    return MetricEngine(dict(zip(("length", "width", "mass", "wb_rear_axle", "a_max"), cfgs[0]["vehicle"])), eng0.dt,
-                        list(eng0.order), eng0.thresholds,
+    return MetricEngine(eng0.vehicle, eng0.dt, list(eng0.order), eng0.thresholds,
                         harm_coeffs={f: getattr(eng0.harm, f) for f, _ in eng0.harm._fields_}, device=eng0.device)
+
+
+def _vehicles(interfaces) -> list:
+    """Each interface's ego vehicle, as its own metric engine holds it (from the interface's ``vehicle_params``)."""
+    return [fi.metrics._core.engine.vehicle for fi in interfaces]
 
 
 def _agents(fi):
@@ -73,9 +76,10 @@ def assess_interfaces(interfaces: Sequence, bundles: Sequence, want_pair: bool =
 
     Each interface's phantom predictions (``agent_manager.predictions``) are taken with the origin rule of
     ``MetricCore.sync_agents`` (the first agent's first position); an interface without phantom agents assesses
-    every trajectory as valid (``Metric.evaluate_metrics``).  The interfaces must agree on device, dt, vehicle
-    parameters, activated metrics, thresholds, harm coefficients and the trajectory length T, else ``ValueError``.
-    No interface's state, cache or prefetch is touched."""
+    every trajectory as valid (``Metric.evaluate_metrics``).  Each interface is assessed with its own ego vehicle
+    (``vehicle_params``), so the vehicles of a mixed fleet share one batch.  The interfaces must agree on device, dt,
+    activated metrics, thresholds, harm coefficients and the trajectory length T, else ``ValueError``.  No interface's
+    state, cache or prefetch is touched."""
     interfaces, bundles = list(interfaces), list(bundles)
     if len(interfaces) != len(bundles):
         raise ValueError(f"{len(interfaces)} interfaces but {len(bundles)} bundles")
@@ -84,7 +88,7 @@ def assess_interfaces(interfaces: Sequence, bundles: Sequence, want_pair: bool =
     egos = [_bundle_array(b) for b in bundles]
     eng = _batch_engine(interfaces, egos)
     agents = [_agents(fi) for fi in interfaces]
-    eng.set_agent_batch([a for a, _ in agents], [o for _, o in agents])
+    eng.set_agent_batch([a for a, _ in agents], [o for _, o in agents], vehicles=_vehicles(interfaces))
     return eng.assess_batch(egos, want_pair=want_pair, want_step=want_step).split()
 
 
@@ -110,7 +114,8 @@ def prefetch_interfaces(interfaces: Sequence, candidates: Sequence) -> list:
     if not live:
         return counts
     agents = [_agents(interfaces[i]) for i in live]
-    eng.set_agent_batch([a for a, _ in agents], [o for _, o in agents])
+    eng.set_agent_batch([a for a, _ in agents], [o for _, o in agents],
+                        vehicles=_vehicles([interfaces[i] for i in live]))
     n = np.array([len(e) for e in egos], dtype=np.int64)
     a = np.array([ag.n_agents if ag.t_stride > 0 else 0 for ag, _ in agents], dtype=np.int64)
     T = max([e.shape[1] for e in egos if len(e)], default=1)

@@ -31,9 +31,11 @@ __device__ __forceinline__ int protection_model(int kind) {  // harm_model.py:15
 }
 
 // One problem of a packing launch: its agents are rows [a_begin, a_begin + A) of the raw arrays (row stride
-// raw.t_stride), its table (stride Tp) starts table_off bytes into the arena.  fo_agents_pack is the one-problem case.
+// raw.t_stride), its table (stride Tp) starts table_off bytes into the arena, m_ego is its ego vehicle's mass (harm
+// mass split).  fo_agents_pack is the one-problem case.
 struct PackProblem {
-  int a_begin, A, Tp, pad_;
+  int a_begin, A, Tp;
+  float m_ego;
   long long table_off;
 };
 
@@ -64,7 +66,7 @@ __global__ void fo_agents_order_kernel(const int32_t* __restrict__ kind_all, Pac
 }
 
 // one thread per (agent slot, state) of a problem; blockIdx.y strides over the problems
-__global__ void fo_agents_pack_kernel(FoAgentsRaw raw, float m_ego, PackProblem one, const PackProblem* many, int P,
+__global__ void fo_agents_pack_kernel(FoAgentsRaw raw, PackProblem one, const PackProblem* many, int P,
                                       unsigned char* arena) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   const int S = raw.t_stride;
@@ -140,18 +142,26 @@ __global__ void fo_agents_pack_kernel(FoAgentsRaw raw, float m_ego, PackProblem 
       q.hw = 0.5f * raw.width[g];
       q.hlb = 0.5f * raw.buf_length[g];
       float mo = obstacle_mass(raw.kind[g], raw.buf_length[g] * raw.buf_width[g]);  // harm_model.py:73,78
-      q.ke = mo / (m_ego + mo);
-      q.ko = m_ego / (m_ego + mo);
+      q.ke = mo / (pp.m_ego + mo);
+      q.ko = pp.m_ego / (pp.m_ego + mo);
       q.pad = sqrtf(q.hl * q.hl + q.hw * q.hw);   // circumradius of the unbuffered rectangle (distance lower bound)
       const_cast<AgentParams*>(v.prm)[slot[idx]] = q;
     }
   }
 }
-static void launch_pack(const FoAgentsRaw& raw, float m_ego, const PackProblem& one, const PackProblem* many, int P,
-                        int max_cells, unsigned char* arena, cudaStream_t st) {
+static void launch_pack(const FoAgentsRaw& raw, const PackProblem& one, const PackProblem* many, int P, int max_cells,
+                        unsigned char* arena, cudaStream_t st) {
   fo_agents_order_kernel<<<P, 256, 0, st>>>(raw.kind, one, many, arena);
   const dim3 grid((max_cells + 255) / 256, P < 65535 ? P : 65535);
-  fo_agents_pack_kernel<<<grid, 256, 0, st>>>(raw, m_ego, one, many, P, arena);
+  fo_agents_pack_kernel<<<grid, 256, 0, st>>>(raw, one, many, P, arena);
+}
+
+// The ego vehicle in kernel units; the single-problem path and every batch descriptor take it from here, so a problem
+// of a batch sees the same float values as alone.
+static void fill_ego_const(const FoVehicle& v, EgoConst& e) {
+  e.hEx = 0.5f * v.length; e.hEy = 0.5f * v.width;
+  e.wb = v.wb_rear_axle; e.a_max = v.a_max;
+  e.L3 = v.length / 3.0f; e.L6 = v.length / 6.0f; e.W2 = v.width / 2.0f;
 }
 
 // Staging of the per-problem descriptors of the batch entry points, per calling thread and device: a ring of slots, each
@@ -234,8 +244,8 @@ extern "C" int fo_agents_pack(const FoAgentsRaw* raw, const FoVehicle* vehicle, 
     fo::set_error("fo_agents_pack: NULL array in FoAgentsRaw");
     return FO_ERR_INVALID_ARG;
   }
-  const fo::PackProblem one{0, A, Tp, 0, 0};
-  fo::launch_pack(*raw, vehicle->mass, one, nullptr, 1, fo::agent_pad(A) * Tp, (unsigned char*)table_dev, (cudaStream_t)stream);
+  const fo::PackProblem one{0, A, Tp, vehicle->mass, 0};
+  fo::launch_pack(*raw, one, nullptr, 1, fo::agent_pad(A) * Tp, (unsigned char*)table_dev, (cudaStream_t)stream);
   fo::count_launch(2);
   FO_CUDA_TRY(cudaGetLastError());
   return FO_OK;
@@ -260,10 +270,10 @@ extern "C" size_t fo_agent_batch_layout(int32_t n_problems, const int32_t* n_age
   return off;
 }
 
-extern "C" int fo_agents_pack_batch(const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
-                                    const FoVehicle* vehicle, void* arena_dev, size_t arena_bytes, void* stream) {
-  const char* fn = "fo_agents_pack_batch";
-  if (!raw || !vehicle || n_problems < 0 || (n_problems > 0 && !problems)) { fo::set_error("%s: bad argument", fn); return FO_ERR_INVALID_ARG; }
+// Problem p is packed with the mass of vehicles[per_problem ? p : 0].
+static int pack_batch_impl(const char* fn, const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
+                           const FoVehicle* vehicles, bool per_problem, void* arena_dev, size_t arena_bytes, void* stream) {
+  if (!raw || !vehicles || n_problems < 0 || (n_problems > 0 && !problems)) { fo::set_error("%s: bad argument", fn); return FO_ERR_INVALID_ARG; }
   if (raw->n_agents < 0 || raw->t_stride < 0) { fo::set_error("%s: negative size", fn); return FO_ERR_INVALID_ARG; }
   if (reinterpret_cast<uintptr_t>(arena_dev) & 15) { fo::set_error("%s: arena must be 16-byte aligned", fn); return FO_ERR_INVALID_ARG; }
   long long total = 0;
@@ -299,17 +309,33 @@ extern "C" int fo_agents_pack_batch(const FoAgentsRaw* raw, int32_t n_problems, 
   int a_begin = 0, j = 0;
   for (int p = 0; p < n_problems; ++p) {
     const FoBatchProblem& q = problems[p];
-    if (q.n_agents > 0) pp[j++] = fo::PackProblem{a_begin, q.n_agents, q.t_stride, 0, (long long)q.table_offset};
+    if (q.n_agents > 0)
+      pp[j++] = fo::PackProblem{a_begin, q.n_agents, q.t_stride, vehicles[per_problem ? p : 0].mass, (long long)q.table_offset};
     a_begin += q.n_agents;
   }
   rc = fo::stage_upload(slot, bytes, st);
   if (rc != FO_OK) return rc;
-  fo::launch_pack(*raw, vehicle->mass, fo::PackProblem{}, reinterpret_cast<const fo::PackProblem*>(slot->dev), n_packed,
-                  max_cells, (unsigned char*)arena_dev, st);
+  fo::launch_pack(*raw, fo::PackProblem{}, reinterpret_cast<const fo::PackProblem*>(slot->dev), n_packed, max_cells,
+                  (unsigned char*)arena_dev, st);
   fo::count_launch(2);
   FO_CUDA_TRY(cudaGetLastError());
   FO_CUDA_TRY(cudaEventRecord(slot->done, st));
   return FO_OK;
+}
+
+extern "C" int fo_agents_pack_batch(const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
+                                    const FoVehicle* vehicle, void* arena_dev, size_t arena_bytes, void* stream) {
+  return pack_batch_impl("fo_agents_pack_batch", raw, n_problems, problems, vehicle, false, arena_dev, arena_bytes, stream);
+}
+
+extern "C" int fo_agents_pack_batch_vehicles(const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
+                                             const FoVehicle* vehicles_host, void* arena_dev, size_t arena_bytes,
+                                             void* stream) {
+  const char* fn = "fo_agents_pack_batch_vehicles";
+  if (n_problems > 0 && !vehicles_host) { fo::set_error("%s: vehicles_host must not be NULL", fn); return FO_ERR_INVALID_ARG; }
+  static const FoVehicle none{};                 // no problems: nothing is read
+  return pack_batch_impl(fn, raw, n_problems, problems, vehicles_host ? vehicles_host : &none, true, arena_dev,
+                         arena_bytes, stream);
 }
 
 // SM count per device (a process may drive several GPUs, one per planner thread): cached per ordinal, racing
@@ -331,9 +357,7 @@ static int num_sms_of_current_device(int* out) {
 static void fill_kargs(const FoMetricArgs* a, fo::MetricKArgs& k) {
   k.ego = a->ego; k.N = a->n_traj; k.T = a->n_states; k.A = a->n_agents; k.Tp = a->t_stride;
   k.tab = fo::agent_table_view(a->agent_table, a->n_agents, a->t_stride);
-  k.hEx = 0.5f * a->vehicle.length; k.hEy = 0.5f * a->vehicle.width;
-  k.wb = a->vehicle.wb_rear_axle; k.a_max = a->vehicle.a_max;
-  k.L3 = a->vehicle.length / 3.0f; k.L6 = a->vehicle.length / 6.0f; k.W2 = a->vehicle.width / 2.0f;
+  fo::fill_ego_const(a->vehicle, k.veh);
   k.hc = a->harm; k.dt = (float)a->dt; k.dtd = a->dt;
   k.mmask = a->metric_mask; k.tmask = a->threshold_mask;
   k.thr_harm = a->thr_harm; k.thr_risk = a->thr_risk; k.thr_be = a->thr_be; k.thr_cp = a->thr_cp;
@@ -459,8 +483,8 @@ static int check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, 
   return FO_OK;
 }
 
-extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
-  const char* fn = "fo_metric_batch";
+// vehicles: problem p's ego vehicle is vehicles[p]; NULL = common.vehicle for every problem
+static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const FoVehicle* vehicles, void* stream) {
   int n_run = 0, a_min = 0;
   {
     const int rc = check_batch(fn, b, false, &n_run, &a_min);
@@ -501,6 +525,7 @@ extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
     const fo::AgentTableView v = fo::agent_table_view(arena + (q.n_agents > 0 ? q.table_offset : 0), q.n_agents, Tp);
     d.t0 = v.t0; d.tv = v.tv; d.aw = v.aw; d.avw = v.avw; d.s0 = v.s0; d.s1 = v.s1; d.s2 = v.s2; d.prm = v.prm;
     d.first = n; d.row0 = (int)q.traj_begin; d.A = q.n_agents; d.Tp = Tp; d.Ap = v.Ap; d.lg = lg;
+    fo::fill_ego_const(vehicles ? vehicles[p] : c.vehicle, d.veh);
     first[i] = n;
     n += q.n_traj;
     ++i;
@@ -529,10 +554,20 @@ extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
   return FO_OK;
 }
 
-extern "C" int fo_metric_batch_detail(const FoMetricBatchArgs* b, void* stream) {
+extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
+  return metric_batch_impl("fo_metric_batch", b, nullptr, stream);
+}
+
+extern "C" int fo_metric_batch_vehicles(const FoMetricBatchArgs* b, const FoVehicle* vehicles_host, void* stream) {
+  const char* fn = "fo_metric_batch_vehicles";
+  if (b && b->n_problems > 0 && !vehicles_host) { fo::set_error("%s: vehicles_host must not be NULL", fn); return FO_ERR_INVALID_ARG; }
+  return metric_batch_impl(fn, b, vehicles_host, stream);
+}
+
+static int metric_batch_detail_impl(const char* fn, const FoMetricBatchArgs* b, const FoVehicle* vehicles, void* stream) {
   int n_run = 0, a_min = 0;
   {
-    const int rc = check_batch("fo_metric_batch_detail", b, true, &n_run, &a_min);
+    const int rc = check_batch(fn, b, true, &n_run, &a_min);
     if (rc != FO_OK || b->common.n_traj == 0) return rc;
   }
   const FoMetricArgs& c = b->common;
@@ -560,6 +595,7 @@ extern "C" int fo_metric_batch_detail(const FoMetricBatchArgs* b, void* stream) 
     d.pair = c.pair ? c.pair + (size_t)pairs * FO_PAIR_K : nullptr;
     d.step = c.step ? c.step + (size_t)pairs * Tm1 * FO_STEP_K : nullptr;
     d.row0 = (int)q.traj_begin; d.A = q.n_agents; d.Tp = Tp; d.Ap = v.Ap;
+    fo::fill_ego_const(vehicles ? vehicles[p] : c.vehicle, d.veh);
     first[i++] = d.row0;
     pairs += (long long)q.n_traj * q.n_agents;
   }
@@ -579,4 +615,14 @@ extern "C" int fo_metric_batch_detail(const FoMetricBatchArgs* b, void* stream) 
   if (rc != FO_OK) return rc;
   FO_CUDA_TRY(cudaEventRecord(slot->done, st));
   return FO_OK;
+}
+
+extern "C" int fo_metric_batch_detail(const FoMetricBatchArgs* b, void* stream) {
+  return metric_batch_detail_impl("fo_metric_batch_detail", b, nullptr, stream);
+}
+
+extern "C" int fo_metric_batch_detail_vehicles(const FoMetricBatchArgs* b, const FoVehicle* vehicles_host, void* stream) {
+  const char* fn = "fo_metric_batch_detail_vehicles";
+  if (b && b->n_problems > 0 && !vehicles_host) { fo::set_error("%s: vehicles_host must not be NULL", fn); return FO_ERR_INVALID_ARG; }
+  return metric_batch_detail_impl(fn, b, vehicles_host, stream);
 }

@@ -102,8 +102,8 @@ __device__ __forceinline__ void dt_harm(const FoHarmCoeffs& hc, int model, const
 // np.round(d, 3) next to a x.xxx5 boundary (dce.py:79): queued candidates are re-rounded from a float64 evaluation, up to
 // 32 at a time and out of line.  A candidate matters only while its float32 rounding is within two units of its pair's
 // running minimum (the float32 value is off by at most one unit); by the time the queue is drained most are not.
-__device__ __forceinline__ void dt_drain_ties_body(const MetricKArgs& k, const float4* t0, const AgentParams* prm,
-                                                   const float* tpsi, int Ap, const float4* egoA, const float2* egoB,
+__device__ __forceinline__ void dt_drain_ties_body(const float4* t0, const AgentParams* prm, const float* tpsi, int Ap,
+                                                   const EgoConst& veh, const float4* egoA, const float2* egoB,
                                                    uint32_t* dkey, const uint2* src, int cnt, int a0, int lane) {
   if (lane < cnt) {
     const uint2 it = src[lane];
@@ -113,7 +113,7 @@ __device__ __forceinline__ void dt_drain_ties_body(const MetricKArgs& k, const f
       const float4 s0 = __ldg(&t0[(size_t)ii * Ap + as]);
       const int4 pa = __ldg(reinterpret_cast<const int4*>(prm + as));
       const float4 EA = egoA[ii];
-      const uint32_t r = obb_round_mm_f64(EA.x, EA.y, egoB[ii].x, k.wb, k.hEx, k.hEy, s0.x, s0.y,
+      const uint32_t r = obb_round_mm_f64(EA.x, EA.y, egoB[ii].x, veh.wb, veh.hEx, veh.hEy, s0.x, s0.y,
                                           __ldg(&tpsi[(size_t)ii * Ap + as]), __int_as_float(pa.z),
                                           __int_as_float(pa.w));
       atomicMin(&dkey[ial], (r << 8) | (uint32_t)ii);
@@ -123,18 +123,21 @@ __device__ __forceinline__ void dt_drain_ties_body(const MetricKArgs& k, const f
 }
 static __device__ __noinline__ void dt_drain_ties(const MetricKArgs& k, const float4* egoA, const float2* egoB,
                                                   uint32_t* dkey, const uint2* src, int cnt, int a0, int lane) {
-  dt_drain_ties_body(k, k.tab.t0, k.tab.prm, k.tab.tpsi, k.tab.Ap, egoA, egoB, dkey, src, cnt, a0, lane);
+  dt_drain_ties_body(k.tab.t0, k.tab.prm, k.tab.tpsi, k.tab.Ap, k.veh, egoA, egoB, dkey, src, cnt, a0, lane);
 }
-// batched kernel: the agent table is the trajectory's problem's, passed in registers
-static __device__ __noinline__ void dt_drain_ties_batch(const MetricKArgs& k, const float4* t0, const AgentParams* prm,
-                                                        const float* tpsi, int Ap, const float4* egoA, const float2* egoB,
-                                                        uint32_t* dkey, const uint2* src, int cnt, int a0, int lane) {
-  dt_drain_ties_body(k, t0, prm, tpsi, Ap, egoA, egoB, dkey, src, cnt, a0, lane);
+// batched kernel: the agent table and the ego box are the trajectory's problem's, passed in registers
+static __device__ __noinline__ void dt_drain_ties_batch(const float4* t0, const AgentParams* prm, const float* tpsi, int Ap,
+                                                        float wb, float hEx, float hEy, const float4* egoA,
+                                                        const float2* egoB, uint32_t* dkey, const uint2* src, int cnt,
+                                                        int a0, int lane) {
+  EgoConst veh;
+  veh.wb = wb; veh.hEx = hEx; veh.hEy = hEy;
+  dt_drain_ties_body(t0, prm, tpsi, Ap, veh, egoA, egoB, dkey, src, cnt, a0, lane);
 }
 
 // MASK != 0: the activated metrics are a compile-time constant (all seven / the default six); 0 = read k.mmask.
-// BATCH: every trajectory takes its agent table, agent count and pair / step blocks from its problem (bv); otherwise
-// from k, whose fields then stay kernel-parameter operands.
+// BATCH: every trajectory takes its agent table, agent count, pair / step blocks and ego vehicle from its problem (bv);
+// otherwise from k, whose fields then stay kernel-parameter operands.
 template <uint32_t MASK, bool BATCH>
 __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailView& bv) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -165,7 +168,7 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
   const bool do_cp = mm & FO_M_CP, do_dce = mm & FO_M_DCE, do_hr = mm & FO_M_HR, do_be = mm & FO_M_BE,
              do_ttc = mm & FO_M_TTC;
   const unsigned lt_mask = (1u << lane) - 1u;
-  const float rE = sqrtf(k.hEx * k.hEx + k.hEy * k.hEy);
+  float rE = sqrtf(k.veh.hEx * k.veh.hEx + k.veh.hEy * k.veh.hEy);   // batched: per trajectory
   bool rows8 = (Tm1 & 1) == 0 && (reinterpret_cast<uintptr_t>(k.step) & 7u) == 0;   // row segments 8-byte aligned
   size_t traj_step = (size_t)k.A * (size_t)Tm1 * FO_STEP_K;
   float* const srow_lane = stage + lane * kDtRow;
@@ -186,6 +189,7 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
         reinterpret_cast<int4*>(sdp)[lane] = __ldg(reinterpret_cast<const int4*>(bv.prob + p) + lane);
       __syncwarp();
       nb = n - sdp->row0;
+      rE = sqrtf(sdp->veh.hEx * sdp->veh.hEx + sdp->veh.hEy * sdp->veh.hEy);
       rows8 = (Tm1 & 1) == 0 && (reinterpret_cast<uintptr_t>(sdp->step) & 7u) == 0;
       traj_step = (size_t)sdp->A * (size_t)Tm1 * FO_STEP_K;
     }
@@ -197,9 +201,10 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
     const int& Ap = BATCH ? sdp->Ap : Apk;
     float* const& pair = BATCH ? sdp->pair : k.pair;
     float* const& step = BATCH ? sdp->step : k.step;
+    const EgoConst& veh = BATCH ? sdp->veh : k.veh;
     const auto drain_ties = [&](const uint2* src, int cnt, int a0) {
       if constexpr (BATCH)
-        dt_drain_ties_batch(k, tab.t0, tab.prm, tab.tpsi, Ap, egoA, egoB, dkey, src, cnt, a0, lane);
+        dt_drain_ties_batch(tab.t0, tab.prm, tab.tpsi, Ap, veh.wb, veh.hEx, veh.hEy, egoA, egoB, dkey, src, cnt, a0, lane);
       else
         dt_drain_ties(k, egoA, egoB, dkey, src, cnt, a0, lane);
     };
@@ -252,7 +257,7 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
           if (i < nA) {
             const float4 s0 = __ldg(t0p);
             const float4 EA = egoA[i];
-            const float dx = fmaf(-k.wb, EA.z, s0.x - EA.x), dy = fmaf(-k.wb, EA.w, s0.y - EA.y);
+            const float dx = fmaf(-veh.wb, EA.z, s0.x - EA.x), dy = fmaf(-veh.wb, EA.w, s0.y - EA.y);
             const float c2 = fmaf(dx, dx, dy * dy);
             if (c2 < U2) { U2 = c2; i_star = i; }
           }
@@ -288,9 +293,9 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
           const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + as));
           const float4 EA = egoA[ii];
           const float c = fmaf(EA.z, s0.z, EA.w * s0.w), s = fmaf(s0.w, EA.z, -s0.z * EA.w);
-          const float dx = (s0.x - EA.x) - k.wb * EA.z, dy = (s0.y - EA.y) - k.wb * EA.w;
+          const float dx = (s0.x - EA.x) - veh.wb * EA.z, dy = (s0.y - EA.y) - veh.wb * EA.w;
           const float rx = fmaf(dx, EA.z, dy * EA.w), ry = fmaf(dy, EA.z, -dx * EA.w);
-          const float d = sqrtf(obb_d2(rx, ry, c, s, k.hEx, k.hEy, __int_as_float(pa.z), __int_as_float(pa.w)));
+          const float d = sqrtf(obb_d2(rx, ry, c, s, veh.hEx, veh.hEy, __int_as_float(pa.z), __int_as_float(pa.w)));
           uint32_t r = (uint32_t)__float2int_rn(fminf(d, 8000.0f) * 1000.0f);   // np.round(d, 3), dce.py:79
           // rounding ties: a candidate for the pair's minimum next to a x.xxx5 boundary is queued for a float64
           // re-rounding (the float32 value is off by at most one unit there); until then r + 1 bounds it from above
@@ -324,8 +329,8 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
           const float4 s1i = __ldg(&tab.s1[idx]);
           const float2 s2i = __ldg(&tab.s2[idx]);
           const float4 Ei = egoA[ii];
-          const float cp = cp_gauss_boxes<false>(s1i.z - Ei.x, s1i.w - Ei.y, Q.hlb * s0i.z, Q.hlb * s0i.w, k.L3 * Ei.z,
-                                          k.L3 * Ei.w, s2i, k.L6, k.W2);
+          const float cp = cp_gauss_boxes<false>(s1i.z - Ei.x, s1i.w - Ei.y, Q.hlb * s0i.z, Q.hlb * s0i.w, veh.L3 * Ei.z,
+                                          veh.L3 * Ei.w, s2i, veh.L6, veh.W2);
           // where the step loop put state t: still in the staging tile, or already in HBM (L2)
           const bool staged = t >= c0;
           float* const srow = stage + ial * kDtRow + 3 * (t - c0);
@@ -410,7 +415,7 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
         const float dxr = s0.x - EA.x, dyr = s0.y - EA.y;
         const float c = fmaf(EA.z, s0.z, EA.w * s0.w);                                // cos(yaw - theta)
         if (do_dce) {
-          const float dx = fmaf(-k.wb, EA.z, dxr), dy = fmaf(-k.wb, EA.w, dyr);       // centre to centre
+          const float dx = fmaf(-veh.wb, EA.z, dxr), dy = fmaf(-veh.wb, EA.w, dyr);   // centre to centre
           const bool need = liveA & (fmaf(dx, dx, dy * dy) < lim2) & (i != i_star);
           const unsigned b = __ballot_sync(kFull, need);
           if (b || last || qn >= 32) {
@@ -501,10 +506,12 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
           const int ns_s = __shfl_sync(kFull, P.n_states, src);
           const float hl_s = __shfl_sync(kFull, P.hl, src), hw_s = __shfl_sync(kFull, P.hw, src);
           BeConst bk = bek;
-          if constexpr (BATCH) { bk.s0 = tab.s0; bk.Tp = Tp; }   // BE bisections read the problem's agent-major states
+          if constexpr (BATCH) {                         // the problem's agent-major states and ego box
+            bk.s0 = tab.s0; bk.Tp = Tp; bk.wb = veh.wb; bk.hEx = veh.hEx; bk.hEy = veh.hEy;
+          }
           const float r = be_bisect<false>(bk, bev, a0 + src, ns_s, hl_s, hw_s, be_lo0, lane, -1.0f).x;
           if (r != r) flags |= FO_F_BE_RANGE;            // NaN: the re-timed path overruns the planned one
-          if (lane == src) { rcd = r; btn = __fdividef(r, k.a_max); }
+          if (lane == src) { rcd = r; btn = __fdividef(r, veh.a_max); }
         }
         acc_rcd = fmaxf(acc_rcd, rcd);     // fmaxf ignores NaN
         acc_btn = fmaxf(acc_btn, btn);
@@ -561,7 +568,7 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
 }
 
 // A batch of independent problems (fo_metric_batch_detail): k.N = all rows of the batch, k.tab / k.A / k.Tp / k.pair /
-// k.step are unused -- every trajectory takes them from its problem.
+// k.step / k.veh are unused -- every trajectory takes them from its problem.
 template <uint32_t MASK>
 __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB)
 fo_metric_batch_detail_kernel(const __grid_constant__ MetricKArgs k, const __grid_constant__ DetailView bv) {

@@ -11,13 +11,19 @@ namespace fo {
 constexpr int kWarpsPerCta = 8;
 constexpr unsigned kFull = 0xffffffffu;
 
+// Constants of the ego vehicle in the units the kernels use (fill_ego_const in fo_metric.cu).  A batch of independent
+// problems carries one per problem (BatchProb / DetailProb::veh).
+struct EgoConst {
+  float hEx, hEy;      // ego half extents
+  float wb, a_max;
+  float L3, L6, W2;    // L/3, L/6, W/2 (CP boxes)
+};
+
 struct MetricKArgs {
   const float* ego;
   int N, T, A, Tp;
   AgentTableView tab;
-  float hEx, hEy;      // ego half extents
-  float wb, a_max;
-  float L3, L6, W2;    // L/3, L/6, W/2 (CP boxes)
+  EgoConst veh;
   FoHarmCoeffs hc;
   float dt;
   double dtd;
@@ -290,7 +296,7 @@ struct BeConst {
   float dt, wb, hEx, hEy;
 };
 __device__ __forceinline__ BeConst be_const(const MetricKArgs& k) {
-  return BeConst{k.tab.s0, k.T, k.Tp, k.dt, k.wb, k.hEx, k.hEy};
+  return BeConst{k.tab.s0, k.T, k.Tp, k.dt, k.veh.wb, k.veh.hEx, k.veh.hEy};
 }
 
 template <bool SEG>
@@ -461,7 +467,7 @@ unsigned int* claim_slot(cudaStream_t st);
 int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st);
 int launch_metric_sweep(const MetricKArgs& k, int num_sms, cudaStream_t st);
 // Batch of independent problems (fo_metric_batch): the trajectories of one launch belong to problems with their own
-// agent tables.  A launch sees the problems of one shape class; `first` numbers their trajectories consecutively.  The
+// agent tables and ego vehicles.  A launch sees the problems of one shape class; `first` numbers their trajectories consecutively.  The
 // table pointers are resolved on the host (agent_table_view of the problem's table in the arena): the kernel loads them
 // and does no address arithmetic of its own per trajectory.
 struct __align__(16) BatchProb {
@@ -477,8 +483,9 @@ struct __align__(16) BatchProb {
   int row0;             // its row in ego / valid / summary / flags
   int A, Tp, Ap;        // agents, table stride, agents padded to 32
   int lg;               // log2 of the agents held by one warp (team shape)
+  EgoConst veh;         // the problem's ego vehicle
 };
-static_assert(sizeof(BatchProb) == 96, "six 16-byte loads");
+static_assert(sizeof(BatchProb) == 128, "eight 16-byte loads");
 struct BatchView {
   const int* first;     // [P] BatchProb::first, strictly increasing (problems without trajectories are left out)
   const BatchProb* prob;
@@ -509,8 +516,9 @@ struct __align__(16) DetailProb {
   float* step;          // [N_p, A_p, T-1, FO_STEP_K]
   int row0;             // the problem's first row in ego / valid / summary / flags
   int A, Tp, Ap;        // agents, table stride, agents padded to 32
+  EgoConst veh;         // the problem's ego vehicle
 };
-static_assert(sizeof(DetailProb) == 96, "six 16-byte loads");
+static_assert(sizeof(DetailProb) == 128, "eight 16-byte loads");
 struct DetailView {
   const int* first;     // [P] DetailProb::row0, strictly increasing (problems without trajectories are left out)
   const DetailProb* prob;

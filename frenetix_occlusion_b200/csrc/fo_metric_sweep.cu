@@ -164,7 +164,10 @@ __device__ __forceinline__ void sw_harm_logits(const MetricKArgs& k, int model, 
 // collision (r <= 1) or lie below the minimum found since (r <= rmin); when no lane holds such an entry the float64
 // code is not entered at all -- in a dense sweep the minimum is 0 after the first collision and the 6 kB stay out of the
 // instruction cache.
-__device__ __forceinline__ uint32_t drain_ties_body(const MetricKArgs& k, const AgentTableView& tab, const int& Tp,
+// K: anything with an EgoConst member veh.  The summary kernel passes its MetricKArgs, whose known 8-byte alignment
+// lets adjacent fields be read with one load.
+template <class K>
+__device__ __forceinline__ uint32_t drain_ties_body(const K& kv, const AgentTableView& tab, const int& Tp,
                                                     const float4* egoA, const float2* egoB, uint32_t* colfirst,
                                                     const uint32_t* src, int cnt, int a0, int lane, uint32_t rmin) {
   uint32_t r = 0xffffffu;
@@ -182,7 +185,7 @@ __device__ __forceinline__ uint32_t drain_ties_body(const MetricKArgs& k, const 
     const float4 s0 = __ldg(&tab.t0[(size_t)ii * tab.Ap + a]);
     const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + a));
     const float4 EA = egoA[ii];
-    r = obb_round_mm_f64(EA.x, EA.y, egoB[ii].x, k.wb, k.hEx, k.hEy, s0.x, s0.y,
+    r = obb_round_mm_f64(EA.x, EA.y, egoB[ii].x, kv.veh.wb, kv.veh.hEx, kv.veh.hEy, s0.x, s0.y,
                          __ldg(&tab.s1[(size_t)a * Tp + ii]).x, __int_as_float(pa.z), __int_as_float(pa.w));
     if (r == 0u) atomicMin(&colfirst[ial], (uint32_t)ii);
   }
@@ -193,14 +196,16 @@ static __device__ __noinline__ uint32_t sw_drain_ties(const MetricKArgs& k, cons
                                                       uint32_t rmin) {
   return drain_ties_body(k, k.tab, k.Tp, egoA, egoB, colfirst, src, cnt, a0, lane, rmin);
 }
-// batched kernel: the agent table is the trajectory's problem's, passed in registers
-static __device__ __noinline__ uint32_t sw_drain_ties_batch(const MetricKArgs& k, const float4* t0, const AgentParams* prm,
-                                                            const float4* s1, int Ap, int Tp, const float4* egoA,
-                                                            const float2* egoB, uint32_t* colfirst, const uint32_t* src,
-                                                            int cnt, int a0, int lane, uint32_t rmin) {
+// batched kernel: the agent table and the ego box are the trajectory's problem's, passed in registers
+static __device__ __noinline__ uint32_t sw_drain_ties_batch(const float4* t0, const AgentParams* prm, const float4* s1,
+                                                            int Ap, int Tp, float wb, float hEx, float hEy,
+                                                            const float4* egoA, const float2* egoB, uint32_t* colfirst,
+                                                            const uint32_t* src, int cnt, int a0, int lane, uint32_t rmin) {
   AgentTableView tab;
   tab.t0 = t0; tab.prm = prm; tab.s1 = s1; tab.Ap = Ap;
-  return drain_ties_body(k, tab, Tp, egoA, egoB, colfirst, src, cnt, a0, lane, rmin);
+  struct { EgoConst veh; } kv;
+  kv.veh.wb = wb; kv.veh.hEx = hEx; kv.veh.hEy = hEy;
+  return drain_ties_body(kv, tab, Tp, egoA, egoB, colfirst, src, cnt, a0, lane, rmin);
 }
 
 // problem of trajectory n: the last p with first[p] <= n
@@ -213,7 +218,8 @@ struct SweepShape {
 // ---------------------------------------------------------------------------------------------
 // UNI: one warp per trajectory and 32 agents per warp pass (the throughput shape): window filter + lane = (agent, window)
 // items, no pooled leftovers (see the header comment).
-// BATCH: every trajectory takes its agent table, agent count and lane grouping from its problem (bv); otherwise from k.
+// BATCH: every trajectory takes its agent table, agent count, lane grouping and ego vehicle from its problem (bv);
+// otherwise from k.
 // tid / block_dim are read in the __global__ function, where the compiler knows their range from the launch bounds.
 template <uint32_t MASK, bool STATS, bool UNI, bool TIES, bool BATCH>
 __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShape shape, const BatchView& bv,
@@ -232,7 +238,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
   const bool do_cp = mm & FO_M_CP, do_dce = mm & FO_M_DCE, do_hr = mm & FO_M_HR, do_be = mm & FO_M_BE,
              do_ttc = mm & FO_M_TTC;
   const unsigned lt_mask = (1u << lane) - 1u;
-  const float rE = sqrtf(k.hEx * k.hEx + k.hEy * k.hEy);   // ego circumradius
+  float rE = sqrtf(k.veh.hEx * k.veh.hEx + k.veh.hEy * k.veh.hEy);   // ego circumradius (batched: per trajectory)
   const float cmax = fmaxf(0.0f, fmaxf(k.hc.rs_side, k.hc.rs_rear));
   int Ap = k.tab.Ap;
   const auto soff = [&](const void* q) { return (uint32_t)(reinterpret_cast<const unsigned char*>(q) - smem_raw); };
@@ -253,6 +259,9 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
   // looks up the problem of the claimed trajectory in the same place.
   __shared__ int s_claim[BATCH ? 2 : 1];               // next trajectory (and, batched, its problem)
   int& s_next = s_claim[0];
+  // batched: the ego vehicle of the current trajectory's problem, read where used (held in registers it would spill)
+  __shared__ EgoConst s_veh;
+  const EgoConst& veh = BATCH ? s_veh : k.veh;
   int p = BATCH ? batch_find(bv, blockIdx.x) : 0;
   for (int n = blockIdx.x; n < k.N;) {
     AgentTableView btab;
@@ -278,7 +287,8 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
     const int& Tp = BATCH ? bTp : k.Tp;
     const auto drain_ties = [&](const uint32_t* src, int cnt, int a0, int lane, uint32_t rmin) {
       if constexpr (BATCH)
-        return sw_drain_ties_batch(k, tab.t0, tab.prm, tab.s1, Ap, Tp, w.egoA, w.egoB, w.colfirst, src, cnt, a0, lane, rmin);
+        return sw_drain_ties_batch(tab.t0, tab.prm, tab.s1, Ap, Tp, veh.wb, veh.hEx, veh.hEy, w.egoA, w.egoB, w.colfirst,
+                                   src, cnt, a0, lane, rmin);
       else
         return sw_drain_ties(k, w.egoA, w.egoB, w.colfirst, src, cnt, a0, lane, rmin);
     };
@@ -286,11 +296,16 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
     const float* eg = k.ego + (size_t)row * T * 5;
     __syncthreads();                                   // previous trajectory fully consumed
     if (tid < 8) w.scal[tid] = 0u;
+    if constexpr (BATCH) {
+      if (tid < (int)(sizeof(EgoConst) / 4))
+        reinterpret_cast<float*>(&s_veh)[tid] = __ldg(reinterpret_cast<const float*>(&bv.prob[p].veh) + tid);
+    }
     if (tid == 0) {
       s_next = k.claim ? (int)(gridDim.x + atomicAdd(k.claim, 1u)) : n + (int)gridDim.x;
       if constexpr (BATCH) s_claim[1] = s_next < k.N ? batch_find(bv, s_next) : 0;
     }
     __syncthreads();
+    if constexpr (BATCH) rE = sqrtf(veh.hEx * veh.hEx + veh.hEy * veh.hEy);
     {
       float amin = 0.0f;
       for (int i = tid; i < T; i += nthr) {
@@ -311,7 +326,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
 #pragma unroll 1
         for (int i = tid * kWinSteps; i < min(T, (tid + 1) * kWinSteps); ++i) {
           const float4 EA = w.egoA[i];
-          const float cx = fmaf(k.wb, EA.z, EA.x), cy = fmaf(k.wb, EA.w, EA.y);     // box centre (dce.py:57-60)
+          const float cx = fmaf(veh.wb, EA.z, EA.x), cy = fmaf(veh.wb, EA.w, EA.y); // box centre (dce.py:57-60)
           xl = fminf(xl, fminf(EA.x, cx)); xh = fmaxf(xh, fmaxf(EA.x, cx));
           yl = fminf(yl, fminf(EA.y, cy)); yh = fmaxf(yh, fmaxf(EA.y, cy));
           vm = fmaxf(vm, fabsf(w.egoB[i].y));
@@ -376,9 +391,9 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           const float dxr = s0.x - EA.x, dyr = s0.y - EA.y;
           if (item & 0x40000000u) {            // exact oriented-box distance, np.round(d, 3) (dce.py:75-79)
             const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + a));
-            const float dx = dxr - k.wb * EA.z, dy = dyr - k.wb * EA.w;
+            const float dx = dxr - veh.wb * EA.z, dy = dyr - veh.wb * EA.w;
             const float rx = fmaf(dx, EA.z, dy * EA.w), ry = fmaf(dy, EA.z, -dx * EA.w);
-            const float d = sqrtf(obb_d2(rx, ry, c, s, k.hEx, k.hEy, __int_as_float(pa.z), __int_as_float(pa.w)));
+            const float d = sqrtf(obb_d2(rx, ry, c, s, veh.hEx, veh.hEy, __int_as_float(pa.z), __int_as_float(pa.w)));
             r = (uint32_t)__float2int_rn(fminf(d, 8000.0f) * 1000.0f);
             // np.round(d, 3) next to a x.xxx5 boundary: a candidate for the minimum is queued for a float64
             // re-rounding (rmin only falls, so "r <= rmin + 2" is a superset of the candidates of the final minimum);
@@ -432,8 +447,8 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           const float4 s1i = __ldg(&tab.s1[idx]);
           const float2 s2i = __ldg(&tab.s2[idx]);
           const float4 Ei = w.egoA[ii];
-          const float cp = cp_gauss_boxes(s1i.z - Ei.x, s1i.w - Ei.y, P.hlb * s0i.z, P.hlb * s0i.w, k.L3 * Ei.z,
-                                          k.L3 * Ei.w, s2i, k.L6, k.W2);
+          const float cp = cp_gauss_boxes(s1i.z - Ei.x, s1i.w - Ei.y, P.hlb * s0i.z, P.hlb * s0i.w, veh.L3 * Ei.z,
+                                          veh.L3 * Ei.w, s2i, veh.L6, veh.W2);
           acc_cp = fmaxf(acc_cp, cp);
           if (do_hr) {                       // risk[t] = harm[t] * cp[t], cp[t] = CP of step t+1 (hr.py:78-79)
             const float4 s0t = __ldg(&tab.s0[idx - 1]);
@@ -498,7 +513,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           const float dxr = s0.x - EA.x, dyr = s0.y - EA.y;
           bool need_obb = false, need_lr = false, ingate = false;
           if (do_dce) {
-            const float dx = fmaf(-k.wb, EA.z, dxr), dy = fmaf(-k.wb, EA.w, dyr);   // centre to centre
+            const float dx = fmaf(-veh.wb, EA.z, dxr), dy = fmaf(-veh.wb, EA.w, dyr);   // centre to centre
             need_obb = live & (fmaf(dx, dx, dy * dy) < lim2);
           }
           if (do_hr) {
@@ -696,12 +711,14 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
 #else
             const float be_floor = rcd_all;
 #endif
-            const float2 be = be_bisect<true>(bek, bev, a, pa.x, __int_as_float(pa.z), __int_as_float(pa.w), be_lo0, lane,
+            BeConst bk = bek;
+            if constexpr (BATCH) { bk.wb = veh.wb; bk.hEx = veh.hEx; bk.hEy = veh.hEy; }
+            const float2 be = be_bisect<true>(bk, bev, a, pa.x, __int_as_float(pa.z), __int_as_float(pa.w), be_lo0, lane,
                                               be_floor);
             const float rcd = be.x;
             if (rcd != rcd) flags |= FO_F_BE_RANGE;      // NaN: the re-timed path overruns the planned one
             rcd_all = fmaxf(rcd_all, rcd);
-            btn_all = fmaxf(btn_all, rcd / k.a_max);
+            btn_all = fmaxf(btn_all, rcd / veh.a_max);
             if (STATS && lane == 0) { st_be += 1; st_probe += (unsigned)__float_as_int(be.y); }
           }
         }
@@ -793,7 +810,7 @@ fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
 }
 
 // One shape class of a batch of independent problems (fo_metric_batch): k.N is the class's trajectory count, k.tab / k.A
-// / k.Tp and shape.lg_agents are unused -- every trajectory takes them from its problem.
+// / k.Tp / k.veh and shape.lg_agents are unused -- every trajectory takes them from its problem.
 template <uint32_t MASK, bool UNI, bool TIES>
 __global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
 fo_metric_batch_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape, const __grid_constant__ BatchView bv) {

@@ -31,6 +31,14 @@ def harm_from_reference_json(coeffs: dict) -> dict:
             "ia_const": ia["const"], "ia_speed": ia["speed"], "ped_const": ped["const"], "ped_speed": ped["speed"]}
 
 
+def vehicle_struct(vehicle_params) -> L.FoVehicle:
+    """An ego vehicle description (dict or object with attributes length, width, mass, wb_rear_axle, a_max) as the
+    C ABI's ``FoVehicle``."""
+    g = (lambda k: float(vehicle_params[k])) if isinstance(vehicle_params, dict) else \
+        (lambda k: float(getattr(vehicle_params, k)))
+    return L.FoVehicle(g("length"), g("width"), g("mass"), g("wb_rear_axle"), g("a_max"))
+
+
 def check_required_metrics(metric_names: Sequence[str]) -> list:
     """Dependency ordering of the activated metrics (reference metrics/metric.py:125-147)."""
     m = list(metric_names)
@@ -176,9 +184,7 @@ class MetricEngine:
         if not torch.cuda.is_available():
             raise RuntimeError("frenetix_occlusion_b200 needs a CUDA device (no CPU fallback)")
         self.device = torch.device(device)
-        g = (lambda k: float(vehicle_params[k])) if isinstance(vehicle_params, dict) else \
-            (lambda k: float(getattr(vehicle_params, k)))
-        self.vehicle = L.FoVehicle(g("length"), g("width"), g("mass"), g("wb_rear_axle"), g("a_max"))
+        self.vehicle = vehicle_struct(vehicle_params)
         self.dt = float(dt)
         self.order = check_required_metrics(activated_metrics)
         if "be" in self.order and "ttc" not in self.order:
@@ -370,11 +376,19 @@ class MetricEngine:
         return g, out
 
     # ---- batches of independent problems ------------------------------------------------------------------------
-    def set_agent_batch(self, agent_sets: Sequence[AgentSet], origins=None):
+    def set_agent_batch(self, agent_sets: Sequence[AgentSet], origins=None, vehicles=None):
         """Upload + pack the phantom predictions of P independent problems (``fo_agents_pack_batch``): one float64
         origin shift per problem, one host-to-device copy of all of them, one pack call.  ``origins``: [P, 2] or None
-        (no shift).  Problem p's table equals what ``set_agents(agent_sets[p], origins[p])`` packs."""
+        (no shift).  ``vehicles``: P ego vehicle descriptions (each a dict or an object with attributes, as the
+        constructor takes them), or None for the engine's own vehicle in every problem; ``assess_batch`` assesses
+        problem p with vehicles[p].  Problem p's table equals what ``set_agents(agent_sets[p], origins[p])`` packs in an
+        engine built with vehicles[p]."""
         P = len(agent_sets)
+        veh = None
+        if vehicles is not None:
+            if len(vehicles) != P:
+                raise ValueError(f"{len(vehicles)} vehicles for {P} problems")
+            veh = (L.FoVehicle * max(P, 1))(*[vehicle_struct(v) for v in vehicles])
         org = np.zeros((P, 2)) if origins is None else np.asarray(origins, dtype=np.float64).reshape(P, 2)
         n_agents = np.array([a.n_agents if a.t_stride > 0 else 0 for a in agent_sets], dtype=np.int32)
         t_stride = np.array([a.t_stride if n else 0 for a, n in zip(agent_sets, n_agents)], dtype=np.int32)
@@ -388,7 +402,7 @@ class MetricEngine:
         A, S = int(n_agents.sum()), int(t_stride.max(initial=0))
         dev = self.device
         self._batch = {"problems": problems, "P": P, "origins": org, "agents": list(agent_sets), "arena": None,
-                       "arena_bytes": arena_bytes, "n_agents": n_agents}
+                       "arena_bytes": arena_bytes, "n_agents": n_agents, "vehicles": veh}
         if A == 0:
             return
         # one host buffer: 6 float rows [A, S] (x, y shifted per problem), 4 float columns [A], 2 int32 columns [A]
@@ -419,9 +433,13 @@ class MetricEngine:
             raw.length, raw.width, raw.buf_length, raw.buf_width = [base + f4 * i * A for i in range(4)]
             raw.n_states, raw.kind = base + f4 * 4 * A, base + f4 * 5 * A
             arena = torch.empty(max(arena_bytes, 16), dtype=torch.uint8, device=dev)
-            L.check(L.lib.fo_agents_pack_batch(C.byref(raw), P, problems, C.byref(self.vehicle),
-                                               C.c_void_p(arena.data_ptr()), arena_bytes, self._stream()),
-                    "fo_agents_pack_batch")
+            if veh is None:
+                L.check(L.lib.fo_agents_pack_batch(C.byref(raw), P, problems, C.byref(self.vehicle),
+                                                   C.c_void_p(arena.data_ptr()), arena_bytes, self._stream()),
+                        "fo_agents_pack_batch")
+            else:
+                L.check(L.lib.fo_agents_pack_batch_vehicles(C.byref(raw), P, problems, veh, C.c_void_p(arena.data_ptr()),
+                                                            arena_bytes, self._stream()), "fo_agents_pack_batch_vehicles")
         self._batch["arena"] = arena
         self._batch["raw_dev"] = d_buf           # keep alive until the stream work is done
 
@@ -455,7 +473,8 @@ class MetricEngine:
         p's [N_p, T, 5] bundle (host array or CUDA tensor, in the caller's frame: it is shifted by the problem's origin).
         Without detail outputs this is ``fo_metric_batch``; with ``want_pair`` / ``want_step`` it is
         ``fo_metric_batch_detail``, and ``split()`` gives problem p what ``set_agents`` + ``assess(want_pair,
-        want_step)`` gives it alone.  ``out``: preallocated outputs of the batch's sizes (valid / summary / flags, and
+        want_step)`` gives it alone (in an engine built with its vehicle, when ``set_agent_batch`` had ``vehicles``).
+        ``out``: preallocated outputs of the batch's sizes (valid / summary / flags, and
         the flat pair / step where wanted).  Asynchronous on the current stream."""
         b = self._batch
         if b is None:
@@ -515,9 +534,12 @@ class MetricEngine:
             # path runs when no detail buffer is left
             a.common.pair = out.pair.data_ptr() if (out.pair is not None and out.pair.numel()) else None
             a.common.step = out.step.data_ptr() if (out.step is not None and out.step.numel()) else None
-            if a.common.pair or a.common.step:
-                L.check(L.lib.fo_metric_batch_detail(C.byref(a), self._stream()), "fo_metric_batch_detail")
+            detail, veh = bool(a.common.pair or a.common.step), b["vehicles"]
+            if veh is None:
+                fn = "fo_metric_batch_detail" if detail else "fo_metric_batch"
+                L.check(getattr(L.lib, fn)(C.byref(a), self._stream()), fn)
             else:
-                L.check(L.lib.fo_metric_batch(C.byref(a), self._stream()), "fo_metric_batch")
+                fn = "fo_metric_batch_detail_vehicles" if detail else "fo_metric_batch_vehicles"
+                L.check(getattr(L.lib, fn)(C.byref(a), veh, self._stream()), fn)
         out._keepalive = (t, b["arena"])
         return out

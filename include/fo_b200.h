@@ -176,7 +176,8 @@ int fo_metric_bundle_host(const float *ego_host, int32_t n_traj, int32_t n_state
  * P problems (one ego each: the vehicles of a multi-agent simulation, the scenes of a re-simulation) assessed by
  * ONE pack call and ONE metric call.  Replaces a loop of Metric.evaluate_metrics / assess_bundle calls, one
  * set_agents + fo_metric_bundle per problem.  Problem p has its own phantom agents (A_p may be 0) and trajectories
- * (N_p may be 0); T, the vehicle, dt, metrics, thresholds and harm coefficients are shared.  Problem p's results
+ * (N_p may be 0); T, dt, metrics, thresholds and harm coefficients are shared.  The ego vehicle is shared by the entry
+ * points below, and per problem with their *_vehicles forms (the vehicles of a mixed fleet).  Problem p's results
  * equal those fo_metric_bundle gives for it alone under FO_TEAM_WARPS set to the batch's team size. */
 typedef struct FoBatchProblem {
   int64_t traj_begin;      /* first row of the problem in ego / valid / summary / flags: rows are contiguous, in problem
@@ -229,6 +230,18 @@ int fo_metric_batch(const FoMetricBatchArgs *args, void *stream);
  * same detail buffers requested; a problem without agents gets what fo_metric_bundle gives it without detail buffers.
  * The descriptors are validated and staged as in fo_metric_batch.  Not capturable in a CUDA graph. */
 int fo_metric_batch_detail(const FoMetricBatchArgs *args, void *stream);
+
+/* The three batch calls with one ego vehicle per problem: vehicles_host is a HOST array of n_problems entries (read
+ * before the call returns), and problem p is assessed with vehicles_host[p] wherever the calls above use the shared
+ * vehicle (pack: its mass enters the harm mass split; metrics: args->common.vehicle is ignored).  Problem p's table
+ * and outputs equal, bit for bit, what fo_agents_pack + fo_metric_bundle give for it alone with
+ * FoMetricArgs.vehicle = vehicles_host[p].  A NULL vehicles_host with n_problems > 0 is FO_ERR_INVALID_ARG, checked
+ * before any device work; otherwise the arguments are validated as in the shared-vehicle calls, which are the case
+ * vehicles_host[p] = the shared vehicle for every p. */
+int fo_agents_pack_batch_vehicles(const FoAgentsRaw *raw, int32_t n_problems, const FoBatchProblem *problems_host,
+                                  const FoVehicle *vehicles_host, void *arena_dev, size_t arena_bytes, void *stream);
+int fo_metric_batch_vehicles(const FoMetricBatchArgs *args, const FoVehicle *vehicles_host, void *stream);
+int fo_metric_batch_detail_vehicles(const FoMetricBatchArgs *args, const FoVehicle *vehicles_host, void *stream);
 
 
 /* ---- stage 1: sensor visibility by ray casting ----------------------------------------------------

@@ -1,9 +1,10 @@
-// Library plumbing: error string, launch counter, version, FP32 probe, host-buffer entry point.
+// Library plumbing: error string, launch counter, version, FP32 probe, host-buffer entry points.
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
 
 #include <atomic>
+#include <vector>
 
 #include "fo_common.cuh"
 
@@ -34,7 +35,7 @@ __global__ void __launch_bounds__(256) fp32_probe_kernel(int iters, float seed, 
   if (r == 123456.789f) sink[0] = r;
 }
 
-// per-thread device workspace for the host-buffer entry point
+// per-thread device workspace of the host-buffer entry points
 constexpr int kHostChunksMax = 16;
 struct HostWs {
   void* dev = nullptr;
@@ -60,7 +61,47 @@ static int ws_reserve(size_t bytes) {
   return FO_OK;
 }
 
+// Error exits of the host-buffer entry points happen with copies / kernels possibly still queued on the workspace
+// streams: wait for them before handing the caller's buffers back (the message of the first failure is kept).
+static int ws_fail(int code) {
+  char keep[sizeof(g_err)];
+  memcpy(keep, g_err, sizeof(keep));
+  cudaStreamSynchronize(g_ws.copy);
+  cudaStreamSynchronize(g_ws.stream);
+  cudaGetLastError();
+  memcpy(g_err, keep, sizeof(keep));
+  return code;
+}
+
+// Upload chunks of N rows of row_bytes each: chunk c is rows [bound[c], bound[c + 1]); returns the chunk count.  The
+// first chunk is small (its copy cannot be hidden), every following one four times larger; rows that take less than two
+// first chunks go in one.
+static int host_chunks(size_t N, size_t row_bytes, size_t bound[kHostChunksMax + 1]) {
+  static const char* chunk_env = getenv("FO_HOST_CHUNK_MB");           // measurement switch: size of the first chunk
+  const size_t first_bytes = (size_t)(chunk_env && atoi(chunk_env) > 0 ? atoi(chunk_env) : 16) << 20;
+  bound[0] = 0; bound[1] = N;
+  if (N * row_bytes < 2 * first_bytes || row_bytes == 0) return 1;
+  size_t step = (first_bytes + row_bytes - 1) / row_bytes, at = 0;
+  int chunks = 0;
+  while (at < N && chunks < kHostChunksMax - 1) {
+    at = (at + step < N) ? at + step : N;
+    bound[++chunks] = at;
+    step *= 4;
+  }
+  if (at < N) bound[++chunks] = N;
+  return chunks;
+}
+
 }  // namespace fo
+
+#define FO_HOST_TRY(expr)                                                                          \
+  do {                                                                                             \
+    cudaError_t _e = (expr);                                                                       \
+    if (_e != cudaSuccess) {                                                                       \
+      fo::set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__);   \
+      return fo::ws_fail(FO_ERR_CUDA);                                                             \
+    }                                                                                              \
+  } while (0)
 
 extern "C" int fo_version(void) { return FO_ABI_VERSION; }
 extern "C" const char* fo_last_error(void) { return fo::g_err; }
@@ -151,25 +192,6 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
   int rc = fo::ws_reserve(total);
   if (rc != FO_OK) return rc;
   cudaStream_t st = fo::g_ws.stream;
-  // Error exits below happen with copies / kernels possibly still queued on the workspace streams: wait for them
-  // before handing the caller's buffers back (the message of the first failure is kept).
-  auto bail = [&](int code) {
-    char keep[sizeof(fo::g_err)];
-    memcpy(keep, fo::g_err, sizeof(keep));
-    cudaStreamSynchronize(fo::g_ws.copy);
-    cudaStreamSynchronize(st);
-    cudaGetLastError();
-    memcpy(fo::g_err, keep, sizeof(keep));
-    return code;
-  };
-#define FO_HOST_TRY(expr)                                                                          \
-  do {                                                                                             \
-    cudaError_t _e = (expr);                                                                       \
-    if (_e != cudaSuccess) {                                                                       \
-      fo::set_error("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__);   \
-      return bail(FO_ERR_CUDA);                                                                    \
-    }                                                                                              \
-  } while (0)
   char* p = (char*)fo::g_ws.dev;
   auto take = [&](size_t b) { char* r = p; p += b; return r; };
   float* d_ego = (float*)take(b_ego);
@@ -179,7 +201,7 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
   for (int i = 0; i < 6; ++i) {
     float* dp = (float*)take(b_f);
     if (A * Tp) {
-      if (!hsrc[i]) { fo::set_error("fo_metric_bundle_host: NULL agent array"); return bail(FO_ERR_INVALID_ARG); }
+      if (!hsrc[i]) { fo::set_error("fo_metric_bundle_host: NULL agent array"); return fo::ws_fail(FO_ERR_INVALID_ARG); }
       FO_HOST_TRY(cudaMemcpyAsync(dp, hsrc[i], A * Tp * 4, cudaMemcpyHostToDevice, st));
     }
     *hdst[i] = dp;
@@ -190,7 +212,7 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
   for (int i = 0; i < 6; ++i) {
     void* dp = take(b_a);
     if (A) {
-      if (!asrc[i]) { fo::set_error("fo_metric_bundle_host: NULL agent array"); return bail(FO_ERR_INVALID_ARG); }
+      if (!asrc[i]) { fo::set_error("fo_metric_bundle_host: NULL agent array"); return fo::ws_fail(FO_ERR_INVALID_ARG); }
       FO_HOST_TRY(cudaMemcpyAsync(dp, asrc[i], A * 4, cudaMemcpyHostToDevice, st));
     }
     *adst[i] = dp;
@@ -215,28 +237,15 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
   m.step = (out_step && T > 1) ? (float*)take(b_step) : nullptr;
   if (A > 0) {
     rc = fo_agents_pack(&d, &m.vehicle, d_tab, b_tab, st);
-    if (rc != FO_OK) return bail(rc);
+    if (rc != FO_OK) return fo::ws_fail(rc);
   }
   // Large bundles are pipelined: the trajectory range is cut into chunks, chunk k+1 crosses PCIe on the copy stream
   // while chunk k is evaluated (trajectories are independent), results follow each chunk back on the compute stream.
   // The first chunk is small (its copy cannot be hidden), every following one four times larger: copying is several
   // times faster than evaluating, and every launch costs a tail of about one trajectory time per warp.
   const size_t traj_bytes = T * 5 * 4;
-  static const char* chunk_env = getenv("FO_HOST_CHUNK_MB");           // measurement switch: size of the first chunk
-  const size_t first_bytes = (size_t)(chunk_env && atoi(chunk_env) > 0 ? atoi(chunk_env) : 16) << 20;
-  size_t bound[fo::kHostChunksMax + 1];
-  int chunks = 1;
-  bound[0] = 0; bound[1] = N;
-  if (N * traj_bytes >= 2 * first_bytes && !m.pair && !m.step && traj_bytes > 0) {
-    size_t step = (first_bytes + traj_bytes - 1) / traj_bytes, at = 0;
-    chunks = 0;
-    while (at < N && chunks < fo::kHostChunksMax - 1) {
-      at = (at + step < N) ? at + step : N;
-      bound[++chunks] = at;
-      step *= 4;
-    }
-    if (at < N) bound[++chunks] = N;
-  }
+  size_t bound[fo::kHostChunksMax + 1] = {0, N};
+  const int chunks = (!m.pair && !m.step) ? fo::host_chunks(N, traj_bytes, bound) : 1;
   for (int c = 0; c < chunks; ++c) {
     const size_t lo = bound[c], hi = bound[c + 1], n = hi - lo;
     if (n == 0) continue;
@@ -253,7 +262,7 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
     if (m.pair) mc.pair = m.pair + lo * A * FO_PAIR_K;
     if (m.step) mc.step = m.step + lo * A * (T - 1) * FO_STEP_K;
     rc = fo_metric_bundle(&mc, st);
-    if (rc != FO_OK) return bail(rc);
+    if (rc != FO_OK) return fo::ws_fail(rc);
     FO_HOST_TRY(cudaMemcpyAsync(out_valid + lo, mc.valid, n, cudaMemcpyDeviceToHost, st));
     if (out_summary)
       FO_HOST_TRY(cudaMemcpyAsync(out_summary + lo * FO_SUMMARY_K, mc.summary, n * FO_SUMMARY_K * 4, cudaMemcpyDeviceToHost, st));
@@ -263,5 +272,146 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
   if (m.step) FO_HOST_TRY(cudaMemcpyAsync(out_step, m.step, N * A * (T - 1) * FO_STEP_K * 4, cudaMemcpyDeviceToHost, st));
   FO_HOST_TRY(cudaStreamSynchronize(st));
   return FO_OK;
-#undef FO_HOST_TRY
+}
+
+extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int32_t n_states, const double* origins_host,
+                                    const FoAgentsRaw* ag, int32_t n_problems, const FoBatchProblem* problems_host,
+                                    const FoVehicle* vehicles_host, const FoMetricArgs* params, uint8_t* out_valid,
+                                    float* out_summary, uint32_t* out_flags, float* out_pair, float* out_step) {
+  const char* fn = "fo_metric_batch_host";
+  const int P = n_problems;
+  // ---- every check before any device work
+  if (!params) { fo::set_error("%s: NULL params", fn); return FO_ERR_INVALID_ARG; }
+  if (params->n_peers != 0) { fo::set_error("%s: peer stores exist on the device entry points only", fn); return FO_ERR_UNSUPPORTED; }
+  if (P > 0 && (!problems_host || !origins_host || !ag)) {
+    fo::set_error("%s: NULL problems / origins / agents with %d problems", fn, P);
+    return FO_ERR_INVALID_ARG;
+  }
+  if (n_traj > 0 && (!ego_host || !out_valid)) { fo::set_error("%s: NULL ego / out_valid", fn); return FO_ERR_INVALID_ARG; }
+  // The library owns the arena: problem p's table goes where fo_agent_batch_layout puts it.  Sizes out of range take no
+  // bytes here; the batch calls' own checks below reject them.
+  std::vector<FoBatchProblem> pr(P > 0 ? P : 0);
+  size_t arena_bytes = 0;
+  for (int p = 0; p < P; ++p) {
+    pr[p] = problems_host[p];
+    pr[p].table_offset = (int64_t)arena_bytes;
+    const int A = pr[p].n_agents, Tp = pr[p].t_stride;
+    if (A > 0 && Tp > 0 && Tp <= FO_MAX_STATES) arena_bytes += (fo::agent_table_bytes(A, Tp) + 15) & ~(size_t)15;
+  }
+  // the workspace is not placed yet: an aligned stand-in takes the place of its buffers in the checks
+  alignas(16) static float stand_in[4];
+  FoMetricBatchArgs b{};
+  b.common = *params;
+  b.common.ego = stand_in; b.common.n_traj = n_traj; b.common.n_states = n_states;
+  b.common.agent_table = stand_in; b.common.n_agents = 0; b.common.t_stride = 1;
+  b.common.valid = (uint8_t*)stand_in; b.common.summary = stand_in; b.common.flags = (uint32_t*)stand_in;
+  b.common.pair = b.common.step = nullptr;
+  b.n_problems = P; b.problems = pr.data(); b.arena_bytes = arena_bytes;
+  int n_run = 0, a_min = 0, n_packed = 0, max_cells = 0;
+  int rc = fo::check_batch(fn, &b, false, &n_run, &a_min);
+  if (rc != FO_OK) return rc;
+  const FoAgentsRaw no_agents{};
+  rc = fo::check_pack_batch(fn, P > 0 ? ag : &no_agents, P, pr.data(), stand_in, arena_bytes, &n_packed, &max_cells);
+  if (rc != FO_OK) return rc;
+  if (n_traj == 0) return FO_OK;
+
+  // ---- workspace: float64 rows, float32 bundle, raw agents, arena, per-problem ingest table, outputs
+  const size_t N = n_traj, T = n_states, A = ag->n_agents, S = ag->t_stride;
+  long long pairs = 0;                           // sum of N_p A_p: the rows of the pair / step blocks
+  for (int p = 0; p < P; ++p) pairs += (long long)pr[p].n_traj * pr[p].n_agents;
+  // as MetricEngine.assess_batch: with no pair or step left to write the summary path runs
+  const bool want_pair = out_pair && pairs > 0, want_step = out_step && pairs > 0 && T > 1;
+  auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  const size_t b_e64 = al(N * T * 5 * 8), b_e32 = al(N * T * 5 * 4), b_f = al(A * S * 4), b_a = al(A * 4 + 4);
+  const size_t b_first = ((size_t)n_run * 4 + 15) & ~(size_t)15, b_idx = al(b_first + (size_t)n_run * 16);
+  const size_t b_arena = al(arena_bytes), b_valid = al(N), b_sum = al(N * FO_SUMMARY_K * 4), b_flags = al(N * 4);
+  const size_t b_pair = want_pair ? al((size_t)pairs * FO_PAIR_K * 4) : 0;
+  const size_t b_step = want_step ? al((size_t)pairs * (T - 1) * FO_STEP_K * 4) : 0;
+  rc = fo::ws_reserve(b_e64 + b_e32 + 6 * b_f + 6 * b_a + b_idx + b_arena + b_valid + b_sum + b_flags + b_pair + b_step);
+  if (rc != FO_OK) return rc;
+  cudaStream_t st = fo::g_ws.stream;
+  char* p = (char*)fo::g_ws.dev;
+  auto take = [&](size_t b) { char* r = p; p += b; return r; };
+  double* d_e64 = (double*)take(b_e64);
+  float* d_e32 = (float*)take(b_e32);
+
+  // ---- agents: upload, then one pack call into the library's arena (overlaps the first ego chunk's upload)
+  FoAgentsRaw d = *ag;
+  const float* hsrc[6] = {ag->x, ag->y, ag->yaw, ag->v, ag->var_x, ag->var_y};
+  const float** hdst[6] = {&d.x, &d.y, &d.yaw, &d.v, &d.var_x, &d.var_y};
+  const void* asrc[6] = {ag->n_states, ag->kind, ag->length, ag->width, ag->buf_length, ag->buf_width};
+  const void** adst[6] = {(const void**)&d.n_states, (const void**)&d.kind, (const void**)&d.length,
+                          (const void**)&d.width, (const void**)&d.buf_length, (const void**)&d.buf_width};
+  for (int i = 0; i < 6; ++i) {
+    float* dp = (float*)take(b_f);
+    if (n_packed) FO_HOST_TRY(cudaMemcpyAsync(dp, hsrc[i], A * S * 4, cudaMemcpyHostToDevice, st));
+    *hdst[i] = dp;
+  }
+  for (int i = 0; i < 6; ++i) {
+    void* dp = take(b_a);
+    if (n_packed) FO_HOST_TRY(cudaMemcpyAsync(dp, asrc[i], A * 4, cudaMemcpyHostToDevice, st));
+    *adst[i] = dp;
+  }
+  // the ingest table: first rows and origins of the problems with trajectories
+  std::vector<unsigned char> idx(b_first + (size_t)n_run * 16);
+  int* first = (int*)idx.data();
+  double* org = (double*)(idx.data() + b_first);
+  for (int q = 0, i = 0; q < P; ++q) {
+    if (pr[q].n_traj == 0) continue;
+    first[i] = (int)pr[q].traj_begin;
+    org[2 * i] = origins_host[2 * q];
+    org[2 * i + 1] = origins_host[2 * q + 1];
+    ++i;
+  }
+  char* d_idx = take(b_idx);
+  FO_HOST_TRY(cudaMemcpyAsync(d_idx, idx.data(), idx.size(), cudaMemcpyHostToDevice, st));
+  void* d_arena = take(b_arena);
+  if (n_packed) {
+    rc = vehicles_host
+             ? fo_agents_pack_batch_vehicles(&d, P, pr.data(), vehicles_host, d_arena, arena_bytes, st)
+             : fo_agents_pack_batch(&d, P, pr.data(), &params->vehicle, d_arena, arena_bytes, st);
+    if (rc != FO_OK) return fo::ws_fail(rc);
+  }
+
+  // ---- ego: chunk k+1 crosses PCIe on the copy stream while chunk k is converted on the compute stream
+  const size_t row_bytes = T * 5 * 8;
+  size_t bound[fo::kHostChunksMax + 1];
+  const int chunks = fo::host_chunks(N, row_bytes, bound);
+  for (int c = 0; c < chunks; ++c) {
+    const size_t lo = bound[c], n = bound[c + 1] - lo;
+    if (n == 0) continue;
+    FO_HOST_TRY(cudaMemcpyAsync(d_e64 + lo * T * 5, ego_host + lo * T * 5, n * row_bytes, cudaMemcpyHostToDevice,
+                                fo::g_ws.copy));
+    FO_HOST_TRY(cudaEventRecord(fo::g_ws.ready[c], fo::g_ws.copy));
+    FO_HOST_TRY(cudaStreamWaitEvent(st, fo::g_ws.ready[c], 0));
+    rc = fo::launch_ego_ingest(d_e64 + lo * T * 5, d_e32 + lo * T * 5, (int)lo, (int)n, (int)T, (const int*)d_idx,
+                               (const double2*)(d_idx + b_first), n_run, st);
+    if (rc != FO_OK) return fo::ws_fail(rc);
+  }
+
+  // ---- the batch call itself, after the last chunk is converted (one W for the whole batch)
+  b.common.ego = d_e32;
+  b.common.agent_table = arena_bytes ? d_arena : nullptr;
+  b.common.valid = (uint8_t*)take(b_valid);
+  b.common.summary = (float*)take(b_sum);
+  b.common.flags = (uint32_t*)take(b_flags);
+  b.common.pair = want_pair ? (float*)take(b_pair) : nullptr;
+  b.common.step = want_step ? (float*)take(b_step) : nullptr;
+  if (want_pair || want_step)
+    rc = vehicles_host ? fo_metric_batch_detail_vehicles(&b, vehicles_host, st) : fo_metric_batch_detail(&b, st);
+  else
+    rc = vehicles_host ? fo_metric_batch_vehicles(&b, vehicles_host, st) : fo_metric_batch(&b, st);
+  if (rc != FO_OK) return fo::ws_fail(rc);
+
+  // ---- results back, then synchronise
+  FO_HOST_TRY(cudaMemcpyAsync(out_valid, b.common.valid, N, cudaMemcpyDeviceToHost, st));
+  if (out_summary)
+    FO_HOST_TRY(cudaMemcpyAsync(out_summary, b.common.summary, N * FO_SUMMARY_K * 4, cudaMemcpyDeviceToHost, st));
+  if (out_flags) FO_HOST_TRY(cudaMemcpyAsync(out_flags, b.common.flags, N * 4, cudaMemcpyDeviceToHost, st));
+  if (want_pair)
+    FO_HOST_TRY(cudaMemcpyAsync(out_pair, b.common.pair, (size_t)pairs * FO_PAIR_K * 4, cudaMemcpyDeviceToHost, st));
+  if (want_step)
+    FO_HOST_TRY(cudaMemcpyAsync(out_step, b.common.step, (size_t)pairs * (T - 1) * FO_STEP_K * 4, cudaMemcpyDeviceToHost, st));
+  FO_HOST_TRY(cudaStreamSynchronize(st));
+  return FO_OK;
 }

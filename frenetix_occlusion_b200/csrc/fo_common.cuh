@@ -11,6 +11,20 @@ namespace fo {
 void set_error(const char* fmt, ...);
 void count_launch(uint64_t n = 1);
 
+// Host-side argument checks of the batch entry points (fo_metric.cu), before any device work; fn names the entry point
+// in the messages.  check_batch: the metric calls (detail: fo_metric_batch_detail's outputs); on success *n_run = the
+// problems with trajectories and *a_min = the fewest agents among them.  check_pack_batch: fo_agents_pack_batch; on
+// success *n_packed = the problems with agents and *max_cells = the most table cells of one of them.
+int check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, int* n_run, int* a_min);
+int check_pack_batch(const char* fn, const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
+                     const void* arena_dev, size_t arena_bytes, int* n_packed, int* max_cells);
+
+// fo_metric_batch_host's float64 -> float32 conversion of ego rows [row0, row0 + n_rows) of a batch ([rows, T, 5], src
+// and dst point at row row0): first_dev[n_first] = the first rows of the problems with trajectories (strictly
+// increasing, first_dev[0] = 0) and origin_dev[n_first] their origins.  One launch (fo_metric.cu).
+int launch_ego_ingest(const double* src, float* dst, int row0, int n_rows, int T, const int* first_dev,
+                      const double2* origin_dev, int n_first, cudaStream_t st);
+
 #define FO_CUDA_TRY(expr)                                                                      \
   do {                                                                                         \
     cudaError_t _e = (expr);                                                                   \

@@ -156,6 +156,57 @@ static void launch_pack(const FoAgentsRaw& raw, const PackProblem& one, const Pa
   fo_agents_pack_kernel<<<grid, 256, 0, st>>>(raw, one, many, P, arena);
 }
 
+// ---------------------------------------------------------------------------------------------
+// fo_metric_batch_host's ego ingest: float64 rows in the caller's world frame -> the float32 bundle of the metric kernels.
+// x and y lose their problem's origin in float64 and are rounded once; theta, v and a are rounded.  The operations are
+// explicit round-to-nearest intrinsics, so no contraction can change a bit: every value equals numpy's float64 difference
+// cast to float32, which is what MetricEngine.assess_batch stages on the host.  A CTA takes a tile of whole rows, finds
+// each row's problem once (find_problem, as the batch kernels do), then streams the tile: coalesced 8-byte loads and
+// 4-byte stores.
+constexpr int kIngestThreads = 256, kIngestTileRows = 256;
+
+__global__ void __launch_bounds__(kIngestThreads)
+fo_ego_ingest_kernel(const double* __restrict__ src, float* __restrict__ dst, int row0, int n_rows, int row_elems,
+                     int tile_rows, const int* __restrict__ first, const double2* __restrict__ origin, int n_first) {
+  __shared__ double2 org[kIngestTileRows];
+  const int n_tiles = (n_rows + tile_rows - 1) / tile_rows;
+  for (int t = blockIdx.x; t < n_tiles; t += gridDim.x) {
+    const int r_lo = t * tile_rows, rows = min(tile_rows, n_rows - r_lo);
+    if ((int)threadIdx.x < rows) org[threadIdx.x] = origin[find_problem(first, n_first, row0 + r_lo + threadIdx.x)];
+    __syncthreads();
+    const double* s = src + (size_t)r_lo * row_elems;
+    float* d = dst + (size_t)r_lo * row_elems;
+    const int m = rows * row_elems;
+    for (int j = threadIdx.x; j < m; j += kIngestThreads) {
+      const double v = s[j];
+      const int col = j % 5;                     // row_elems = 5 T: every row starts at a multiple of 5
+      float o;
+      if (col < 2) {
+        const double2 g = org[j / row_elems];
+        o = __double2float_rn(__dsub_rn(v, col == 0 ? g.x : g.y));
+      } else {
+        o = __double2float_rn(v);
+      }
+      d[j] = o;
+    }
+    __syncthreads();
+  }
+}
+
+int launch_ego_ingest(const double* src, float* dst, int row0, int n_rows, int T, const int* first_dev,
+                      const double2* origin_dev, int n_first, cudaStream_t st) {
+  if (n_rows <= 0) return FO_OK;
+  const int row_elems = 5 * T;
+  // about 2048 elements per tile, so short horizons still give every thread several
+  const int tile_rows = max(1, min(kIngestTileRows, 2048 / row_elems));
+  const int n_tiles = (n_rows + tile_rows - 1) / tile_rows;
+  fo_ego_ingest_kernel<<<min(n_tiles, 4096), kIngestThreads, 0, st>>>(src, dst, row0, n_rows, row_elems, tile_rows,
+                                                                     first_dev, origin_dev, n_first);
+  count_launch();
+  FO_CUDA_TRY(cudaGetLastError());
+  return FO_OK;
+}
+
 // The ego vehicle in kernel units; the single-problem path and every batch descriptor take it from here, so a problem
 // of a batch sees the same float values as alone.
 static void fill_ego_const(const FoVehicle& v, EgoConst& e) {
@@ -270,14 +321,14 @@ extern "C" size_t fo_agent_batch_layout(int32_t n_problems, const int32_t* n_age
   return off;
 }
 
-// Problem p is packed with the mass of vehicles[per_problem ? p : 0].
-static int pack_batch_impl(const char* fn, const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
-                           const FoVehicle* vehicles, bool per_problem, void* arena_dev, size_t arena_bytes, void* stream) {
-  if (!raw || !vehicles || n_problems < 0 || (n_problems > 0 && !problems)) { fo::set_error("%s: bad argument", fn); return FO_ERR_INVALID_ARG; }
+int fo::check_pack_batch(const char* fn, const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
+                         const void* arena_dev, size_t arena_bytes, int* n_packed_out, int* max_cells_out) {
+  if (!raw || n_problems < 0 || (n_problems > 0 && !problems)) { fo::set_error("%s: bad argument", fn); return FO_ERR_INVALID_ARG; }
   if (raw->n_agents < 0 || raw->t_stride < 0) { fo::set_error("%s: negative size", fn); return FO_ERR_INVALID_ARG; }
   if (reinterpret_cast<uintptr_t>(arena_dev) & 15) { fo::set_error("%s: arena must be 16-byte aligned", fn); return FO_ERR_INVALID_ARG; }
   long long total = 0;
   int n_packed = 0, max_cells = 0;
+  *n_packed_out = 0;
   for (int p = 0; p < n_problems; ++p) {
     const FoBatchProblem& q = problems[p];
     if (q.n_agents < 0) { fo::set_error("%s: problem %d has %d agents", fn, p, q.n_agents); return FO_ERR_INVALID_ARG; }
@@ -299,6 +350,20 @@ static int pack_batch_impl(const char* fn, const FoAgentsRaw* raw, int32_t n_pro
       !raw->length || !raw->width || !raw->buf_length || !raw->buf_width) {
     fo::set_error("%s: NULL array in FoAgentsRaw", fn);
     return FO_ERR_INVALID_ARG;
+  }
+  *n_packed_out = n_packed;
+  *max_cells_out = max_cells;
+  return FO_OK;
+}
+
+// Problem p is packed with the mass of vehicles[per_problem ? p : 0].
+static int pack_batch_impl(const char* fn, const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
+                           const FoVehicle* vehicles, bool per_problem, void* arena_dev, size_t arena_bytes, void* stream) {
+  if (!vehicles) { fo::set_error("%s: bad argument", fn); return FO_ERR_INVALID_ARG; }
+  int n_packed = 0, max_cells = 0;
+  {
+    const int rc = fo::check_pack_batch(fn, raw, n_problems, problems, arena_dev, arena_bytes, &n_packed, &max_cells);
+    if (rc != FO_OK || n_packed == 0) return rc;
   }
   cudaStream_t st = (cudaStream_t)stream;
   const size_t bytes = (size_t)n_packed * sizeof(fo::PackProblem);
@@ -430,7 +495,7 @@ static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, 
 // Host-side checks of the batch entry points, before any device work: the outputs each one accepts, row order and
 // contiguity, rows inside n_traj, tables inside the arena, alignment, stride and T limits, 'be' needs 'ttc'.  On success
 // *n_run = the problems with trajectories and *a_min = the fewest agents among them.
-static int check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, int* n_run, int* a_min) {
+int fo::check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, int* n_run, int* a_min) {
   if (!b) { fo::set_error("%s: NULL args", fn); return FO_ERR_INVALID_ARG; }
   const FoMetricArgs& c = b->common;
   const int P = b->n_problems;
@@ -487,7 +552,7 @@ static int check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, 
 static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const FoVehicle* vehicles, void* stream) {
   int n_run = 0, a_min = 0;
   {
-    const int rc = check_batch(fn, b, false, &n_run, &a_min);
+    const int rc = fo::check_batch(fn, b, false, &n_run, &a_min);
     if (rc != FO_OK || b->common.n_traj == 0) return rc;
   }
   const FoMetricArgs& c = b->common;
@@ -567,7 +632,7 @@ extern "C" int fo_metric_batch_vehicles(const FoMetricBatchArgs* b, const FoVehi
 static int metric_batch_detail_impl(const char* fn, const FoMetricBatchArgs* b, const FoVehicle* vehicles, void* stream) {
   int n_run = 0, a_min = 0;
   {
-    const int rc = check_batch(fn, b, true, &n_run, &a_min);
+    const int rc = fo::check_batch(fn, b, true, &n_run, &a_min);
     if (rc != FO_OK || b->common.n_traj == 0) return rc;
   }
   const FoMetricArgs& c = b->common;

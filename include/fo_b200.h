@@ -243,6 +243,34 @@ int fo_agents_pack_batch_vehicles(const FoAgentsRaw *raw, int32_t n_problems, co
 int fo_metric_batch_vehicles(const FoMetricBatchArgs *args, const FoVehicle *vehicles_host, void *stream);
 int fo_metric_batch_detail_vehicles(const FoMetricBatchArgs *args, const FoVehicle *vehicles_host, void *stream);
 
+/* A batch driven from HOST buffers (pinned or pageable), for embedders without a CUDA runtime of their own: the
+ * planner's float64 ego rows in the caller's world frame and one float64 origin per problem in, results in host arrays
+ * out, synchronised.  The library shifts every row by its problem's origin on the device, in float64, and only then
+ * rounds to float32: (float)(x - origin_p.x), (float)(y - origin_p.y), (float)theta, (float)v, (float)a -- what
+ * MetricEngine.assess_batch stages on the host.  It then packs the agents into a library-owned arena and makes the
+ * batch call, so the results equal, bit for bit, fo_agents_pack_batch[_vehicles] + fo_metric_batch[_vehicles] on that
+ * bundle, or fo_metric_batch_detail[_vehicles] when out_pair or out_step is non-NULL and there is a pair / step block
+ * to write (some problem has trajectories and agents; for step also T > 1) -- otherwise the summary path runs and the
+ * detail outputs are not touched.  out_pair / out_step are laid out as in fo_metric_batch_detail and need no alignment;
+ * out_summary / out_flags may be NULL.
+ *   ego_host      [n_traj, T, 5] (x, y, theta, v, a), rows of the problems contiguous in problem order
+ *   origins_host  [n_problems, 2] problem p's origin
+ *   agents_host   HOST pointers: the agents of all problems concatenated in problem order, positions already relative
+ *                 to their problem's origin, row stride t_stride >= every problem's t_stride (as fo_agents_pack_batch)
+ *   problems_host traj_begin, n_traj, n_agents, t_stride; table_offset is ignored (the library places the tables)
+ *   vehicles_host [n_problems] or NULL: params->vehicle for every problem
+ *   params        vehicle, harm, dt, metric / threshold masks and thresholds; its device pointers (ego, agent_table,
+ *                 valid, summary, flags, pair, step) and sizes are ignored; n_peers != 0 is FO_ERR_UNSUPPORTED
+ * Every argument is validated before any device work, with the checks and messages of the device batch calls; NULL
+ * problems_host, origins_host or agents_host with n_problems > 0, and NULL ego_host or out_valid with n_traj > 0, are
+ * FO_ERR_INVALID_ARG.  The float64 rows cross PCIe in chunks (FO_HOST_CHUNK_MB, as fo_metric_bundle_host), each
+ * converted while the next one is copied; the metric call follows the last chunk.  Device workspace as
+ * fo_metric_bundle_host's (per calling thread, grown on demand). */
+int fo_metric_batch_host(const double *ego_host, int32_t n_traj, int32_t n_states, const double *origins_host,
+                         const FoAgentsRaw *agents_host, int32_t n_problems, const FoBatchProblem *problems_host,
+                         const FoVehicle *vehicles_host, const FoMetricArgs *params, uint8_t *out_valid,
+                         float *out_summary, uint32_t *out_flags, float *out_pair, float *out_step);
+
 
 /* ---- stage 1: sensor visibility by ray casting ----------------------------------------------------
  * Replaces SensorModel.calc_visible_and_occluded_area (sensor_model.py:41-193): the reference clips

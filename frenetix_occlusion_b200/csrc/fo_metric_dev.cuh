@@ -39,7 +39,7 @@ struct MetricKArgs {
   uint32_t* flags;
   float* pair;
   float* step;
-  unsigned long long* stats;   // optional [8] work counters (see fo_metric_stats), NULL in production launches
+  unsigned long long* stats;   // optional [FO_STATS_K] work counters (see fo_metric_stats), NULL in production launches
   unsigned int* claim;         // zeroed per launch: next-trajectory counter of the summary kernel (NULL = static striding)
   int n_peers;                 // summary kernel: results are also stored at these byte offsets (peer-mapped gather buffers)
   long long peer_delta[FO_MAX_PEERS];
@@ -356,22 +356,86 @@ __device__ __forceinline__ float be_arclen(float dt, float v0, float v1, float s
   return (i == 0) ? 0.0f : dt * (v0 + fmaf(m, v1, -0.5f * step * m * (m - 1.0f)));
 }
 
-// Returns (required constant deceleration, number of probes as int bits); the deceleration is NaN when the re-timed
-// path overruns the planned one (the reference raises, be.py:117-124).
-// floor_rcd (summary kernel; negative = off): the caller keeps only the MAXIMUM over a trajectory's pairs.  The bracket
-// [lo, hi] only shrinks and the result is its last midpoint, so once hi <= floor_rcd this pair cannot raise the maximum
-// and the bisection stops -- provided no later probe could overrun the planned path: dist_new[T-1] falls with the
-// deceleration, the smallest deceleration the rest of the bisection can probe is the end of its all-miss branch, and
-// that one is checked (with a margin for the float32 closed form; inside the margin the bisection simply runs on).
+// number of positive terms of the clipped series at the probe step = deceleration * dt; step in [4e-4, 0.5]:
+// v1 * rcp == __fdividef(v1, step) bit for bit
+__device__ __forceinline__ float be_mpos(float v1, float step) {
+  return (step > 0.0f) ? fmaxf(floorf(v1 * rcp_approx(step)) + 1.0f, 0.0f) : 1.0e9f;
+}
+
+// Re-timed ego reference point (x, y) and heading (sin, cos) of step i at the probe (step, mpos) (be.py:109-130).
+struct BePose {
+  float x, y, s, c;
+};
 template <bool SEG>
-static __device__ __noinline__ float2 be_bisect(const BeConst k, const BeView v, int a, int n_states, float hl, float hw,
-                                                float lo0, int lane, float floor_rcd) {
+__device__ __forceinline__ BePose be_pose(const BeView& v, int T, float dt, float v0, float v1, float inv_w, float step,
+                                          float mpos, int i) {
   extern __shared__ __align__(16) unsigned char fo_dyn_smem[];
   const float4* const egoA = reinterpret_cast<const float4*>(fo_dyn_smem + v.egoA);
   const float2* const egoB = reinterpret_cast<const float2*>(fo_dyn_smem + v.egoB);
   const float* const dist = reinterpret_cast<const float*>(fo_dyn_smem + v.dist);
   const uint8_t* const inv_tab = fo_dyn_smem + v.inv;
   const float4* const seg = reinterpret_cast<const float4*>(fo_dyn_smem + v.seg);
+  const float q = be_arclen(dt, v0, v1, step, mpos, i);
+  // numpy.interp: j = last index with dist[j] <= q.  The bucket of q brackets it: j0 = inv[b] (stepped one bucket
+  // down when float32 rounding of the bucket index put it too high), j1 = inv[b + 1]; a bisection of [j0, j1] --
+  // most buckets hold at most one state -- and a final upward check for a q that rounded across the bucket's end
+  int b = min(__float2int_rd(q * inv_w), kBeBuckets - 1);
+  int j = inv_tab[b];
+  if (dist[j] > q) { b = max(b - 1, 0); j = inv_tab[b]; }
+  int jh = inv_tab[b + 1];
+  while (j < jh) {
+    const int mid = (j + jh + 1) >> 1;
+    if (dist[mid] <= q) j = mid; else jh = mid - 1;
+  }
+  while (j < T - 1 && dist[j + 1] <= q) ++j;
+  const float dj = dist[j];
+  const float4 A0 = egoA[j];
+  float xn = A0.x, yn = A0.y, tn = egoB[j].x;
+  if (j != T - 1 && dj != q) {
+    const float wq = q - dj;
+    if (SEG) {
+      const float4 sl = seg[j];
+      xn = fmaf(sl.x, wq, A0.x);
+      yn = fmaf(sl.y, wq, A0.y);
+      tn = fmaf(sl.z, wq, tn);
+    } else {
+      const float4 A1 = egoA[j + 1];
+      const float inv = 1.0f / (dist[j + 1] - dj);
+      xn = fmaf((A1.x - A0.x) * inv, wq, A0.x);
+      yn = fmaf((A1.y - A0.y) * inv, wq, A0.y);
+      tn = fmaf((egoB[j + 1].x - tn) * inv, wq, tn);
+    }
+  }
+  BePose p;
+  p.x = xn;
+  p.y = yn;
+  __sincosf(tn, &p.s, &p.c);
+  return p;
+}
+
+// the agent's state s0 at that step against the ego box at the re-timed pose (be.py:181)
+__device__ __forceinline__ bool be_hit(const BeConst& k, const BePose& p, const float4 s0, float hl, float hw) {
+  const float dx = (s0.x - p.x) - k.wb * p.c;
+  const float dy = (s0.y - p.y) - k.wb * p.s;
+  const float rx = fmaf(dx, p.c, dy * p.s), ry = fmaf(dy, p.c, -dx * p.s);
+  const float c = fmaf(p.c, s0.z, p.s * s0.w), s = fmaf(s0.w, p.c, -s0.z * p.s);
+  return obb_hit(rx, ry, c, s, k.hEx, k.hEy, hl, hw);
+}
+
+// BE of one pair: returns (required constant deceleration, number of probes as int bits); the deceleration is NaN
+// when the re-timed path overruns the planned one (the reference raises, be.py:117-124).
+// floor_rcd (team shape of the summary kernel; negative = off): the caller keeps only the MAXIMUM over a trajectory's
+// pairs.  The bracket [lo, hi] only shrinks and the result is its last midpoint, so once hi <= floor_rcd this pair
+// cannot raise the maximum and the bisection stops -- provided no later probe could overrun the planned path:
+// dist_new[T-1] falls with the deceleration, the smallest deceleration the rest of the bisection can probe is the end
+// of its all-miss branch, and that one is checked (with a margin for the float32 closed form; inside the margin the
+// bisection simply runs on).
+template <bool SEG>
+static __device__ __noinline__ float2 be_bisect(const BeConst k, const BeView v, int a, int n_states, float hl, float hw,
+                                                float lo0, int lane, float floor_rcd) {
+  extern __shared__ __align__(16) unsigned char fo_dyn_smem[];
+  const float2* const egoB = reinterpret_cast<const float2*>(fo_dyn_smem + v.egoB);
+  const float* const dist = reinterpret_cast<const float*>(fo_dyn_smem + v.dist);
   const int T = k.T;
   const int nA = min(T, n_states);
   const float v0 = egoB[0].y, v1 = egoB[T > 1 ? 1 : 0].y;
@@ -389,8 +453,7 @@ static __device__ __noinline__ float2 be_bisect(const BeConst k, const BeView v,
     cur = 0.5f * (lo + hi);
     ++probes;
     const float step = cur * k.dt;
-    // step in [4e-4, 0.5]: v1 * rcp == __fdividef(v1, step) bit for bit
-    const float mpos = (step > 0.0f) ? fmaxf(floorf(v1 * rcp_approx(step)) + 1.0f, 0.0f) : 1.0e9f;
+    const float mpos = be_mpos(v1, step);
     if (be_arclen(k.dt, v0, v1, step, mpos, T - 1) > dmax) return make_float2(CUDART_NAN_F, __int_as_float(probes));
     bool any_hit = false;
 #pragma unroll 1
@@ -398,45 +461,8 @@ static __device__ __noinline__ float2 be_bisect(const BeConst k, const BeView v,
       const int i = i0 + lane;
       bool hit = false;
       if (i < nA) {
-        const float q = be_arclen(k.dt, v0, v1, step, mpos, i);
-        // numpy.interp: j = last index with dist[j] <= q.  The bucket of q brackets it: j0 = inv[b] (stepped one bucket
-        // down when float32 rounding of the bucket index put it too high), j1 = inv[b + 1]; a bisection of [j0, j1] --
-        // most buckets hold at most one state -- and a final upward check for a q that rounded across the bucket's end
-        int b = min(__float2int_rd(q * inv_w), kBeBuckets - 1);
-        int j = inv_tab[b];
-        if (dist[j] > q) { b = max(b - 1, 0); j = inv_tab[b]; }
-        int jh = inv_tab[b + 1];
-        while (j < jh) {
-          const int mid = (j + jh + 1) >> 1;
-          if (dist[mid] <= q) j = mid; else jh = mid - 1;
-        }
-        while (j < T - 1 && dist[j + 1] <= q) ++j;
-        const float dj = dist[j];
-        const float4 A0 = egoA[j];
-        float xn = A0.x, yn = A0.y, tn = egoB[j].x;
-        if (j != T - 1 && dj != q) {
-          const float wq = q - dj;
-          if (SEG) {
-            const float4 sl = seg[j];
-            xn = fmaf(sl.x, wq, A0.x);
-            yn = fmaf(sl.y, wq, A0.y);
-            tn = fmaf(sl.z, wq, tn);
-          } else {
-            const float4 A1 = egoA[j + 1];
-            const float inv = 1.0f / (dist[j + 1] - dj);
-            xn = fmaf((A1.x - A0.x) * inv, wq, A0.x);
-            yn = fmaf((A1.y - A0.y) * inv, wq, A0.y);
-            tn = fmaf((egoB[j + 1].x - tn) * inv, wq, tn);
-          }
-        }
-        float sn, cn;
-        __sincosf(tn, &sn, &cn);
-        const float4 s0 = (i0 == 0) ? pre0 : ((i0 == 32) ? pre1 : __ldg(sa + i));
-        const float dx = (s0.x - xn) - k.wb * cn;
-        const float dy = (s0.y - yn) - k.wb * sn;
-        const float rx = fmaf(dx, cn, dy * sn), ry = fmaf(dy, cn, -dx * sn);
-        const float c = fmaf(cn, s0.z, sn * s0.w), s = fmaf(s0.w, cn, -s0.z * sn);
-        hit = obb_hit(rx, ry, c, s, k.hEx, k.hEy, hl, hw);
+        const BePose p = be_pose<SEG>(v, T, k.dt, v0, v1, inv_w, step, mpos, i);
+        hit = be_hit(k, p, (i0 == 0) ? pre0 : ((i0 == 32) ? pre1 : __ldg(sa + i)), hl, hw);
       }
       any_hit = __any_sync(kFull, hit);
     }
@@ -450,11 +476,123 @@ static __device__ __noinline__ float2 be_bisect(const BeConst k, const BeView v,
         if (h - lo < 0.1f) break;
       }
       const float st = c * k.dt;
-      const float mp = (st > 0.0f) ? fmaxf(floorf(v1 * rcp_approx(st)) + 1.0f, 0.0f) : 1.0e9f;
-      if (be_arclen(k.dt, v0, v1, st, mp, T - 1) < dmax * 0.99999f) break;
+      if (be_arclen(k.dt, v0, v1, st, be_mpos(v1, st), T - 1) < dmax * 0.99999f) break;
     }
   }
   return make_float2(cur, __int_as_float(probes));
+}
+
+// ---- BE of the summary kernels: the maximum over a trajectory's colliding pairs, one walk over one bisection tree ---
+// Every pair starts from the bracket [lo0, 5] and follows the same midpoint and stop rules, so all probes of a
+// trajectory are nodes of one binary tree, and each pair's bisection is one root-to-leaf path through it.  be_walk
+// visits that tree depth first.  The re-timed ego path of a node is computed once, 32 steps at a time (lane = step),
+// and every pair that reaches the node is tested against it, with the per-chunk early exit of be_bisect: the pairs
+// that hit move to the right child (cur, hi), the others to the left child (lo, cur).  A pair sees the probes of its
+// own bisection and decides each from the same operations on the same inputs (be_pose, be_hit), so it ends in the
+// same leaf; only the maximum over the leaves leaves the kernel.
+// Floor: the maximum so far.  A pending node whose bracket lies at or below it cannot raise it (a result is the last
+// midpoint, inside the bracket) and is dropped -- provided no probe below it could overrun the planned path:
+// dist_new[T-1] falls with the deceleration, the smallest deceleration below the node is the end of its all-miss
+// branch, and that one is checked with a margin for the float32 closed form (inside the margin the walk goes on).
+// The hit child is visited first: high decelerations raise the floor soonest.  A range error ends the walk (the
+// outputs are NaN, the trajectory invalid).
+// k.s0 / prm: the tile's first agent; list: byte offset of the tile's pair list (agent-in-tile indices, reordered in
+// place).  Pending nodes sit one per lane (at most one per depth, depth <= 10): no local memory.
+// Used by the one-warp throughput shape.  The team (latency) shape keeps one be_bisect per pair: there a warp holds one
+// or two pairs, and the walk's per-node loads of the pair parameters and states lengthen the critical path (DESIGN.md 5.1).
+struct BeWalk {
+  float rcd;                       // maximum of the floor and the leaves' decelerations
+  bool range;                      // a probe overran the planned path (be.py:117-124)
+  unsigned tests, nodes, chunks;   // STATS: pair tests (probes of be_bisect), nodes visited, ego-path chunks computed
+};
+template <bool STATS>
+static __device__ __noinline__ BeWalk be_walk(const BeConst k, const AgentParams* prm, const BeView v, uint32_t list, int n,
+                                              float lo0, float rcd, int lane) {
+  extern __shared__ __align__(16) unsigned char fo_dyn_smem[];
+  uint16_t* const lst = reinterpret_cast<uint16_t*>(fo_dyn_smem + list);
+  const float2* const egoB = reinterpret_cast<const float2*>(fo_dyn_smem + v.egoB);
+  const float* const dist = reinterpret_cast<const float*>(fo_dyn_smem + v.dist);
+  const int T = k.T;
+  const float v0 = egoB[0].y, v1 = egoB[T > 1 ? 1 : 0].y;
+  const float dmax = dist[T - 1];
+  const float inv_w = dmax > 0.0f ? (float)kBeBuckets / dmax : 0.0f;
+  BeWalk r;
+  r.range = false;
+  if (STATS) r.tests = r.nodes = r.chunks = 0u;
+  float lo = lo0, hi = 5.0f;
+  int b = 0, e = n, d = 0;               // node: bracket, its pairs lst[b, e), probes above it
+  float st_lo = 0.0f, st_hi = 0.0f;      // lane j: pending node j
+  int st_n = 0, sp = 0;
+  bool below = false;                    // the node lies at or below the floor: is it safe to drop?
+  for (;;) {
+    // the probe of the node, or (below) the end of its all-miss branch; one closed-form path length serves both tests
+    float cur = 0.5f * (lo + hi);
+    if (below)
+      for (int j = d + 1; j < 10 && !(cur - lo < 0.1f); ++j) cur = 0.5f * (lo + cur);
+    const float step = cur * k.dt;
+    const float mpos = be_mpos(v1, step);
+    const float len = be_arclen(k.dt, v0, v1, step, mpos, T - 1);
+    bool pop = true;
+    if (below) {
+      below = false;
+      pop = len < dmax * 0.99999f;       // dropped; otherwise visited next time round
+    } else {
+      if (len > dmax) { r.range = true; break; }
+      if (STATS) { ++r.nodes; r.tests += (unsigned)(e - b); }
+      int m = e;                         // lst[b, m): no hit so far
+#pragma unroll 1
+      for (int i0 = 0; m > b; i0 += 32) {
+        const int i = i0 + lane;
+        const BePose p = be_pose<true>(v, T, k.dt, v0, v1, inv_w, step, mpos, i);
+        if (STATS) ++r.chunks;
+        bool more = false;               // a pair without a hit has steps after this chunk
+#pragma unroll 1
+        for (int s = b; s < m;) {
+          const int al = lst[s];
+          const int4 pa = __ldg(reinterpret_cast<const int4*>(prm + al));
+          const int nA = min(T, pa.x);
+          bool hit = nA == 0;            // be.py:74-77 (an agent that never exists counts as a hit)
+          if (i < nA) hit = be_hit(k, p, __ldg(k.s0 + al * k.Tp + i), __int_as_float(pa.z), __int_as_float(pa.w));
+          if (__any_sync(kFull, hit)) {  // to the hit end of the node's pairs
+            --m;
+            if (lane == 0) { lst[s] = lst[m]; lst[m] = (uint16_t)al; }
+            __syncwarp();
+          } else {
+            more |= nA > i0 + 32;
+            ++s;
+          }
+        }
+        if (!more) break;
+      }
+      // children: misses lst[b, m) with (lo, cur), hits lst[m, e) with (cur, hi).  A child at the stop rule (be.py:79)
+      // or after the tenth probe is a leaf: its pairs' result is cur.  Pushed left first: the hit child is popped first.
+      ++d;
+#pragma unroll 1
+      for (int h = 0; h < 2; ++h) {
+        const float cl = h ? cur : lo, ch = h ? hi : cur;
+        const int cb = h ? m : b, ce = h ? e : m;
+        if (cb < ce) {
+          if (ch - cl < 0.1f || d == 10) {
+            rcd = fmaxf(rcd, cur);
+          } else {
+            if (lane == sp) { st_lo = cl; st_hi = ch; st_n = cb | ce << 9 | d << 18; }
+            ++sp;
+          }
+        }
+      }
+    }
+    if (pop) {
+      if (sp == 0) break;
+      --sp;
+      lo = __shfl_sync(kFull, st_lo, sp);
+      hi = __shfl_sync(kFull, st_hi, sp);
+      const int nd = __shfl_sync(kFull, st_n, sp);
+      b = nd & 0x1ff; e = (nd >> 9) & 0x1ff; d = nd >> 18;
+      below = hi <= rcd;
+    }
+  }
+  r.rcd = rcd;
+  return r;
 }
 
 struct EgoState {

@@ -25,8 +25,10 @@
 //     out of five items never reach it;
 //   * the running minimum distance and the running maximum logits are WARP-SHARED (REDUX after every drain), so a
 //     near agent found by one lane prunes the work of all 32;
-//   * colliding pairs are collected in a team list and their BE bisections (be.py:66-193) are dealt round-robin to
-//     the warps; per-trajectory results are order-independent min/max reductions (lane -> warp REDUX -> team).
+//   * colliding pairs are collected in a team list for the brake evaluation (BE, be.py:66-193): the one-warp shape walks
+//     their common bisection tree (be_walk: one re-timed ego path per probe value instead of one per pair and probe),
+//     the team shape deals one bisection per pair round-robin to its warps (be_bisect); per-trajectory results are
+//     order-independent min/max reductions (lane -> warp REDUX -> team).
 //
 // All bounds are exact (a skipped evaluation cannot change a min / max / threshold decision); results equal the detail
 // kernel's.  The kernel is instruction-issue- and instruction-cache-bound (DESIGN.md 6): code that exists twice after
@@ -253,6 +255,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
   const int s_lo = (wib * (32 >> lg) + ls) * L;
   const int s_hi = min(T, s_lo + L);
   unsigned long long st_dense = 0, st_obb = 0, st_lr = 0, st_cp = 0, st_be = 0, st_probe = 0, st_win = 0, st_wkeep = 0;
+  unsigned long long st_node = 0, st_path = 0;
 
   // Trajectories are claimed from a device counter (their cost varies several-fold with the number of near agents and
   // braking pairs); the claim for the next one is issued here and read at the bottom, so its latency is hidden.  A batch
@@ -701,25 +704,33 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
             be_ready = true;
           }
           const float be_lo0 = rintf(__uint_as_float(w.scal[0]) * 100.0f) / 100.0f;   // be.py:68
-          // only max over the pairs is kept: a bisection stops as soon as its bracket lies below the running maximum
-          // (be_bisect), and a range error makes every further one moot (the outputs are NaN, the trajectory invalid)
-          for (int q = wib; q < n_be && !(flags & FO_F_BE_RANGE); q += W) {   // bisections dealt round-robin to the warps
-            const int a = a0 + (int)w.be_list[q];
-            const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + a));
-#ifdef FO_BE_NO_FLOOR
-            const float be_floor = -1.0f;
-#else
-            const float be_floor = rcd_all;
-#endif
-            BeConst bk = bek;
-            if constexpr (BATCH) { bk.wb = veh.wb; bk.hEx = veh.hEx; bk.hEy = veh.hEy; }
-            const float2 be = be_bisect<true>(bk, bev, a, pa.x, __int_as_float(pa.z), __int_as_float(pa.w), be_lo0, lane,
-                                              be_floor);
-            const float rcd = be.x;
-            if (rcd != rcd) flags |= FO_F_BE_RANGE;      // NaN: the re-timed path overruns the planned one
-            rcd_all = fmaxf(rcd_all, rcd);
-            btn_all = fmaxf(btn_all, rcd / veh.a_max);
-            if (STATS && lane == 0) { st_be += 1; st_probe += (unsigned)__float_as_int(be.y); }
+          BeConst bk = bek;
+          if constexpr (BATCH) { bk.wb = veh.wb; bk.hEx = veh.hEx; bk.hEy = veh.hEy; }
+          if constexpr (UNI) {
+            // one walk over the bisection tree of the tile's pairs (be_walk); only the maximum over the pairs is kept,
+            // and after a range error no further pair matters (the outputs are NaN, the trajectory invalid)
+            if (!(flags & FO_F_BE_RANGE)) {
+              bk.s0 += (size_t)a0 * bk.Tp;               // the tile's first agent
+              const BeWalk be = be_walk<STATS>(bk, tab.prm + a0, bev, soff(w.be_list), n_be, be_lo0, rcd_all, lane);
+              if (be.range) flags |= FO_F_BE_RANGE;
+              rcd_all = be.rcd;
+              btn_all = fmaxf(btn_all, rcd_all / veh.a_max);   // division is monotone: the maximum of the quotients
+              if (STATS && lane == 0) { st_be += n_be; st_probe += be.tests; st_node += be.nodes; st_path += be.chunks; }
+            }
+          } else {
+            // team shape: bisections dealt round-robin to the warps; a bisection stops as soon as its bracket lies
+            // below the running maximum (be_bisect), and a range error makes every further one moot
+            for (int q = wib; q < n_be && !(flags & FO_F_BE_RANGE); q += W) {
+              const int a = a0 + (int)w.be_list[q];
+              const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + a));
+              const float2 be = be_bisect<true>(bk, bev, a, pa.x, __int_as_float(pa.z), __int_as_float(pa.w), be_lo0,
+                                                lane, rcd_all);
+              const float rcd = be.x;
+              if (rcd != rcd) flags |= FO_F_BE_RANGE;    // NaN: the re-timed path overruns the planned one
+              rcd_all = fmaxf(rcd_all, rcd);
+              btn_all = fmaxf(btn_all, rcd / veh.a_max);
+              if (STATS && lane == 0) { st_be += 1; st_probe += (unsigned)__float_as_int(be.y); }
+            }
           }
         }
         __syncthreads();                               // list consumed before the next tile refills it
@@ -794,11 +805,12 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
     };
     const unsigned long long s6 = wsum(st_win), s7 = wsum(st_wkeep);
     const unsigned long long s0 = wsum(st_dense), s1 = wsum(st_obb), s2 = wsum(st_lr), s3 = wsum(st_cp);
-    st_be = wsum(st_be); st_probe = wsum(st_probe);
+    st_be = wsum(st_be); st_probe = wsum(st_probe); st_node = wsum(st_node); st_path = wsum(st_path);
     if (lane == 0) {
       atomicAdd(&k.stats[0], s0); atomicAdd(&k.stats[1], s1); atomicAdd(&k.stats[2], s2); atomicAdd(&k.stats[3], s3);
       atomicAdd(&k.stats[4], st_be); atomicAdd(&k.stats[5], st_probe);
       atomicAdd(&k.stats[6], s6); atomicAdd(&k.stats[7], s7);
+      atomicAdd(&k.stats[8], st_node); atomicAdd(&k.stats[9], st_path);
     }
   }
 }

@@ -309,8 +309,9 @@ class MetricEngine:
 
     def work_stats(self, ego) -> dict:
         """How much of the algorithmic work survives the exact bounds (``fo_metric_stats``): counts of visited
-        (trajectory, agent, step) evaluations, exact box distances, LR4S logits, CP evaluations, BE bisections and
-        probes for one pass over ``ego``.  Used by bench.py's flop model; synchronises."""
+        (trajectory, agent, step) evaluations, exact box distances, LR4S logits, CP evaluations, BE pairs and pair
+        tests (probes), BE tree nodes walked and re-timed ego-path chunks computed for one pass over ``ego``.  Used by
+        bench.py's flop model; synchronises."""
         t = self.to_device_bundle(ego)
         N = int(t.shape[0])
         dev = self.device
@@ -320,11 +321,11 @@ class MetricEngine:
                                torch.empty((N, L.FO_SUMMARY_K), dtype=torch.float32, device=dev),
                                torch.empty(N, dtype=torch.int32, device=dev))
             a = self._args(t, out)
-            cnt = torch.zeros(8, dtype=torch.int64, device=dev)
+            cnt = torch.zeros(10, dtype=torch.int64, device=dev)   # FO_STATS_K
             L.check(L.lib.fo_metric_stats(C.byref(a), C.c_void_p(cnt.data_ptr()), self._stream()), "fo_metric_stats")
             c = cnt.cpu().tolist()
         return {"visited": c[0], "obb": c[1], "lr4s": c[2], "cp": c[3], "be": c[4], "be_probes": c[5],
-                "windows": c[6], "windows_kept": c[7]}
+                "windows": c[6], "windows_kept": c[7], "be_nodes": c[8], "be_path_chunks": c[9]}
 
     def assess(self, ego, want_pair: bool = False, want_step: bool = False, out: Optional[BundleResult] = None
                ) -> BundleResult:

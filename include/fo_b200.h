@@ -154,10 +154,11 @@ int fo_metric_bundle(const FoMetricArgs *args, void *stream);
  * step must be NULL): how much of the algorithmic work survives the exact bounds.  bench.py uses them for the
  * flop model behind roofline.achieved.  counters_dev[FO_STATS_K] (device, zeroed by the call) =
  * { (trajectory, agent, step) evaluations visited, exact oriented-box distances, LR4S impact-angle logits,
- *   collision-probability evaluations (inside the 5 m gate), BE bisections, BE probes,
- *   (agent, 8-step window) items tested by the window filter, items it kept }  -- the last two are 0 when the bundle
- *   is small enough for the multi-warp team shape, which has no window filter. */
-#define FO_STATS_K 8
+ *   collision-probability evaluations (inside the 5 m gate), BE pairs, BE pair tests (the probes of one bisection
+ *   per pair), (agent, 8-step window) items tested by the window filter, items it kept, BE tree nodes walked, BE
+ *   re-timed ego-path chunks of 32 steps computed }  -- the window and tree counters are 0 when the bundle is small
+ *   enough for the multi-warp team shape, which has no window filter and bisects one BE pair at a time. */
+#define FO_STATS_K 10
 int fo_metric_stats(const FoMetricArgs *args, uint64_t *counters_dev, void *stream);
 
 /* Same computation driven from HOST buffers (pinned or pageable): copies ego / agents to the

@@ -22,6 +22,9 @@ print({k: v for k, v in st.items()}, "evals", evals)
 for k in ("obb", "lr4s", "cp"):
     print(k, "per visited evaluation:", st[k] / max(st["visited"], 1))
 print("be pairs per pair:", st["be"] / (n * a), "probes per be:", st["be_probes"] / max(st["be"], 1))
+# the BE tree walks (one per warp and agent tile with colliding pairs): nodes visited and re-timed ego-path chunks
+# computed, per trajectory -- scripts/be_tree_count.py gives the float64 count model of the same walk
+print("be tree nodes per trajectory:", st["be_nodes"] / n, "ego-path chunks per trajectory:", st["be_path_chunks"] / n)
 if st.get("windows"):
     print("window filter: kept", st["windows_kept"] / st["windows"], "of", st["windows"], "(agent, window) items;",
           "visited", st["visited"] / evals, "of the evaluations")

@@ -157,6 +157,10 @@ _PROTOS = {
     "fo_agents_pack": (C.c_int, [C.POINTER(FoAgentsRaw), C.POINTER(FoVehicle), C.c_void_p, C.c_size_t, C.c_void_p]),
     "fo_metric_bundle": (C.c_int, [C.POINTER(FoMetricArgs), C.c_void_p]),
     "fo_metric_stats": (C.c_int, [C.POINTER(FoMetricArgs), C.c_void_p, C.c_void_p]),
+    "fo_agent_table_bytes_corr": (C.c_size_t, [C.c_int32, C.c_int32]),
+    "fo_agents_pack_corr": (C.c_int, [C.POINTER(FoAgentsRaw), C.c_void_p, C.POINTER(FoVehicle), C.c_void_p, C.c_size_t,
+                                      C.c_void_p]),
+    "fo_metric_bundle_corr": (C.c_int, [C.POINTER(FoMetricArgs), C.c_void_p]),
     "fo_metric_bundle_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(FoAgentsRaw),
                                         C.POINTER(FoMetricArgs), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_void_p]),

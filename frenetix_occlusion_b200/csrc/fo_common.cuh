@@ -100,4 +100,14 @@ __host__ __device__ inline AgentTableView agent_table_view(const void* base, int
   return v;
 }
 
+// Correlated tables (fo_agents_pack_corr): the table above, then, 16-byte aligned, one more agent-major section
+//   s3[i] = (1/sigma_x, 1/sigma_y, rho, 0) of covariance i-1, slot order (rho NaN when the covariance is not positive definite)
+__host__ __device__ inline size_t agent_corr_offset(int A, int Tp) { return (agent_table_bytes(A, Tp) + 15) & ~(size_t)15; }
+__host__ __device__ inline size_t agent_table_bytes_corr(int A, int Tp) {
+  return agent_corr_offset(A, Tp) + (size_t)A * Tp * sizeof(float4);
+}
+__host__ __device__ inline const float4* agent_corr_view(const void* base, int A, int Tp) {
+  return reinterpret_cast<const float4*>(reinterpret_cast<const unsigned char*>(base) + agent_corr_offset(A, Tp));
+}
+
 }  // namespace fo

@@ -156,6 +156,30 @@ static void launch_pack(const FoAgentsRaw& raw, const PackProblem& one, const Pa
   fo_agents_pack_kernel<<<grid, 256, 0, st>>>(raw, one, many, P, arena);
 }
 
+// The s3 section of a correlated table (fo_agents_pack_corr), one thread per (agent, state), after the two launches of
+// launch_pack (it reads their slot map): (1/sigma_x, 1/sigma_y, rho) of covariance i-1 in float64, then rounded.  The
+// zero rule of the diagonal pack applies to the all-zero matrix; a covariance that is not positive definite gets
+// rho = NaN (|rho| >= 1, a zero variance with a non-zero covariance: +-inf / NaN here), so its CP values are NaN.
+__global__ void fo_agents_corr_kernel(FoAgentsRaw raw, const float* __restrict__ cov_xy, int A, int Tp,
+                                      unsigned char* table) {
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= A * Tp) return;
+  const int a = idx / Tp, i = idx - a * Tp;
+  const int32_t* slot = agent_table_view(table, A, Tp).slot;
+  float4 o = make_float4(1, 1, 0, 0);
+  if (i < raw.n_states[a]) {
+    const size_t r = (size_t)a * raw.t_stride + i, ip = i > 0 ? r - 1 : r;
+    float vx = raw.var_x[ip], vy = raw.var_y[ip];
+    const float c = cov_xy[ip];
+    if (vx == 0.0f && vy == 0.0f && c == 0.0f) { vx = 0.1f; vy = 0.1f; }   // collision_probability.py:85-87
+    const double sx = sqrt((double)vx), sy = sqrt((double)vy);
+    double rho = (double)c / (sx * sy);
+    if (!(fabs(rho) < 1.0)) rho = CUDART_NAN;
+    o = make_float4((float)(1.0 / sx), (float)(1.0 / sy), (float)rho, 0.0f);
+  }
+  const_cast<float4*>(agent_corr_view(table, A, Tp))[(size_t)slot[a] * Tp + i] = o;
+}
+
 // ---------------------------------------------------------------------------------------------
 // fo_metric_batch_host's ego ingest: float64 rows in the caller's world frame -> the float32 bundle of the metric kernels.
 // x and y lose their problem's origin in float64 and are rounded once; theta, v and a are rounded.  The operations are
@@ -298,6 +322,32 @@ extern "C" int fo_agents_pack(const FoAgentsRaw* raw, const FoVehicle* vehicle, 
   const fo::PackProblem one{0, A, Tp, vehicle->mass, 0};
   fo::launch_pack(*raw, one, nullptr, 1, fo::agent_pad(A) * Tp, (unsigned char*)table_dev, (cudaStream_t)stream);
   fo::count_launch(2);
+  FO_CUDA_TRY(cudaGetLastError());
+  return FO_OK;
+}
+
+extern "C" size_t fo_agent_table_bytes_corr(int32_t n_agents, int32_t t_stride) {
+  if (n_agents < 0 || t_stride < 0) return 0;
+  return fo::agent_table_bytes_corr(n_agents, t_stride);
+}
+
+extern "C" int fo_agents_pack_corr(const FoAgentsRaw* raw, const float* cov_xy, const FoVehicle* vehicle, void* table_dev,
+                                   size_t table_bytes, void* stream) {
+  const char* fn = "fo_agents_pack_corr";
+  if (!raw || !vehicle || !cov_xy) { fo::set_error("%s: NULL argument", fn); return FO_ERR_INVALID_ARG; }
+  const int A = raw->n_agents, Tp = raw->t_stride;
+  if (A < 0 || Tp < 0) { fo::set_error("%s: negative size", fn); return FO_ERR_INVALID_ARG; }
+  if (A == 0 || Tp == 0) return FO_OK;
+  if (Tp > FO_MAX_STATES) { fo::set_error("%s: t_stride %d > FO_MAX_STATES", fn, Tp); return FO_ERR_UNSUPPORTED; }
+  if (!table_dev || table_bytes < fo::agent_table_bytes_corr(A, Tp)) {
+    fo::set_error("%s: table buffer too small (%zu < %zu)", fn, table_bytes, fo::agent_table_bytes_corr(A, Tp));
+    return FO_ERR_INVALID_ARG;
+  }
+  const int rc = fo_agents_pack(raw, vehicle, table_dev, table_bytes, stream);   // the diagonal table, byte for byte
+  if (rc != FO_OK) return rc;
+  fo::fo_agents_corr_kernel<<<(A * Tp + 255) / 256, 256, 0, (cudaStream_t)stream>>>(*raw, cov_xy, A, Tp,
+                                                                                   (unsigned char*)table_dev);
+  fo::count_launch();
   FO_CUDA_TRY(cudaGetLastError());
   return FO_OK;
 }
@@ -446,11 +496,17 @@ static void fill_kargs(const FoMetricArgs* a, fo::MetricKArgs& k) {
   k.claim = nullptr;
   k.n_peers = 0;
   for (int p = 0; p < FO_MAX_PEERS; ++p) k.peer_delta[p] = 0;
+  k.corr = false;
 }
 
-static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, void* stream);
+static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, void* stream, bool corr = false);
 
 extern "C" int fo_metric_bundle(const FoMetricArgs* a, void* stream) { return metric_bundle_impl(a, nullptr, stream); }
+
+extern "C" int fo_metric_bundle_corr(const FoMetricArgs* a, void* stream) {
+  if (a && a->n_peers != 0) { fo::set_error("fo_metric_bundle_corr: no peer stores on correlated tables"); return FO_ERR_UNSUPPORTED; }
+  return metric_bundle_impl(a, nullptr, stream, true);
+}
 
 extern "C" int fo_metric_stats(const FoMetricArgs* a, uint64_t* counters_dev, void* stream) {
   if (!counters_dev) { fo::set_error("fo_metric_stats: counters_dev must not be NULL"); return FO_ERR_INVALID_ARG; }
@@ -459,7 +515,7 @@ extern "C" int fo_metric_stats(const FoMetricArgs* a, uint64_t* counters_dev, vo
   return metric_bundle_impl(a, reinterpret_cast<unsigned long long*>(counters_dev), stream);
 }
 
-static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, void* stream) {
+static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, void* stream, bool corr) {
   if (!a) { fo::set_error("fo_metric_bundle: NULL args"); return FO_ERR_INVALID_ARG; }
   if (a->n_traj < 0 || a->n_states < 0 || a->n_agents < 0) { fo::set_error("fo_metric_bundle: negative size"); return FO_ERR_INVALID_ARG; }
   if (a->n_traj == 0) return FO_OK;
@@ -486,6 +542,7 @@ static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, 
   if (a->n_peers > 0 && (a->pair || a->step || stats)) { fo::set_error("fo_metric_bundle: peer stores exist on the summary path only"); return FO_ERR_UNSUPPORTED; }
   k.n_peers = a->n_peers;
   for (int p = 0; p < FO_MAX_PEERS; ++p) k.peer_delta[p] = p < a->n_peers ? (long long)a->peer_delta[p] : 0;
+  k.corr = corr;
 
   cudaStream_t st = (cudaStream_t)stream;
   if (k.pair || k.step) return fo::launch_metric_detail(k, g_num_sms, st);

@@ -138,7 +138,9 @@ static __device__ __noinline__ void dt_drain_ties_batch(const float4* t0, const 
 // MASK != 0: the activated metrics are a compile-time constant (all seven / the default six); 0 = read k.mmask.
 // BATCH: every trajectory takes its agent table, agent count, pair / step blocks and ego vehicle from its problem (bv);
 // otherwise from k, whose fields then stay kernel-parameter operands.
-template <uint32_t MASK, bool BATCH>
+// CORR: correlated table (fo_metric_bundle_corr): every CP term is the float64 rectangle mass of the full covariance
+// (cp_bvn_boxes, the table's s3 section).
+template <uint32_t MASK, bool BATCH, bool CORR = false>
 __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailView& bv) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -160,6 +162,7 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
   const auto soff = [&](const void* q) { return (uint32_t)(reinterpret_cast<const unsigned char*>(q) - smem_raw); };
   const BeView bev{soff(egoA), soff(egoB), soff(dist), soff(inv), 0u};
   const BeConst bek = be_const(k);                // batched: the table and its stride are set per bisection
+  const float4* const s3 = CORR ? agent_corr_view(k.tab.s0, k.A, k.Tp) : nullptr;
   // batched: the warp's copy of its problem's descriptor, behind the per-warp regions (read where used, not held in
   // registers across the trajectory)
   DetailProb* const sdp = reinterpret_cast<DetailProb*>(smem_raw + kDtWarps * detail_warp_bytes(T)) + wib;
@@ -327,10 +330,16 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
           const size_t idx = (size_t)as * Tp + ii;
           const float4 s0i = __ldg(&tab.s0[idx]);
           const float4 s1i = __ldg(&tab.s1[idx]);
-          const float2 s2i = __ldg(&tab.s2[idx]);
           const float4 Ei = egoA[ii];
-          const float cp = cp_gauss_boxes<false>(s1i.z - Ei.x, s1i.w - Ei.y, Q.hlb * s0i.z, Q.hlb * s0i.w, veh.L3 * Ei.z,
-                                          veh.L3 * Ei.w, s2i, veh.L6, veh.W2);
+          float cp;
+          if constexpr (CORR) {
+            cp = cp_bvn_boxes(s1i.z - Ei.x, s1i.w - Ei.y, Q.hlb * s0i.z, Q.hlb * s0i.w, veh.L3 * Ei.z, veh.L3 * Ei.w,
+                              __ldg(&s3[idx]), veh.L6, veh.W2);
+          } else {
+            const float2 s2i = __ldg(&tab.s2[idx]);
+            cp = cp_gauss_boxes<false>(s1i.z - Ei.x, s1i.w - Ei.y, Q.hlb * s0i.z, Q.hlb * s0i.w, veh.L3 * Ei.z,
+                                       veh.L3 * Ei.w, s2i, veh.L6, veh.W2);
+          }
           // where the step loop put state t: still in the staging tile, or already in HBM (L2)
           const bool staged = t >= c0;
           float* const srow = stage + ial * kDtRow + 3 * (t - c0);
@@ -567,6 +576,11 @@ __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_ke
   detail_body<MASK, false>(k, DetailView{});
 }
 
+// Correlated tables (fo_metric_bundle_corr), runtime metric mask.
+__global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB) fo_metric_detail_corr_kernel(const __grid_constant__ MetricKArgs k) {
+  detail_body<0u, false, true>(k, DetailView{});
+}
+
 // A batch of independent problems (fo_metric_batch_detail): k.N = all rows of the batch, k.tab / k.A / k.Tp / k.pair /
 // k.step / k.veh are unused -- every trajectory takes them from its problem.
 template <uint32_t MASK>
@@ -616,6 +630,7 @@ int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st) {
     set_error("fo_metric_bundle: step must be 4-byte aligned");
     return FO_ERR_INVALID_ARG;
   }
+  if (k.corr) return launch_detail_kernel<fo_metric_detail_corr_kernel>(k, num_sms, 0, st);
   if (k.mmask == kDtAll) return launch_detail_kernel<fo_metric_detail_kernel<kDtAll>>(k, num_sms, 0, st);
   if (k.mmask == kDtDefault) return launch_detail_kernel<fo_metric_detail_kernel<kDtDefault>>(k, num_sms, 0, st);
   return launch_detail_kernel<fo_metric_detail_kernel<0u>>(k, num_sms, 0, st);

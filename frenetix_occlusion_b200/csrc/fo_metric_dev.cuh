@@ -34,6 +34,8 @@ struct MetricKArgs {
   //   ttc < thr_ttc   <=>  first colliding step < thr_ttc_col  (np.round(step * dt, 3), ttc.py:43, metric.py:85-89)
   uint32_t thr_dce_mm, thr_ttc_col;
   bool exact_dce;      // summary kernel: re-round np.round(d, 3) ties in float64 even when no threshold needs it (FO_EXACT_DCE=1)
+  bool corr;           // the table is a correlated one (fo_metric_bundle_corr): the CORR kernels read its s3 section
+                       // (agent_corr_view).  Sits in padding: MetricKArgs and every parameter offset keep their size / place.
   uint8_t* valid;
   float* summary;
   uint32_t* flags;
@@ -258,6 +260,110 @@ __device__ __forceinline__ float cp_gauss_boxes(float mx, float my, float hx, fl
     fm = (m == 0) ? 1.0f : -1.0f;
   }
   return prob * (1.0f / 3.0f);
+}
+
+// ---- collision probability with a full 2x2 covariance (fo_metric_bundle_corr) ---------------------------------------
+// Gauss-Legendre nodes (negative half) and weights of orders 6, 12 and 20, at offsets 0, 3 and 9.
+static __constant__ double kBvnX[19] = {
+    -0.9324695142031519, -0.6612093864662645, -0.2386191860831969,
+    -0.9815606342467192, -0.9041172563704748, -0.7699026741943047, -0.5873179542866175, -0.3678314989981802,
+    -0.1252334085114689,
+    -0.993128599185095, -0.9639719272779138, -0.912234428251326, -0.8391169718222188, -0.7463319064601508,
+    -0.636053680726515, -0.5108670019508271, -0.37370608871541955, -0.22778585114164507, -0.07652652113349734};
+static __constant__ double kBvnW[19] = {
+    0.17132449237917027, 0.3607615730481387, 0.46791393457269104,
+    0.04717533638651141, 0.10693932599531907, 0.16007832854334642, 0.20316742672306573, 0.2334925365383546,
+    0.2491470458134027,
+    0.017614007139150893, 0.040601429800386446, 0.06267204833410879, 0.08327674157670471, 0.1019301198172407,
+    0.1181945319615186, 0.1316886384491769, 0.1420961093183824, 0.14917298647260424, 0.15275338713072628};
+
+// One out-of-line copy each of the float64 normal CDF and exp: bvn_upper evaluates them at seven and five sites.
+static __device__ __noinline__ double bvn_phi(double x) { return normcdf(x); }
+static __device__ __noinline__ double bvn_exp(double x) { return exp(x); }
+
+// P(X > h, Y > k) of a standard bivariate normal with correlation r, |r| < 1: Genz's BVNU (Drezner-Wesolowsky with
+// 6 / 12 / 20-point Gauss-Legendre by |r|, and the expansion around |r| = 1 above 0.925), float64.
+__device__ __forceinline__ double bvn_upper(double h, double k, double r) {
+  constexpr double kTwoPi = 6.283185307179586;
+  const double ar = fabs(r);
+  const int g0 = ar < 0.3 ? 0 : (ar < 0.75 ? 3 : 9), lg = ar < 0.3 ? 3 : (ar < 0.75 ? 6 : 10);
+  double hk = h * k, bvn = 0.0;
+  if (ar < 0.925) {
+    // sinpi: the argument is at most pi/2, so sin's Payne-Hanek reduction (8 kB of code) is not needed
+    const double hs = 0.5 * (h * h + k * k), asr = asin(r), asr_pi = asr * (0.5 / CUDART_PI);
+#pragma unroll 1
+    for (int i = 0; i < 2 * lg; ++i) {
+      const double x = (i & 1) ? -kBvnX[g0 + (i >> 1)] : kBvnX[g0 + (i >> 1)];
+      const double sn = sinpi(asr_pi * (x + 1.0));
+      bvn += kBvnW[g0 + (i >> 1)] * bvn_exp((sn * hk - hs) / (1.0 - sn * sn));
+    }
+    return bvn * asr / (2.0 * kTwoPi) + bvn_phi(-h) * bvn_phi(-k);
+  }
+  if (r < 0.0) { k = -k; hk = -hk; }
+  const double as = (1.0 - r) * (1.0 + r);
+  double a = sqrt(as);
+  const double bs = (h - k) * (h - k), c = (4.0 - hk) / 8.0, d = (12.0 - hk) / 16.0;
+  bvn = a * bvn_exp(-0.5 * (bs / as + hk)) * (1.0 - c * (bs - as) * (1.0 - d * bs / 5.0) / 3.0 + c * d * as * as / 5.0);
+  if (hk > -160.0) {
+    const double b = sqrt(bs);
+    bvn -= bvn_exp(-0.5 * hk) * sqrt(kTwoPi) * bvn_phi(-b / a) * b * (1.0 - c * bs * (1.0 - d * bs / 5.0) / 3.0);
+  }
+  a *= 0.5;
+#pragma unroll 1
+  for (int i = 0; i < 2 * lg; ++i) {
+    const double x = (i & 1) ? -kBvnX[g0 + (i >> 1)] : kBvnX[g0 + (i >> 1)];
+    const double xs = (a * (x + 1.0)) * (a * (x + 1.0)), rs = sqrt(1.0 - xs);
+    bvn += a * kBvnW[g0 + (i >> 1)] *
+           (bvn_exp(-bs / (2.0 * xs) - hk / (1.0 + rs)) / rs - bvn_exp(-0.5 * (bs / xs + hk)) * (1.0 + c * xs * (1.0 + d * xs)));
+  }
+  bvn = -bvn / kTwoPi;
+  if (r > 0.0) return bvn + bvn_phi(-fmax(h, k));
+  bvn = -bvn;
+  if (k > h) bvn += h < 0.0 ? bvn_phi(k) - bvn_phi(h) : bvn_phi(-h) - bvn_phi(-k);
+  return bvn;
+}
+
+// Mass of a standard bivariate normal with correlation r over [a1, b1] x [a2, b2] (a < b), float64.  The four corners
+// are combined on the tails: a coordinate whose interval lies mostly below the mean is reflected (r changes sign), so a
+// box far from the mean is a difference of small upper-orthant masses and keeps its relative accuracy.  NaN unless
+// |r| < 1 (a covariance that is not positive definite).
+static __device__ __noinline__ double bvn_rect(double a1, double b1, double a2, double b2, double r) {
+  if (!(fabs(r) < 1.0)) return CUDART_NAN;
+  if (a1 + b1 < 0.0) { const double t = a1; a1 = -b1; b1 = -t; r = -r; }
+  if (a2 + b2 < 0.0) { const double t = a2; a2 = -b2; b2 = -t; r = -r; }
+  double p = 0.0;
+#pragma unroll 1
+  for (int q = 0; q < 4; ++q) {
+    const double u = bvn_upper((q & 1) ? b1 : a1, (q & 2) ? b2 : a2, r);
+    p += (q == 0 || q == 3) ? u : -u;
+  }
+  return p;
+}
+
+// cp_gauss_boxes with the correlated covariance s3 = (1/sigma_x, 1/sigma_y, rho, 0) of the state (fo_agents_pack_corr):
+// the same nine box x point terms and the same float32 box limits, each term the float64 rectangle mass.  No cut-off:
+// the 4.7-sigma rule of the diagonal path bounds each axis factor of a product, which a correlated mass is not.
+__device__ __forceinline__ float cp_bvn_boxes(float mx, float my, float hx, float hy, float bx, float by, float4 s3,
+                                              float L6, float W2) {
+  const double isx = s3.x, isy = s3.y;
+  double prob = 0.0;
+  float fm = 0.0f;                 // obstacle point: centre, front, back
+#pragma unroll 1
+  for (int m = 0; m < 3; ++m) {
+    const float uy = fmaf(fm, hy, my), ux = fmaf(fm, hx, mx);
+    float fb = 0.0f;               // ego box: middle, front, rear
+#pragma unroll 1
+    for (int bb = 0; bb < 3; ++bb) {
+      const float cyb = fb * by, cxb = fb * bx;
+      fb = (bb == 0) ? 1.0f : -1.0f;
+      prob += bvn_rect((double)(cxb - L6 - ux) * isx, (double)(cxb + L6 - ux) * isx, (double)(cyb - W2 - uy) * isy,
+                       (double)(cyb + W2 - uy) * isy, (double)s3.z);
+    }
+    fm = (m == 0) ? 1.0f : -1.0f;
+  }
+  // the inclusion-exclusion can leave -1e-20 where the mass is 0: the result is +0 there (the summary kernel's maximum
+  // compares bit patterns), and a NaN (not positive definite) stays NaN
+  return (float)(prob > 0.0 ? prob / 3.0 : (prob == prob ? 0.0 : prob));
 }
 
 __device__ __forceinline__ float logistic_neg(float z) {  // 1 / (1 + exp(z))

@@ -131,6 +131,8 @@ __device__ __forceinline__ float ord2f(uint32_t u) {
   return __uint_as_float(u ^ ((u >> 31) ? 0x80000000u : 0xffffffffu));
 }
 __device__ __forceinline__ float warp_max_signed(float v) { return ord2f(__reduce_max_sync(kFull, f2ord(v))); }
+// maximum of values >= 0 or NaN that keeps a NaN (bit order: every NaN above +inf); umaxf is its warp form
+__device__ __forceinline__ float nan_maxf(float a, float b) { return __uint_as_float(max(__float_as_uint(a), __float_as_uint(b))); }
 
 __device__ __forceinline__ float sw_sigmoid(float z) { return rcp_approx(1.0f + __expf(-z)); }   // 1 + exp >= 1: same bits as __fdividef(1, .)
 
@@ -222,8 +224,11 @@ struct SweepShape {
 // items, no pooled leftovers (see the header comment).
 // BATCH: every trajectory takes its agent table, agent count, lane grouping and ego vehicle from its problem (bv);
 // otherwise from k.
+// CORR: the table is a correlated one (fo_agents_pack_corr): the CP drain evaluates the nine rectangle masses of the
+// full covariance (cp_bvn_boxes, the table's s3 section) instead of cp_gauss_boxes; a NaN CP (a covariance that is not
+// positive definite) is carried into max_collision_probability_all.
 // tid / block_dim are read in the __global__ function, where the compiler knows their range from the launch bounds.
-template <uint32_t MASK, bool STATS, bool UNI, bool TIES, bool BATCH>
+template <uint32_t MASK, bool STATS, bool UNI, bool TIES, bool BATCH, bool CORR = false>
 __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShape shape, const BatchView& bv,
                                            const int tid, const int block_dim) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -245,6 +250,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
   int Ap = k.tab.Ap;
   const auto soff = [&](const void* q) { return (uint32_t)(reinterpret_cast<const unsigned char*>(q) - smem_raw); };
   const BeView bev{soff(w.egoA), soff(w.egoB), soff(w.dist), soff(w.inv), soff(w.seg)};
+  const float4* const s3 = CORR ? agent_corr_view(k.tab.s0, k.A, k.Tp) : nullptr;
   BeConst bek = be_const(k);                       // batched: the table and its stride are set per trajectory
   // lane -> (agent within the lane group, time slice); every (warp, slice) owns a contiguous range of steps
   const int lg = shape.lg_agents;
@@ -448,11 +454,18 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           const size_t idx = (size_t)a * Tp + ii;
           const float4 s0i = __ldg(&tab.s0[idx]);
           const float4 s1i = __ldg(&tab.s1[idx]);
-          const float2 s2i = __ldg(&tab.s2[idx]);
           const float4 Ei = w.egoA[ii];
-          const float cp = cp_gauss_boxes(s1i.z - Ei.x, s1i.w - Ei.y, P.hlb * s0i.z, P.hlb * s0i.w, veh.L3 * Ei.z,
-                                          veh.L3 * Ei.w, s2i, veh.L6, veh.W2);
-          acc_cp = fmaxf(acc_cp, cp);
+          float cp;
+          if constexpr (CORR) {
+            cp = cp_bvn_boxes(s1i.z - Ei.x, s1i.w - Ei.y, P.hlb * s0i.z, P.hlb * s0i.w, veh.L3 * Ei.z, veh.L3 * Ei.w,
+                              __ldg(&s3[idx]), veh.L6, veh.W2);
+            acc_cp = nan_maxf(acc_cp, cp);
+          } else {
+            const float2 s2i = __ldg(&tab.s2[idx]);
+            cp = cp_gauss_boxes(s1i.z - Ei.x, s1i.w - Ei.y, P.hlb * s0i.z, P.hlb * s0i.w, veh.L3 * Ei.z, veh.L3 * Ei.w,
+                                s2i, veh.L6, veh.W2);
+            acc_cp = fmaxf(acc_cp, cp);
+          }
           if (do_hr) {                       // risk[t] = harm[t] * cp[t], cp[t] = CP of step t+1 (hr.py:78-79)
             const float4 s0t = __ldg(&tab.s0[idx - 1]);
             const float4 s1t = __ldg(&tab.s1[idx - 1]);
@@ -757,7 +770,8 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
       uint32_t rmin_t = 0xffffffu, col = 0xffffffffu, fl = 0u;
       for (int q = 0; q < W; ++q) {
         const float* r = w.red + q * 16;
-        er = fmaxf(er, r[0]); orr = fmaxf(orr, r[1]); cpm = fmaxf(cpm, r[2]); hwc_all = fmaxf(hwc_all, r[3]);
+        er = fmaxf(er, r[0]); orr = fmaxf(orr, r[1]); cpm = CORR ? nan_maxf(cpm, r[2]) : fmaxf(cpm, r[2]);
+        hwc_all = fmaxf(hwc_all, r[3]);
         ze = fmaxf(ze, r[4]); zo = fmaxf(zo, r[5]);
         rmin_t = min(rmin_t, __float_as_uint(r[6])); col = min(col, __float_as_uint(r[7])); fl |= __float_as_uint(r[8]);
         btn = fmaxf(btn, r[9]); rcd = fmaxf(rcd, r[10]);
@@ -819,6 +833,13 @@ template <uint32_t MASK, bool STATS, bool UNI, bool TIES>
 __global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
 fo_metric_sweep_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape) {
   sweep_body<MASK, STATS, UNI, TIES, false>(k, shape, BatchView{}, threadIdx.x, blockDim.x);
+}
+
+// Correlated tables (fo_metric_bundle_corr): the runtime metric mask, both shapes, with and without the tie path.
+template <bool UNI, bool TIES>
+__global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
+fo_metric_sweep_corr_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape) {
+  sweep_body<0u, false, UNI, TIES, false, true>(k, shape, BatchView{}, threadIdx.x, blockDim.x);
 }
 
 // One shape class of a batch of independent problems (fo_metric_batch): k.N is the class's trajectory count, k.tab / k.A
@@ -940,6 +961,17 @@ constexpr uint32_t kAllMetrics = FO_M_CP | FO_M_DCE | FO_M_TTC | FO_M_HR | FO_M_
 constexpr uint32_t kDefaultMetrics = kAllMetrics & ~FO_M_BE;   // occlusion.yaml:12-18
 
 int launch_metric_sweep(const MetricKArgs& k, int num_sms, cudaStream_t st) {
+  if (k.corr) {
+    int W = 1;
+    SweepShape shape;
+    pick_shape(k, num_sms, W, shape);
+    const bool ties = needs_ties(k);
+    const bool uni = W == 1 && shape.lg_agents == 5;
+    if (uni) return ties ? launch_team_kernel<fo_metric_sweep_corr_kernel<true, true>>(k, num_sms, W, uni, ties, st, shape)
+                         : launch_team_kernel<fo_metric_sweep_corr_kernel<true, false>>(k, num_sms, W, uni, ties, st, shape);
+    return ties ? launch_team_kernel<fo_metric_sweep_corr_kernel<false, true>>(k, num_sms, W, uni, ties, st, shape)
+                : launch_team_kernel<fo_metric_sweep_corr_kernel<false, false>>(k, num_sms, W, uni, ties, st, shape);
+  }
   if (k.stats) return launch_sweep_inst<0u, true>(k, num_sms, st);
   if (k.mmask == kAllMetrics) return launch_sweep_inst<kAllMetrics, false>(k, num_sms, st);
   if (k.mmask == kDefaultMetrics) return launch_sweep_inst<kDefaultMetrics, false>(k, num_sms, st);

@@ -75,6 +75,8 @@ class AgentSet:
     buf_length: np.ndarray
     buf_width: np.ndarray
     agent_types: list = field(default_factory=list)
+    # off-diagonal term of every covariance [A, t_stride], aligned with var_x / var_y; None = all diagonal
+    cov_xy: Optional[np.ndarray] = None
 
     @property
     def n_agents(self) -> int:
@@ -95,6 +97,7 @@ class AgentSet:
         A = len(agents)
         Tp = max([len(np.asarray(a["yaw"])) for a in agents], default=0)
         x, y, yaw, v, vx, vy = cls._alloc(A, Tp)
+        cxy = np.zeros((A, Tp), dtype=np.float64)
         ns = np.zeros(A, dtype=np.int32)
         kind = np.zeros(A, dtype=np.int32)
         dims = np.zeros((4, A), dtype=np.float64)
@@ -107,15 +110,22 @@ class AgentSet:
             yaw[k, :n], v[k, :n] = a["yaw"], a["v"]
             if "cov" in a:
                 cov = np.asarray(a["cov"], dtype=np.float64)
-                if np.any(cov[:, 0, 1] != 0) or np.any(cov[:, 1, 0] != 0):
-                    raise ValueError("only diagonal prediction covariances are supported on the GPU path")
-                vx[k, :n], vy[k, :n] = cov[:, 0, 0], cov[:, 1, 1]
+                c01, c10, c00, c11 = cov[:, 0, 1], cov[:, 1, 0], cov[:, 0, 0], cov[:, 1, 1]
+                if np.any(c01 != c10):
+                    raise ValueError(f"agent {k}: prediction covariance is not symmetric")
+                # positive definite where there is a correlation (scipy's mvn raises otherwise); diagonal states keep
+                # the rules of the diagonal path (an all-zero matrix is 0.1 I)
+                bad = (c01 != 0) & ~((c00 > 0) & (c11 > 0) & (c01 * c01 < c00 * c11))
+                if np.any(bad):
+                    raise ValueError(f"agent {k}: prediction covariance of state {int(np.argmax(bad))} is not positive definite")
+                vx[k, :n], vy[k, :n], cxy[k, :n] = c00, c11, c01
             else:
                 vx[k, :n] = vy[k, :n] = a["var"]
             kind[k] = L.KINDS[a["agent_type"].lower()]
             types.append(a["agent_type"])
             dims[:, k] = (a["length"], a["width"], a["buf_length"], a["buf_width"])
-        return cls(list(range(A)), x, y, yaw, v, vx, vy, ns, kind, dims[0], dims[1], dims[2], dims[3], types)
+        return cls(list(range(A)), x, y, yaw, v, vx, vy, ns, kind, dims[0], dims[1], dims[2], dims[3], types,
+                   cxy if np.any(cxy != 0) else None)
 
     @classmethod
     def from_predictions(cls, predictions: dict, agent_by_prediction_id) -> "AgentSet":
@@ -203,6 +213,7 @@ class MetricEngine:
         self.origin = np.zeros(2)
         self.agents: Optional[AgentSet] = None
         self._table = None
+        self._corr = False            # the table is a correlated one (fo_agents_pack_corr / fo_metric_bundle_corr)
         self._raw_dev = None
         self.n_agents = 0
         self.t_stride = 0
@@ -229,6 +240,7 @@ class MetricEngine:
         A, Tp = agents.n_agents, agents.t_stride
         self.n_agents, self.t_stride = A, Tp
         self._table = None
+        self._corr = False
         self._pack_pending = False
         if A == 0 or Tp == 0:
             self.n_agents = 0
@@ -243,8 +255,9 @@ class MetricEngine:
             return
         self._pack_pending = False
         agents, A, Tp = self.agents, self.n_agents, self.t_stride
-        fl = np.stack([agents.x - self.origin[0], agents.y - self.origin[1], agents.yaw, agents.v,
-                       agents.var_x, agents.var_y]).astype(np.float32)
+        corr = agents.cov_xy is not None
+        rows = [agents.x - self.origin[0], agents.y - self.origin[1], agents.yaw, agents.v, agents.var_x, agents.var_y]
+        fl = np.stack(rows + ([agents.cov_xy] if corr else [])).astype(np.float32)
         pa = np.stack([agents.length, agents.width, agents.buf_length, agents.buf_width]).astype(np.float32)
         ia = np.stack([agents.n_states, agents.kind]).astype(np.int32)
         with torch.cuda.device(self.device):
@@ -256,10 +269,18 @@ class MetricEngine:
             raw.x, raw.y, raw.yaw, raw.v, raw.var_x, raw.var_y = [d_fl[i].data_ptr() for i in range(6)]
             raw.n_states, raw.kind = d_ia[0].data_ptr(), d_ia[1].data_ptr()
             raw.length, raw.width, raw.buf_length, raw.buf_width = [d_pa[i].data_ptr() for i in range(4)]
-            nbytes = L.lib.fo_agent_table_bytes(A, Tp)
-            self._table = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
-            L.check(L.lib.fo_agents_pack(C.byref(raw), C.byref(self.vehicle), C.c_void_p(self._table.data_ptr()),
-                                         nbytes, self._stream()), "fo_agents_pack")
+            if corr:
+                nbytes = L.lib.fo_agent_table_bytes_corr(A, Tp)
+                self._table = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+                L.check(L.lib.fo_agents_pack_corr(C.byref(raw), C.c_void_p(d_fl[6].data_ptr()), C.byref(self.vehicle),
+                                                  C.c_void_p(self._table.data_ptr()), nbytes, self._stream()),
+                        "fo_agents_pack_corr")
+            else:
+                nbytes = L.lib.fo_agent_table_bytes(A, Tp)
+                self._table = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+                L.check(L.lib.fo_agents_pack(C.byref(raw), C.byref(self.vehicle), C.c_void_p(self._table.data_ptr()),
+                                             nbytes, self._stream()), "fo_agents_pack")
+            self._corr = corr
             self._raw_dev = (d_fl, d_pa, d_ia)  # keep alive until the stream work is done
 
     # ------------------------------------------------------------------------------------------
@@ -311,7 +332,9 @@ class MetricEngine:
         """How much of the algorithmic work survives the exact bounds (``fo_metric_stats``): counts of visited
         (trajectory, agent, step) evaluations, exact box distances, LR4S logits, CP evaluations, BE pairs and pair
         tests (probes), BE tree nodes walked and re-timed ego-path chunks computed for one pass over ``ego``.  Used by
-        bench.py's flop model; synchronises."""
+        bench.py's flop model; synchronises.  Diagonal covariances only."""
+        if self.agents is not None and self.agents.cov_xy is not None and self.n_agents > 0:
+            raise ValueError("work_stats() takes diagonal prediction covariances only")
         t = self.to_device_bundle(ego)
         N = int(t.shape[0])
         dev = self.device
@@ -351,7 +374,8 @@ class MetricEngine:
             a = self._args(t, out)
             a.pair = out.pair.data_ptr() if (out.pair is not None and A > 0) else None
             a.step = out.step.data_ptr() if (out.step is not None and A > 0 and T > 1) else None
-            L.check(L.lib.fo_metric_bundle(C.byref(a), self._stream()), "fo_metric_bundle")
+            fn = "fo_metric_bundle_corr" if self._corr else "fo_metric_bundle"
+            L.check(getattr(L.lib, fn)(C.byref(a), self._stream()), fn)
         out._keepalive = t
         return out
 
@@ -383,8 +407,11 @@ class MetricEngine:
         (no shift).  ``vehicles``: P ego vehicle descriptions (each a dict or an object with attributes, as the
         constructor takes them), or None for the engine's own vehicle in every problem; ``assess_batch`` assesses
         problem p with vehicles[p].  Problem p's table equals what ``set_agents(agent_sets[p], origins[p])`` packs in an
-        engine built with vehicles[p]."""
+        engine built with vehicles[p].  Diagonal prediction covariances only (``AgentSet.cov_xy`` None)."""
         P = len(agent_sets)
+        if any(a.cov_xy is not None for a in agent_sets):
+            raise ValueError("batches take diagonal prediction covariances only; assess a correlated set with "
+                             "set_agents() + assess()")
         veh = None
         if vehicles is not None:
             if len(vehicles) != P:

@@ -55,7 +55,8 @@ class MetricCore:
             pos = np.ascontiguousarray(v.get("pos_list"), dtype=np.float64)
             items.append((k, pos.shape, hash(pos.tobytes()),
                           hash(np.ascontiguousarray(v.get("orientation_list"), dtype=np.float64).tobytes()),
-                          hash(np.ascontiguousarray(v.get("v_list"), dtype=np.float64).tobytes())))
+                          hash(np.ascontiguousarray(v.get("v_list"), dtype=np.float64).tobytes()),
+                          hash(np.ascontiguousarray(v.get("cov_list"), dtype=np.float64).tobytes())))
         return ("c", tuple(items))
 
     def sync_agents(self, origin=None):

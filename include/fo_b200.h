@@ -161,6 +161,25 @@ int fo_metric_bundle(const FoMetricArgs *args, void *stream);
 #define FO_STATS_K 10
 int fo_metric_stats(const FoMetricArgs *args, uint64_t *counters_dev, void *stream);
 
+/* Predictions with full 2x2 covariances [[var_x, cov_xy], [cov_xy, var_y]] (a learned predictor's correlated ones):
+ * the collision probability of each gated step is the mass of N(mu, Sigma) with the full Sigma of covariance i-1 over
+ * each of the three ego boxes, per obstacle point, / 3 -- the reference's mvnun (collision_probability.py:94-122).
+ * Everything else (5 m gate, index offsets, ego boxes, the all-zero matrix -> 0.1 I rule) is as on the diagonal path.
+ *
+ * fo_agent_table_bytes_corr: fo_agent_table_bytes plus one appended per-(agent, state) section; the layout of the
+ * diagonal table in front of it is unchanged.
+ * fo_agents_pack_corr: `cov_xy` is a device array [A, t_stride] aligned with raw->var_x / var_y.  Writes what
+ * fo_agents_pack writes, byte for byte, plus the correlation section.  PRECONDITION: every covariance of a state the
+ * agent has is symmetric positive definite (or all zero); the device data is not inspected by the host, and a state
+ * that violates it (|rho| >= 1, a zero variance with a non-zero covariance) gets NaN collision probabilities.
+ * fo_metric_bundle_corr: fo_metric_bundle on a table written by fo_agents_pack_corr, with its outputs, checks and
+ * CUDA-graph capture behaviour.  Each CP term is a float64 bivariate-normal rectangle mass.  n_peers > 0 returns
+ * FO_ERR_UNSUPPORTED.  Batches, fo_metric_bundle_host and fo_metric_stats take diagonal tables only. */
+size_t fo_agent_table_bytes_corr(int32_t n_agents, int32_t t_stride);
+int fo_agents_pack_corr(const FoAgentsRaw *raw, const float *cov_xy, const FoVehicle *vehicle, void *table_dev,
+                        size_t table_bytes, void *stream);
+int fo_metric_bundle_corr(const FoMetricArgs *args, void *stream);
+
 /* Same computation driven from HOST buffers (pinned or pageable): copies ego / agents to the
  * device, runs fo_agents_pack + fo_metric_bundle, copies valid/summary/flags back and synchronises.
  * This is the call a non-torch embedder of the reference would make; device workspace is owned by

@@ -173,6 +173,12 @@ _PROTOS = {
                                                 C.POINTER(FoVehicle), C.c_void_p, C.c_size_t, C.c_void_p]),
     "fo_metric_batch_vehicles": (C.c_int, [C.POINTER(FoMetricBatchArgs), C.POINTER(FoVehicle), C.c_void_p]),
     "fo_metric_batch_detail_vehicles": (C.c_int, [C.POINTER(FoMetricBatchArgs), C.POINTER(FoVehicle), C.c_void_p]),
+    "fo_agent_batch_layout_corr": (C.c_size_t, [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fo_agents_pack_batch_corr": (C.c_int, [C.POINTER(FoAgentsRaw), C.c_void_p, C.c_int32, C.POINTER(FoBatchProblem),
+                                            C.c_void_p, C.POINTER(FoVehicle), C.c_void_p, C.c_size_t, C.c_void_p]),
+    "fo_metric_batch_corr": (C.c_int, [C.POINTER(FoMetricBatchArgs), C.c_void_p, C.POINTER(FoVehicle), C.c_void_p]),
+    "fo_metric_batch_detail_corr": (C.c_int, [C.POINTER(FoMetricBatchArgs), C.c_void_p, C.POINTER(FoVehicle),
+                                              C.c_void_p]),
     "fo_metric_batch_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(FoAgentsRaw), C.c_int32,
                                        C.POINTER(FoBatchProblem), C.POINTER(FoVehicle), C.POINTER(FoMetricArgs),
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

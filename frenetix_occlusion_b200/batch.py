@@ -4,7 +4,8 @@ A multi-agent simulation runs one planner and one ``FOInterface`` per vehicle; a
 many scenes side by side.  Instead of one ``assess_bundle`` per interface (an agent upload, two pack launches and a
 metric launch each), ``assess_interfaces`` packs the phantom agents of all interfaces with one
 ``fo_agents_pack_batch`` call and evaluates all candidate bundles with one ``fo_metric_batch`` (or, with pair / step
-detail, ``fo_metric_batch_detail``) call.  ``prefetch_interfaces`` does the same for the reference's per-trajectory
+detail, ``fo_metric_batch_detail``) call -- their ``_corr`` forms when some interface's predictions carry correlated
+covariances, which are then assessed as that interface assesses them.  ``prefetch_interfaces`` does the same for the reference's per-trajectory
 protocol: it is ``prefetch_assessments`` for all interfaces at once.
 """
 from __future__ import annotations
@@ -77,7 +78,8 @@ def assess_interfaces(interfaces: Sequence, bundles: Sequence, want_pair: bool =
     Each interface's phantom predictions (``agent_manager.predictions``) are taken with the origin rule of
     ``MetricCore.sync_agents`` (the first agent's first position); an interface without phantom agents assesses
     every trajectory as valid (``Metric.evaluate_metrics``).  Each interface is assessed with its own ego vehicle
-    (``vehicle_params``), so the vehicles of a mixed fleet share one batch.  The interfaces must agree on device, dt,
+    (``vehicle_params``), so the vehicles of a mixed fleet share one batch, and with its own predictions' covariances,
+    diagonal or correlated.  The interfaces must agree on device, dt,
     activated metrics, thresholds, harm coefficients and the trajectory length T, else ``ValueError``.  No interface's
     state, cache or prefetch is touched."""
     interfaces, bundles = list(interfaces), list(bundles)
@@ -88,13 +90,14 @@ def assess_interfaces(interfaces: Sequence, bundles: Sequence, want_pair: bool =
     egos = [_bundle_array(b) for b in bundles]
     eng = _batch_engine(interfaces, egos)
     agents = [_agents(fi) for fi in interfaces]
-    eng.set_agent_batch([a for a, _ in agents], [o for _, o in agents], vehicles=_vehicles(interfaces))
+    eng.set_agent_batch([a for a, _ in agents], [o for _, o in agents], vehicles=_vehicles(interfaces), correlated=True)
     return eng.assess_batch(egos, want_pair=want_pair, want_step=want_step).split()
 
 
 def prefetch_interfaces(interfaces: Sequence, candidates: Sequence) -> list:
     """``interfaces[i].prefetch_assessments(candidates[i])`` for every interface at once: one ``fo_agents_pack_batch``,
-    one ``fo_metric_batch_detail`` and one device-to-host copy of all results.  Afterwards
+    one ``fo_metric_batch_detail`` and one device-to-host copy of all results (with correlated predictions the ``_corr``
+    calls: a third pack launch, and one detail launch each for the diagonal and the correlated interfaces).  Afterwards
     ``interfaces[i].trajectory_safety_assessment(t)`` for every ``t`` in ``candidates[i]`` (trajectory objects with
     ``.cartesian.x / y / theta / v / a``) returns what it would after the interface's own prefetch, without a launch.
     Returns the per-interface counts ``prefetch_assessments`` returns (0 for an interface without phantom agents or
@@ -115,7 +118,7 @@ def prefetch_interfaces(interfaces: Sequence, candidates: Sequence) -> list:
         return counts
     agents = [_agents(interfaces[i]) for i in live]
     eng.set_agent_batch([a for a, _ in agents], [o for _, o in agents],
-                        vehicles=_vehicles([interfaces[i] for i in live]))
+                        vehicles=_vehicles([interfaces[i] for i in live]), correlated=True)
     n = np.array([len(e) for e in egos], dtype=np.int64)
     a = np.array([ag.n_agents if ag.t_stride > 0 else 0 for ag, _ in agents], dtype=np.int64)
     T = max([e.shape[1] for e in egos if len(e)], default=1)

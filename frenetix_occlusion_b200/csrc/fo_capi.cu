@@ -308,10 +308,10 @@ extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int3
   b.common.pair = b.common.step = nullptr;
   b.n_problems = P; b.problems = pr.data(); b.arena_bytes = arena_bytes;
   int n_run = 0, a_min = 0, n_packed = 0, max_cells = 0;
-  int rc = fo::check_batch(fn, &b, false, &n_run, &a_min);
+  int rc = fo::check_batch(fn, &b, nullptr, false, &n_run, &a_min);
   if (rc != FO_OK) return rc;
   const FoAgentsRaw no_agents{};
-  rc = fo::check_pack_batch(fn, P > 0 ? ag : &no_agents, P, pr.data(), stand_in, arena_bytes, &n_packed, &max_cells);
+  rc = fo::check_pack_batch(fn, P > 0 ? ag : &no_agents, P, pr.data(), nullptr, stand_in, arena_bytes, &n_packed, &max_cells);
   if (rc != FO_OK) return rc;
   if (n_traj == 0) return FO_OK;
 

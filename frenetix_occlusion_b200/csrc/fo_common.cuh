@@ -14,10 +14,11 @@ void count_launch(uint64_t n = 1);
 // Host-side argument checks of the batch entry points (fo_metric.cu), before any device work; fn names the entry point
 // in the messages.  check_batch: the metric calls (detail: fo_metric_batch_detail's outputs); on success *n_run = the
 // problems with trajectories and *a_min = the fewest agents among them.  check_pack_batch: fo_agents_pack_batch; on
-// success *n_packed = the problems with agents and *max_cells = the most table cells of one of them.
-int check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, int* n_run, int* a_min);
+// success *n_packed = the problems with agents and *max_cells = the most table cells of one of them.  corr: NULL = every
+// table is diagonal, else corr[p] != 0 = problem p's table is a correlated one (fo_agent_table_bytes_corr bytes).
+int check_batch(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, bool detail, int* n_run, int* a_min);
 int check_pack_batch(const char* fn, const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
-                     const void* arena_dev, size_t arena_bytes, int* n_packed, int* max_cells);
+                     const uint8_t* corr, const void* arena_dev, size_t arena_bytes, int* n_packed, int* max_cells);
 
 // fo_metric_batch_host's float64 -> float32 conversion of ego rows [row0, row0 + n_rows) of a batch ([rows, T, 5], src
 // and dst point at row row0): first_dev[n_first] = the first rows of the problems with trajectories (strictly

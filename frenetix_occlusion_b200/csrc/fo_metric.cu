@@ -160,24 +160,35 @@ static void launch_pack(const FoAgentsRaw& raw, const PackProblem& one, const Pa
 // launch_pack (it reads their slot map): (1/sigma_x, 1/sigma_y, rho) of covariance i-1 in float64, then rounded.  The
 // zero rule of the diagonal pack applies to the all-zero matrix; a covariance that is not positive definite gets
 // rho = NaN (|rho| >= 1, a zero variance with a non-zero covariance: +-inf / NaN here), so its CP values are NaN.
-__global__ void fo_agents_corr_kernel(FoAgentsRaw raw, const float* __restrict__ cov_xy, int A, int Tp,
-                                      unsigned char* table) {
+// Problems as in fo_agents_pack_kernel (blockIdx.y strides over them); fo_agents_pack_corr is the one-problem case.
+__global__ void fo_agents_corr_kernel(FoAgentsRaw raw, const float* __restrict__ cov_xy, PackProblem one,
+                                      const PackProblem* many, int P, unsigned char* arena) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= A * Tp) return;
-  const int a = idx / Tp, i = idx - a * Tp;
-  const int32_t* slot = agent_table_view(table, A, Tp).slot;
-  float4 o = make_float4(1, 1, 0, 0);
-  if (i < raw.n_states[a]) {
-    const size_t r = (size_t)a * raw.t_stride + i, ip = i > 0 ? r - 1 : r;
-    float vx = raw.var_x[ip], vy = raw.var_y[ip];
-    const float c = cov_xy[ip];
-    if (vx == 0.0f && vy == 0.0f && c == 0.0f) { vx = 0.1f; vy = 0.1f; }   // collision_probability.py:85-87
-    const double sx = sqrt((double)vx), sy = sqrt((double)vy);
-    double rho = (double)c / (sx * sy);
-    if (!(fabs(rho) < 1.0)) rho = CUDART_NAN;
-    o = make_float4((float)(1.0 / sx), (float)(1.0 / sy), (float)rho, 0.0f);
+  for (int p = blockIdx.y; p < P; p += gridDim.y) {
+    const PackProblem pp = many ? many[p] : one;
+    const int A = pp.A, Tp = pp.Tp;
+    if (idx >= A * Tp) continue;
+    const int a = idx / Tp, i = idx - a * Tp;
+    unsigned char* const table = arena + pp.table_off;
+    const int32_t* slot = agent_table_view(table, A, Tp).slot;
+    float4 o = make_float4(1, 1, 0, 0);
+    if (i < raw.n_states[pp.a_begin + a]) {
+      const size_t r = ((size_t)pp.a_begin + a) * raw.t_stride + i, ip = i > 0 ? r - 1 : r;
+      float vx = raw.var_x[ip], vy = raw.var_y[ip];
+      const float c = cov_xy[ip];
+      if (vx == 0.0f && vy == 0.0f && c == 0.0f) { vx = 0.1f; vy = 0.1f; }   // collision_probability.py:85-87
+      const double sx = sqrt((double)vx), sy = sqrt((double)vy);
+      double rho = (double)c / (sx * sy);
+      if (!(fabs(rho) < 1.0)) rho = CUDART_NAN;
+      o = make_float4((float)(1.0 / sx), (float)(1.0 / sy), (float)rho, 0.0f);
+    }
+    const_cast<float4*>(agent_corr_view(table, A, Tp))[(size_t)slot[a] * Tp + i] = o;
   }
-  const_cast<float4*>(agent_corr_view(table, A, Tp))[(size_t)slot[a] * Tp + i] = o;
+}
+static void launch_corr(const FoAgentsRaw& raw, const float* cov_xy, const PackProblem& one, const PackProblem* many,
+                        int P, int max_cells, unsigned char* arena, cudaStream_t st) {
+  const dim3 grid((max_cells + 255) / 256, P < 65535 ? P : 65535);
+  fo_agents_corr_kernel<<<grid, 256, 0, st>>>(raw, cov_xy, one, many, P, arena);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -283,13 +294,15 @@ static int stage_upload(StageSlot* s, size_t bytes, cudaStream_t st) {
   return FO_OK;
 }
 
-// Checks the table of one problem against the arena (A > 0): stride range, 16-byte alignment, bounds.
-static int check_table(const char* fn, int p, int A, int Tp, int64_t off, size_t arena_bytes) {
+// Checks the table of one problem against the arena (A > 0): stride range, 16-byte alignment, bounds (of a correlated
+// table when corr).
+static int check_table(const char* fn, int p, int A, int Tp, int64_t off, size_t arena_bytes, bool corr) {
   if (Tp < 1) { set_error("%s: problem %d has agents but t_stride %d", fn, p, Tp); return FO_ERR_INVALID_ARG; }
   if (Tp > FO_MAX_STATES) { set_error("%s: problem %d t_stride %d > FO_MAX_STATES", fn, p, Tp); return FO_ERR_UNSUPPORTED; }
-  if (off < 0 || (off & 15) || (size_t)off > arena_bytes || arena_bytes - (size_t)off < agent_table_bytes(A, Tp)) {
-    set_error("%s: table of problem %d (offset %lld, %zu bytes) misaligned or outside the arena (%zu bytes)", fn, p,
-              (long long)off, agent_table_bytes(A, Tp), arena_bytes);
+  const size_t need = corr ? agent_table_bytes_corr(A, Tp) : agent_table_bytes(A, Tp);
+  if (off < 0 || (off & 15) || (size_t)off > arena_bytes || arena_bytes - (size_t)off < need) {
+    set_error("%s: %stable of problem %d (offset %lld, %zu bytes) misaligned or outside the arena (%zu bytes)", fn,
+              corr ? "correlated " : "", p, (long long)off, need, arena_bytes);
     return FO_ERR_INVALID_ARG;
   }
   return FO_OK;
@@ -345,34 +358,49 @@ extern "C" int fo_agents_pack_corr(const FoAgentsRaw* raw, const float* cov_xy, 
   }
   const int rc = fo_agents_pack(raw, vehicle, table_dev, table_bytes, stream);   // the diagonal table, byte for byte
   if (rc != FO_OK) return rc;
-  fo::fo_agents_corr_kernel<<<(A * Tp + 255) / 256, 256, 0, (cudaStream_t)stream>>>(*raw, cov_xy, A, Tp,
-                                                                                   (unsigned char*)table_dev);
+  fo::launch_corr(*raw, cov_xy, fo::PackProblem{0, A, Tp, vehicle->mass, 0}, nullptr, 1, A * Tp, (unsigned char*)table_dev,
+                  (cudaStream_t)stream);
   fo::count_launch();
   FO_CUDA_TRY(cudaGetLastError());
   return FO_OK;
 }
 
-extern "C" size_t fo_agent_batch_layout(int32_t n_problems, const int32_t* n_agents, const int32_t* t_stride,
-                                        int64_t* table_offset) {
+// corr: NULL = every table diagonal (fo_agent_batch_layout)
+static size_t batch_layout(const char* fn, int32_t n_problems, const int32_t* n_agents, const int32_t* t_stride,
+                           const uint8_t* corr, int64_t* table_offset) {
   if (n_problems < 0 || (n_problems > 0 && (!n_agents || !t_stride || !table_offset))) {
-    fo::set_error("fo_agent_batch_layout: bad argument");
+    fo::set_error("%s: bad argument", fn);
     return 0;
   }
   size_t off = 0;
   for (int p = 0; p < n_problems; ++p) {
     const int A = n_agents[p], Tp = t_stride[p];
     if (A < 0 || Tp < 0 || Tp > FO_MAX_STATES) {
-      fo::set_error("fo_agent_batch_layout: problem %d: n_agents %d / t_stride %d out of range", p, A, Tp);
+      fo::set_error("%s: problem %d: n_agents %d / t_stride %d out of range", fn, p, A, Tp);
       return 0;
     }
     table_offset[p] = (int64_t)off;
-    if (A > 0 && Tp > 0) off += (fo::agent_table_bytes(A, Tp) + 15) & ~(size_t)15;
+    if (A > 0 && Tp > 0)
+      off += ((corr && corr[p] ? fo::agent_table_bytes_corr(A, Tp) : fo::agent_table_bytes(A, Tp)) + 15) & ~(size_t)15;
   }
   return off;
 }
 
+extern "C" size_t fo_agent_batch_layout(int32_t n_problems, const int32_t* n_agents, const int32_t* t_stride,
+                                        int64_t* table_offset) {
+  return batch_layout("fo_agent_batch_layout", n_problems, n_agents, t_stride, nullptr, table_offset);
+}
+
+extern "C" size_t fo_agent_batch_layout_corr(int32_t n_problems, const int32_t* n_agents, const int32_t* t_stride,
+                                             const uint8_t* corr_host, int64_t* table_offset) {
+  const char* fn = "fo_agent_batch_layout_corr";
+  if (n_problems > 0 && !corr_host) { fo::set_error("%s: corr_host must not be NULL", fn); return 0; }
+  return batch_layout(fn, n_problems, n_agents, t_stride, corr_host, table_offset);
+}
+
 int fo::check_pack_batch(const char* fn, const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
-                         const void* arena_dev, size_t arena_bytes, int* n_packed_out, int* max_cells_out) {
+                         const uint8_t* corr, const void* arena_dev, size_t arena_bytes, int* n_packed_out,
+                         int* max_cells_out) {
   if (!raw || n_problems < 0 || (n_problems > 0 && !problems)) { fo::set_error("%s: bad argument", fn); return FO_ERR_INVALID_ARG; }
   if (raw->n_agents < 0 || raw->t_stride < 0) { fo::set_error("%s: negative size", fn); return FO_ERR_INVALID_ARG; }
   if (reinterpret_cast<uintptr_t>(arena_dev) & 15) { fo::set_error("%s: arena must be 16-byte aligned", fn); return FO_ERR_INVALID_ARG; }
@@ -384,7 +412,8 @@ int fo::check_pack_batch(const char* fn, const FoAgentsRaw* raw, int32_t n_probl
     if (q.n_agents < 0) { fo::set_error("%s: problem %d has %d agents", fn, p, q.n_agents); return FO_ERR_INVALID_ARG; }
     total += q.n_agents;
     if (q.n_agents == 0) continue;
-    const int rc = fo::check_table(fn, p, q.n_agents, q.t_stride, q.table_offset, arena_dev ? arena_bytes : 0);
+    const int rc = fo::check_table(fn, p, q.n_agents, q.t_stride, q.table_offset, arena_dev ? arena_bytes : 0,
+                                   corr && corr[p]);
     if (rc != FO_OK) return rc;
     if (q.t_stride > raw->t_stride) { fo::set_error("%s: problem %d t_stride %d > raw row stride %d", fn, p, q.t_stride, raw->t_stride); return FO_ERR_INVALID_ARG; }
     ++n_packed;
@@ -406,33 +435,50 @@ int fo::check_pack_batch(const char* fn, const FoAgentsRaw* raw, int32_t n_probl
   return FO_OK;
 }
 
-// Problem p is packed with the mass of vehicles[per_problem ? p : 0].
+// Problem p is packed with the mass of vehicles[per_problem ? p : 0]; corr / cov_xy: the correlated problems
+// (fo_agents_pack_batch_corr), NULL for none.
 static int pack_batch_impl(const char* fn, const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
-                           const FoVehicle* vehicles, bool per_problem, void* arena_dev, size_t arena_bytes, void* stream) {
+                           const FoVehicle* vehicles, bool per_problem, const uint8_t* corr, const float* cov_xy,
+                           void* arena_dev, size_t arena_bytes, void* stream) {
   if (!vehicles) { fo::set_error("%s: bad argument", fn); return FO_ERR_INVALID_ARG; }
   int n_packed = 0, max_cells = 0;
   {
-    const int rc = fo::check_pack_batch(fn, raw, n_problems, problems, arena_dev, arena_bytes, &n_packed, &max_cells);
+    const int rc = fo::check_pack_batch(fn, raw, n_problems, problems, corr, arena_dev, arena_bytes, &n_packed, &max_cells);
     if (rc != FO_OK || n_packed == 0) return rc;
   }
+  int n_corr = 0, corr_cells = 0;               // the correlated problems with agents, the most (agent, state) cells of one
+  for (int p = 0; corr && p < n_problems; ++p) {
+    const FoBatchProblem& q = problems[p];
+    if (!corr[p] || q.n_agents == 0) continue;
+    ++n_corr;
+    if (q.n_agents * q.t_stride > corr_cells) corr_cells = q.n_agents * q.t_stride;
+  }
+  if (n_corr > 0 && !cov_xy) { fo::set_error("%s: cov_xy must not be NULL with correlated problems", fn); return FO_ERR_INVALID_ARG; }
   cudaStream_t st = (cudaStream_t)stream;
-  const size_t bytes = (size_t)n_packed * sizeof(fo::PackProblem);
+  // staged: the descriptors of all packed problems, then those of the correlated ones again (the s3 launch)
+  const size_t bytes = (size_t)(n_packed + n_corr) * sizeof(fo::PackProblem);
   fo::StageSlot* slot = nullptr;
   int rc = fo::stage_acquire(bytes, &slot);
   if (rc != FO_OK) return rc;
   fo::PackProblem* pp = reinterpret_cast<fo::PackProblem*>(slot->host);
-  int a_begin = 0, j = 0;
+  int a_begin = 0, j = 0, jc = n_packed;
   for (int p = 0; p < n_problems; ++p) {
     const FoBatchProblem& q = problems[p];
-    if (q.n_agents > 0)
+    if (q.n_agents > 0) {
       pp[j++] = fo::PackProblem{a_begin, q.n_agents, q.t_stride, vehicles[per_problem ? p : 0].mass, (long long)q.table_offset};
+      if (corr && corr[p]) pp[jc++] = pp[j - 1];
+    }
     a_begin += q.n_agents;
   }
   rc = fo::stage_upload(slot, bytes, st);
   if (rc != FO_OK) return rc;
-  fo::launch_pack(*raw, fo::PackProblem{}, reinterpret_cast<const fo::PackProblem*>(slot->dev), n_packed, max_cells,
-                  (unsigned char*)arena_dev, st);
+  const fo::PackProblem* pp_dev = reinterpret_cast<const fo::PackProblem*>(slot->dev);
+  fo::launch_pack(*raw, fo::PackProblem{}, pp_dev, n_packed, max_cells, (unsigned char*)arena_dev, st);
   fo::count_launch(2);
+  if (n_corr > 0) {
+    fo::launch_corr(*raw, cov_xy, fo::PackProblem{}, pp_dev + n_packed, n_corr, corr_cells, (unsigned char*)arena_dev, st);
+    fo::count_launch();
+  }
   FO_CUDA_TRY(cudaGetLastError());
   FO_CUDA_TRY(cudaEventRecord(slot->done, st));
   return FO_OK;
@@ -440,7 +486,8 @@ static int pack_batch_impl(const char* fn, const FoAgentsRaw* raw, int32_t n_pro
 
 extern "C" int fo_agents_pack_batch(const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
                                     const FoVehicle* vehicle, void* arena_dev, size_t arena_bytes, void* stream) {
-  return pack_batch_impl("fo_agents_pack_batch", raw, n_problems, problems, vehicle, false, arena_dev, arena_bytes, stream);
+  return pack_batch_impl("fo_agents_pack_batch", raw, n_problems, problems, vehicle, false, nullptr, nullptr, arena_dev,
+                         arena_bytes, stream);
 }
 
 extern "C" int fo_agents_pack_batch_vehicles(const FoAgentsRaw* raw, int32_t n_problems, const FoBatchProblem* problems,
@@ -449,8 +496,22 @@ extern "C" int fo_agents_pack_batch_vehicles(const FoAgentsRaw* raw, int32_t n_p
   const char* fn = "fo_agents_pack_batch_vehicles";
   if (n_problems > 0 && !vehicles_host) { fo::set_error("%s: vehicles_host must not be NULL", fn); return FO_ERR_INVALID_ARG; }
   static const FoVehicle none{};                 // no problems: nothing is read
-  return pack_batch_impl(fn, raw, n_problems, problems, vehicles_host ? vehicles_host : &none, true, arena_dev,
-                         arena_bytes, stream);
+  return pack_batch_impl(fn, raw, n_problems, problems, vehicles_host ? vehicles_host : &none, true, nullptr, nullptr,
+                         arena_dev, arena_bytes, stream);
+}
+
+extern "C" int fo_agents_pack_batch_corr(const FoAgentsRaw* raw, const float* cov_xy, int32_t n_problems,
+                                         const FoBatchProblem* problems, const uint8_t* corr_host,
+                                         const FoVehicle* vehicles_host, void* arena_dev, size_t arena_bytes,
+                                         void* stream) {
+  const char* fn = "fo_agents_pack_batch_corr";
+  if (n_problems > 0 && (!corr_host || !vehicles_host)) {
+    fo::set_error("%s: corr_host and vehicles_host must not be NULL", fn);
+    return FO_ERR_INVALID_ARG;
+  }
+  static const FoVehicle none{};                 // no problems: nothing is read
+  return pack_batch_impl(fn, raw, n_problems, problems, vehicles_host ? vehicles_host : &none, true, corr_host, cov_xy,
+                         arena_dev, arena_bytes, stream);
 }
 
 // SM count per device (a process may drive several GPUs, one per planner thread): cached per ordinal, racing
@@ -552,7 +613,7 @@ static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, 
 // Host-side checks of the batch entry points, before any device work: the outputs each one accepts, row order and
 // contiguity, rows inside n_traj, tables inside the arena, alignment, stride and T limits, 'be' needs 'ttc'.  On success
 // *n_run = the problems with trajectories and *a_min = the fewest agents among them.
-int fo::check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, int* n_run, int* a_min) {
+int fo::check_batch(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, bool detail, int* n_run, int* a_min) {
   if (!b) { fo::set_error("%s: NULL args", fn); return FO_ERR_INVALID_ARG; }
   const FoMetricArgs& c = b->common;
   const int P = b->n_problems;
@@ -590,8 +651,14 @@ int fo::check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, int
     next_row += q.n_traj;
     if (next_row > c.n_traj) { fo::set_error("%s: problem %d ends at row %lld > n_traj %d", fn, p, next_row, c.n_traj); return FO_ERR_INVALID_ARG; }
     if (q.n_agents > 0) {
-      const int rc = fo::check_table(fn, p, q.n_agents, q.t_stride, q.table_offset, c.agent_table ? b->arena_bytes : 0);
+      const bool qc = corr && corr[p];
+      const int rc = fo::check_table(fn, p, q.n_agents, q.t_stride, q.table_offset, c.agent_table ? b->arena_bytes : 0, qc);
       if (rc != FO_OK) return rc;
+      // the detail descriptor holds the s3 section's place as a 32-bit offset from s0 in 16-byte units
+      if (qc && detail && (fo::agent_corr_offset(q.n_agents, q.t_stride) >> 4) > 0xffffffffull) {
+        fo::set_error("%s: correlated table of problem %d too large for a batch", fn, p);
+        return FO_ERR_UNSUPPORTED;
+      }
     }
     if (q.n_traj > 0) {
       ++*n_run;
@@ -605,11 +672,13 @@ int fo::check_batch(const char* fn, const FoMetricBatchArgs* b, bool detail, int
   return FO_OK;
 }
 
-// vehicles: problem p's ego vehicle is vehicles[p]; NULL = common.vehicle for every problem
-static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const FoVehicle* vehicles, void* stream) {
+// vehicles: problem p's ego vehicle is vehicles[p]; NULL = common.vehicle for every problem.  corr: problem p's table is a
+// correlated one when corr[p] != 0; NULL = none is.
+static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles,
+                             void* stream) {
   int n_run = 0, a_min = 0;
   {
-    const int rc = fo::check_batch(fn, b, false, &n_run, &a_min);
+    const int rc = fo::check_batch(fn, b, corr, false, &n_run, &a_min);
     if (rc != FO_OK || b->common.n_traj == 0) return rc;
   }
   const FoMetricArgs& c = b->common;
@@ -617,15 +686,17 @@ static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const F
   int num_sms = 0;
   { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
   // one team size for the whole batch, as fo_metric_bundle picks it; with W = 1 problems with >= 17 agents run the
-  // window-filter shape, the others the team shape with their own lane grouping
+  // window-filter shape, the others the team shape with their own lane grouping.  Classes: 0 / 1 diagonal window-filter
+  // / team shape, 2 / 3 the same for correlated tables; one launch per non-empty class, each numbering its trajectories
   const int W = fo::pick_team_warps(c.n_traj, c.n_states, a_min, num_sms);
-  int n_uni = 0;
-  for (int p = 0; p < P; ++p) {
-    const FoBatchProblem& q = b->problems[p];
-    if (q.n_traj > 0 && W == 1 && fo::lane_group_log2(q.n_agents) == 5) ++n_uni;
-  }
-  const int n_team = n_run - n_uni;
-  // staged: first[] of both classes, then their descriptors (16-byte aligned)
+  const auto class_of = [&](int p) {
+    return (corr && corr[p] ? 2 : 0) + (W == 1 && fo::lane_group_log2(b->problems[p].n_agents) == 5 ? 0 : 1);
+  };
+  int cnt[4] = {0, 0, 0, 0};
+  for (int p = 0; p < P; ++p)
+    if (b->problems[p].n_traj > 0) ++cnt[class_of(p)];
+  const int start[4] = {0, cnt[0], cnt[0] + cnt[1], cnt[0] + cnt[1] + cnt[2]};
+  // staged: first[] of all classes, then their descriptors (16-byte aligned), class by class
   const size_t first_bytes = ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15;
   const size_t bytes = first_bytes + (size_t)n_run * sizeof(fo::BatchProb);
   fo::StageSlot* slot = nullptr;
@@ -634,23 +705,23 @@ static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const F
   int* first = reinterpret_cast<int*>(slot->host);
   fo::BatchProb* prob = reinterpret_cast<fo::BatchProb*>(slot->host + first_bytes);
   const unsigned char* arena = reinterpret_cast<const unsigned char*>(c.agent_table);
-  int iu = 0, it = n_uni, nu = 0, nt = 0;       // uni class first, team class after it
+  int next[4] = {start[0], start[1], start[2], start[3]}, n_cls[4] = {0, 0, 0, 0};
   for (int p = 0; p < P; ++p) {
     const FoBatchProblem& q = b->problems[p];
     if (q.n_traj == 0) continue;
-    const int lg = fo::lane_group_log2(q.n_agents);
-    const bool uni = W == 1 && lg == 5;
-    int& i = uni ? iu : it;
-    int& n = uni ? nu : nt;
+    const int cl = class_of(p);
+    const int i = next[cl]++;
+    int& n = n_cls[cl];
     fo::BatchProb& d = prob[i];
     const int Tp = q.n_agents > 0 ? q.t_stride : 1;
-    const fo::AgentTableView v = fo::agent_table_view(arena + (q.n_agents > 0 ? q.table_offset : 0), q.n_agents, Tp);
+    const unsigned char* tab = arena + (q.n_agents > 0 ? q.table_offset : 0);
+    const fo::AgentTableView v = fo::agent_table_view(tab, q.n_agents, Tp);
     d.t0 = v.t0; d.tv = v.tv; d.aw = v.aw; d.avw = v.avw; d.s0 = v.s0; d.s1 = v.s1; d.s2 = v.s2; d.prm = v.prm;
-    d.first = n; d.row0 = (int)q.traj_begin; d.A = q.n_agents; d.Tp = Tp; d.Ap = v.Ap; d.lg = lg;
+    d.first = n; d.row0 = (int)q.traj_begin; d.A = q.n_agents; d.Tp = Tp; d.Ap = v.Ap; d.lg = fo::lane_group_log2(q.n_agents);
     fo::fill_ego_const(vehicles ? vehicles[p] : c.vehicle, d.veh);
+    d.s3 = cl >= 2 && q.n_agents > 0 ? fo::agent_corr_view(tab, q.n_agents, Tp) : nullptr;
     first[i] = n;
     n += q.n_traj;
-    ++i;
   }
   cudaStream_t st = (cudaStream_t)stream;
   rc = fo::stage_upload(slot, bytes, st);
@@ -662,14 +733,11 @@ static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const F
   fill_kargs(&ca, k);
   const int* first_dev = reinterpret_cast<const int*>(slot->dev);
   const fo::BatchProb* prob_dev = reinterpret_cast<const fo::BatchProb*>(slot->dev + first_bytes);
-  if (n_uni > 0) {
-    k.N = nu;
-    rc = fo::launch_metric_batch(k, num_sms, W, true, fo::BatchView{first_dev, prob_dev, n_uni}, st);
-    if (rc != FO_OK) return rc;
-  }
-  if (n_team > 0) {
-    k.N = nt;
-    rc = fo::launch_metric_batch(k, num_sms, W, false, fo::BatchView{first_dev + n_uni, prob_dev + n_uni, n_team}, st);
+  for (int cl = 0; cl < 4; ++cl) {
+    if (cnt[cl] == 0) continue;
+    k.N = n_cls[cl];
+    k.corr = cl >= 2;
+    rc = fo::launch_metric_batch(k, num_sms, W, (cl & 1) == 0, fo::BatchView{first_dev + start[cl], prob_dev + start[cl], cnt[cl]}, st);
     if (rc != FO_OK) return rc;
   }
   FO_CUDA_TRY(cudaEventRecord(slot->done, st));
@@ -677,28 +745,47 @@ static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const F
 }
 
 extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
-  return metric_batch_impl("fo_metric_batch", b, nullptr, stream);
+  return metric_batch_impl("fo_metric_batch", b, nullptr, nullptr, stream);
 }
 
 extern "C" int fo_metric_batch_vehicles(const FoMetricBatchArgs* b, const FoVehicle* vehicles_host, void* stream) {
   const char* fn = "fo_metric_batch_vehicles";
   if (b && b->n_problems > 0 && !vehicles_host) { fo::set_error("%s: vehicles_host must not be NULL", fn); return FO_ERR_INVALID_ARG; }
-  return metric_batch_impl(fn, b, vehicles_host, stream);
+  return metric_batch_impl(fn, b, nullptr, vehicles_host, stream);
 }
 
-static int metric_batch_detail_impl(const char* fn, const FoMetricBatchArgs* b, const FoVehicle* vehicles, void* stream) {
+// corr as in metric_batch_impl.  The diagonal problems run fo_metric_batch_detail_kernel, which takes its launch's rows
+// to be [0, k.N) with the problems' first rows in first[]: where correlated problems sit between diagonal ones, their rows
+// enter that launch as problems without agents (valid / summary / flags only), and the correlated launch that follows on
+// the stream writes them again with their own results.  The correlated launch numbers its trajectories itself
+// (fo_metric_batch_detail_corr_kernel), so it touches its own rows only.
+static int metric_batch_detail_impl(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr,
+                                    const FoVehicle* vehicles, void* stream) {
   int n_run = 0, a_min = 0;
   {
-    const int rc = fo::check_batch(fn, b, true, &n_run, &a_min);
+    const int rc = fo::check_batch(fn, b, corr, true, &n_run, &a_min);
     if (rc != FO_OK || b->common.n_traj == 0) return rc;
   }
   const FoMetricArgs& c = b->common;
   const int P = b->n_problems, Tm1 = c.n_states - 1;
   int num_sms = 0;
   { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
-  // staged: the problems' first rows, then their descriptors (16-byte aligned)
-  const size_t first_bytes = ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15;
-  const size_t bytes = first_bytes + (size_t)n_run * sizeof(fo::DetailProb);
+  // the diagonal launch covers the rows up to the end of its last problem; its descriptors: every problem with
+  // trajectories up to there (the correlated ones as stand-ins without agents).  The correlated launch: its problems.
+  long long diag_rows = 0;
+  int n_diag = 0, n_corr = 0;
+  for (int p = 0; p < P; ++p) {
+    const FoBatchProblem& q = b->problems[p];
+    if (q.n_traj == 0) continue;
+    if (corr && corr[p]) { ++n_corr; continue; }
+    diag_rows = q.traj_begin + q.n_traj;
+  }
+  for (int p = 0; p < P; ++p)
+    if (b->problems[p].n_traj > 0 && b->problems[p].traj_begin < diag_rows) ++n_diag;
+  const int n_desc = n_diag + n_corr;
+  // staged: the first[] of both launches, then their descriptors (16-byte aligned)
+  const size_t first_bytes = ((size_t)n_desc * sizeof(int) + 15) & ~(size_t)15;
+  const size_t bytes = first_bytes + (size_t)n_desc * sizeof(fo::DetailProb);
   fo::StageSlot* slot = nullptr;
   int rc = fo::stage_acquire(bytes, &slot);
   if (rc != FO_OK) return rc;
@@ -706,19 +793,33 @@ static int metric_batch_detail_impl(const char* fn, const FoMetricBatchArgs* b, 
   fo::DetailProb* prob = reinterpret_cast<fo::DetailProb*>(slot->host + first_bytes);
   const unsigned char* arena = reinterpret_cast<const unsigned char*>(c.agent_table);
   long long pairs = 0;                           // sum of N_q A_q over the problems before p: the offset of p's blocks
-  int i = 0;
+  // problem p's descriptor; a stand-in has no agents and no detail blocks
+  const auto fill = [&](fo::DetailProb& d, int p, bool stand_in) {
+    const FoBatchProblem& q = b->problems[p];
+    const int A = stand_in ? 0 : q.n_agents;
+    const int Tp = A > 0 ? q.t_stride : 1;
+    const fo::AgentTableView v = fo::agent_table_view(arena + (A > 0 ? q.table_offset : 0), A, Tp);
+    d.t0 = v.t0; d.tv = v.tv; d.s0 = v.s0; d.s1 = v.s1; d.s2 = v.s2; d.prm = v.prm; d.orig = v.orig; d.tpsi = v.tpsi;
+    d.pair = c.pair && !stand_in ? c.pair + (size_t)pairs * FO_PAIR_K : nullptr;
+    d.step = c.step && !stand_in ? c.step + (size_t)pairs * Tm1 * FO_STEP_K : nullptr;
+    d.row0 = (int)q.traj_begin; d.A = A; d.Tp = Tp; d.Ap = v.Ap;
+    fo::fill_ego_const(vehicles ? vehicles[p] : c.vehicle, d.veh);
+    d.s3_off = corr && corr[p] && A > 0 ? (uint32_t)(fo::agent_corr_offset(A, Tp) >> 4) : 0u;
+  };
+  int i = 0, ic = n_diag, nc = 0;                // next diagonal / correlated descriptor; trajectories of the latter
   for (int p = 0; p < P; ++p) {
     const FoBatchProblem& q = b->problems[p];
     if (q.n_traj == 0) continue;
-    const int Tp = q.n_agents > 0 ? q.t_stride : 1;
-    const fo::AgentTableView v = fo::agent_table_view(arena + (q.n_agents > 0 ? q.table_offset : 0), q.n_agents, Tp);
-    fo::DetailProb& d = prob[i];
-    d.t0 = v.t0; d.tv = v.tv; d.s0 = v.s0; d.s1 = v.s1; d.s2 = v.s2; d.prm = v.prm; d.orig = v.orig; d.tpsi = v.tpsi;
-    d.pair = c.pair ? c.pair + (size_t)pairs * FO_PAIR_K : nullptr;
-    d.step = c.step ? c.step + (size_t)pairs * Tm1 * FO_STEP_K : nullptr;
-    d.row0 = (int)q.traj_begin; d.A = q.n_agents; d.Tp = Tp; d.Ap = v.Ap;
-    fo::fill_ego_const(vehicles ? vehicles[p] : c.vehicle, d.veh);
-    first[i++] = d.row0;
+    const bool qc = corr && corr[p];
+    if (!qc || q.traj_begin < diag_rows) {
+      fill(prob[i], p, qc);
+      first[i++] = (int)q.traj_begin;
+    }
+    if (qc) {
+      fill(prob[ic], p, false);
+      first[ic++] = nc;
+      nc += q.n_traj;
+    }
     pairs += (long long)q.n_traj * q.n_agents;
   }
   cudaStream_t st = (cudaStream_t)stream;
@@ -730,21 +831,52 @@ static int metric_batch_detail_impl(const char* fn, const FoMetricBatchArgs* b, 
   ca.agent_table = nullptr;
   ca.pair = ca.step = nullptr;
   fill_kargs(&ca, k);
-  rc = fo::launch_metric_batch_detail(k, num_sms,
-                                      fo::DetailView{reinterpret_cast<const int*>(slot->dev),
-                                                     reinterpret_cast<const fo::DetailProb*>(slot->dev + first_bytes), n_run},
-                                      st);
-  if (rc != FO_OK) return rc;
+  const int* first_dev = reinterpret_cast<const int*>(slot->dev);
+  const fo::DetailProb* prob_dev = reinterpret_cast<const fo::DetailProb*>(slot->dev + first_bytes);
+  if (n_diag > 0) {                          // first: the correlated launch overwrites its stand-ins' rows
+    k.N = (int)diag_rows;
+    rc = fo::launch_metric_batch_detail(k, num_sms, fo::DetailView{first_dev, prob_dev, n_diag}, st);
+    if (rc != FO_OK) return rc;
+  }
+  if (n_corr > 0) {
+    k.N = nc;
+    k.corr = true;
+    rc = fo::launch_metric_batch_detail(k, num_sms, fo::DetailView{first_dev + n_diag, prob_dev + n_diag, n_corr}, st);
+    if (rc != FO_OK) return rc;
+  }
   FO_CUDA_TRY(cudaEventRecord(slot->done, st));
   return FO_OK;
 }
 
 extern "C" int fo_metric_batch_detail(const FoMetricBatchArgs* b, void* stream) {
-  return metric_batch_detail_impl("fo_metric_batch_detail", b, nullptr, stream);
+  return metric_batch_detail_impl("fo_metric_batch_detail", b, nullptr, nullptr, stream);
 }
 
 extern "C" int fo_metric_batch_detail_vehicles(const FoMetricBatchArgs* b, const FoVehicle* vehicles_host, void* stream) {
   const char* fn = "fo_metric_batch_detail_vehicles";
   if (b && b->n_problems > 0 && !vehicles_host) { fo::set_error("%s: vehicles_host must not be NULL", fn); return FO_ERR_INVALID_ARG; }
-  return metric_batch_detail_impl(fn, b, vehicles_host, stream);
+  return metric_batch_detail_impl(fn, b, nullptr, vehicles_host, stream);
+}
+
+// Correlated and diagonal problems in one batch: corr_host[p] != 0 = problem p's table is a correlated one.
+static int check_corr_args(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr_host, const FoVehicle* vehicles_host) {
+  if (b && b->n_problems > 0 && (!corr_host || !vehicles_host)) {
+    fo::set_error("%s: corr_host and vehicles_host must not be NULL", fn);
+    return FO_ERR_INVALID_ARG;
+  }
+  return FO_OK;
+}
+
+extern "C" int fo_metric_batch_corr(const FoMetricBatchArgs* b, const uint8_t* corr_host, const FoVehicle* vehicles_host,
+                                    void* stream) {
+  const char* fn = "fo_metric_batch_corr";
+  const int rc = check_corr_args(fn, b, corr_host, vehicles_host);
+  return rc != FO_OK ? rc : metric_batch_impl(fn, b, corr_host, vehicles_host, stream);
+}
+
+extern "C" int fo_metric_batch_detail_corr(const FoMetricBatchArgs* b, const uint8_t* corr_host,
+                                           const FoVehicle* vehicles_host, void* stream) {
+  const char* fn = "fo_metric_batch_detail_corr";
+  const int rc = check_corr_args(fn, b, corr_host, vehicles_host);
+  return rc != FO_OK ? rc : metric_batch_detail_impl(fn, b, corr_host, vehicles_host, stream);
 }

@@ -162,7 +162,8 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
   const auto soff = [&](const void* q) { return (uint32_t)(reinterpret_cast<const unsigned char*>(q) - smem_raw); };
   const BeView bev{soff(egoA), soff(egoB), soff(dist), soff(inv), 0u};
   const BeConst bek = be_const(k);                // batched: the table and its stride are set per bisection
-  const float4* const s3 = CORR ? agent_corr_view(k.tab.s0, k.A, k.Tp) : nullptr;
+  // batched: the trajectory's problem's s3 section, set per trajectory
+  const float4* s3 = (CORR && !BATCH) ? agent_corr_view(k.tab.s0, k.A, k.Tp) : nullptr;
   // batched: the warp's copy of its problem's descriptor, behind the per-warp regions (read where used, not held in
   // registers across the trajectory)
   DetailProb* const sdp = reinterpret_cast<DetailProb*>(smem_raw + kDtWarps * detail_warp_bytes(T)) + wib;
@@ -187,11 +188,18 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
       if constexpr (BATCH) p_next = n_next < k.N ? find_problem(bv.first, bv.P, n_next) : 0;
     }
     int nb = n;                                        // the trajectory's index in its pair / step block
+    int row = n;                                       // its row in ego / valid / summary / flags
     if constexpr (BATCH) {
       if (lane < (int)(sizeof(DetailProb) / 16))
         reinterpret_cast<int4*>(sdp)[lane] = __ldg(reinterpret_cast<const int4*>(bv.prob + p) + lane);
       __syncwarp();
-      nb = n - sdp->row0;
+      if constexpr (CORR) {                            // n numbers the trajectories of the launch's problems
+        nb = n - __ldg(bv.first + p);
+        row = sdp->row0 + nb;
+        s3 = sdp->s0 + sdp->s3_off;
+      } else {
+        nb = n - sdp->row0;
+      }
       rE = sqrtf(sdp->veh.hEx * sdp->veh.hEx + sdp->veh.hEy * sdp->veh.hEy);
       rows8 = (Tm1 & 1) == 0 && (reinterpret_cast<uintptr_t>(sdp->step) & 7u) == 0;
       traj_step = (size_t)sdp->A * (size_t)Tm1 * FO_STEP_K;
@@ -212,7 +220,7 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
         dt_drain_ties(k, egoA, egoB, dkey, src, cnt, a0, lane);
     };
     // ---- stage the ego trajectory (this warp only) ---------------------------------------------------------------
-    const float* eg = k.ego + (size_t)n * T * 5;
+    const float* eg = k.ego + (size_t)row * T * 5;
     float amin = 0.0f;
     for (int i = lane; i < T; i += 32) {
       const float x = __ldg(eg + i * 5 + 0), y = __ldg(eg + i * 5 + 1), th = __ldg(eg + i * 5 + 2);
@@ -553,10 +561,10 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
           if (do_dce && (k.tmask & FO_T_DCE) && rmin != 0xffffffu && rmin < k.thr_dce_mm) ok = false;
           if (fl & FO_F_BE_RANGE) ok = false;
         }
-        k.valid[n] = ok ? 1 : 0;
-        if (k.flags) k.flags[n] = fl;
+        k.valid[row] = ok ? 1 : 0;
+        if (k.flags) k.flags[row] = fl;
         if (k.summary) {
-          float* sm = k.summary + (size_t)n * FO_SUMMARY_K;
+          float* sm = k.summary + (size_t)row * FO_SUMMARY_K;
           sm[0] = er; sm[1] = orr; sm[2] = eh; sm[3] = oh; sm[4] = cpm; sm[5] = hwc_all;
           sm[6] = (rmin == 0xffffffu || !do_dce) ? CUDART_INF_F : mm_to_m(rmin);
           sm[7] = has_col ? step_to_s(col, k.dtd) : CUDART_INF_F;
@@ -587,6 +595,14 @@ template <uint32_t MASK>
 __global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB)
 fo_metric_batch_detail_kernel(const __grid_constant__ MetricKArgs k, const __grid_constant__ DetailView bv) {
   detail_body<MASK, true>(k, bv);
+}
+
+// The correlated problems of a batch (fo_metric_batch_detail_corr), runtime metric mask: fo_metric_batch_detail_kernel with
+// fo_metric_detail_corr_kernel's CP terms.  Its problems' rows need not be contiguous: bv.first numbers the trajectories
+// of the launch (k.N = their count), and DetailProb::row0 places each problem's rows.
+__global__ void __launch_bounds__(kDtWarps * 32, FO_DT_MINB)
+fo_metric_batch_detail_corr_kernel(const __grid_constant__ MetricKArgs k, const __grid_constant__ DetailView bv) {
+  detail_body<0u, true, true>(k, bv);
 }
 
 // Persistent launch of one detail-kernel instantiation: as many CTAs as fit on the device, warps claiming trajectories.
@@ -639,6 +655,7 @@ int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st) {
 // k.N = the batch's rows; the caller has validated the descriptors and the alignment of every pair / step block
 int launch_metric_batch_detail(const MetricKArgs& k, int num_sms, const DetailView& bv, cudaStream_t st) {
   constexpr size_t x = kDtWarps * sizeof(DetailProb);   // the warps' descriptor copies
+  if (k.corr) return launch_detail_kernel<fo_metric_batch_detail_corr_kernel>(k, num_sms, x, st, bv);
   if (k.mmask == kDtAll) return launch_detail_kernel<fo_metric_batch_detail_kernel<kDtAll>>(k, num_sms, x, st, bv);
   if (k.mmask == kDtDefault) return launch_detail_kernel<fo_metric_batch_detail_kernel<kDtDefault>>(k, num_sms, x, st, bv);
   return launch_detail_kernel<fo_metric_batch_detail_kernel<0u>>(k, num_sms, x, st, bv);

@@ -728,6 +728,7 @@ struct __align__(16) BatchProb {
   int A, Tp, Ap;        // agents, table stride, agents padded to 32
   int lg;               // log2 of the agents held by one warp (team shape)
   EgoConst veh;         // the problem's ego vehicle
+  const float4* s3;     // correlated tables (fo_metric_batch_corr): the s3 section (agent_corr_view); NULL otherwise
 };
 static_assert(sizeof(BatchProb) == 128, "eight 16-byte loads");
 struct BatchView {
@@ -761,16 +762,18 @@ struct __align__(16) DetailProb {
   int row0;             // the problem's first row in ego / valid / summary / flags
   int A, Tp, Ap;        // agents, table stride, agents padded to 32
   EgoConst veh;         // the problem's ego vehicle
+  uint32_t s3_off;      // correlated tables (fo_metric_batch_detail_corr): s3 = s0 + s3_off (float4 units); 0 otherwise
 };
 static_assert(sizeof(DetailProb) == 128, "eight 16-byte loads");
 struct DetailView {
-  const int* first;     // [P] DetailProb::row0, strictly increasing (problems without trajectories are left out)
+  const int* first;     // [P] DetailProb::row0, strictly increasing (problems without trajectories are left out); the
+                        // correlated kernel numbers its trajectories within the launch instead, as BatchView::first
   const DetailProb* prob;
   int P;
 };
 int launch_metric_batch_detail(const MetricKArgs& k, int num_sms, const DetailView& bv, cudaStream_t st);
 // summary kernel over one shape class of a batch (uni: the one-warp window-filter shape, W == 1); k.N = the class's
-// trajectory count
+// trajectory count.  k.corr: the class's tables are correlated ones (fo_metric_batch_corr_kernel), in both batch launches
 int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st);
 int lane_group_log2(int A);                                  // team shape: a warp holds 1 << lg agents
 int pick_team_warps(int N, int T, int A, int num_sms);       // team size W (FO_TEAM_WARPS overrides)

@@ -250,7 +250,8 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
   int Ap = k.tab.Ap;
   const auto soff = [&](const void* q) { return (uint32_t)(reinterpret_cast<const unsigned char*>(q) - smem_raw); };
   const BeView bev{soff(w.egoA), soff(w.egoB), soff(w.dist), soff(w.inv), soff(w.seg)};
-  const float4* const s3 = CORR ? agent_corr_view(k.tab.s0, k.A, k.Tp) : nullptr;
+  // batched: the trajectory's problem's s3 section, set per trajectory
+  const float4* s3 = (CORR && !BATCH) ? agent_corr_view(k.tab.s0, k.A, k.Tp) : nullptr;
   BeConst bek = be_const(k);                       // batched: the table and its stride are set per trajectory
   // lane -> (agent within the lane group, time slice); every (warp, slice) owns a contiguous range of steps
   const int lg = shape.lg_agents;
@@ -289,6 +290,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
       const int bL = (T + W * (32 >> bp.lg) - 1) / (W * (32 >> bp.lg));
       b_slo = (wib * (32 >> bp.lg) + (lane >> bp.lg)) * bL;
       b_shi = min(T, b_slo + bL);
+      if constexpr (CORR) s3 = bp.s3;
     }
     // references into the kernel parameters when not batched: their uses stay constant-bank operands
     const AgentTableView& tab = BATCH ? btab : k.tab;
@@ -850,6 +852,14 @@ fo_metric_batch_kernel(const __grid_constant__ MetricKArgs k, const SweepShape s
   sweep_body<MASK, false, UNI, TIES, true>(k, shape, bv, threadIdx.x, blockDim.x);
 }
 
+// One shape class of the correlated problems of a batch (fo_metric_batch_corr): fo_metric_batch_kernel's problem lookup
+// with fo_metric_sweep_corr_kernel's CP drain; every trajectory reads its problem's s3 section (BatchProb::s3).
+template <bool UNI, bool TIES>
+__global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
+fo_metric_batch_corr_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape, const __grid_constant__ BatchView bv) {
+  sweep_body<0u, false, UNI, TIES, true, true>(k, shape, bv, threadIdx.x, blockDim.x);
+}
+
 // Team shape.  lg_agents: a warp holds min(32, next power of two >= A) agents, the remaining lanes are time slices.
 // W: as many warps per trajectory as keeps the whole bundle resident in one wave (the latency of a bundle is its
 // slowest trajectory), as long as every (warp, slice) still owns at least 4 steps.
@@ -989,6 +999,14 @@ static int launch_batch_inst(const MetricKArgs& k, int num_sms, int W, bool uni,
 }
 
 int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st) {
+  if (k.corr) {
+    const SweepShape shape{0};
+    const bool ties = needs_ties(k);
+    if (uni) return ties ? launch_team_kernel<fo_metric_batch_corr_kernel<true, true>>(k, num_sms, W, uni, ties, st, shape, bv)
+                         : launch_team_kernel<fo_metric_batch_corr_kernel<true, false>>(k, num_sms, W, uni, ties, st, shape, bv);
+    return ties ? launch_team_kernel<fo_metric_batch_corr_kernel<false, true>>(k, num_sms, W, uni, ties, st, shape, bv)
+                : launch_team_kernel<fo_metric_batch_corr_kernel<false, false>>(k, num_sms, W, uni, ties, st, shape, bv);
+  }
   if (k.mmask == kAllMetrics) return launch_batch_inst<kAllMetrics>(k, num_sms, W, uni, bv, st);
   if (k.mmask == kDefaultMetrics) return launch_batch_inst<kDefaultMetrics>(k, num_sms, W, uni, bv, st);
   return launch_batch_inst<0u>(k, num_sms, W, uni, bv, st);

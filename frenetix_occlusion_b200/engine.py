@@ -401,17 +401,21 @@ class MetricEngine:
         return g, out
 
     # ---- batches of independent problems ------------------------------------------------------------------------
-    def set_agent_batch(self, agent_sets: Sequence[AgentSet], origins=None, vehicles=None):
+    def set_agent_batch(self, agent_sets: Sequence[AgentSet], origins=None, vehicles=None, correlated: bool = False):
         """Upload + pack the phantom predictions of P independent problems (``fo_agents_pack_batch``): one float64
         origin shift per problem, one host-to-device copy of all of them, one pack call.  ``origins``: [P, 2] or None
         (no shift).  ``vehicles``: P ego vehicle descriptions (each a dict or an object with attributes, as the
         constructor takes them), or None for the engine's own vehicle in every problem; ``assess_batch`` assesses
         problem p with vehicles[p].  Problem p's table equals what ``set_agents(agent_sets[p], origins[p])`` packs in an
-        engine built with vehicles[p].  Diagonal prediction covariances only (``AgentSet.cov_xy`` None)."""
+        engine built with vehicles[p].
+
+        ``correlated``: sets with correlated prediction covariances (``AgentSet.cov_xy`` set) are accepted and packed
+        as ``set_agents`` packs them (``fo_agents_pack_batch_corr``); their collision probabilities cost many times the
+        diagonal ones.  Without it such a set raises ``ValueError``.  A batch without one makes the diagonal calls."""
         P = len(agent_sets)
-        if any(a.cov_xy is not None for a in agent_sets):
-            raise ValueError("batches take diagonal prediction covariances only; assess a correlated set with "
-                             "set_agents() + assess()")
+        if not correlated and any(a.cov_xy is not None for a in agent_sets):
+            raise ValueError("batches take diagonal prediction covariances only unless correlated=True; assess a "
+                             "correlated set with set_agents() + assess()")
         veh = None
         if vehicles is not None:
             if len(vehicles) != P:
@@ -422,22 +426,33 @@ class MetricEngine:
         t_stride = np.array([a.t_stride if n else 0 for a, n in zip(agent_sets, n_agents)], dtype=np.int32)
         if np.any(t_stride > L.FO_MAX_STATES):
             raise ValueError(f"predictions longer than {L.FO_MAX_STATES} states are not supported")
+        # the correlated problems (with agents, as set_agents packs them); None = the diagonal calls
+        corr = np.array([a.cov_xy is not None and n > 0 for a, n in zip(agent_sets, n_agents)], dtype=np.uint8)
+        corr = corr if corr.any() else None
+        if corr is not None and veh is None:
+            veh = (L.FoVehicle * P)(*[self.vehicle] * P)
         offsets = np.zeros(P, dtype=np.int64)
-        arena_bytes = L.lib.fo_agent_batch_layout(P, n_agents.ctypes.data, t_stride.ctypes.data, offsets.ctypes.data)
+        if corr is None:
+            arena_bytes = L.lib.fo_agent_batch_layout(P, n_agents.ctypes.data, t_stride.ctypes.data, offsets.ctypes.data)
+        else:
+            arena_bytes = L.lib.fo_agent_batch_layout_corr(P, n_agents.ctypes.data, t_stride.ctypes.data,
+                                                           corr.ctypes.data, offsets.ctypes.data)
         problems = (L.FoBatchProblem * max(P, 1))()
         for p in range(P):
             problems[p].n_agents, problems[p].t_stride, problems[p].table_offset = int(n_agents[p]), int(t_stride[p]), int(offsets[p])
         A, S = int(n_agents.sum()), int(t_stride.max(initial=0))
         dev = self.device
         self._batch = {"problems": problems, "P": P, "origins": org, "agents": list(agent_sets), "arena": None,
-                       "arena_bytes": arena_bytes, "n_agents": n_agents, "vehicles": veh}
+                       "arena_bytes": arena_bytes, "n_agents": n_agents, "vehicles": veh, "corr": corr}
         if A == 0:
             return
-        # one host buffer: 6 float rows [A, S] (x, y shifted per problem), 4 float columns [A], 2 int32 columns [A]
-        buf = np.zeros(6 * A * S + 6 * A, dtype=np.float32)
-        fl = buf[:6 * A * S].reshape(6, A, S)
-        pa = buf[6 * A * S:6 * A * S + 4 * A].reshape(4, A)
-        ia = buf[6 * A * S + 4 * A:].view(np.int32).reshape(2, A)
+        # one host buffer: 6 float rows [A, S] (x, y shifted per problem; a seventh, cov_xy, with correlated problems),
+        # 4 float columns [A], 2 int32 columns [A]
+        R = 6 if corr is None else 7
+        buf = np.zeros(R * A * S + 6 * A, dtype=np.float32)
+        fl = buf[:R * A * S].reshape(R, A, S)
+        pa = buf[R * A * S:R * A * S + 4 * A].reshape(4, A)
+        ia = buf[R * A * S + 4 * A:].view(np.int32).reshape(2, A)
         a0 = 0
         for p, ag in enumerate(agent_sets):
             n, tp = int(n_agents[p]), int(t_stride[p])
@@ -447,6 +462,8 @@ class MetricEngine:
             fl[0, rows, :tp] = ag.x - org[p, 0]
             fl[1, rows, :tp] = ag.y - org[p, 1]
             fl[2, rows, :tp], fl[3, rows, :tp], fl[4, rows, :tp], fl[5, rows, :tp] = ag.yaw, ag.v, ag.var_x, ag.var_y
+            if corr is not None and corr[p]:
+                fl[6, rows, :tp] = ag.cov_xy
             pa[:, rows] = (ag.length, ag.width, ag.buf_length, ag.buf_width)
             ia[:, rows] = (ag.n_states, ag.kind)
             a0 += n
@@ -457,11 +474,15 @@ class MetricEngine:
             raw = L.FoAgentsRaw()
             raw.n_agents, raw.t_stride = A, S
             raw.x, raw.y, raw.yaw, raw.v, raw.var_x, raw.var_y = [ptr + f4 * i * A * S for i in range(6)]
-            base = ptr + f4 * 6 * A * S
+            base = ptr + f4 * R * A * S
             raw.length, raw.width, raw.buf_length, raw.buf_width = [base + f4 * i * A for i in range(4)]
             raw.n_states, raw.kind = base + f4 * 4 * A, base + f4 * 5 * A
             arena = torch.empty(max(arena_bytes, 16), dtype=torch.uint8, device=dev)
-            if veh is None:
+            if corr is not None:
+                L.check(L.lib.fo_agents_pack_batch_corr(C.byref(raw), C.c_void_p(ptr + f4 * 6 * A * S), P, problems,
+                                                        corr.ctypes.data, veh, C.c_void_p(arena.data_ptr()), arena_bytes,
+                                                        self._stream()), "fo_agents_pack_batch_corr")
+            elif veh is None:
                 L.check(L.lib.fo_agents_pack_batch(C.byref(raw), P, problems, C.byref(self.vehicle),
                                                    C.c_void_p(arena.data_ptr()), arena_bytes, self._stream()),
                         "fo_agents_pack_batch")
@@ -500,7 +521,7 @@ class MetricEngine:
         """One pass over every problem of the batch set by ``set_agent_batch`` in one metric call.  ``egos[p]``: problem
         p's [N_p, T, 5] bundle (host array or CUDA tensor, in the caller's frame: it is shifted by the problem's origin).
         Without detail outputs this is ``fo_metric_batch``; with ``want_pair`` / ``want_step`` it is
-        ``fo_metric_batch_detail``, and ``split()`` gives problem p what ``set_agents`` + ``assess(want_pair,
+        ``fo_metric_batch_detail`` (their ``_corr`` forms when the batch has a correlated problem), and ``split()`` gives problem p what ``set_agents`` + ``assess(want_pair,
         want_step)`` gives it alone (in an engine built with its vehicle, when ``set_agent_batch`` had ``vehicles``).
         ``out``: preallocated outputs of the batch's sizes (valid / summary / flags, and
         the flat pair / step where wanted).  Asynchronous on the current stream."""
@@ -562,8 +583,11 @@ class MetricEngine:
             # path runs when no detail buffer is left
             a.common.pair = out.pair.data_ptr() if (out.pair is not None and out.pair.numel()) else None
             a.common.step = out.step.data_ptr() if (out.step is not None and out.step.numel()) else None
-            detail, veh = bool(a.common.pair or a.common.step), b["vehicles"]
-            if veh is None:
+            detail, veh, corr = bool(a.common.pair or a.common.step), b["vehicles"], b["corr"]
+            if corr is not None:
+                fn = "fo_metric_batch_detail_corr" if detail else "fo_metric_batch_corr"
+                L.check(getattr(L.lib, fn)(C.byref(a), corr.ctypes.data, veh, self._stream()), fn)
+            elif veh is None:
                 fn = "fo_metric_batch_detail" if detail else "fo_metric_batch"
                 L.check(getattr(L.lib, fn)(C.byref(a), self._stream()), fn)
             else:

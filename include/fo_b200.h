@@ -174,7 +174,8 @@ int fo_metric_stats(const FoMetricArgs *args, uint64_t *counters_dev, void *stre
  * that violates it (|rho| >= 1, a zero variance with a non-zero covariance) gets NaN collision probabilities.
  * fo_metric_bundle_corr: fo_metric_bundle on a table written by fo_agents_pack_corr, with its outputs, checks and
  * CUDA-graph capture behaviour.  Each CP term is a float64 bivariate-normal rectangle mass.  n_peers > 0 returns
- * FO_ERR_UNSUPPORTED.  Batches, fo_metric_bundle_host and fo_metric_stats take diagonal tables only. */
+ * FO_ERR_UNSUPPORTED.  Batches take correlated tables through their *_corr forms (fo_agents_pack_batch_corr, below);
+ * fo_metric_bundle_host, fo_metric_batch_host and fo_metric_stats take diagonal tables only. */
 size_t fo_agent_table_bytes_corr(int32_t n_agents, int32_t t_stride);
 int fo_agents_pack_corr(const FoAgentsRaw *raw, const float *cov_xy, const FoVehicle *vehicle, void *table_dev,
                         size_t table_bytes, void *stream);
@@ -262,6 +263,33 @@ int fo_agents_pack_batch_vehicles(const FoAgentsRaw *raw, int32_t n_problems, co
                                   const FoVehicle *vehicles_host, void *arena_dev, size_t arena_bytes, void *stream);
 int fo_metric_batch_vehicles(const FoMetricBatchArgs *args, const FoVehicle *vehicles_host, void *stream);
 int fo_metric_batch_detail_vehicles(const FoMetricBatchArgs *args, const FoVehicle *vehicles_host, void *stream);
+
+/* Correlated and diagonal problems in one batch (predictions with full 2x2 covariances, fo_agents_pack_corr).
+ * corr_host is a HOST array of n_problems flags: nonzero = problem p's table is a correlated one; vehicles_host is as in
+ * the *_vehicles calls.  Problem p's table and outputs equal, bit for bit, what fo_agents_pack_corr +
+ * fo_metric_bundle_corr (flagged) or fo_agents_pack + fo_metric_bundle (not flagged) give for it alone with its vehicle
+ * and FO_TEAM_WARPS set to the batch's team size W, chosen as in fo_metric_batch from all problems.  A NULL corr_host or
+ * vehicles_host with n_problems > 0 is FO_ERR_INVALID_ARG; every argument is validated before any device work, as in
+ * the calls above, with a flagged table checked against fo_agent_table_bytes_corr.
+ *
+ * fo_agent_batch_layout_corr: fo_agent_batch_layout, except that a flagged problem with agents takes
+ * fo_agent_table_bytes_corr bytes (rounded up to 16); with every flag 0 the same offsets and size.
+ * fo_agents_pack_batch_corr: fo_agents_pack_batch_vehicles plus one launch that writes the correlation sections of
+ * all flagged problems.  cov_xy is a device array [raw->n_agents, raw->t_stride] aligned with raw->var_x / var_y; it
+ * may be NULL when no flagged problem has agents.  The positive-definiteness precondition of fo_agents_pack_corr holds.
+ * fo_metric_batch_corr / fo_metric_batch_detail_corr: fo_metric_batch_vehicles / fo_metric_batch_detail_vehicles over
+ * such an arena, with their outputs, layout and checks.  The summary call makes one launch per non-empty class of
+ * problems (diagonal or correlated x window-filter or team shape), the detail call one per non-empty class (diagonal,
+ * correlated).  n_peers != 0 is FO_ERR_UNSUPPORTED; not capturable in a CUDA graph. */
+size_t fo_agent_batch_layout_corr(int32_t n_problems, const int32_t *n_agents_host, const int32_t *t_stride_host,
+                                  const uint8_t *corr_host, int64_t *table_offset_host);
+int fo_agents_pack_batch_corr(const FoAgentsRaw *raw, const float *cov_xy, int32_t n_problems,
+                              const FoBatchProblem *problems_host, const uint8_t *corr_host,
+                              const FoVehicle *vehicles_host, void *arena_dev, size_t arena_bytes, void *stream);
+int fo_metric_batch_corr(const FoMetricBatchArgs *args, const uint8_t *corr_host, const FoVehicle *vehicles_host,
+                         void *stream);
+int fo_metric_batch_detail_corr(const FoMetricBatchArgs *args, const uint8_t *corr_host, const FoVehicle *vehicles_host,
+                                void *stream);
 
 /* A batch driven from HOST buffers (pinned or pageable), for embedders without a CUDA runtime of their own: the
  * planner's float64 ego rows in the caller's world frame and one float64 origin per problem in, results in host arrays

@@ -182,6 +182,10 @@ _PROTOS = {
     "fo_metric_batch_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(FoAgentsRaw), C.c_int32,
                                        C.POINTER(FoBatchProblem), C.POINTER(FoVehicle), C.POINTER(FoMetricArgs),
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fo_metric_batch_host_corr": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(FoAgentsRaw),
+                                            C.c_void_p, C.c_int32, C.POINTER(FoBatchProblem), C.c_void_p,
+                                            C.POINTER(FoVehicle), C.POINTER(FoMetricArgs), C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_void_p]),
     "fo_visibility_raycast": (C.c_int, [C.POINTER(FoVisibilityArgs), C.c_void_p]),
     "fo_visibility_stats": (C.c_int, [C.POINTER(FoVisibilityArgs), C.c_void_p, C.c_void_p]),
     "fo_visibility_points": (C.c_int, [C.POINTER(FoPointQueryArgs), C.c_void_p]),

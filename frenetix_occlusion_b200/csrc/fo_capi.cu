@@ -274,11 +274,14 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
   return FO_OK;
 }
 
-extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int32_t n_states, const double* origins_host,
-                                    const FoAgentsRaw* ag, int32_t n_problems, const FoBatchProblem* problems_host,
-                                    const FoVehicle* vehicles_host, const FoMetricArgs* params, uint8_t* out_valid,
-                                    float* out_summary, uint32_t* out_flags, float* out_pair, float* out_step) {
-  const char* fn = "fo_metric_batch_host";
+// fo_metric_batch_host and fo_metric_batch_host_corr.  corr: NULL = every table diagonal (the diagonal pack and metric
+// calls); else corr[p] != 0 = problem p's table is a correlated one, its off-diagonal terms in cov_xy (host, aligned with
+// ag->var_x / var_y), and the *_corr pack and metric calls run.
+static int metric_batch_host_impl(const char* fn, const double* ego_host, int32_t n_traj, int32_t n_states,
+                                  const double* origins_host, const FoAgentsRaw* ag, const float* cov_xy, int32_t n_problems,
+                                  const FoBatchProblem* problems_host, const uint8_t* corr, const FoVehicle* vehicles_host,
+                                  const FoMetricArgs* params, uint8_t* out_valid, float* out_summary, uint32_t* out_flags,
+                                  float* out_pair, float* out_step) {
   const int P = n_problems;
   // ---- every check before any device work
   if (!params) { fo::set_error("%s: NULL params", fn); return FO_ERR_INVALID_ARG; }
@@ -288,15 +291,16 @@ extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int3
     return FO_ERR_INVALID_ARG;
   }
   if (n_traj > 0 && (!ego_host || !out_valid)) { fo::set_error("%s: NULL ego / out_valid", fn); return FO_ERR_INVALID_ARG; }
-  // The library owns the arena: problem p's table goes where fo_agent_batch_layout puts it.  Sizes out of range take no
-  // bytes here; the batch calls' own checks below reject them.
+  // The library owns the arena: problem p's table goes where fo_agent_batch_layout[_corr] puts it.  Sizes out of range
+  // take no bytes here; the batch calls' own checks below reject them.
   std::vector<FoBatchProblem> pr(P > 0 ? P : 0);
   size_t arena_bytes = 0;
   for (int p = 0; p < P; ++p) {
     pr[p] = problems_host[p];
     pr[p].table_offset = (int64_t)arena_bytes;
     const int A = pr[p].n_agents, Tp = pr[p].t_stride;
-    if (A > 0 && Tp > 0 && Tp <= FO_MAX_STATES) arena_bytes += (fo::agent_table_bytes(A, Tp) + 15) & ~(size_t)15;
+    if (A > 0 && Tp > 0 && Tp <= FO_MAX_STATES)
+      arena_bytes += ((corr && corr[p] ? fo::agent_table_bytes_corr(A, Tp) : fo::agent_table_bytes(A, Tp)) + 15) & ~(size_t)15;
   }
   // the workspace is not placed yet: an aligned stand-in takes the place of its buffers in the checks
   alignas(16) static float stand_in[4];
@@ -308,14 +312,37 @@ extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int3
   b.common.pair = b.common.step = nullptr;
   b.n_problems = P; b.problems = pr.data(); b.arena_bytes = arena_bytes;
   int n_run = 0, a_min = 0, n_packed = 0, max_cells = 0;
-  int rc = fo::check_batch(fn, &b, nullptr, false, &n_run, &a_min);
+  int rc = fo::check_batch(fn, &b, corr, false, &n_run, &a_min);
   if (rc != FO_OK) return rc;
   const FoAgentsRaw no_agents{};
-  rc = fo::check_pack_batch(fn, P > 0 ? ag : &no_agents, P, pr.data(), nullptr, stand_in, arena_bytes, &n_packed, &max_cells);
+  rc = fo::check_pack_batch(fn, P > 0 ? ag : &no_agents, P, pr.data(), corr, stand_in, arena_bytes, &n_packed, &max_cells);
   if (rc != FO_OK) return rc;
+  // The correlated problems with agents: their covariances are in host memory here, so the states the correlation pack
+  // reads (covariance i-1 of every state i < min(n_states, t_stride_p), as fo_agents_corr_kernel) are checked now, with
+  // its own predicate, and a covariance that would give NaN collision probabilities on the device is an error.
+  int n_corr = 0;
+  for (int p = 0, a0 = 0; corr && p < P; a0 += pr[p].n_agents, ++p) {
+    if (!corr[p] || pr[p].n_agents == 0) continue;
+    if (!cov_xy) { fo::set_error("%s: cov_xy must not be NULL with correlated problems (problem %d)", fn, p); return FO_ERR_INVALID_ARG; }
+    ++n_corr;
+    const int Tp = pr[p].t_stride;
+    for (int a = 0; a < pr[p].n_agents; ++a) {
+      const int n = ag->n_states[a0 + a] < Tp ? ag->n_states[a0 + a] : Tp;
+      const size_t row = (size_t)(a0 + a) * ag->t_stride;
+      for (int i = 0; i < n; ++i) {
+        const size_t ip = row + (i > 0 ? i - 1 : 0);
+        double sx, sy, rho;
+        if (!fo::corr_terms(ag->var_x[ip], ag->var_y[ip], cov_xy[ip], &sx, &sy, &rho)) {
+          fo::set_error("%s: problem %d, agent %d: covariance %d is not positive definite", fn, p, a, i > 0 ? i - 1 : 0);
+          return FO_ERR_INVALID_ARG;
+        }
+      }
+    }
+  }
   if (n_traj == 0) return FO_OK;
 
-  // ---- workspace: float64 rows, float32 bundle, raw agents, arena, per-problem ingest table, outputs
+  // ---- workspace: float64 rows, float32 bundle, raw agents (with cov_xy when correlated), arena, per-problem ingest
+  // table, outputs
   const size_t N = n_traj, T = n_states, A = ag->n_agents, S = ag->t_stride;
   long long pairs = 0;                           // sum of N_p A_p: the rows of the pair / step blocks
   for (int p = 0; p < P; ++p) pairs += (long long)pr[p].n_traj * pr[p].n_agents;
@@ -327,7 +354,9 @@ extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int3
   const size_t b_arena = al(arena_bytes), b_valid = al(N), b_sum = al(N * FO_SUMMARY_K * 4), b_flags = al(N * 4);
   const size_t b_pair = want_pair ? al((size_t)pairs * FO_PAIR_K * 4) : 0;
   const size_t b_step = want_step ? al((size_t)pairs * (T - 1) * FO_STEP_K * 4) : 0;
-  rc = fo::ws_reserve(b_e64 + b_e32 + 6 * b_f + 6 * b_a + b_idx + b_arena + b_valid + b_sum + b_flags + b_pair + b_step);
+  const size_t b_cov = corr ? b_f : 0;
+  rc = fo::ws_reserve(b_e64 + b_e32 + 6 * b_f + b_cov + 6 * b_a + b_idx + b_arena + b_valid + b_sum + b_flags + b_pair +
+                      b_step);
   if (rc != FO_OK) return rc;
   cudaStream_t st = fo::g_ws.stream;
   char* p = (char*)fo::g_ws.dev;
@@ -352,6 +381,8 @@ extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int3
     if (n_packed) FO_HOST_TRY(cudaMemcpyAsync(dp, asrc[i], A * 4, cudaMemcpyHostToDevice, st));
     *adst[i] = dp;
   }
+  float* d_cov = corr ? (float*)take(b_cov) : nullptr;
+  if (n_corr) FO_HOST_TRY(cudaMemcpyAsync(d_cov, cov_xy, A * S * 4, cudaMemcpyHostToDevice, st));
   // the ingest table: first rows and origins of the problems with trajectories
   std::vector<unsigned char> idx(b_first + (size_t)n_run * 16);
   int* first = (int*)idx.data();
@@ -366,10 +397,16 @@ extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int3
   char* d_idx = take(b_idx);
   FO_HOST_TRY(cudaMemcpyAsync(d_idx, idx.data(), idx.size(), cudaMemcpyHostToDevice, st));
   void* d_arena = take(b_arena);
+  // the *_corr calls take one vehicle per problem: params->vehicle for every one unless the caller gives them
+  std::vector<FoVehicle> shared(corr && !vehicles_host ? P : 0, params->vehicle);
+  const FoVehicle* veh = corr && !vehicles_host ? shared.data() : vehicles_host;
   if (n_packed) {
-    rc = vehicles_host
-             ? fo_agents_pack_batch_vehicles(&d, P, pr.data(), vehicles_host, d_arena, arena_bytes, st)
-             : fo_agents_pack_batch(&d, P, pr.data(), &params->vehicle, d_arena, arena_bytes, st);
+    if (corr)
+      rc = fo_agents_pack_batch_corr(&d, n_corr ? d_cov : nullptr, P, pr.data(), corr, veh, d_arena, arena_bytes, st);
+    else
+      rc = vehicles_host
+               ? fo_agents_pack_batch_vehicles(&d, P, pr.data(), vehicles_host, d_arena, arena_bytes, st)
+               : fo_agents_pack_batch(&d, P, pr.data(), &params->vehicle, d_arena, arena_bytes, st);
     if (rc != FO_OK) return fo::ws_fail(rc);
   }
 
@@ -397,7 +434,9 @@ extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int3
   b.common.flags = (uint32_t*)take(b_flags);
   b.common.pair = want_pair ? (float*)take(b_pair) : nullptr;
   b.common.step = want_step ? (float*)take(b_step) : nullptr;
-  if (want_pair || want_step)
+  if (corr)
+    rc = (want_pair || want_step) ? fo_metric_batch_detail_corr(&b, corr, veh, st) : fo_metric_batch_corr(&b, corr, veh, st);
+  else if (want_pair || want_step)
     rc = vehicles_host ? fo_metric_batch_detail_vehicles(&b, vehicles_host, st) : fo_metric_batch_detail(&b, st);
   else
     rc = vehicles_host ? fo_metric_batch_vehicles(&b, vehicles_host, st) : fo_metric_batch(&b, st);
@@ -414,4 +453,25 @@ extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int3
     FO_HOST_TRY(cudaMemcpyAsync(out_step, b.common.step, (size_t)pairs * (T - 1) * FO_STEP_K * 4, cudaMemcpyDeviceToHost, st));
   FO_HOST_TRY(cudaStreamSynchronize(st));
   return FO_OK;
+}
+
+extern "C" int fo_metric_batch_host(const double* ego_host, int32_t n_traj, int32_t n_states, const double* origins_host,
+                                    const FoAgentsRaw* ag, int32_t n_problems, const FoBatchProblem* problems_host,
+                                    const FoVehicle* vehicles_host, const FoMetricArgs* params, uint8_t* out_valid,
+                                    float* out_summary, uint32_t* out_flags, float* out_pair, float* out_step) {
+  return metric_batch_host_impl("fo_metric_batch_host", ego_host, n_traj, n_states, origins_host, ag, nullptr, n_problems,
+                                problems_host, nullptr, vehicles_host, params, out_valid, out_summary, out_flags, out_pair,
+                                out_step);
+}
+
+extern "C" int fo_metric_batch_host_corr(const double* ego_host, int32_t n_traj, int32_t n_states,
+                                         const double* origins_host, const FoAgentsRaw* ag, const float* cov_xy_host,
+                                         int32_t n_problems, const FoBatchProblem* problems_host, const uint8_t* corr_host,
+                                         const FoVehicle* vehicles_host, const FoMetricArgs* params, uint8_t* out_valid,
+                                         float* out_summary, uint32_t* out_flags, float* out_pair, float* out_step) {
+  const char* fn = "fo_metric_batch_host_corr";
+  if (n_problems > 0 && !corr_host) { fo::set_error("%s: corr_host must not be NULL", fn); return FO_ERR_INVALID_ARG; }
+  // (with no problems there is nothing to assess: NULL flags reach no pack or metric call)
+  return metric_batch_host_impl(fn, ego_host, n_traj, n_states, origins_host, ag, cov_xy_host, n_problems, problems_host,
+                                corr_host, vehicles_host, params, out_valid, out_summary, out_flags, out_pair, out_step);
 }

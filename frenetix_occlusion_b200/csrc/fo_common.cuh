@@ -111,4 +111,15 @@ __host__ __device__ inline const float4* agent_corr_view(const void* base, int A
   return reinterpret_cast<const float4*>(reinterpret_cast<const unsigned char*>(base) + agent_corr_offset(A, Tp));
 }
 
+// sigma_x, sigma_y and rho of the covariance [[vx, c], [c, vy]] in float64, the all-zero matrix taken as 0.1 I
+// (collision_probability.py:85-87); true when it is positive definite (|rho| < 1).  The one predicate of both places
+// that look at it: fo_agents_corr_kernel writes rho = NaN where it is false, fo_metric_batch_host_corr rejects the call.
+__host__ __device__ inline bool corr_terms(float vx, float vy, float c, double* sx, double* sy, double* rho) {
+  if (vx == 0.0f && vy == 0.0f && c == 0.0f) { vx = 0.1f; vy = 0.1f; }
+  *sx = sqrt((double)vx);
+  *sy = sqrt((double)vy);
+  *rho = (double)c / (*sx * *sy);
+  return fabs(*rho) < 1.0;
+}
+
 }  // namespace fo

@@ -174,12 +174,8 @@ __global__ void fo_agents_corr_kernel(FoAgentsRaw raw, const float* __restrict__
     float4 o = make_float4(1, 1, 0, 0);
     if (i < raw.n_states[pp.a_begin + a]) {
       const size_t r = ((size_t)pp.a_begin + a) * raw.t_stride + i, ip = i > 0 ? r - 1 : r;
-      float vx = raw.var_x[ip], vy = raw.var_y[ip];
-      const float c = cov_xy[ip];
-      if (vx == 0.0f && vy == 0.0f && c == 0.0f) { vx = 0.1f; vy = 0.1f; }   // collision_probability.py:85-87
-      const double sx = sqrt((double)vx), sy = sqrt((double)vy);
-      double rho = (double)c / (sx * sy);
-      if (!(fabs(rho) < 1.0)) rho = CUDART_NAN;
+      double sx, sy, rho;
+      if (!corr_terms(raw.var_x[ip], raw.var_y[ip], cov_xy[ip], &sx, &sy, &rho)) rho = CUDART_NAN;
       o = make_float4((float)(1.0 / sx), (float)(1.0 / sy), (float)rho, 0.0f);
     }
     const_cast<float4*>(agent_corr_view(table, A, Tp))[(size_t)slot[a] * Tp + i] = o;

@@ -174,8 +174,9 @@ int fo_metric_stats(const FoMetricArgs *args, uint64_t *counters_dev, void *stre
  * that violates it (|rho| >= 1, a zero variance with a non-zero covariance) gets NaN collision probabilities.
  * fo_metric_bundle_corr: fo_metric_bundle on a table written by fo_agents_pack_corr, with its outputs, checks and
  * CUDA-graph capture behaviour.  Each CP term is a float64 bivariate-normal rectangle mass.  n_peers > 0 returns
- * FO_ERR_UNSUPPORTED.  Batches take correlated tables through their *_corr forms (fo_agents_pack_batch_corr, below);
- * fo_metric_bundle_host, fo_metric_batch_host and fo_metric_stats take diagonal tables only. */
+ * FO_ERR_UNSUPPORTED.  Batches take correlated tables through their *_corr forms (fo_agents_pack_batch_corr, below), and
+ * so do batches from host memory (fo_metric_batch_host_corr, below); fo_metric_bundle_host, fo_metric_batch_host and
+ * fo_metric_stats take diagonal tables only. */
 size_t fo_agent_table_bytes_corr(int32_t n_agents, int32_t t_stride);
 int fo_agents_pack_corr(const FoAgentsRaw *raw, const float *cov_xy, const FoVehicle *vehicle, void *table_dev,
                         size_t table_bytes, void *stream);
@@ -318,6 +319,31 @@ int fo_metric_batch_host(const double *ego_host, int32_t n_traj, int32_t n_state
                          const FoAgentsRaw *agents_host, int32_t n_problems, const FoBatchProblem *problems_host,
                          const FoVehicle *vehicles_host, const FoMetricArgs *params, uint8_t *out_valid,
                          float *out_summary, uint32_t *out_flags, float *out_pair, float *out_step);
+
+/* fo_metric_batch_host with correlated predictions (full 2x2 covariances), for host-memory embedders: the arguments,
+ * outputs, float64 ingest, workspace and checks of fo_metric_batch_host, plus
+ *   cov_xy_host   [agents_host->n_agents, agents_host->t_stride] float32, the off-diagonal term of every covariance,
+ *                 aligned with var_x / var_y (cov_list[..., 0, 1] of the reference); may be NULL when no flagged problem
+ *                 has agents
+ *   corr_host     [n_problems]: nonzero = problem p is correlated (no effect on a problem without agents); NULL with
+ *                 n_problems > 0 is FO_ERR_INVALID_ARG
+ * Tables are placed as fo_agent_batch_layout_corr places them and packed by fo_agents_pack_batch_corr; the metric call is
+ * fo_metric_batch_corr, or fo_metric_batch_detail_corr under fo_metric_batch_host's rule for the detail path, with
+ * vehicles_host or, when it is NULL, params->vehicle for every problem.  The results equal, bit for bit, those calls on
+ * the bundle fo_metric_batch_host's ingest produces.  One correlated planner is the case n_problems = 1: its team size is
+ * the one fo_metric_bundle_corr picks, so it gets fo_agents_pack_corr + fo_metric_bundle_corr bit for bit.
+ * The covariances are checked on the host before any device work: every covariance the correlation pack reads (covariance
+ * i-1 of every state i < min(n_states[a], t_stride_p) of a flagged problem's agents; state 0 reads covariance 0) must be
+ * positive definite by the predicate under which fo_agents_pack_corr writes NaN -- the all-zero matrix is 0.1 I, and
+ * otherwise |cov_xy / sqrt(var_x var_y)| < 1 in float64 -- else FO_ERR_INVALID_ARG names the problem, the agent within it
+ * and the covariance index.  This rejects a state with one zero variance and zero covariance, which the reference's
+ * diagonal rule accepts but which gives NaN collision probabilities on the correlated path.  Covariances the pack never
+ * reads (index n_states - 1, the padding up to t_stride) are not checked.  n_peers != 0 is FO_ERR_UNSUPPORTED. */
+int fo_metric_batch_host_corr(const double *ego_host, int32_t n_traj, int32_t n_states, const double *origins_host,
+                              const FoAgentsRaw *agents_host, const float *cov_xy_host, int32_t n_problems,
+                              const FoBatchProblem *problems_host, const uint8_t *corr_host,
+                              const FoVehicle *vehicles_host, const FoMetricArgs *params, uint8_t *out_valid,
+                              float *out_summary, uint32_t *out_flags, float *out_pair, float *out_step);
 
 
 /* ---- stage 1: sensor visibility by ray casting ----------------------------------------------------

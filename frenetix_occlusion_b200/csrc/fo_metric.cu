@@ -558,6 +558,13 @@ static void fill_kargs(const FoMetricArgs* a, fo::MetricKArgs& k) {
 
 static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, void* stream, bool corr = false);
 
+// Peer stores: n_peers in [0, FO_MAX_PEERS], and only on the summary path (no pair / step, no work counters).
+static int check_peers(const char* fn, const FoMetricArgs* a, bool stats) {
+  if (a->n_peers < 0 || a->n_peers > FO_MAX_PEERS) { fo::set_error("%s: n_peers %d outside [0, %d]", fn, a->n_peers, FO_MAX_PEERS); return FO_ERR_INVALID_ARG; }
+  if (a->n_peers > 0 && (a->pair || a->step || stats)) { fo::set_error("%s: peer stores exist on the summary path only", fn); return FO_ERR_UNSUPPORTED; }
+  return FO_OK;
+}
+
 extern "C" int fo_metric_bundle(const FoMetricArgs* a, void* stream) { return metric_bundle_impl(a, nullptr, stream); }
 
 extern "C" int fo_metric_bundle_corr(const FoMetricArgs* a, void* stream) {
@@ -565,11 +572,25 @@ extern "C" int fo_metric_bundle_corr(const FoMetricArgs* a, void* stream) {
   return metric_bundle_impl(a, nullptr, stream, true);
 }
 
-extern "C" int fo_metric_stats(const FoMetricArgs* a, uint64_t* counters_dev, void* stream) {
-  if (!counters_dev) { fo::set_error("fo_metric_stats: counters_dev must not be NULL"); return FO_ERR_INVALID_ARG; }
-  if (a && (a->pair || a->step)) { fo::set_error("fo_metric_stats: summary outputs only"); return FO_ERR_INVALID_ARG; }
+// The peer checks run here before any device query, so a bad n_peers is reported without a device.
+extern "C" int fo_metric_bundle_corr_peers(const FoMetricArgs* a, void* stream) {
+  const int rc = a ? check_peers("fo_metric_bundle_corr_peers", a, false) : FO_OK;
+  return rc != FO_OK ? rc : metric_bundle_impl(a, nullptr, stream, true);
+}
+
+static int metric_stats_impl(const char* fn, const FoMetricArgs* a, uint64_t* counters_dev, void* stream, bool corr) {
+  if (!counters_dev) { fo::set_error("%s: counters_dev must not be NULL", fn); return FO_ERR_INVALID_ARG; }
+  if (a && (a->pair || a->step)) { fo::set_error("%s: summary outputs only", fn); return FO_ERR_INVALID_ARG; }
   FO_CUDA_TRY(cudaMemsetAsync(counters_dev, 0, FO_STATS_K * sizeof(uint64_t), (cudaStream_t)stream));
-  return metric_bundle_impl(a, reinterpret_cast<unsigned long long*>(counters_dev), stream);
+  return metric_bundle_impl(a, reinterpret_cast<unsigned long long*>(counters_dev), stream, corr);
+}
+
+extern "C" int fo_metric_stats(const FoMetricArgs* a, uint64_t* counters_dev, void* stream) {
+  return metric_stats_impl("fo_metric_stats", a, counters_dev, stream, false);
+}
+
+extern "C" int fo_metric_stats_corr(const FoMetricArgs* a, uint64_t* counters_dev, void* stream) {
+  return metric_stats_impl("fo_metric_stats_corr", a, counters_dev, stream, true);
 }
 
 static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, void* stream, bool corr) {
@@ -595,8 +616,7 @@ static int metric_bundle_impl(const FoMetricArgs* a, unsigned long long* stats, 
   fill_kargs(a, k);
   k.stats = stats;
   if (a->summary && (reinterpret_cast<uintptr_t>(a->summary) & 7u)) { fo::set_error("fo_metric_bundle: summary must be 8-byte aligned"); return FO_ERR_INVALID_ARG; }
-  if (a->n_peers < 0 || a->n_peers > FO_MAX_PEERS) { fo::set_error("fo_metric_bundle: n_peers %d outside [0, %d]", a->n_peers, FO_MAX_PEERS); return FO_ERR_INVALID_ARG; }
-  if (a->n_peers > 0 && (a->pair || a->step || stats)) { fo::set_error("fo_metric_bundle: peer stores exist on the summary path only"); return FO_ERR_UNSUPPORTED; }
+  { const int rc = check_peers("fo_metric_bundle", a, stats != nullptr); if (rc != FO_OK) return rc; }
   k.n_peers = a->n_peers;
   for (int p = 0; p < FO_MAX_PEERS; ++p) k.peer_delta[p] = p < a->n_peers ? (long long)a->peer_delta[p] : 0;
   k.corr = corr;

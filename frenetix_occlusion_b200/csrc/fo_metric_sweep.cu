@@ -844,6 +844,15 @@ fo_metric_sweep_corr_kernel(const __grid_constant__ MetricKArgs k, const SweepSh
   sweep_body<0u, false, UNI, TIES, false, true>(k, shape, BatchView{}, threadIdx.x, blockDim.x);
 }
 
+// Work counters on correlated tables (fo_metric_stats_corr): fo_metric_sweep_corr_kernel with the counters of
+// fo_metric_sweep_kernel<0, true>.  They count geometric work and queue items only, so on the same geometry they equal
+// the diagonal table's (DESIGN.md 5.13: where the team shape's warp order makes some of them vary, on both tables).
+template <bool UNI, bool TIES>
+__global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
+fo_metric_sweep_corr_stats_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape) {
+  sweep_body<0u, true, UNI, TIES, false, true>(k, shape, BatchView{}, threadIdx.x, blockDim.x);
+}
+
 // One shape class of a batch of independent problems (fo_metric_batch): k.N is the class's trajectory count, k.tab / k.A
 // / k.Tp / k.veh and shape.lg_agents are unused -- every trajectory takes them from its problem.
 template <uint32_t MASK, bool UNI, bool TIES>
@@ -977,6 +986,12 @@ int launch_metric_sweep(const MetricKArgs& k, int num_sms, cudaStream_t st) {
     pick_shape(k, num_sms, W, shape);
     const bool ties = needs_ties(k);
     const bool uni = W == 1 && shape.lg_agents == 5;
+    if (k.stats) {
+      if (uni) return ties ? launch_team_kernel<fo_metric_sweep_corr_stats_kernel<true, true>>(k, num_sms, W, uni, ties, st, shape)
+                           : launch_team_kernel<fo_metric_sweep_corr_stats_kernel<true, false>>(k, num_sms, W, uni, ties, st, shape);
+      return ties ? launch_team_kernel<fo_metric_sweep_corr_stats_kernel<false, true>>(k, num_sms, W, uni, ties, st, shape)
+                  : launch_team_kernel<fo_metric_sweep_corr_stats_kernel<false, false>>(k, num_sms, W, uni, ties, st, shape);
+    }
     if (uni) return ties ? launch_team_kernel<fo_metric_sweep_corr_kernel<true, true>>(k, num_sms, W, uni, ties, st, shape)
                          : launch_team_kernel<fo_metric_sweep_corr_kernel<true, false>>(k, num_sms, W, uni, ties, st, shape);
     return ties ? launch_team_kernel<fo_metric_sweep_corr_kernel<false, true>>(k, num_sms, W, uni, ties, st, shape)

@@ -328,13 +328,20 @@ class MetricEngine:
                 a.peer_delta[i] = int(d)
         return a
 
-    def work_stats(self, ego) -> dict:
+    def work_stats(self, ego, correlated: bool = False) -> dict:
         """How much of the algorithmic work survives the exact bounds (``fo_metric_stats``): counts of visited
         (trajectory, agent, step) evaluations, exact box distances, LR4S logits, CP evaluations, BE pairs and pair
         tests (probes), BE tree nodes walked and re-timed ego-path chunks computed for one pass over ``ego``.  Used by
-        bench.py's flop model; synchronises.  Diagonal covariances only."""
-        if self.agents is not None and self.agents.cov_xy is not None and self.n_agents > 0:
-            raise ValueError("work_stats() takes diagonal prediction covariances only")
+        bench.py's flop model; synchronises.
+
+        ``correlated``: a set with correlated prediction covariances is counted by ``fo_metric_stats_corr``, which costs
+        one pass of the correlated summary path (many times the diagonal one, DESIGN.md §5.10).  The counters do not
+        depend on the covariances, so they equal those of the same set with ``cov_xy = None`` (in multi-warp team shapes
+        "obb", "lr4s", "be" and "be_probes" vary from run to run on either path, DESIGN.md §5.13).  Without the flag
+        such a set raises ``ValueError``; with it a diagonal set is counted exactly as without it."""
+        corr = self.agents is not None and self.agents.cov_xy is not None and self.n_agents > 0
+        if corr and not correlated:
+            raise ValueError("work_stats() takes diagonal prediction covariances only unless correlated=True")
         t = self.to_device_bundle(ego)
         N = int(t.shape[0])
         dev = self.device
@@ -345,7 +352,8 @@ class MetricEngine:
                                torch.empty(N, dtype=torch.int32, device=dev))
             a = self._args(t, out)
             cnt = torch.zeros(10, dtype=torch.int64, device=dev)   # FO_STATS_K
-            L.check(L.lib.fo_metric_stats(C.byref(a), C.c_void_p(cnt.data_ptr()), self._stream()), "fo_metric_stats")
+            fn = "fo_metric_stats_corr" if self._corr else "fo_metric_stats"
+            L.check(getattr(L.lib, fn)(C.byref(a), C.c_void_p(cnt.data_ptr()), self._stream()), fn)
             c = cnt.cpu().tolist()
         return {"visited": c[0], "obb": c[1], "lr4s": c[2], "cp": c[3], "be": c[4], "be_probes": c[5],
                 "windows": c[6], "windows_kept": c[7], "be_nodes": c[8], "be_path_chunks": c[9]}
@@ -374,7 +382,9 @@ class MetricEngine:
             a = self._args(t, out)
             a.pair = out.pair.data_ptr() if (out.pair is not None and A > 0) else None
             a.step = out.step.data_ptr() if (out.step is not None and A > 0 and T > 1) else None
-            fn = "fo_metric_bundle_corr" if self._corr else "fo_metric_bundle"
+            # a correlated table with peer stores (parallel.PeerResultGatherer) takes the call that honours them
+            fn = ("fo_metric_bundle_corr_peers" if out.peer_delta else "fo_metric_bundle_corr") if self._corr \
+                else "fo_metric_bundle"
             L.check(getattr(L.lib, fn)(C.byref(a), self._stream()), fn)
         out._keepalive = t
         return out

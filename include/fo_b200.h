@@ -174,13 +174,27 @@ int fo_metric_stats(const FoMetricArgs *args, uint64_t *counters_dev, void *stre
  * that violates it (|rho| >= 1, a zero variance with a non-zero covariance) gets NaN collision probabilities.
  * fo_metric_bundle_corr: fo_metric_bundle on a table written by fo_agents_pack_corr, with its outputs, checks and
  * CUDA-graph capture behaviour.  Each CP term is a float64 bivariate-normal rectangle mass.  n_peers > 0 returns
- * FO_ERR_UNSUPPORTED.  Batches take correlated tables through their *_corr forms (fo_agents_pack_batch_corr, below), and
- * so do batches from host memory (fo_metric_batch_host_corr, below); fo_metric_bundle_host, fo_metric_batch_host and
- * fo_metric_stats take diagonal tables only. */
+ * FO_ERR_UNSUPPORTED; fo_metric_bundle_corr_peers (below) takes peer stores.  fo_metric_stats_corr (below) gives the work
+ * counters of a correlated table.  Batches take correlated tables through their *_corr forms (fo_agents_pack_batch_corr,
+ * below), and so do batches from host memory (fo_metric_batch_host_corr, below); fo_metric_bundle_host,
+ * fo_metric_batch_host and fo_metric_stats take diagonal tables only. */
 size_t fo_agent_table_bytes_corr(int32_t n_agents, int32_t t_stride);
 int fo_agents_pack_corr(const FoAgentsRaw *raw, const float *cov_xy, const FoVehicle *vehicle, void *table_dev,
                         size_t table_bytes, void *stream);
 int fo_metric_bundle_corr(const FoMetricArgs *args, void *stream);
+
+/* fo_metric_bundle_corr with the fused result exchange of a trajectory-sharded sweep: n_peers / peer_delta are honoured
+ * on the summary path as fo_metric_bundle honours them.  n_peers outside [0, FO_MAX_PEERS] is FO_ERR_INVALID_ARG and
+ * n_peers > 0 with pair / step is FO_ERR_UNSUPPORTED, both checked before any device query; with n_peers = 0 it is
+ * fo_metric_bundle_corr. */
+int fo_metric_bundle_corr_peers(const FoMetricArgs *args, void *stream);
+
+/* fo_metric_stats on a table written by fo_agents_pack_corr: the same checks, zeroed counters, summary outputs only and
+ * no peers.  The FO_STATS_K counters do not depend on the covariances (gate, window filter, BE pairs, probes and tree
+ * walk, drained CP items), so they equal fo_metric_stats' on the diagonal table of the same agents.  (With a team of
+ * W > 1 warps the box-distance, LR4S, BE-pair and BE-probe counts depend on the order in which the warps pool their
+ * work, and vary from run to run on either table; the others do not.)  Costs one pass of the correlated summary path. */
+int fo_metric_stats_corr(const FoMetricArgs *args, uint64_t *counters_dev, void *stream);
 
 /* Same computation driven from HOST buffers (pinned or pageable): copies ego / agents to the
  * device, runs fo_agents_pack + fo_metric_bundle, copies valid/summary/flags back and synchronises.

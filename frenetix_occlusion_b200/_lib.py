@@ -17,6 +17,7 @@ FO_MAX_PEERS = 8
 FO_SUMMARY_K = 10
 FO_PAIR_K = 12
 FO_STEP_K = 3
+FO_VALID_SKIPPED = 2     # fo_metric_batch_select: a row ranked after its problem's first valid row, not assessed
 
 # metric bits (FO_M_*), threshold bits (FO_T_*), kinds (FO_KIND_*), flags (FO_F_*)
 M_BITS = {"cp": 1 << 0, "dce": 1 << 1, "ttc": 1 << 2, "hr": 1 << 3, "be": 1 << 4, "ttce": 1 << 5, "wttc": 1 << 6}
@@ -181,6 +182,8 @@ _PROTOS = {
     "fo_metric_batch_corr": (C.c_int, [C.POINTER(FoMetricBatchArgs), C.c_void_p, C.POINTER(FoVehicle), C.c_void_p]),
     "fo_metric_batch_detail_corr": (C.c_int, [C.POINTER(FoMetricBatchArgs), C.c_void_p, C.POINTER(FoVehicle),
                                               C.c_void_p]),
+    "fo_metric_batch_select": (C.c_int, [C.POINTER(FoMetricBatchArgs), C.c_void_p, C.POINTER(FoVehicle), C.c_void_p,
+                                         C.c_void_p]),
     "fo_metric_batch_host": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(FoAgentsRaw), C.c_int32,
                                        C.POINTER(FoBatchProblem), C.POINTER(FoVehicle), C.POINTER(FoMetricArgs),
                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -6,7 +6,8 @@ metric launch each), ``assess_interfaces`` packs the phantom agents of all inter
 ``fo_agents_pack_batch`` call and evaluates all candidate bundles with one ``fo_metric_batch`` (or, with pair / step
 detail, ``fo_metric_batch_detail``) call -- their ``_corr`` forms when some interface's predictions carry correlated
 covariances, which are then assessed as that interface assesses them.  ``prefetch_interfaces`` does the same for the reference's per-trajectory
-protocol: it is ``prefetch_assessments`` for all interfaces at once.
+protocol: it is ``prefetch_assessments`` for all interfaces at once, and ``select_interfaces`` gives each interface the
+first candidate that passes, as ``FOInterface.select_trajectory`` does.
 """
 from __future__ import annotations
 
@@ -150,4 +151,24 @@ def prefetch_interfaces(interfaces: Sequence, candidates: Sequence) -> list:
     return counts
 
 
-__all__ = ["assess_interfaces", "prefetch_interfaces", "BundleResult"]
+def select_interfaces(interfaces: Sequence, candidates: Sequence) -> list:
+    """``interfaces[i].select_trajectory(candidates[i])`` for every interface in one pack and one
+    ``fo_metric_batch_select`` call: per interface the index of the first candidate (in the order given, the planner's
+    cost order) that passes, or None when none does.  Configuration rule, vehicles, covariances and ``ValueError`` as in
+    ``assess_interfaces``; an interface without phantom agents or metrics gets 0 (None for no candidates).  Synchronises
+    on one int per interface; no interface's state, cache or prefetch is touched."""
+    interfaces, candidates = list(interfaces), list(candidates)
+    if len(interfaces) != len(candidates):
+        raise ValueError(f"{len(interfaces)} interfaces but {len(candidates)} candidate lists")
+    if not interfaces:
+        return []
+    egos = [_bundle_array(c) if len(c) else np.zeros((0, 1, 5)) for c in candidates]
+    eng = _batch_engine(interfaces, egos)
+    agents = [_agents(fi) for fi in interfaces]
+    eng.set_agent_batch([a for a, _ in agents], [o for _, o in agents], vehicles=_vehicles(interfaces), correlated=True)
+    r = eng.select_batch(egos)
+    sel = r.selected.cpu().numpy()
+    return [int(k) if k < n else None for k, n in zip(sel, np.diff(r.offsets))]
+
+
+__all__ = ["assess_interfaces", "prefetch_interfaces", "select_interfaces", "BundleResult"]

@@ -2,7 +2,9 @@
 #include <math.h>
 #include <stdlib.h>
 
+#include <algorithm>
 #include <atomic>
+#include <vector>
 
 #include "fo_metric_dev.cuh"
 
@@ -688,46 +690,55 @@ int fo::check_batch(const char* fn, const FoMetricBatchArgs* b, const uint8_t* c
   return FO_OK;
 }
 
+// The staged descriptors of a summary batch call (metric_batch_impl, metric_batch_select_impl): one team size for the
+// whole batch, as fo_metric_bundle picks it; with W = 1 problems with >= 17 agents run the window-filter shape, the
+// others the team shape with their own lane grouping.  Classes: 0 / 1 diagonal window-filter / team shape, 2 / 3 the
+// same for correlated tables; one launch per non-empty class, each numbering its trajectories.
+struct BatchStage {
+  int W = 1;
+  int cnt[4] = {0, 0, 0, 0}, start[4] = {0, 0, 0, 0}, n_cls[4] = {0, 0, 0, 0};
+  fo::StageSlot* slot = nullptr;
+  size_t prob_off = 0;              // offset of the descriptors behind first[]
+  size_t bytes = 0;                 // first[] and the descriptors; a caller's own data follows at this offset
+  std::vector<int> problem;         // problem of each descriptor
+};
+
 // vehicles: problem p's ego vehicle is vehicles[p]; NULL = common.vehicle for every problem.  corr: problem p's table is a
-// correlated one when corr[p] != 0; NULL = none is.
-static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles,
-                             void* stream) {
-  int n_run = 0, a_min = 0;
-  {
-    const int rc = fo::check_batch(fn, b, corr, false, &n_run, &a_min);
-    if (rc != FO_OK || b->common.n_traj == 0) return rc;
-  }
+// correlated one when corr[p] != 0; NULL = none is.  by_size: within a class the descriptors are sorted by N_p in
+// descending order (stable), else they are in problem order.  Stages first[] of all classes, then their descriptors
+// (16-byte aligned), class by class, and reserves extra_bytes behind them; the caller uploads.
+static int stage_batch(const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles, int n_run, int a_min,
+                       int num_sms, bool by_size, size_t extra_bytes, BatchStage& s) {
   const FoMetricArgs& c = b->common;
   const int P = b->n_problems;
-  int num_sms = 0;
-  { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
-  // one team size for the whole batch, as fo_metric_bundle picks it; with W = 1 problems with >= 17 agents run the
-  // window-filter shape, the others the team shape with their own lane grouping.  Classes: 0 / 1 diagonal window-filter
-  // / team shape, 2 / 3 the same for correlated tables; one launch per non-empty class, each numbering its trajectories
-  const int W = fo::pick_team_warps(c.n_traj, c.n_states, a_min, num_sms);
+  s.W = fo::pick_team_warps(c.n_traj, c.n_states, a_min, num_sms);
   const auto class_of = [&](int p) {
-    return (corr && corr[p] ? 2 : 0) + (W == 1 && fo::lane_group_log2(b->problems[p].n_agents) == 5 ? 0 : 1);
+    return (corr && corr[p] ? 2 : 0) + (s.W == 1 && fo::lane_group_log2(b->problems[p].n_agents) == 5 ? 0 : 1);
   };
-  int cnt[4] = {0, 0, 0, 0};
+  s.problem.clear();
   for (int p = 0; p < P; ++p)
-    if (b->problems[p].n_traj > 0) ++cnt[class_of(p)];
-  const int start[4] = {0, cnt[0], cnt[0] + cnt[1], cnt[0] + cnt[1] + cnt[2]};
-  // staged: first[] of all classes, then their descriptors (16-byte aligned), class by class
-  const size_t first_bytes = ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15;
-  const size_t bytes = first_bytes + (size_t)n_run * sizeof(fo::BatchProb);
-  fo::StageSlot* slot = nullptr;
-  int rc = fo::stage_acquire(bytes, &slot);
+    if (b->problems[p].n_traj > 0) {
+      ++s.cnt[class_of(p)];
+      s.problem.push_back(p);
+    }
+  std::stable_sort(s.problem.begin(), s.problem.end(), [&](int p, int q) {
+    const int cp = class_of(p), cq = class_of(q);
+    if (cp != cq) return cp < cq;
+    return by_size && b->problems[p].n_traj > b->problems[q].n_traj;
+  });
+  s.start[1] = s.cnt[0]; s.start[2] = s.start[1] + s.cnt[1]; s.start[3] = s.start[2] + s.cnt[2];
+  s.prob_off = ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15;
+  s.bytes = s.prob_off + (size_t)n_run * sizeof(fo::BatchProb);
+  int rc = fo::stage_acquire(s.bytes + extra_bytes, &s.slot);
   if (rc != FO_OK) return rc;
-  int* first = reinterpret_cast<int*>(slot->host);
-  fo::BatchProb* prob = reinterpret_cast<fo::BatchProb*>(slot->host + first_bytes);
+  int* first = reinterpret_cast<int*>(s.slot->host);
+  fo::BatchProb* prob = reinterpret_cast<fo::BatchProb*>(s.slot->host + s.prob_off);
   const unsigned char* arena = reinterpret_cast<const unsigned char*>(c.agent_table);
-  int next[4] = {start[0], start[1], start[2], start[3]}, n_cls[4] = {0, 0, 0, 0};
-  for (int p = 0; p < P; ++p) {
+  for (int i = 0; i < n_run; ++i) {
+    const int p = s.problem[i];
     const FoBatchProblem& q = b->problems[p];
-    if (q.n_traj == 0) continue;
     const int cl = class_of(p);
-    const int i = next[cl]++;
-    int& n = n_cls[cl];
+    int& n = s.n_cls[cl];
     fo::BatchProb& d = prob[i];
     const int Tp = q.n_agents > 0 ? q.t_stride : 1;
     const unsigned char* tab = arena + (q.n_agents > 0 ? q.table_offset : 0);
@@ -739,24 +750,113 @@ static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const u
     first[i] = n;
     n += q.n_traj;
   }
-  cudaStream_t st = (cudaStream_t)stream;
-  rc = fo::stage_upload(slot, bytes, st);
-  if (rc != FO_OK) return rc;
-  fo::MetricKArgs k;
+  return FO_OK;
+}
+
+// Kernel arguments shared by the classes of a summary batch call: the tables are per problem.
+static void batch_kargs(const FoMetricArgs& c, fo::MetricKArgs& k) {
   FoMetricArgs ca = c;
-  ca.n_agents = 0;                           // per problem
+  ca.n_agents = 0;
   ca.agent_table = nullptr;
   fill_kargs(&ca, k);
-  const int* first_dev = reinterpret_cast<const int*>(slot->dev);
-  const fo::BatchProb* prob_dev = reinterpret_cast<const fo::BatchProb*>(slot->dev + first_bytes);
+}
+
+static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles,
+                             void* stream) {
+  int n_run = 0, a_min = 0;
+  {
+    const int rc = fo::check_batch(fn, b, corr, false, &n_run, &a_min);
+    if (rc != FO_OK || b->common.n_traj == 0) return rc;
+  }
+  int num_sms = 0;
+  { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
+  BatchStage s;
+  int rc = stage_batch(b, corr, vehicles, n_run, a_min, num_sms, false, 0, s);
+  if (rc != FO_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = fo::stage_upload(s.slot, s.bytes, st);
+  if (rc != FO_OK) return rc;
+  fo::MetricKArgs k;
+  batch_kargs(b->common, k);
+  const int* first_dev = reinterpret_cast<const int*>(s.slot->dev);
+  const fo::BatchProb* prob_dev = reinterpret_cast<const fo::BatchProb*>(s.slot->dev + s.prob_off);
   for (int cl = 0; cl < 4; ++cl) {
-    if (cnt[cl] == 0) continue;
-    k.N = n_cls[cl];
+    if (s.cnt[cl] == 0) continue;
+    k.N = s.n_cls[cl];
     k.corr = cl >= 2;
-    rc = fo::launch_metric_batch(k, num_sms, W, (cl & 1) == 0, fo::BatchView{first_dev + start[cl], prob_dev + start[cl], cnt[cl]}, st);
+    rc = fo::launch_metric_batch(k, num_sms, s.W, (cl & 1) == 0, fo::BatchView{first_dev + s.start[cl], prob_dev + s.start[cl], s.cnt[cl]}, st);
     if (rc != FO_OK) return rc;
   }
-  FO_CUDA_TRY(cudaEventRecord(slot->done, st));
+  FO_CUDA_TRY(cudaEventRecord(s.slot->done, st));
+  return FO_OK;
+}
+
+// fo_metric_batch_select: metric_batch_impl's classes and descriptors, sorted by N_p within each class.  Staged behind
+// them: the rank segments of every class (at most one per descriptor), the problem index of each descriptor and N_p of
+// every problem, which is copied into selected_dev before the launches.
+static int metric_batch_select_impl(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr,
+                                    const FoVehicle* vehicles, int32_t* selected_dev, void* stream) {
+  int n_run = 0, a_min = 0;
+  {
+    const int rc = fo::check_batch(fn, b, corr, false, &n_run, &a_min);
+    if (rc != FO_OK) return rc;
+  }
+  const int P = b->n_problems;
+  if (P > 0 && (!selected_dev || (reinterpret_cast<uintptr_t>(selected_dev) & 3u))) {
+    fo::set_error("%s: selected_dev must be a 4-byte aligned device array of n_problems int32", fn);
+    return FO_ERR_INVALID_ARG;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (b->common.n_traj == 0) {                     // every N_p is 0
+    if (P > 0) FO_CUDA_TRY(cudaMemsetAsync(selected_dev, 0, (size_t)P * sizeof(int32_t), st));
+    return FO_OK;
+  }
+  int num_sms = 0;
+  { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
+  const size_t seg_bytes = (size_t)n_run * sizeof(int4), out_bytes = ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15;
+  BatchStage s;
+  int rc = stage_batch(b, corr, vehicles, n_run, a_min, num_sms, true, seg_bytes + out_bytes + (size_t)P * sizeof(int32_t), s);
+  if (rc != FO_OK) return rc;
+  int4* seg = reinterpret_cast<int4*>(s.slot->host + s.bytes);
+  int* out = reinterpret_cast<int*>(s.slot->host + s.bytes + seg_bytes);
+  int32_t* init = reinterpret_cast<int32_t*>(s.slot->host + s.bytes + seg_bytes + out_bytes);
+  for (int p = 0; p < P; ++p) init[p] = b->problems[p].n_traj;
+  for (int i = 0; i < n_run; ++i) out[i] = s.problem[i];
+  // class cl: descriptors start[cl] .. with N descending; the ranks in [N of descriptor m, N of descriptor m - 1) have
+  // the first m descriptors active
+  int seg_start[4] = {0, 0, 0, 0}, n_seg[4] = {0, 0, 0, 0}, ns = 0;
+  for (int cl = 0; cl < 4; ++cl) {
+    seg_start[cl] = ns;
+    int claims = 0, prev = 0;
+    for (int m = s.cnt[cl]; m >= 1; --m) {
+      const int hi = b->problems[s.problem[s.start[cl] + m - 1]].n_traj;
+      if (hi <= prev) continue;
+      seg[ns++] = make_int4(claims, prev, m, 0);
+      claims += (hi - prev) * m;
+      prev = hi;
+    }
+    n_seg[cl] = ns - seg_start[cl];
+  }
+  rc = fo::stage_upload(s.slot, s.bytes + seg_bytes + out_bytes + (size_t)P * sizeof(int32_t), st);
+  if (rc != FO_OK) return rc;
+  FO_CUDA_TRY(cudaMemcpyAsync(selected_dev, s.slot->dev + s.bytes + seg_bytes + out_bytes, (size_t)P * sizeof(int32_t),
+                              cudaMemcpyDeviceToDevice, st));
+  fo::MetricKArgs k;
+  batch_kargs(b->common, k);
+  const int* first_dev = reinterpret_cast<const int*>(s.slot->dev);
+  const fo::BatchProb* prob_dev = reinterpret_cast<const fo::BatchProb*>(s.slot->dev + s.prob_off);
+  const int4* seg_dev = reinterpret_cast<const int4*>(s.slot->dev + s.bytes);
+  const int* out_dev = reinterpret_cast<const int*>(s.slot->dev + s.bytes + seg_bytes);
+  for (int cl = 0; cl < 4; ++cl) {
+    if (s.cnt[cl] == 0) continue;
+    k.N = s.n_cls[cl];
+    k.corr = cl >= 2;
+    rc = fo::launch_metric_batch_select(k, num_sms, s.W, (cl & 1) == 0,
+                                        fo::BatchView{first_dev + s.start[cl], prob_dev + s.start[cl], s.cnt[cl]},
+                                        fo::SelectView{seg_dev + seg_start[cl], out_dev + s.start[cl], selected_dev, n_seg[cl]}, st);
+    if (rc != FO_OK) return rc;
+  }
+  FO_CUDA_TRY(cudaEventRecord(s.slot->done, st));
   return FO_OK;
 }
 
@@ -895,4 +995,9 @@ extern "C" int fo_metric_batch_detail_corr(const FoMetricBatchArgs* b, const uin
   const char* fn = "fo_metric_batch_detail_corr";
   const int rc = check_corr_args(fn, b, corr_host, vehicles_host);
   return rc != FO_OK ? rc : metric_batch_detail_impl(fn, b, corr_host, vehicles_host, stream);
+}
+
+extern "C" int fo_metric_batch_select(const FoMetricBatchArgs* b, const uint8_t* corr_host, const FoVehicle* vehicles_host,
+                                      int32_t* selected_dev, void* stream) {
+  return metric_batch_select_impl("fo_metric_batch_select", b, corr_host, vehicles_host, selected_dev, stream);
 }

@@ -775,6 +775,17 @@ int launch_metric_batch_detail(const MetricKArgs& k, int num_sms, const DetailVi
 // summary kernel over one shape class of a batch (uni: the one-warp window-filter shape, W == 1); k.N = the class's
 // trajectory count.  k.corr: the class's tables are correlated ones (fo_metric_batch_corr_kernel), in both batch launches
 int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st);
+// First valid row per problem (fo_metric_batch_select): one launch's state besides its BatchView.  The launch's
+// descriptors are sorted by N_p in descending order, so the problems with a row of rank j are a prefix of them; claims
+// run rank-major, and the ranks split into segments over which that prefix is the same.
+struct SelectView {
+  const int4* seg;      // [S] (first claim, first rank, active descriptors, 0) of each segment, in rank order
+  const int* out;       // [descriptors] the problem index of each descriptor (its entry of selected)
+  int32_t* selected;    // [n_problems] smallest rank whose row completed valid; initialised to N_p
+  int S;
+};
+int launch_metric_batch_select(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv,
+                               const SelectView& sv, cudaStream_t st);
 int lane_group_log2(int A);                                  // team shape: a warp holds 1 << lg agents
 int pick_team_warps(int N, int T, int A, int num_sms);       // team size W (FO_TEAM_WARPS overrides)
 

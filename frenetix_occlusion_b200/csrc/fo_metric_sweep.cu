@@ -215,6 +215,26 @@ static __device__ __noinline__ uint32_t sw_drain_ties_batch(const float4* t0, co
 // problem of trajectory n: the last p with first[p] <= n
 __device__ __forceinline__ int batch_find(const BatchView& b, int n) { return find_problem(b.first, b.P, n); }
 
+// claim n of a select launch -> (descriptor, rank): the segment of n (the last s with seg[s].x <= n), then rank-major
+// within it over the segment's active descriptors
+__device__ __forceinline__ int2 select_find(const SelectView& s, int n) {
+  int lo = 0, hi = s.S - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(&s.seg[mid].x) <= n) lo = mid; else hi = mid - 1;
+  }
+  const int4 g = __ldg(s.seg + lo);
+  const int d = n - g.x;
+  return make_int2(d % g.z, g.y + d / g.z);
+}
+
+// selected[p] as other teams' atomicMin left it: a relaxed load that does not stop in L1
+__device__ __forceinline__ int ld_relaxed(const int32_t* p) {
+  int v;
+  asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p));
+  return v;
+}
+
 struct SweepShape {
   int lg_agents;   // log2 of the agents held by one warp (0..5); a warp has 32 >> lg_agents time slices
 };
@@ -227,10 +247,14 @@ struct SweepShape {
 // CORR: the table is a correlated one (fo_agents_pack_corr): the CP drain evaluates the nine rectangle masses of the
 // full covariance (cp_bvn_boxes, the table's s3 section) instead of cp_gauss_boxes; a NaN CP (a covariance that is not
 // positive definite) is carried into max_collision_probability_all.
+// SELECT (with BATCH): claims map to (descriptor, rank) rank-major (sv, select_find), and a row whose rank exceeds its
+// problem's sv.selected is not assessed -- checked when it is claimed, before each agent tile and before the BE walk --
+// but written as valid = FO_VALID_SKIPPED.  A row that completes valid lowers selected to its rank.  Whether a row runs
+// is all SELECT decides: a completed row equals the BATCH kernels' row.
 // tid / block_dim are read in the __global__ function, where the compiler knows their range from the launch bounds.
-template <uint32_t MASK, bool STATS, bool UNI, bool TIES, bool BATCH, bool CORR = false>
+template <uint32_t MASK, bool STATS, bool UNI, bool TIES, bool BATCH, bool CORR = false, bool SELECT = false>
 __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShape shape, const BatchView& bv,
-                                           const int tid, const int block_dim) {
+                                           const int tid, const int block_dim, const SelectView& sv = SelectView{}) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   // the one-warp shape is launched with 32 threads: warp index, team size and lane are compile-time facts there (the
   // queue addresses become immediates instead of being re-derived from %tid wherever registers are short)
@@ -267,18 +291,27 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
   // Trajectories are claimed from a device counter (their cost varies several-fold with the number of near agents and
   // braking pairs); the claim for the next one is issued here and read at the bottom, so its latency is hidden.  A batch
   // looks up the problem of the claimed trajectory in the same place.
-  __shared__ int s_claim[BATCH ? 2 : 1];               // next trajectory (and, batched, its problem)
+  // select: [2] the next claim's rank, [3] skip the claimed row, [4] stop the row in progress (a slot of its own: no
+  // barrier separates the reads of [3] from the first write of [4])
+  __shared__ int s_claim[BATCH ? (SELECT ? 5 : 2) : 1];   // next trajectory (and, batched, its problem)
   int& s_next = s_claim[0];
   // batched: the ego vehicle of the current trajectory's problem, read where used (held in registers it would spill)
   __shared__ EgoConst s_veh;
   const EgoConst& veh = BATCH ? s_veh : k.veh;
-  int p = BATCH ? batch_find(bv, blockIdx.x) : 0;
+  int p = (BATCH && !SELECT) ? batch_find(bv, blockIdx.x) : 0;
+  int rank = 0;
+  if constexpr (SELECT) {
+    const int2 q = select_find(sv, blockIdx.x);
+    p = q.x; rank = q.y;
+  }
   for (int n = blockIdx.x; n < k.N;) {
     AgentTableView btab;
     int row = n, bA = 0, bTp = 0, b_group = 1, b_la = 0, b_slo = 0, b_shi = 0;
+    int32_t* sel = nullptr;                          // select: the problem's entry of sv.selected
     if constexpr (BATCH) {
       const BatchProb bp = bv.prob[p];
-      row = bp.row0 + (n - bp.first);
+      row = bp.row0 + (SELECT ? rank : n - bp.first);
+      if constexpr (SELECT) sel = sv.selected + __ldg(sv.out + p);
       bA = bp.A; bTp = bp.Tp;
       btab.t0 = bp.t0; btab.tv = bp.tv; btab.aw = bp.aw; btab.avw = bp.avw;
       btab.s0 = bp.s0; btab.s1 = bp.s1; btab.s2 = bp.s2; btab.prm = bp.prm;
@@ -313,9 +346,28 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
     }
     if (tid == 0) {
       s_next = k.claim ? (int)(gridDim.x + atomicAdd(k.claim, 1u)) : n + (int)gridDim.x;
-      if constexpr (BATCH) s_claim[1] = s_next < k.N ? batch_find(bv, s_next) : 0;
+      if constexpr (SELECT) {
+        if (s_next < k.N) {
+          const int2 q = select_find(sv, s_next);
+          s_claim[1] = q.x; s_claim[2] = q.y;
+        }
+        s_claim[3] = ld_relaxed(sel) < rank;
+        s_claim[4] = 0;
+      } else if constexpr (BATCH) {
+        s_claim[1] = s_next < k.N ? batch_find(bv, s_next) : 0;
+      }
     }
     __syncthreads();
+    // select: a row ranked after its problem's valid row so far is written as skipped, not staged
+    const auto skip_row = [&]() {
+      if (tid == 0) k.valid[row] = FO_VALID_SKIPPED;
+      n = s_next;
+      p = s_claim[1];
+      rank = s_claim[2];
+    };
+    if constexpr (SELECT) {
+      if (s_claim[3]) { skip_row(); continue; }
+    }
     if constexpr (BATCH) rE = sqrtf(veh.hEx * veh.hEx + veh.hEy * veh.hEy);
     {
       float amin = 0.0f;
@@ -359,7 +411,13 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
     for (int a0 = 0; a0 < A; a0 += kSwTile) {
       const int nAt = min(kSwTile, A - a0);
       for (int j = tid; j < nAt; j += nthr) { w.pairkey[j] = 0ull; w.colfirst[j] = 0xffffffffu; }
+      if constexpr (SELECT) {                          // before the tile's sweep and queued drains
+        if (tid == 0) s_claim[4] = ld_relaxed(sel) < rank;
+      }
       __syncthreads();                                 // ego staged, pair arrays cleared
+      if constexpr (SELECT) {
+        if (s_claim[4]) break;
+      }
       int qn = 0, qc = 0, qt = 0;
       // per-lane bound state of the current lane group (refreshed after every drain)
       float lim0 = 0.0f, lim2 = 0.0f, thr2 = CUDART_INF_F;
@@ -710,7 +768,13 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           w.be_list[atomicAdd(&w.scal[1], 1u)] = (uint16_t)j;
       }
       if (do_be && do_ttc) {
+        if constexpr (SELECT) {                        // before the BE walk
+          if (tid == 0) s_claim[4] = ld_relaxed(sel) < rank;
+        }
         __syncthreads();                               // BE list complete
+        if constexpr (SELECT) {
+          if (s_claim[4]) break;
+        }
         const int n_be = (int)w.scal[1];
         if (n_be > 0) {
           if (!be_ready) {
@@ -752,6 +816,9 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
         if (tid == 0) w.scal[1] = 0u;
       }
     }  // agent tiles
+    if constexpr (SELECT) {
+      if (s_claim[4]) { skip_row(); continue; }
+    }
 
     // ---- per-trajectory reduction (warp, then team) and threshold mask (metric.py:50-98) --------------------
     {
@@ -810,9 +877,13 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           sm[4] = make_float2(o8, o9);
         }
       }
+      if constexpr (SELECT) {
+        if (ok) atomicMin(sel, rank);
+      }
     }
     n = s_next;
     if constexpr (BATCH) p = s_claim[1];
+    if constexpr (SELECT) rank = s_claim[2];
   }
   if (STATS && k.stats) {
     auto wsum = [&](unsigned long long v) {
@@ -867,6 +938,15 @@ template <bool UNI, bool TIES>
 __global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
 fo_metric_batch_corr_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape, const __grid_constant__ BatchView bv) {
   sweep_body<0u, false, UNI, TIES, true, true>(k, shape, bv, threadIdx.x, blockDim.x);
+}
+
+// One shape class of a batch for its problems' first valid rows (fo_metric_batch_select): fo_metric_batch_kernel<0> /
+// fo_metric_batch_corr_kernel with rank-major claims and early exit.
+template <bool UNI, bool TIES, bool CORR>
+__global__ void __launch_bounds__(kSwMaxWarps * 32, FO_SW_MINB)
+fo_metric_batch_select_kernel(const __grid_constant__ MetricKArgs k, const SweepShape shape,
+                              const __grid_constant__ BatchView bv, const __grid_constant__ SelectView sv) {
+  sweep_body<0u, false, UNI, TIES, true, CORR, true>(k, shape, bv, threadIdx.x, blockDim.x, sv);
 }
 
 // Team shape.  lg_agents: a warp holds min(32, next power of two >= A) agents, the remaining lanes are time slices.
@@ -1025,6 +1105,23 @@ int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, cons
   if (k.mmask == kAllMetrics) return launch_batch_inst<kAllMetrics>(k, num_sms, W, uni, bv, st);
   if (k.mmask == kDefaultMetrics) return launch_batch_inst<kDefaultMetrics>(k, num_sms, W, uni, bv, st);
   return launch_batch_inst<0u>(k, num_sms, W, uni, bv, st);
+}
+
+template <bool CORR>
+static int launch_select_inst(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv,
+                              const SelectView& sv, cudaStream_t st) {
+  const SweepShape shape{0};
+  const bool ties = needs_ties(k);
+  if (uni) return ties ? launch_team_kernel<fo_metric_batch_select_kernel<true, true, CORR>>(k, num_sms, W, uni, ties, st, shape, bv, sv)
+                       : launch_team_kernel<fo_metric_batch_select_kernel<true, false, CORR>>(k, num_sms, W, uni, ties, st, shape, bv, sv);
+  return ties ? launch_team_kernel<fo_metric_batch_select_kernel<false, true, CORR>>(k, num_sms, W, uni, ties, st, shape, bv, sv)
+              : launch_team_kernel<fo_metric_batch_select_kernel<false, false, CORR>>(k, num_sms, W, uni, ties, st, shape, bv, sv);
+}
+
+int launch_metric_batch_select(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv,
+                               const SelectView& sv, cudaStream_t st) {
+  return k.corr ? launch_select_inst<true>(k, num_sms, W, uni, bv, sv, st)
+                : launch_select_inst<false>(k, num_sms, W, uni, bv, sv, st);
 }
 
 }  // namespace fo

@@ -168,6 +168,7 @@ class BatchResult:
     step: Optional[torch.Tensor] = None     # float32 [sum_p N_p A_p (T-1) FO_STEP_K]
     n_agents: Optional[np.ndarray] = None   # A_p, with pair / step
     n_states: int = 0                       # T, with pair / step
+    selected: Optional[torch.Tensor] = None  # int32 [P], select_batch / select: each problem's first valid rank (N_p: none)
 
     def split(self) -> list:
         """Per-problem ``BundleResult`` views of the batch tensors (no copies): pair [N_p, A_p, FO_PAIR_K] and step
@@ -536,8 +537,77 @@ class MetricEngine:
         ``out``: preallocated outputs of the batch's sizes (valid / summary / flags, and
         the flat pair / step where wanted).  Asynchronous on the current stream."""
         b = self._batch
+        a, out, t = self._batch_args("assess_batch", egos, want_pair, want_step, out)
+        with torch.cuda.device(self.device):
+            detail, veh, corr = bool(a.common.pair or a.common.step), b["vehicles"], b["corr"]
+            if corr is not None:
+                fn = "fo_metric_batch_detail_corr" if detail else "fo_metric_batch_corr"
+                L.check(getattr(L.lib, fn)(C.byref(a), corr.ctypes.data, veh, self._stream()), fn)
+            elif veh is None:
+                fn = "fo_metric_batch_detail" if detail else "fo_metric_batch"
+                L.check(getattr(L.lib, fn)(C.byref(a), self._stream()), fn)
+            else:
+                fn = "fo_metric_batch_detail_vehicles" if detail else "fo_metric_batch_vehicles"
+                L.check(getattr(L.lib, fn)(C.byref(a), veh, self._stream()), fn)
+        out._keepalive = (t, b["arena"])
+        return out
+
+    def select_batch(self, egos: Sequence, out: Optional[BatchResult] = None) -> BatchResult:
+        """The first valid row of every problem of the batch set by ``set_agent_batch`` (``fo_metric_batch_select``), for
+        a planner that stacks each problem's candidates in priority order and takes the first that passes.  ``egos`` and
+        ``out`` as in ``assess_batch`` (without detail).  Returns the ``BatchResult`` with ``selected``: int32 [P] on
+        the device, problem p's smallest rank whose row ``assess_batch`` marks valid, or N_p when none is.  Rows ranked
+        after it may hold ``FO_VALID_SKIPPED`` instead of their results; the others equal ``assess_batch``'s bit for bit.
+        Asynchronous on the current stream."""
+        b = self._batch
+        a, out, t = self._batch_args("select_batch", egos, False, False, out)
+        with torch.cuda.device(self.device):
+            out.selected = torch.empty(b["P"], dtype=torch.int32, device=self.device)
+            corr = b["corr"]
+            L.check(L.lib.fo_metric_batch_select(C.byref(a), corr.ctypes.data if corr is not None else None,
+                                                 b["vehicles"], C.c_void_p(out.selected.data_ptr()), self._stream()),
+                    "fo_metric_batch_select")
+        out._keepalive = (t, b["arena"])
+        return out
+
+    def select(self, ego) -> BatchResult:
+        """``select_batch`` for the engine's own agents (``set_agents``) and one bundle in priority order: the batch of
+        one problem over the engine's table, so the rows it assesses equal ``assess(ego)``'s.  ``selected[0]`` is the
+        first valid row, N when none is.  Asynchronous on the current stream."""
+        t = self.to_device_bundle(ego)
+        if t.ndim != 3 or t.shape[2] != 5:
+            raise ValueError("trajectory bundle must have shape [N, T, 5] (x, y, theta, v, a)")
+        N, T = int(t.shape[0]), int(t.shape[1])
+        if T > L.FO_MAX_STATES:
+            raise ValueError(f"trajectories longer than {L.FO_MAX_STATES} states are not supported")
+        dev = self.device
+        self._pack_agents()
+        problems = (L.FoBatchProblem * 1)()
+        problems[0].traj_begin, problems[0].n_traj = 0, N
+        problems[0].n_agents, problems[0].t_stride, problems[0].table_offset = self.n_agents, max(self.t_stride, 1), 0
+        corr = np.ones(1, dtype=np.uint8) if self._corr else None
+        with torch.cuda.device(dev):
+            out = BatchResult(torch.empty(N, dtype=torch.uint8, device=dev),
+                              torch.empty((N, L.FO_SUMMARY_K), dtype=torch.float32, device=dev),
+                              torch.empty(N, dtype=torch.int32, device=dev), np.array([0, N], dtype=np.int64),
+                              selected=torch.empty(1, dtype=torch.int32, device=dev))
+            a = L.FoMetricBatchArgs()
+            a.common = self._args(t, BundleResult(out.valid, out.summary, out.flags))
+            a.common.n_agents, a.common.t_stride = 0, 1
+            a.n_problems, a.problems = 1, problems
+            a.arena_bytes = self._table.numel() if self._table is not None else 0
+            L.check(L.lib.fo_metric_batch_select(C.byref(a), corr.ctypes.data if corr is not None else None, None,
+                                                 C.c_void_p(out.selected.data_ptr()), self._stream()),
+                    "fo_metric_batch_select")
+        out._keepalive = (t, self._table)
+        return out
+
+    def _batch_args(self, fn, egos, want_pair, want_step, out):
+        """The batch call's arguments for ``egos`` over the batch set by ``set_agent_batch``: the staged bundle, the
+        outputs (allocated unless ``out`` is given) and ``FoMetricBatchArgs`` with pair / step where wanted."""
+        b = self._batch
         if b is None:
-            raise RuntimeError("assess_batch() needs set_agent_batch() first")
+            raise RuntimeError(f"{fn}() needs set_agent_batch() first")
         P = b["P"]
         if len(egos) != P:
             raise ValueError(f"{len(egos)} bundles for {P} problems")
@@ -593,15 +663,4 @@ class MetricEngine:
             # path runs when no detail buffer is left
             a.common.pair = out.pair.data_ptr() if (out.pair is not None and out.pair.numel()) else None
             a.common.step = out.step.data_ptr() if (out.step is not None and out.step.numel()) else None
-            detail, veh, corr = bool(a.common.pair or a.common.step), b["vehicles"], b["corr"]
-            if corr is not None:
-                fn = "fo_metric_batch_detail_corr" if detail else "fo_metric_batch_corr"
-                L.check(getattr(L.lib, fn)(C.byref(a), corr.ctypes.data, veh, self._stream()), fn)
-            elif veh is None:
-                fn = "fo_metric_batch_detail" if detail else "fo_metric_batch"
-                L.check(getattr(L.lib, fn)(C.byref(a), self._stream()), fn)
-            else:
-                fn = "fo_metric_batch_detail_vehicles" if detail else "fo_metric_batch_vehicles"
-                L.check(getattr(L.lib, fn)(C.byref(a), veh, self._stream()), fn)
-        out._keepalive = (t, b["arena"])
-        return out
+        return a, out, t

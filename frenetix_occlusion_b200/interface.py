@@ -181,6 +181,13 @@ class FOInterface:
         (``engine.BundleResult``); every trajectory is valid when there are no phantom agents (metric.py:44-45)."""
         return self.metrics.evaluate_bundle(trajectories, want_pair=want_pair, want_step=want_step)
 
+    def select_trajectory(self, trajectories):
+        """The planner's protocol in one call: ``trajectories`` sorted by cost (as ``assess_bundle`` takes them), the
+        index of the first one ``trajectory_safety_assessment`` would pass, or None when none passes.  Only the
+        candidates up to that one need to be assessed.  For the chosen candidate's result dict call
+        ``trajectory_safety_assessment(trajectories[k])``; the prefetch is not touched."""
+        return self.metrics.select(trajectories)
+
     def _update_time_step(self, timestep):
         self.timestep = timestep
         self.sensor_model.timestep = timestep

@@ -175,6 +175,15 @@ class MetricCore:
         self.sync_agents()
         return self.engine.assess(ego, want_pair=want_pair, want_step=want_step)
 
+    # ---- the first valid row of a bundle in priority order --------------------------------------------
+    def select(self, ego):
+        """Index of the first valid row of ``ego`` (``MetricEngine.select``), None when no row is valid; synchronises
+        on one int.  The prefetch and the per-trajectory cache are left as they are."""
+        self.sync_agents()
+        n = int(ego.shape[0])
+        k = int(self.engine.select(ego).selected.item())
+        return k if k < n else None
+
 
 _cores = {}
 

@@ -78,6 +78,25 @@ class Metric:
             trajectories = np.stack([trajectory_to_array(t) for t in trajectories])
         return self._core.bundle(trajectories, want_pair=want_pair, want_step=want_step)
 
+    def select(self, trajectories):
+        """Index of the first of ``trajectories`` (in priority order: [N, T, 5] tensor / array or a sequence of
+        trajectory objects) that ``evaluate_metrics`` finds safe, None when none is; 0 without phantom agents or
+        metrics (metric.py:44-45), None for an empty list.  Only the rows up to the answer need to be assessed
+        (``MetricEngine.select``); synchronises on one int, and leaves the prefetch untouched."""
+        import numpy as np
+        import torch
+        from .core import trajectory_to_array
+        if not isinstance(trajectories, (np.ndarray, torch.Tensor)):
+            trajectories = list(trajectories)
+            if not trajectories:
+                return None
+            trajectories = np.stack([trajectory_to_array(t) for t in trajectories])
+        if int(trajectories.shape[0]) == 0:
+            return None
+        if not self.agent_manager.phantom_agents or not self.metrics:
+            return 0
+        return self._core.select(trajectories)
+
     def prefetch(self, trajectories):
         """Evaluate all candidates of this planning cycle in one launch; the ``evaluate_metrics`` calls that follow are
         served from the host copy (see ``MetricCore.prefetch``)."""

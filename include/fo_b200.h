@@ -306,6 +306,23 @@ int fo_metric_batch_corr(const FoMetricBatchArgs *args, const uint8_t *corr_host
 int fo_metric_batch_detail_corr(const FoMetricBatchArgs *args, const uint8_t *corr_host, const FoVehicle *vehicles_host,
                                 void *stream);
 
+/* The first valid row of every problem of a batch, for a planner that takes the first candidate of a cost-ordered list
+ * that passes.  Problem p's rows are in priority order: row traj_begin is the most preferred.  selected_dev (DEVICE
+ * int32 [n_problems], 4-byte aligned) receives the smallest rank r in [0, N_p) whose valid byte fo_metric_batch_corr
+ * writes as 1 for the same arguments (fo_metric_batch_vehicles / fo_metric_batch without flags / vehicles), and N_p
+ * when no row passes (so 0 for N_p = 0; a problem without agents or metrics gets 0).  corr_host: NULL = no correlated
+ * problem; vehicles_host: NULL = common.vehicle for every problem.
+ * Rows of rank <= selected_dev[p] hold exactly what fo_metric_batch_corr writes (all rows when none passes); every later
+ * row holds either that, or valid = FO_VALID_SKIPPED with its summary / flags left unwritten.  Every valid byte is
+ * written.  Team size and shape classes are fo_metric_batch's, so a row that is assessed equals the batch call's row;
+ * rows ranked after a row already known valid are skipped, which is where the call saves time.
+ * Argument checks as in fo_metric_batch_corr, plus a NULL selected_dev with n_problems > 0 or a misaligned one
+ * (FO_ERR_INVALID_ARG); pair / step / n_peers != 0 are FO_ERR_UNSUPPORTED.  All checks run before any device work.  Not
+ * capturable in a CUDA graph. */
+#define FO_VALID_SKIPPED 2
+int fo_metric_batch_select(const FoMetricBatchArgs *args, const uint8_t *corr_host, const FoVehicle *vehicles_host,
+                           int32_t *selected_dev, void *stream);
+
 /* A batch driven from HOST buffers (pinned or pageable), for embedders without a CUDA runtime of their own: the
  * planner's float64 ego rows in the caller's world frame and one float64 origin per problem in, results in host arrays
  * out, synchronised.  The library shifts every row by its problem's origin on the device, in float64, and only then

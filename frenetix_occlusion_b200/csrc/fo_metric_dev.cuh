@@ -205,11 +205,8 @@ __device__ __forceinline__ float ex2_approx(float x) {
 
 // erfc(z), z >= 0, fractional error < 1.2e-7 in exact arithmetic (Chebyshev fit of Numerical Recipes' erfcc:
 // t = 1/(1 + z/2), erfc = t exp(-z^2 + P9(t))); about 4e-6 relative in float32 because of the exponent's
-// magnitude -- two orders below the 1e-4 parity tolerance.  17 instructions instead of erfcf's ~45.
-// RAW_EXP: exp as one FMUL + MUFU.EX2 (flushes results below 2^-126 to zero).  The summary kernel's cut-off keeps one end
-// of every evaluated interval within 4.7, so a flushed far end (< 1e-38 against >= 3e-11) cannot change a bit of the
-// factor; the detail kernel (no cut-off, per-step values compared for their first index) keeps the guarded __expf.
-template <bool RAW_EXP>
+// magnitude -- two orders below the 1e-4 parity tolerance.  17 instructions instead of erfcf's ~45.  This form (guarded
+// __expf) serves the detail kernel; the summary kernel evaluates the same chain two at a time (erf_span2).
 __device__ __forceinline__ float erfc_pos_fast(float z) {
   const float t = rcp_approx(fmaf(0.5f, z, 1.0f));      // 1 + z/2 >= 1: same bits as __fdividef(1, .)
   float p = 0.17087277f;
@@ -223,7 +220,39 @@ __device__ __forceinline__ float erfc_pos_fast(float z) {
   p = fmaf(p, t, 1.00002368f);
   p = fmaf(p, t, -1.26551223f);
   const float a = fmaf(-z, z, p);
-  return t * (RAW_EXP ? ex2_approx(a * 1.4426950216293334961f) : __expf(a));
+  return t * __expf(a);
+}
+
+// Packed float32 (sm_100 FFMA2 / FADD2 / FMUL2): two IEEE operations in one issue slot, each lane bit-identical to the
+// scalar FFMA / FADD / FMUL.  ptxas does not form them itself.  A scalar operand is broadcast without a move (f2).
+__device__ __forceinline__ float2 f2(float v) { return make_float2(v, v); }
+__device__ __forceinline__ float2 fma2(float2 a, float2 b, float2 c) { return __ffma2_rn(a, b, c); }
+__device__ __forceinline__ float2 add2(float2 a, float2 b) { return __fadd2_rn(a, b); }
+__device__ __forceinline__ float2 mul2(float2 a, float2 b) { return __fmul2_rn(a, b); }
+
+// erf(b) - erf(a), a < b, from erfc(|a|) and erfc(|b|) of erfc_pos_fast's chain, the two chains packed into one.
+// exp is one FMUL + MUFU.EX2 (flushes results below 2^-126 to zero): the summary kernel's cut-off keeps one end of every
+// evaluated interval within 4.7, so a flushed far end (< 1e-38 against >= 3e-11) cannot change a bit of the factor.
+// The last products are formed as the scalar chains' contractions formed them, so the result keeps their bits:
+// erfc(|b|) = t.y * e.y rounded once, erfc(|a|) = t.x * e.x fused into both combinations.  A packed product of the two
+// would round erfc(|a|) as well.
+__device__ __forceinline__ float erf_span2(float a, float b) {
+  const float2 z = make_float2(fabsf(a), fabsf(b));
+  const float2 d = fma2(f2(0.5f), z, f2(1.0f));
+  const float2 t = make_float2(rcp_approx(d.x), rcp_approx(d.y));
+  float2 p = fma2(f2(0.17087277f), t, f2(-0.82215223f));
+  p = fma2(p, t, f2(1.48851587f));
+  p = fma2(p, t, f2(-1.13520398f));
+  p = fma2(p, t, f2(0.27886807f));
+  p = fma2(p, t, f2(-0.18628806f));
+  p = fma2(p, t, f2(0.09678418f));
+  p = fma2(p, t, f2(0.37409196f));
+  p = fma2(p, t, f2(1.00002368f));
+  p = fma2(p, t, f2(-1.26551223f));
+  const float2 x = mul2(fma2(make_float2(-z.x, -z.y), z, p), f2(1.4426950216293334961f));
+  const float2 e = make_float2(ex2_approx(x.x), ex2_approx(x.y));
+  const float eb = __fmul_rn(t.y, e.y);
+  return ((a > 0.0f) == (b > 0.0f)) ? fabsf(fmaf(t.x, e.x, -eb)) : __fsub_rn(fmaf(-t.x, e.x, 2.0f), eb);
 }
 
 // Collision probability of one gated step (collision_probability.py:94-122): Gaussian mass of the 3 obstacle
@@ -245,17 +274,27 @@ __device__ __forceinline__ float cp_gauss_boxes(float mx, float my, float hx, fl
     float fb = 0.0f;               // ego box: middle, front, rear
 #pragma unroll 1
     for (int bb = 0; bb < 3; ++bb) {
-      const float cyb = fb * by, cxb = fb * bx;
+      const float f = fb;
       fb = (bb == 0) ? 1.0f : -1.0f;
-      const float ya = (cyb - W2 - uy) * s2.y, yb = (cyb + W2 - uy) * s2.y;     // ya < yb
-      if (CUT && (ya > kFar || yb < -kFar)) continue;
-      const float xa = (cxb - L6 - ux) * s2.x, xb = (cxb + L6 - ux) * s2.x;
-      if (CUT && (xa > kFar || xb < -kFar)) continue;
-      const float eya = erfc_pos_fast<CUT>(fabsf(ya)), eyb = erfc_pos_fast<CUT>(fabsf(yb));
-      const float py = ((ya > 0.0f) == (yb > 0.0f)) ? fabsf(eya - eyb) : (2.0f - eya - eyb);
-      const float exa = erfc_pos_fast<CUT>(fabsf(xa)), exb = erfc_pos_fast<CUT>(fabsf(xb));
-      const float px = ((xa > 0.0f) == (xb > 0.0f)) ? fabsf(exa - exb) : (2.0f - exa - exb);
-      prob = fmaf(0.25f * px, py, prob);
+      if constexpr (CUT) {
+        // both ends of an interval as one packed pair: (f b -+ half) - u, times s2 (the scalar code's contraction)
+        const float2 y = mul2(add2(fma2(f2(f), f2(by), make_float2(-W2, W2)), f2(-uy)), f2(s2.y));   // y.x < y.y
+        if (y.x > kFar || y.y < -kFar) continue;
+        const float2 x = mul2(add2(fma2(f2(f), f2(bx), make_float2(-L6, L6)), f2(-ux)), f2(s2.x));
+        if (x.x > kFar || x.y < -kFar) continue;
+        const float py = erf_span2(y.x, y.y);
+        const float px = erf_span2(x.x, x.y);
+        prob = fmaf(0.25f * px, py, prob);
+      } else {
+        const float cyb = f * by, cxb = f * bx;
+        const float ya = (cyb - W2 - uy) * s2.y, yb = (cyb + W2 - uy) * s2.y;     // ya < yb
+        const float xa = (cxb - L6 - ux) * s2.x, xb = (cxb + L6 - ux) * s2.x;
+        const float eya = erfc_pos_fast(fabsf(ya)), eyb = erfc_pos_fast(fabsf(yb));
+        const float py = ((ya > 0.0f) == (yb > 0.0f)) ? fabsf(eya - eyb) : (2.0f - eya - eyb);
+        const float exa = erfc_pos_fast(fabsf(xa)), exb = erfc_pos_fast(fabsf(xb));
+        const float px = ((xa > 0.0f) == (xb > 0.0f)) ? fabsf(exa - exb) : (2.0f - exa - exb);
+        prob = fmaf(0.25f * px, py, prob);
+      }
     }
     fm = (m == 0) ? 1.0f : -1.0f;
   }

@@ -586,11 +586,11 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           const int ie = min(i, T - 1);
           const float4 EA = w.egoA[ie];
           const float ve = w.egoB[ie].y;
-          const float dxr = s0.x - EA.x, dyr = s0.y - EA.y;
           bool need_obb = false, need_lr = false, ingate = false;
           if (do_dce) {
-            const float dx = fmaf(-veh.wb, EA.z, dxr), dy = fmaf(-veh.wb, EA.w, dyr);   // centre to centre
-            need_obb = live & (fmaf(dx, dx, dy * dy) < lim2);
+            const float2 d = fma2(f2(-veh.wb), make_float2(EA.z, EA.w),
+                                  add2(make_float2(s0.x, s0.y), make_float2(-EA.x, -EA.y)));   // centre to centre
+            need_obb = live & (fmaf(d.x, d.x, d.y * d.y) < lim2);
           }
           if (do_hr) {
             const float c = fmaf(EA.z, s0.z, EA.w * s0.w);                            // cos(yaw - theta)
@@ -601,7 +601,8 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           }
           if (do_cp) {                                                                // 5 m gate, collision_probability.py:61-78
             // min over the points p, p +- h u of |. - e|^2  =  |m|^2 + min(0, h^2 - 2 h |m.u|),  m = p_{i-1} - e_i
-            const float mx = pxp - EA.x, my = pyp - EA.y;
+            const float2 m = add2(make_float2(pxp, pyp), make_float2(-EA.x, -EA.y));
+            const float mx = m.x, my = m.y;
             const float mu = fmaf(mx, s0.z, my * s0.w);
             const float dmin = fmaf(mx, mx, my * my) + fminf(fmaf(hlbm2, fabsf(mu), hlb2), 0.0f);
             ingate = live & (i >= 1) & (dmin <= 25.0f);

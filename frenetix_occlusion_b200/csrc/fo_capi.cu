@@ -274,9 +274,9 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
   return FO_OK;
 }
 
-// fo_metric_batch_host and fo_metric_batch_host_corr.  corr: NULL = every table diagonal (the diagonal pack and metric
-// calls); else corr[p] != 0 = problem p's table is a correlated one, its off-diagonal terms in cov_xy (host, aligned with
-// ag->var_x / var_y), and the *_corr pack and metric calls run.
+// fo_metric_batch_host and fo_metric_batch_host_corr.  corr: NULL = every table diagonal; else corr[p] != 0 = problem
+// p's table is a correlated one, its off-diagonal terms in cov_xy (host, aligned with ag->var_x / var_y).  The pack and
+// metric calls are the *_corr ones either way.
 static int metric_batch_host_impl(const char* fn, const double* ego_host, int32_t n_traj, int32_t n_states,
                                   const double* origins_host, const FoAgentsRaw* ag, const float* cov_xy, int32_t n_problems,
                                   const FoBatchProblem* problems_host, const uint8_t* corr, const FoVehicle* vehicles_host,
@@ -397,16 +397,14 @@ static int metric_batch_host_impl(const char* fn, const double* ego_host, int32_
   char* d_idx = take(b_idx);
   FO_HOST_TRY(cudaMemcpyAsync(d_idx, idx.data(), idx.size(), cudaMemcpyHostToDevice, st));
   void* d_arena = take(b_arena);
-  // the *_corr calls take one vehicle per problem: params->vehicle for every one unless the caller gives them
-  std::vector<FoVehicle> shared(corr && !vehicles_host ? P : 0, params->vehicle);
-  const FoVehicle* veh = corr && !vehicles_host ? shared.data() : vehicles_host;
+  // the *_corr calls take a flag and a vehicle per problem: without corr none is correlated, without vehicles_host every
+  // problem has params->vehicle (with every flag 0 they make the launches of the diagonal calls)
+  const std::vector<uint8_t> no_corr(corr ? 0 : P, 0);
+  const uint8_t* corr_flags = corr ? corr : no_corr.data();
+  const std::vector<FoVehicle> shared(vehicles_host ? 0 : P, params->vehicle);
+  const FoVehicle* veh = vehicles_host ? vehicles_host : shared.data();
   if (n_packed) {
-    if (corr)
-      rc = fo_agents_pack_batch_corr(&d, n_corr ? d_cov : nullptr, P, pr.data(), corr, veh, d_arena, arena_bytes, st);
-    else
-      rc = vehicles_host
-               ? fo_agents_pack_batch_vehicles(&d, P, pr.data(), vehicles_host, d_arena, arena_bytes, st)
-               : fo_agents_pack_batch(&d, P, pr.data(), &params->vehicle, d_arena, arena_bytes, st);
+    rc = fo_agents_pack_batch_corr(&d, n_corr ? d_cov : nullptr, P, pr.data(), corr_flags, veh, d_arena, arena_bytes, st);
     if (rc != FO_OK) return fo::ws_fail(rc);
   }
 
@@ -434,12 +432,8 @@ static int metric_batch_host_impl(const char* fn, const double* ego_host, int32_
   b.common.flags = (uint32_t*)take(b_flags);
   b.common.pair = want_pair ? (float*)take(b_pair) : nullptr;
   b.common.step = want_step ? (float*)take(b_step) : nullptr;
-  if (corr)
-    rc = (want_pair || want_step) ? fo_metric_batch_detail_corr(&b, corr, veh, st) : fo_metric_batch_corr(&b, corr, veh, st);
-  else if (want_pair || want_step)
-    rc = vehicles_host ? fo_metric_batch_detail_vehicles(&b, vehicles_host, st) : fo_metric_batch_detail(&b, st);
-  else
-    rc = vehicles_host ? fo_metric_batch_vehicles(&b, vehicles_host, st) : fo_metric_batch(&b, st);
+  rc = (want_pair || want_step) ? fo_metric_batch_detail_corr(&b, corr_flags, veh, st)
+                                 : fo_metric_batch_corr(&b, corr_flags, veh, st);
   if (rc != FO_OK) return fo::ws_fail(rc);
 
   // ---- results back, then synchronise

@@ -690,10 +690,10 @@ int fo::check_batch(const char* fn, const FoMetricBatchArgs* b, const uint8_t* c
   return FO_OK;
 }
 
-// The staged descriptors of a summary batch call (metric_batch_impl, metric_batch_select_impl): one team size for the
-// whole batch, as fo_metric_bundle picks it; with W = 1 problems with >= 17 agents run the window-filter shape, the
-// others the team shape with their own lane grouping.  Classes: 0 / 1 diagonal window-filter / team shape, 2 / 3 the
-// same for correlated tables; one launch per non-empty class, each numbering its trajectories.
+// The staged descriptors of a summary batch call (metric_batch_impl): one team size for the whole batch, as
+// fo_metric_bundle picks it; with W = 1 problems with >= 17 agents run the window-filter shape, the others the team
+// shape with their own lane grouping.  Classes: 0 / 1 diagonal window-filter / team shape, 2 / 3 the same for
+// correlated tables; one launch per non-empty class, each numbering its trajectories.
 struct BatchStage {
   int W = 1;
   int cnt[4] = {0, 0, 0, 0}, start[4] = {0, 0, 0, 0}, n_cls[4] = {0, 0, 0, 0};
@@ -761,86 +761,62 @@ static void batch_kargs(const FoMetricArgs& c, fo::MetricKArgs& k) {
   fill_kargs(&ca, k);
 }
 
+// select (fo_metric_batch_select): the descriptors are sorted by N_p within each class, and staged behind them are the
+// rank segments of every class (at most one per descriptor), the problem index of each descriptor and N_p of every
+// problem, which is copied into selected_dev before the launches.
 static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles,
-                             void* stream) {
-  int n_run = 0, a_min = 0;
-  {
-    const int rc = fo::check_batch(fn, b, corr, false, &n_run, &a_min);
-    if (rc != FO_OK || b->common.n_traj == 0) return rc;
-  }
-  int num_sms = 0;
-  { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
-  BatchStage s;
-  int rc = stage_batch(b, corr, vehicles, n_run, a_min, num_sms, false, 0, s);
-  if (rc != FO_OK) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  rc = fo::stage_upload(s.slot, s.bytes, st);
-  if (rc != FO_OK) return rc;
-  fo::MetricKArgs k;
-  batch_kargs(b->common, k);
-  const int* first_dev = reinterpret_cast<const int*>(s.slot->dev);
-  const fo::BatchProb* prob_dev = reinterpret_cast<const fo::BatchProb*>(s.slot->dev + s.prob_off);
-  for (int cl = 0; cl < 4; ++cl) {
-    if (s.cnt[cl] == 0) continue;
-    k.N = s.n_cls[cl];
-    k.corr = cl >= 2;
-    rc = fo::launch_metric_batch(k, num_sms, s.W, (cl & 1) == 0, fo::BatchView{first_dev + s.start[cl], prob_dev + s.start[cl], s.cnt[cl]}, st);
-    if (rc != FO_OK) return rc;
-  }
-  FO_CUDA_TRY(cudaEventRecord(s.slot->done, st));
-  return FO_OK;
-}
-
-// fo_metric_batch_select: metric_batch_impl's classes and descriptors, sorted by N_p within each class.  Staged behind
-// them: the rank segments of every class (at most one per descriptor), the problem index of each descriptor and N_p of
-// every problem, which is copied into selected_dev before the launches.
-static int metric_batch_select_impl(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr,
-                                    const FoVehicle* vehicles, int32_t* selected_dev, void* stream) {
+                             bool select, int32_t* selected_dev, void* stream) {
   int n_run = 0, a_min = 0;
   {
     const int rc = fo::check_batch(fn, b, corr, false, &n_run, &a_min);
     if (rc != FO_OK) return rc;
   }
   const int P = b->n_problems;
-  if (P > 0 && (!selected_dev || (reinterpret_cast<uintptr_t>(selected_dev) & 3u))) {
+  if (select && P > 0 && (!selected_dev || (reinterpret_cast<uintptr_t>(selected_dev) & 3u))) {
     fo::set_error("%s: selected_dev must be a 4-byte aligned device array of n_problems int32", fn);
     return FO_ERR_INVALID_ARG;
   }
   cudaStream_t st = (cudaStream_t)stream;
   if (b->common.n_traj == 0) {                     // every N_p is 0
-    if (P > 0) FO_CUDA_TRY(cudaMemsetAsync(selected_dev, 0, (size_t)P * sizeof(int32_t), st));
+    if (select && P > 0) FO_CUDA_TRY(cudaMemsetAsync(selected_dev, 0, (size_t)P * sizeof(int32_t), st));
     return FO_OK;
   }
   int num_sms = 0;
   { const int rc = num_sms_of_current_device(&num_sms); if (rc != FO_OK) return rc; }
-  const size_t seg_bytes = (size_t)n_run * sizeof(int4), out_bytes = ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15;
+  const size_t seg_bytes = select ? (size_t)n_run * sizeof(int4) : 0;
+  const size_t out_bytes = select ? ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15 : 0;
+  const size_t init_bytes = select ? (size_t)P * sizeof(int32_t) : 0;
   BatchStage s;
-  int rc = stage_batch(b, corr, vehicles, n_run, a_min, num_sms, true, seg_bytes + out_bytes + (size_t)P * sizeof(int32_t), s);
+  int rc = stage_batch(b, corr, vehicles, n_run, a_min, num_sms, select, seg_bytes + out_bytes + init_bytes, s);
   if (rc != FO_OK) return rc;
-  int4* seg = reinterpret_cast<int4*>(s.slot->host + s.bytes);
-  int* out = reinterpret_cast<int*>(s.slot->host + s.bytes + seg_bytes);
-  int32_t* init = reinterpret_cast<int32_t*>(s.slot->host + s.bytes + seg_bytes + out_bytes);
-  for (int p = 0; p < P; ++p) init[p] = b->problems[p].n_traj;
-  for (int i = 0; i < n_run; ++i) out[i] = s.problem[i];
   // class cl: descriptors start[cl] .. with N descending; the ranks in [N of descriptor m, N of descriptor m - 1) have
   // the first m descriptors active
-  int seg_start[4] = {0, 0, 0, 0}, n_seg[4] = {0, 0, 0, 0}, ns = 0;
-  for (int cl = 0; cl < 4; ++cl) {
-    seg_start[cl] = ns;
-    int claims = 0, prev = 0;
-    for (int m = s.cnt[cl]; m >= 1; --m) {
-      const int hi = b->problems[s.problem[s.start[cl] + m - 1]].n_traj;
-      if (hi <= prev) continue;
-      seg[ns++] = make_int4(claims, prev, m, 0);
-      claims += (hi - prev) * m;
-      prev = hi;
+  int seg_start[4] = {0, 0, 0, 0}, n_seg[4] = {0, 0, 0, 0};
+  if (select) {
+    int4* seg = reinterpret_cast<int4*>(s.slot->host + s.bytes);
+    int* out = reinterpret_cast<int*>(s.slot->host + s.bytes + seg_bytes);
+    int32_t* init = reinterpret_cast<int32_t*>(s.slot->host + s.bytes + seg_bytes + out_bytes);
+    for (int p = 0; p < P; ++p) init[p] = b->problems[p].n_traj;
+    for (int i = 0; i < n_run; ++i) out[i] = s.problem[i];
+    int ns = 0;
+    for (int cl = 0; cl < 4; ++cl) {
+      seg_start[cl] = ns;
+      int claims = 0, prev = 0;
+      for (int m = s.cnt[cl]; m >= 1; --m) {
+        const int hi = b->problems[s.problem[s.start[cl] + m - 1]].n_traj;
+        if (hi <= prev) continue;
+        seg[ns++] = make_int4(claims, prev, m, 0);
+        claims += (hi - prev) * m;
+        prev = hi;
+      }
+      n_seg[cl] = ns - seg_start[cl];
     }
-    n_seg[cl] = ns - seg_start[cl];
   }
-  rc = fo::stage_upload(s.slot, s.bytes + seg_bytes + out_bytes + (size_t)P * sizeof(int32_t), st);
+  rc = fo::stage_upload(s.slot, s.bytes + seg_bytes + out_bytes + init_bytes, st);
   if (rc != FO_OK) return rc;
-  FO_CUDA_TRY(cudaMemcpyAsync(selected_dev, s.slot->dev + s.bytes + seg_bytes + out_bytes, (size_t)P * sizeof(int32_t),
-                              cudaMemcpyDeviceToDevice, st));
+  if (select)
+    FO_CUDA_TRY(cudaMemcpyAsync(selected_dev, s.slot->dev + s.bytes + seg_bytes + out_bytes, init_bytes,
+                                cudaMemcpyDeviceToDevice, st));
   fo::MetricKArgs k;
   batch_kargs(b->common, k);
   const int* first_dev = reinterpret_cast<const int*>(s.slot->dev);
@@ -851,9 +827,10 @@ static int metric_batch_select_impl(const char* fn, const FoMetricBatchArgs* b, 
     if (s.cnt[cl] == 0) continue;
     k.N = s.n_cls[cl];
     k.corr = cl >= 2;
-    rc = fo::launch_metric_batch_select(k, num_sms, s.W, (cl & 1) == 0,
-                                        fo::BatchView{first_dev + s.start[cl], prob_dev + s.start[cl], s.cnt[cl]},
-                                        fo::SelectView{seg_dev + seg_start[cl], out_dev + s.start[cl], selected_dev, n_seg[cl]}, st);
+    const fo::SelectView sv = select ? fo::SelectView{seg_dev + seg_start[cl], out_dev + s.start[cl], selected_dev, n_seg[cl]}
+                                     : fo::SelectView{};
+    rc = fo::launch_metric_batch(k, num_sms, s.W, (cl & 1) == 0,
+                                 fo::BatchView{first_dev + s.start[cl], prob_dev + s.start[cl], s.cnt[cl]}, sv, st);
     if (rc != FO_OK) return rc;
   }
   FO_CUDA_TRY(cudaEventRecord(s.slot->done, st));
@@ -861,13 +838,13 @@ static int metric_batch_select_impl(const char* fn, const FoMetricBatchArgs* b, 
 }
 
 extern "C" int fo_metric_batch(const FoMetricBatchArgs* b, void* stream) {
-  return metric_batch_impl("fo_metric_batch", b, nullptr, nullptr, stream);
+  return metric_batch_impl("fo_metric_batch", b, nullptr, nullptr, false, nullptr, stream);
 }
 
 extern "C" int fo_metric_batch_vehicles(const FoMetricBatchArgs* b, const FoVehicle* vehicles_host, void* stream) {
   const char* fn = "fo_metric_batch_vehicles";
   if (b && b->n_problems > 0 && !vehicles_host) { fo::set_error("%s: vehicles_host must not be NULL", fn); return FO_ERR_INVALID_ARG; }
-  return metric_batch_impl(fn, b, nullptr, vehicles_host, stream);
+  return metric_batch_impl(fn, b, nullptr, vehicles_host, false, nullptr, stream);
 }
 
 // corr as in metric_batch_impl.  The diagonal problems run fo_metric_batch_detail_kernel, which takes its launch's rows
@@ -987,7 +964,7 @@ extern "C" int fo_metric_batch_corr(const FoMetricBatchArgs* b, const uint8_t* c
                                     void* stream) {
   const char* fn = "fo_metric_batch_corr";
   const int rc = check_corr_args(fn, b, corr_host, vehicles_host);
-  return rc != FO_OK ? rc : metric_batch_impl(fn, b, corr_host, vehicles_host, stream);
+  return rc != FO_OK ? rc : metric_batch_impl(fn, b, corr_host, vehicles_host, false, nullptr, stream);
 }
 
 extern "C" int fo_metric_batch_detail_corr(const FoMetricBatchArgs* b, const uint8_t* corr_host,
@@ -999,5 +976,5 @@ extern "C" int fo_metric_batch_detail_corr(const FoMetricBatchArgs* b, const uin
 
 extern "C" int fo_metric_batch_select(const FoMetricBatchArgs* b, const uint8_t* corr_host, const FoVehicle* vehicles_host,
                                       int32_t* selected_dev, void* stream) {
-  return metric_batch_select_impl("fo_metric_batch_select", b, corr_host, vehicles_host, selected_dev, stream);
+  return metric_batch_impl("fo_metric_batch_select", b, corr_host, vehicles_host, true, selected_dev, stream);
 }

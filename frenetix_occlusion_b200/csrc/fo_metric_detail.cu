@@ -27,9 +27,6 @@
 //     one 32-byte sector per lane and step: the (cp, ego_harm, obst_harm) triples of 16 steps are transposed through
 //     a per-warp shared-memory tile and leave as 192-byte row segments (8-byte stores when T-1 is even);
 //   * colliding pairs run the warp-cooperative BE bisection of the summary kernel (be_bisect, lanes = steps).
-#include <atomic>
-#include <mutex>
-
 #include "fo_metric_dev.cuh"
 
 namespace fo {
@@ -605,38 +602,7 @@ fo_metric_batch_detail_corr_kernel(const __grid_constant__ MetricKArgs k, const 
   detail_body<0u, true, true>(k, bv);
 }
 
-// Persistent launch of one detail-kernel instantiation: as many CTAs as fit on the device, warps claiming trajectories.
-template <auto KERNEL, class... Extra>
-static int launch_detail_kernel(const MetricKArgs& k, int num_sms, size_t smem_extra, cudaStream_t st,
-                                const Extra&... extra) {
-  const size_t smem = (size_t)kDtWarps * detail_warp_bytes(k.T) + smem_extra;
-  constexpr int kMaxDev = 64;
-  static std::atomic<size_t> configured[kMaxDev];
-  int dev = 0;
-  FO_CUDA_TRY(cudaGetDevice(&dev));
-  const bool tracked = dev >= 0 && dev < kMaxDev;
-  if (!tracked || smem > configured[dev].load(std::memory_order_acquire)) {
-    FO_CUDA_TRY(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (tracked) configured[dev].store(smem, std::memory_order_release);
-  }
-  int per_sm = 1;
-  FO_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, KERNEL, kDtWarps * 32, smem));
-  if (per_sm < 1) per_sm = 1;
-  const int full = num_sms * per_sm;
-  const int need = (k.N + kDtWarps - 1) / kDtWarps;
-  const int grid = need < full ? need : full;
-  MetricKArgs kk = k;
-  kk.claim = (k.N > grid * kDtWarps) ? claim_slot(st) : nullptr;     // trajectories differ several-fold in cost
-  if (kk.claim) FO_CUDA_TRY(cudaMemsetAsync(kk.claim, 0, sizeof(unsigned int), st));
-  KERNEL<<<grid, kDtWarps * 32, smem, st>>>(kk, extra...);
-  count_launch();
-  FO_CUDA_TRY(cudaGetLastError());
-  return FO_OK;
-}
-
-constexpr uint32_t kDtAll = FO_M_CP | FO_M_DCE | FO_M_TTC | FO_M_HR | FO_M_BE | FO_M_TTCE | FO_M_WTTC;
-constexpr uint32_t kDtDefault = kDtAll & ~FO_M_BE;   // occlusion.yaml:12-18
-
+// Persistent launches: as many CTAs as fit on the device, their warps claiming trajectories independently.
 int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st) {
   if (k.pair && (reinterpret_cast<uintptr_t>(k.pair) & 15u)) {
     set_error("fo_metric_bundle: pair must be 16-byte aligned");
@@ -646,19 +612,22 @@ int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st) {
     set_error("fo_metric_bundle: step must be 4-byte aligned");
     return FO_ERR_INVALID_ARG;
   }
-  if (k.corr) return launch_detail_kernel<fo_metric_detail_corr_kernel>(k, num_sms, 0, st);
-  if (k.mmask == kDtAll) return launch_detail_kernel<fo_metric_detail_kernel<kDtAll>>(k, num_sms, 0, st);
-  if (k.mmask == kDtDefault) return launch_detail_kernel<fo_metric_detail_kernel<kDtDefault>>(k, num_sms, 0, st);
-  return launch_detail_kernel<fo_metric_detail_kernel<0u>>(k, num_sms, 0, st);
+  const size_t smem = (size_t)kDtWarps * detail_warp_bytes(k.T);
+  if (k.corr) return launch_persistent<fo_metric_detail_corr_kernel>(k, num_sms, kDtWarps * 32, kDtWarps, smem, false, st);
+  return with_mask(k.mmask, [&](auto m) {
+    return launch_persistent<fo_metric_detail_kernel<m>>(k, num_sms, kDtWarps * 32, kDtWarps, smem, false, st);
+  });
 }
 
-// k.N = the batch's rows; the caller has validated the descriptors and the alignment of every pair / step block
+// k.N = the batch's rows; the caller has validated the descriptors and the alignment of every pair / step block.  Each
+// warp keeps a copy of its problem's descriptor behind the warps' own shared memory.
 int launch_metric_batch_detail(const MetricKArgs& k, int num_sms, const DetailView& bv, cudaStream_t st) {
-  constexpr size_t x = kDtWarps * sizeof(DetailProb);   // the warps' descriptor copies
-  if (k.corr) return launch_detail_kernel<fo_metric_batch_detail_corr_kernel>(k, num_sms, x, st, bv);
-  if (k.mmask == kDtAll) return launch_detail_kernel<fo_metric_batch_detail_kernel<kDtAll>>(k, num_sms, x, st, bv);
-  if (k.mmask == kDtDefault) return launch_detail_kernel<fo_metric_batch_detail_kernel<kDtDefault>>(k, num_sms, x, st, bv);
-  return launch_detail_kernel<fo_metric_batch_detail_kernel<0u>>(k, num_sms, x, st, bv);
+  const size_t smem = (size_t)kDtWarps * (detail_warp_bytes(k.T) + sizeof(DetailProb));
+  if (k.corr)
+    return launch_persistent<fo_metric_batch_detail_corr_kernel>(k, num_sms, kDtWarps * 32, kDtWarps, smem, false, st, bv);
+  return with_mask(k.mmask, [&](auto m) {
+    return launch_persistent<fo_metric_batch_detail_kernel<m>>(k, num_sms, kDtWarps * 32, kDtWarps, smem, false, st, bv);
+  });
 }
 
 }  // namespace fo

@@ -3,6 +3,9 @@
 #pragma once
 #include <math_constants.h>
 
+#include <atomic>
+#include <type_traits>
+
 #include "fo_common.cuh"
 
 namespace fo {
@@ -747,6 +750,51 @@ struct EgoState {
 
 // one zeroed-per-launch device counter (trajectory claims of the persistent kernels), see fo_metric_sweep.cu
 unsigned int* claim_slot(cudaStream_t st);
+
+// The metric sets with instantiations of their own; any other set is read from MetricKArgs::mmask at run time (MASK 0).
+constexpr uint32_t kAllMetrics = FO_M_CP | FO_M_DCE | FO_M_TTC | FO_M_HR | FO_M_BE | FO_M_TTCE | FO_M_WTTC;
+constexpr uint32_t kDefaultMetrics = kAllMetrics & ~FO_M_BE;   // occlusion.yaml:12-18
+
+// f(std::integral_constant<uint32_t, MASK>) with the MASK the kernels are instantiated for when mmask is asked for
+template <class F>
+int with_mask(uint32_t mmask, F&& f) {
+  if (mmask == kAllMetrics) return f(std::integral_constant<uint32_t, kAllMetrics>{});
+  if (mmask == kDefaultMetrics) return f(std::integral_constant<uint32_t, kDefaultMetrics>{});
+  return f(std::integral_constant<uint32_t, 0u>{});
+}
+
+constexpr int kMaxDev = 64;   // devices with per-device host state (claim slots, function attributes)
+
+// Persistent launch of one metric-kernel instantiation: as many CTAs of `threads` threads as fit on the device, each
+// owning traj_per_cta trajectories at a time.  When one wave does not cover k.N, the trajectories are claimed from a
+// device counter (their cost varies several-fold), unless static_stride: then the CTAs stride over them.
+template <auto KERNEL, class... Extra>
+int launch_persistent(const MetricKArgs& k, int num_sms, int threads, int traj_per_cta, size_t smem, bool static_stride,
+                      cudaStream_t st, const Extra&... extra) {
+  // the opt-in shared-memory size is a per-device function attribute: remember what each device has been given
+  static std::atomic<size_t> configured[kMaxDev];
+  int dev = 0;
+  FO_CUDA_TRY(cudaGetDevice(&dev));
+  const bool tracked = dev >= 0 && dev < kMaxDev;
+  if (!tracked || smem > configured[dev].load(std::memory_order_acquire)) {
+    FO_CUDA_TRY(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (tracked) configured[dev].store(smem, std::memory_order_release);
+  }
+  int per_sm = 1;
+  FO_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, KERNEL, threads, smem));
+  if (per_sm < 1) per_sm = 1;
+  const int full = num_sms * per_sm;
+  const int need = (k.N + traj_per_cta - 1) / traj_per_cta;
+  const int grid = need < full ? need : full;
+  MetricKArgs kk = k;
+  kk.claim = (k.N > grid * traj_per_cta && !static_stride) ? claim_slot(st) : nullptr;
+  if (kk.claim) FO_CUDA_TRY(cudaMemsetAsync(kk.claim, 0, sizeof(unsigned int), st));
+  KERNEL<<<grid, threads, smem, st>>>(kk, extra...);
+  count_launch();
+  FO_CUDA_TRY(cudaGetLastError());
+  return FO_OK;
+}
+
 int launch_metric_detail(const MetricKArgs& k, int num_sms, cudaStream_t st);
 int launch_metric_sweep(const MetricKArgs& k, int num_sms, cudaStream_t st);
 // Batch of independent problems (fo_metric_batch): the trajectories of one launch belong to problems with their own
@@ -811,9 +859,6 @@ struct DetailView {
   int P;
 };
 int launch_metric_batch_detail(const MetricKArgs& k, int num_sms, const DetailView& bv, cudaStream_t st);
-// summary kernel over one shape class of a batch (uni: the one-warp window-filter shape, W == 1); k.N = the class's
-// trajectory count.  k.corr: the class's tables are correlated ones (fo_metric_batch_corr_kernel), in both batch launches
-int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st);
 // First valid row per problem (fo_metric_batch_select): one launch's state besides its BatchView.  The launch's
 // descriptors are sorted by N_p in descending order, so the problems with a row of rank j are a prefix of them; claims
 // run rank-major, and the ranks split into segments over which that prefix is the same.
@@ -823,8 +868,11 @@ struct SelectView {
   int32_t* selected;    // [n_problems] smallest rank whose row completed valid; initialised to N_p
   int S;
 };
-int launch_metric_batch_select(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv,
-                               const SelectView& sv, cudaStream_t st);
+// summary kernel over one shape class of a batch (uni: the one-warp window-filter shape, W == 1); k.N = the class's
+// trajectory count.  k.corr: the class's tables are correlated ones.  sv.selected != NULL: the select launch
+// (fo_metric_batch_select_kernel), else fo_metric_batch[_corr]_kernel.
+int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, const SelectView& sv,
+                        cudaStream_t st);
 int lane_group_log2(int A);                                  // team shape: a warp holds 1 << lg agents
 int pick_team_warps(int N, int T, int A, int num_sms);       // team size W (FO_TEAM_WARPS overrides)
 

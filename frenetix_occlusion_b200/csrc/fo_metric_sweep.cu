@@ -35,7 +35,6 @@
 // inlining costs more than a flag in a loop, hence the single call sites of the drains and the noinline helpers.  Reference semantics: SURVEY.md appendix A; citations on the helpers in fo_metric_dev.cuh.
 #include <stdlib.h>
 
-#include <atomic>
 #include <mutex>
 
 #include "fo_metric_dev.cuh"
@@ -973,16 +972,11 @@ int pick_team_warps(int N, int T, int A, int num_sms) {
   return w;
 }
 
-static void pick_shape(const MetricKArgs& k, int num_sms, int& W, SweepShape& shape) {
-  shape.lg_agents = lane_group_log2(k.A);
-  W = pick_team_warps(k.N, k.T, k.A, num_sms);
-}
-
 // Claim counters: one 4-byte slot per launch, zeroed in-stream before the kernel.  Eager launches rotate through a ring
 // (a slot is reused kClaimRing launches later); a launch recorded into a CUDA graph keeps a slot of its own for the
 // life of the process, because the graph may be replayed while later eager launches are in flight.  When the graph
 // slots run out the kernel falls back to static striding (claim == NULL).
-constexpr int kClaimRing = 1024, kClaimGraph = 3072, kMaxDev = 64;
+constexpr int kClaimRing = 1024, kClaimGraph = 3072;
 unsigned int* claim_slot(cudaStream_t st) {
   static std::mutex mu;
   static unsigned int* pool[kMaxDev] = {};
@@ -1009,120 +1003,60 @@ unsigned int* claim_slot(cudaStream_t st) {
   return pool[dev] + s;
 }
 
-// Persistent launch of one summary-kernel instantiation: as many teams as fit on the device, claiming trajectories.
-template <auto KERNEL, class... Extra>
-static int launch_team_kernel(const MetricKArgs& k, int num_sms, int W, bool uni, bool ties, cudaStream_t st,
-                              const SweepShape& shape, const Extra&... extra) {
-  const size_t smem = sweep_smem_bytes(k.T, W, uni, ties);
-  // the opt-in shared-memory size is a per-device function attribute: remember what each device has been given
-  static std::atomic<size_t> configured[kMaxDev];
-  int dev = 0;
-  FO_CUDA_TRY(cudaGetDevice(&dev));
-  const bool tracked = dev >= 0 && dev < kMaxDev;
-  if (!tracked || smem > configured[dev].load(std::memory_order_acquire)) {
-    FO_CUDA_TRY(cudaFuncSetAttribute(KERNEL, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    if (tracked) configured[dev].store(smem, std::memory_order_release);
-  }
-  int per_sm = 1;
-  FO_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, KERNEL, W * 32, smem));
-  if (per_sm < 1) per_sm = 1;
-  const int full = num_sms * per_sm;
-  const int grid = k.N < full ? k.N : full;       // persistent: teams claim trajectories
-  MetricKArgs kk = k;
-  const char* fixed = getenv("FO_STATIC_STRIDE");          // A/B switch: teams stride over trajectories instead
-  kk.claim = (k.N > grid && !(fixed && fixed[0] == '1')) ? claim_slot(st) : nullptr;
-  if (kk.claim) FO_CUDA_TRY(cudaMemsetAsync(kk.claim, 0, sizeof(unsigned int), st));
-  KERNEL<<<grid, W * 32, smem, st>>>(kk, shape, extra...);
-  count_launch();
-  FO_CUDA_TRY(cudaGetLastError());
-  return FO_OK;
-}
-
 // Float64 re-rounding of np.round(d, 3) ties is compiled into the variants that run when a clause of the validity mask
 // hangs on a rounded distance (dce / ttc / be thresholds armed, or the caller asked for it): there the mask is the
 // float64 reference's.  With those thresholds null (the deployment default, occlusion.yaml:20-28) only the last
 // digit of the reported min_dce could differ, and the kernel without the tie path is a quarter faster (DESIGN.md 5.1).
 static bool needs_ties(const MetricKArgs& k) { return (k.tmask & (FO_T_DCE | FO_T_TTC | FO_T_BE)) != 0 || k.exact_dce; }
 
-template <uint32_t MASK, bool STATS>
-static int launch_sweep_inst(const MetricKArgs& k, int num_sms, cudaStream_t st) {
-  int W = 1;
-  SweepShape shape;
-  pick_shape(k, num_sms, W, shape);
-  const bool ties = needs_ties(k);
-  const bool uni = W == 1 && shape.lg_agents == 5;
-  if (uni) return ties ? launch_team_kernel<fo_metric_sweep_kernel<MASK, STATS, true, true>>(k, num_sms, W, uni, ties, st, shape)
-                       : launch_team_kernel<fo_metric_sweep_kernel<MASK, STATS, true, false>>(k, num_sms, W, uni, ties, st, shape);
-  return ties ? launch_team_kernel<fo_metric_sweep_kernel<MASK, STATS, false, true>>(k, num_sms, W, uni, ties, st, shape)
-              : launch_team_kernel<fo_metric_sweep_kernel<MASK, STATS, false, false>>(k, num_sms, W, uni, ties, st, shape);
+// FO_STATIC_STRIDE=1: teams stride over the trajectories instead of claiming them (A/B switch, summary kernels only)
+static bool static_stride() {
+  const char* fixed = getenv("FO_STATIC_STRIDE");
+  return fixed && fixed[0] == '1';
 }
 
-constexpr uint32_t kAllMetrics = FO_M_CP | FO_M_DCE | FO_M_TTC | FO_M_HR | FO_M_BE | FO_M_TTCE | FO_M_WTTC;
-constexpr uint32_t kDefaultMetrics = kAllMetrics & ~FO_M_BE;   // occlusion.yaml:12-18
+// f(UNI, TIES) as std::bool_constants: the shape and tie-path variant of a summary-kernel family
+template <class F>
+static int with_shape(bool uni, bool ties, F&& f) {
+  if (uni) return ties ? f(std::true_type{}, std::true_type{}) : f(std::true_type{}, std::false_type{});
+  return ties ? f(std::false_type{}, std::true_type{}) : f(std::false_type{}, std::false_type{});
+}
 
+// One team of W warps per trajectory (persistent: as many teams as fit on the device, claiming trajectories).
 int launch_metric_sweep(const MetricKArgs& k, int num_sms, cudaStream_t st) {
-  if (k.corr) {
-    int W = 1;
-    SweepShape shape;
-    pick_shape(k, num_sms, W, shape);
-    const bool ties = needs_ties(k);
-    const bool uni = W == 1 && shape.lg_agents == 5;
-    if (k.stats) {
-      if (uni) return ties ? launch_team_kernel<fo_metric_sweep_corr_stats_kernel<true, true>>(k, num_sms, W, uni, ties, st, shape)
-                           : launch_team_kernel<fo_metric_sweep_corr_stats_kernel<true, false>>(k, num_sms, W, uni, ties, st, shape);
-      return ties ? launch_team_kernel<fo_metric_sweep_corr_stats_kernel<false, true>>(k, num_sms, W, uni, ties, st, shape)
-                  : launch_team_kernel<fo_metric_sweep_corr_stats_kernel<false, false>>(k, num_sms, W, uni, ties, st, shape);
-    }
-    if (uni) return ties ? launch_team_kernel<fo_metric_sweep_corr_kernel<true, true>>(k, num_sms, W, uni, ties, st, shape)
-                         : launch_team_kernel<fo_metric_sweep_corr_kernel<true, false>>(k, num_sms, W, uni, ties, st, shape);
-    return ties ? launch_team_kernel<fo_metric_sweep_corr_kernel<false, true>>(k, num_sms, W, uni, ties, st, shape)
-                : launch_team_kernel<fo_metric_sweep_corr_kernel<false, false>>(k, num_sms, W, uni, ties, st, shape);
-  }
-  if (k.stats) return launch_sweep_inst<0u, true>(k, num_sms, st);
-  if (k.mmask == kAllMetrics) return launch_sweep_inst<kAllMetrics, false>(k, num_sms, st);
-  if (k.mmask == kDefaultMetrics) return launch_sweep_inst<kDefaultMetrics, false>(k, num_sms, st);
-  return launch_sweep_inst<0u, false>(k, num_sms, st);
+  const SweepShape shape{lane_group_log2(k.A)};
+  const int W = pick_team_warps(k.N, k.T, k.A, num_sms);
+  const bool uni = W == 1 && shape.lg_agents == 5, ties = needs_ties(k);
+  const size_t smem = sweep_smem_bytes(k.T, W, uni, ties);
+  const bool fixed = static_stride();
+  return with_shape(uni, ties, [&](auto u, auto t) {
+    if (k.corr && k.stats)
+      return launch_persistent<fo_metric_sweep_corr_stats_kernel<u, t>>(k, num_sms, W * 32, 1, smem, fixed, st, shape);
+    if (k.corr) return launch_persistent<fo_metric_sweep_corr_kernel<u, t>>(k, num_sms, W * 32, 1, smem, fixed, st, shape);
+    if (k.stats)
+      return launch_persistent<fo_metric_sweep_kernel<0u, true, u, t>>(k, num_sms, W * 32, 1, smem, fixed, st, shape);
+    return with_mask(k.mmask, [&](auto m) {
+      return launch_persistent<fo_metric_sweep_kernel<m, false, u, t>>(k, num_sms, W * 32, 1, smem, fixed, st, shape);
+    });
+  });
 }
 
-template <uint32_t MASK>
-static int launch_batch_inst(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st) {
+int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, const SelectView& sv,
+                        cudaStream_t st) {
   const SweepShape shape{0};
   const bool ties = needs_ties(k);
-  if (uni) return ties ? launch_team_kernel<fo_metric_batch_kernel<MASK, true, true>>(k, num_sms, W, uni, ties, st, shape, bv)
-                       : launch_team_kernel<fo_metric_batch_kernel<MASK, true, false>>(k, num_sms, W, uni, ties, st, shape, bv);
-  return ties ? launch_team_kernel<fo_metric_batch_kernel<MASK, false, true>>(k, num_sms, W, uni, ties, st, shape, bv)
-              : launch_team_kernel<fo_metric_batch_kernel<MASK, false, false>>(k, num_sms, W, uni, ties, st, shape, bv);
-}
-
-int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv, cudaStream_t st) {
-  if (k.corr) {
-    const SweepShape shape{0};
-    const bool ties = needs_ties(k);
-    if (uni) return ties ? launch_team_kernel<fo_metric_batch_corr_kernel<true, true>>(k, num_sms, W, uni, ties, st, shape, bv)
-                         : launch_team_kernel<fo_metric_batch_corr_kernel<true, false>>(k, num_sms, W, uni, ties, st, shape, bv);
-    return ties ? launch_team_kernel<fo_metric_batch_corr_kernel<false, true>>(k, num_sms, W, uni, ties, st, shape, bv)
-                : launch_team_kernel<fo_metric_batch_corr_kernel<false, false>>(k, num_sms, W, uni, ties, st, shape, bv);
-  }
-  if (k.mmask == kAllMetrics) return launch_batch_inst<kAllMetrics>(k, num_sms, W, uni, bv, st);
-  if (k.mmask == kDefaultMetrics) return launch_batch_inst<kDefaultMetrics>(k, num_sms, W, uni, bv, st);
-  return launch_batch_inst<0u>(k, num_sms, W, uni, bv, st);
-}
-
-template <bool CORR>
-static int launch_select_inst(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv,
-                              const SelectView& sv, cudaStream_t st) {
-  const SweepShape shape{0};
-  const bool ties = needs_ties(k);
-  if (uni) return ties ? launch_team_kernel<fo_metric_batch_select_kernel<true, true, CORR>>(k, num_sms, W, uni, ties, st, shape, bv, sv)
-                       : launch_team_kernel<fo_metric_batch_select_kernel<true, false, CORR>>(k, num_sms, W, uni, ties, st, shape, bv, sv);
-  return ties ? launch_team_kernel<fo_metric_batch_select_kernel<false, true, CORR>>(k, num_sms, W, uni, ties, st, shape, bv, sv)
-              : launch_team_kernel<fo_metric_batch_select_kernel<false, false, CORR>>(k, num_sms, W, uni, ties, st, shape, bv, sv);
-}
-
-int launch_metric_batch_select(const MetricKArgs& k, int num_sms, int W, bool uni, const BatchView& bv,
-                               const SelectView& sv, cudaStream_t st) {
-  return k.corr ? launch_select_inst<true>(k, num_sms, W, uni, bv, sv, st)
-                : launch_select_inst<false>(k, num_sms, W, uni, bv, sv, st);
+  const size_t smem = sweep_smem_bytes(k.T, W, uni, ties);
+  const bool fixed = static_stride();
+  return with_shape(uni, ties, [&](auto u, auto t) {
+    if (sv.selected && k.corr)
+      return launch_persistent<fo_metric_batch_select_kernel<u, t, true>>(k, num_sms, W * 32, 1, smem, fixed, st, shape, bv, sv);
+    if (sv.selected)
+      return launch_persistent<fo_metric_batch_select_kernel<u, t, false>>(k, num_sms, W * 32, 1, smem, fixed, st, shape, bv, sv);
+    if (k.corr) return launch_persistent<fo_metric_batch_corr_kernel<u, t>>(k, num_sms, W * 32, 1, smem, fixed, st, shape, bv);
+    return with_mask(k.mmask, [&](auto m) {
+      return launch_persistent<fo_metric_batch_kernel<m, u, t>>(k, num_sms, W * 32, 1, smem, fixed, st, shape, bv);
+    });
+  });
 }
 
 }  // namespace fo

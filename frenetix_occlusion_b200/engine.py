@@ -413,7 +413,7 @@ class MetricEngine:
 
     # ---- batches of independent problems ------------------------------------------------------------------------
     def set_agent_batch(self, agent_sets: Sequence[AgentSet], origins=None, vehicles=None, correlated: bool = False):
-        """Upload + pack the phantom predictions of P independent problems (``fo_agents_pack_batch``): one float64
+        """Upload + pack the phantom predictions of P independent problems (``fo_agents_pack_batch_corr``): one float64
         origin shift per problem, one host-to-device copy of all of them, one pack call.  ``origins``: [P, 2] or None
         (no shift).  ``vehicles``: P ego vehicle descriptions (each a dict or an object with attributes, as the
         constructor takes them), or None for the engine's own vehicle in every problem; ``assess_batch`` assesses
@@ -421,33 +421,26 @@ class MetricEngine:
         engine built with vehicles[p].
 
         ``correlated``: sets with correlated prediction covariances (``AgentSet.cov_xy`` set) are accepted and packed
-        as ``set_agents`` packs them (``fo_agents_pack_batch_corr``); their collision probabilities cost many times the
-        diagonal ones.  Without it such a set raises ``ValueError``.  A batch without one makes the diagonal calls."""
+        as ``set_agents`` packs them; their collision probabilities cost many times the diagonal ones.  Without it such
+        a set raises ``ValueError``."""
         P = len(agent_sets)
         if not correlated and any(a.cov_xy is not None for a in agent_sets):
             raise ValueError("batches take diagonal prediction covariances only unless correlated=True; assess a "
                              "correlated set with set_agents() + assess()")
-        veh = None
-        if vehicles is not None:
-            if len(vehicles) != P:
-                raise ValueError(f"{len(vehicles)} vehicles for {P} problems")
-            veh = (L.FoVehicle * max(P, 1))(*[vehicle_struct(v) for v in vehicles])
+        if vehicles is not None and len(vehicles) != P:
+            raise ValueError(f"{len(vehicles)} vehicles for {P} problems")
+        veh = [self.vehicle] * P if vehicles is None else [vehicle_struct(v) for v in vehicles]
+        veh = (L.FoVehicle * max(P, 1))(*veh)
         org = np.zeros((P, 2)) if origins is None else np.asarray(origins, dtype=np.float64).reshape(P, 2)
         n_agents = np.array([a.n_agents if a.t_stride > 0 else 0 for a in agent_sets], dtype=np.int32)
         t_stride = np.array([a.t_stride if n else 0 for a, n in zip(agent_sets, n_agents)], dtype=np.int32)
         if np.any(t_stride > L.FO_MAX_STATES):
             raise ValueError(f"predictions longer than {L.FO_MAX_STATES} states are not supported")
-        # the correlated problems (with agents, as set_agents packs them); None = the diagonal calls
+        # the correlated problems (with agents, as set_agents packs them)
         corr = np.array([a.cov_xy is not None and n > 0 for a, n in zip(agent_sets, n_agents)], dtype=np.uint8)
-        corr = corr if corr.any() else None
-        if corr is not None and veh is None:
-            veh = (L.FoVehicle * P)(*[self.vehicle] * P)
         offsets = np.zeros(P, dtype=np.int64)
-        if corr is None:
-            arena_bytes = L.lib.fo_agent_batch_layout(P, n_agents.ctypes.data, t_stride.ctypes.data, offsets.ctypes.data)
-        else:
-            arena_bytes = L.lib.fo_agent_batch_layout_corr(P, n_agents.ctypes.data, t_stride.ctypes.data,
-                                                           corr.ctypes.data, offsets.ctypes.data)
+        arena_bytes = L.lib.fo_agent_batch_layout_corr(P, n_agents.ctypes.data, t_stride.ctypes.data, corr.ctypes.data,
+                                                       offsets.ctypes.data)
         problems = (L.FoBatchProblem * max(P, 1))()
         for p in range(P):
             problems[p].n_agents, problems[p].t_stride, problems[p].table_offset = int(n_agents[p]), int(t_stride[p]), int(offsets[p])
@@ -459,7 +452,7 @@ class MetricEngine:
             return
         # one host buffer: 6 float rows [A, S] (x, y shifted per problem; a seventh, cov_xy, with correlated problems),
         # 4 float columns [A], 2 int32 columns [A]
-        R = 6 if corr is None else 7
+        R = 7 if corr.any() else 6
         buf = np.zeros(R * A * S + 6 * A, dtype=np.float32)
         fl = buf[:R * A * S].reshape(R, A, S)
         pa = buf[R * A * S:R * A * S + 4 * A].reshape(4, A)
@@ -473,7 +466,7 @@ class MetricEngine:
             fl[0, rows, :tp] = ag.x - org[p, 0]
             fl[1, rows, :tp] = ag.y - org[p, 1]
             fl[2, rows, :tp], fl[3, rows, :tp], fl[4, rows, :tp], fl[5, rows, :tp] = ag.yaw, ag.v, ag.var_x, ag.var_y
-            if corr is not None and corr[p]:
+            if corr[p]:
                 fl[6, rows, :tp] = ag.cov_xy
             pa[:, rows] = (ag.length, ag.width, ag.buf_length, ag.buf_width)
             ia[:, rows] = (ag.n_states, ag.kind)
@@ -489,17 +482,10 @@ class MetricEngine:
             raw.length, raw.width, raw.buf_length, raw.buf_width = [base + f4 * i * A for i in range(4)]
             raw.n_states, raw.kind = base + f4 * 4 * A, base + f4 * 5 * A
             arena = torch.empty(max(arena_bytes, 16), dtype=torch.uint8, device=dev)
-            if corr is not None:
-                L.check(L.lib.fo_agents_pack_batch_corr(C.byref(raw), C.c_void_p(ptr + f4 * 6 * A * S), P, problems,
-                                                        corr.ctypes.data, veh, C.c_void_p(arena.data_ptr()), arena_bytes,
-                                                        self._stream()), "fo_agents_pack_batch_corr")
-            elif veh is None:
-                L.check(L.lib.fo_agents_pack_batch(C.byref(raw), P, problems, C.byref(self.vehicle),
-                                                   C.c_void_p(arena.data_ptr()), arena_bytes, self._stream()),
-                        "fo_agents_pack_batch")
-            else:
-                L.check(L.lib.fo_agents_pack_batch_vehicles(C.byref(raw), P, problems, veh, C.c_void_p(arena.data_ptr()),
-                                                            arena_bytes, self._stream()), "fo_agents_pack_batch_vehicles")
+            cov_xy = C.c_void_p(ptr + f4 * 6 * A * S) if R == 7 else None
+            L.check(L.lib.fo_agents_pack_batch_corr(C.byref(raw), cov_xy, P, problems, corr.ctypes.data, veh,
+                                                    C.c_void_p(arena.data_ptr()), arena_bytes, self._stream()),
+                    "fo_agents_pack_batch_corr")
         self._batch["arena"] = arena
         self._batch["raw_dev"] = d_buf           # keep alive until the stream work is done
 
@@ -531,24 +517,16 @@ class MetricEngine:
                      out: Optional[BatchResult] = None) -> BatchResult:
         """One pass over every problem of the batch set by ``set_agent_batch`` in one metric call.  ``egos[p]``: problem
         p's [N_p, T, 5] bundle (host array or CUDA tensor, in the caller's frame: it is shifted by the problem's origin).
-        Without detail outputs this is ``fo_metric_batch``; with ``want_pair`` / ``want_step`` it is
-        ``fo_metric_batch_detail`` (their ``_corr`` forms when the batch has a correlated problem), and ``split()`` gives problem p what ``set_agents`` + ``assess(want_pair,
+        Without detail outputs this is ``fo_metric_batch_corr``; with ``want_pair`` / ``want_step`` it is
+        ``fo_metric_batch_detail_corr``, and ``split()`` gives problem p what ``set_agents`` + ``assess(want_pair,
         want_step)`` gives it alone (in an engine built with its vehicle, when ``set_agent_batch`` had ``vehicles``).
         ``out``: preallocated outputs of the batch's sizes (valid / summary / flags, and
         the flat pair / step where wanted).  Asynchronous on the current stream."""
         b = self._batch
         a, out, t = self._batch_args("assess_batch", egos, want_pair, want_step, out)
         with torch.cuda.device(self.device):
-            detail, veh, corr = bool(a.common.pair or a.common.step), b["vehicles"], b["corr"]
-            if corr is not None:
-                fn = "fo_metric_batch_detail_corr" if detail else "fo_metric_batch_corr"
-                L.check(getattr(L.lib, fn)(C.byref(a), corr.ctypes.data, veh, self._stream()), fn)
-            elif veh is None:
-                fn = "fo_metric_batch_detail" if detail else "fo_metric_batch"
-                L.check(getattr(L.lib, fn)(C.byref(a), self._stream()), fn)
-            else:
-                fn = "fo_metric_batch_detail_vehicles" if detail else "fo_metric_batch_vehicles"
-                L.check(getattr(L.lib, fn)(C.byref(a), veh, self._stream()), fn)
+            fn = "fo_metric_batch_detail_corr" if (a.common.pair or a.common.step) else "fo_metric_batch_corr"
+            L.check(getattr(L.lib, fn)(C.byref(a), b["corr"].ctypes.data, b["vehicles"], self._stream()), fn)
         out._keepalive = (t, b["arena"])
         return out
 
@@ -563,9 +541,8 @@ class MetricEngine:
         a, out, t = self._batch_args("select_batch", egos, False, False, out)
         with torch.cuda.device(self.device):
             out.selected = torch.empty(b["P"], dtype=torch.int32, device=self.device)
-            corr = b["corr"]
-            L.check(L.lib.fo_metric_batch_select(C.byref(a), corr.ctypes.data if corr is not None else None,
-                                                 b["vehicles"], C.c_void_p(out.selected.data_ptr()), self._stream()),
+            L.check(L.lib.fo_metric_batch_select(C.byref(a), b["corr"].ctypes.data, b["vehicles"],
+                                                 C.c_void_p(out.selected.data_ptr()), self._stream()),
                     "fo_metric_batch_select")
         out._keepalive = (t, b["arena"])
         return out

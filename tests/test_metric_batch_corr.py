@@ -225,7 +225,7 @@ def _assert_mixed_batch_equals_single(probs, fleet, want_pair=False, want_step=F
     import torch
     eng = _engine(probs[0][3])
     eng.set_agent_batch([p[0] for p in probs], [p[1] for p in probs], vehicles=fleet, correlated=True)
-    assert eng._batch["corr"] is not None
+    assert eng._batch["corr"].any()
     parts = eng.assess_batch([p[2] for p in probs], want_pair=want_pair, want_step=want_step).split()
     fields = ("valid", "flags", "summary") + (("pair",) if want_pair else ()) + (("step",) if want_step else ())
     for i, ((ag, origin, ego, case), veh, got) in enumerate(zip(probs, fleet, parts)):
@@ -328,7 +328,8 @@ class _Recorder:
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("detail", [False, True])
-def test_all_diagonal_batch_with_correlated_allowed_makes_the_diagonal_calls(detail, cuda_device, monkeypatch):
+def test_all_diagonal_batch_with_correlated_allowed_makes_the_diagonal_launches(detail, cuda_device, monkeypatch):
+    import torch
     from frenetix_occlusion_b200 import _lib as L
     monkeypatch.setenv("FO_TEAM_WARPS", "1")
     probs, fleet = _mixed(79, 31, n_set=(1, 64), n_problems=8, every=0)
@@ -337,15 +338,24 @@ def test_all_diagonal_batch_with_correlated_allowed_makes_the_diagonal_calls(det
         rec = _Recorder(L.lib)
         monkeypatch.setattr(L, "lib", rec)
         eng = _engine(probs[0][3])
-        eng.set_agent_batch([p[0] for p in probs], [p[1] for p in probs], vehicles=fleet, correlated=correlated)
-        got = eng.assess_batch([p[2] for p in probs], want_pair=detail, want_step=detail)
+        with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+            eng.set_agent_batch([p[0] for p in probs], [p[1] for p in probs], vehicles=fleet, correlated=correlated)
+            got = eng.assess_batch([p[2] for p in probs], want_pair=detail, want_step=detail)
+            torch.cuda.synchronize()
         monkeypatch.setattr(L, "lib", rec._lib)
-        return [c for c in rec.calls if c.startswith("fo_") and c not in ("fo_last_error",)], got
-    calls_c, got_c = run(True)
-    calls_d, got_d = run(False)
+        assert not eng._batch["corr"].any()
+        kernels = [e.name for e in sorted(prof.events(), key=lambda e: e.time_range.start)
+                   if e.device_type == torch.autograd.DeviceType.CUDA and "fo::" in e.name]
+        return [c for c in rec.calls if c.startswith("fo_") and c not in ("fo_last_error",)], kernels, got
+    calls_c, kernels_c, got_c = run(True)
+    calls_d, kernels_d, got_d = run(False)
     assert calls_c == calls_d
-    assert calls_c == ["fo_agent_batch_layout", "fo_agents_pack_batch_vehicles",
-                       "fo_metric_batch_detail_vehicles" if detail else "fo_metric_batch_vehicles"]
+    assert calls_c == ["fo_agent_batch_layout_corr", "fo_agents_pack_batch_corr",
+                       "fo_metric_batch_detail_corr" if detail else "fo_metric_batch_corr"]
+    # with every flag 0 the _corr calls make the launches of the diagonal ones: no correlated kernel runs
+    assert kernels_c == kernels_d
+    assert kernels_c and not any("corr" in k for k in kernels_c), kernels_c
+    assert any(("fo_metric_batch_detail_kernel" if detail else "fo_metric_batch_kernel") in k for k in kernels_c), kernels_c
     for f in ("valid", "flags", "summary") + (("pair", "step") if detail else ()):
         _assert_equal(getattr(got_c, f), getattr(got_d, f), f)
     for (ag, origin, ego, case), veh, g in zip(probs, fleet, got_c.split()):

@@ -75,6 +75,89 @@ def agent_table(n_agents: int, n_states: int, dt: float = 0.1, seed: int = SEED 
     return out
 
 
+# Every obstacle type of the reference's ObstacleType that the metric core distinguishes (``_lib.KINDS``), with a
+# plausible raw length / width / speed and the buffer factors of the nearest kind of AGENT_DEFAULTS.  The car-mass
+# kinds keep a buffered area far above the 3.3 m^2 below which -1333.5 + 526.9 size^0.8 is not positive.
+VARIED_KINDS = {
+    "Pedestrian": AGENT_DEFAULTS["Pedestrian"], "Bicycle": AGENT_DEFAULTS["Bicycle"], "Car": AGENT_DEFAULTS["Car"],
+    "Truck": AGENT_DEFAULTS["Truck"],
+    "Bus": {"length": 12.0, "width": 2.55, "v": 8.0, "fl": 1.2, "fw": 1.3},
+    "Motorcycle": {"length": 2.2, "width": 0.8, "v": 12.0, "fl": 1.4, "fw": 2.5},
+    "PriorityVehicle": {"length": 5.2, "width": 2.0, "v": 14.0, "fl": 1.2, "fw": 1.3},
+    "ParkedVehicle": {"length": 4.5, "width": 1.8, "v": 0.0, "fl": 1.2, "fw": 1.3},
+    "Taxi": {"length": 4.8, "width": 1.9, "v": 9.0, "fl": 1.2, "fw": 1.3},
+    "Train": {"length": 30.0, "width": 3.0, "v": 10.0, "fl": 1.2, "fw": 1.3},
+    "Unknown": {"length": 1.0, "width": 1.0, "v": 2.0, "fl": 1.2, "fw": 1.3},
+}
+
+
+def varied_agents(n_agents: int, n_states: int, seed: int, *, jitter: bool = False, ragged: bool = True,
+                  dt: float = 0.1, area=((-20.0, 50.0), (-25.0, 25.0)), variance_factor: float = 1.05):
+    """Case-format predictions that turn, change speed and carry per-axis variances, cycling through every kind of
+    VARIED_KINDS.  ``agent_table`` keeps heading, speed and var_x = var_y constant, so a kernel that reads a heading,
+    speed or variance from the wrong step or axis agrees with it; these agents tell such mistakes apart.
+
+    * kinematic (default): heading yaw0 + w t with w ~ U(-0.6, 0.6) rad/s, speed max(v0 + a t, 0) with
+      a ~ U(-3, 2) (ParkedVehicle: 0), positions integrated from both; every third agent starts within 0.15 rad of
+      +-pi and turns outwards, so its heading leaves [-pi, pi].
+    * ``jitter``: heading, speed and variances drawn independently per step, positions a random walk -- any index
+      offset then gives a large error, not a second-order one.
+    * per state var_x, var_y = 0.1 * 1.05^k * U(0.3, 3) each, both zero on about 10 % of the states, carried as a
+      diagonal ``cov`` [T_a, 2, 2] (``var`` is var_x).
+    * ``ragged``: every fifth agent has 1, 2, 8, 9 or n_states + 20 (at most 128) states instead of n_states.
+    All values are float32-representable."""
+    rng = np.random.default_rng(seed)
+    kinds = list(VARIED_KINDS)
+    out = []
+    for i in range(n_agents):
+        kind = kinds[i % len(kinds)]
+        d = VARIED_KINDS[kind]
+        n = n_states
+        if ragged and i % 5 == 4:
+            n = [1, 2, 8, 9, min(n_states + 20, 128)][(i // 5) % 5]
+        t = np.arange(n) * dt
+        x0, y0 = rng.uniform(*area[0]), rng.uniform(*area[1])
+        if i % 3 == 0:
+            sgn = rng.choice((-1.0, 1.0))
+            yaw0, w = sgn * (np.pi - rng.uniform(0.0, 0.15)), sgn * rng.uniform(0.2, 0.6)
+        else:
+            yaw0, w = rng.uniform(-np.pi, np.pi), rng.uniform(-0.6, 0.6)
+        if jitter:
+            yaw = yaw0 + rng.uniform(-1.5, 1.5, n)
+            v = rng.uniform(0.0, 1.5 * d["v"] + 0.5, n) * (d["v"] > 0)
+            x = x0 + np.cumsum(rng.normal(0.0, 0.4, n))
+            y = y0 + np.cumsum(rng.normal(0.0, 0.4, n))
+        else:
+            yaw = yaw0 + w * t
+            v = np.maximum(d["v"] + rng.uniform(-3.0, 2.0) * t, 0.0) * (d["v"] > 0)   # a parked vehicle stays
+            x = x0 + np.concatenate(([0.0], np.cumsum(v[:-1] * np.cos(yaw[:-1]) * dt)))
+            y = y0 + np.concatenate(([0.0], np.cumsum(v[:-1] * np.sin(yaw[:-1]) * dt)))
+        base = 0.1 * np.power(variance_factor, np.arange(n))
+        vx, vy = _f32(base * rng.uniform(0.3, 3.0, n)), _f32(base * rng.uniform(0.3, 3.0, n))
+        zero = rng.random(n) < 0.1
+        vx[zero] = vy[zero] = 0.0
+        cov = np.zeros((n, 2, 2))
+        cov[:, 0, 0], cov[:, 1, 1] = vx, vy
+        out.append({"agent_type": kind, "length": float(_f32(d["length"])), "width": float(_f32(d["width"])),
+                    "buf_length": float(_f32(d["length"] * d["fl"])), "buf_width": float(_f32(d["width"] * d["fw"])),
+                    "pos": _f32(np.stack((x, y), -1)), "yaw": _f32(yaw), "v": _f32(v), "var": vx, "cov": cov})
+    return out
+
+
+def rotate_bundle(ego: np.ndarray, seed: int) -> np.ndarray:
+    """``ego`` [N, T, 5] with every trajectory turned about the origin by its own heading ~ U(-pi, pi): the arcs of
+    ``ego_bundle`` all start along +x, so their collision-probability boxes mostly travel along x; turned, both axes
+    of an agent's covariance matter."""
+    ego = np.asarray(ego, dtype=np.float64)
+    h = np.random.default_rng(seed).uniform(-np.pi, np.pi, len(ego))[:, None]
+    c, s = np.cos(h), np.sin(h)
+    out = ego.copy()
+    out[..., 0] = c * ego[..., 0] - s * ego[..., 1]
+    out[..., 1] = s * ego[..., 0] + c * ego[..., 1]
+    out[..., 2] = ego[..., 2] + h
+    return _f32(out)
+
+
 def make_case(n_traj: int, n_agents: int, n_states: int, dt: float = 0.1, seed: int = SEED,
               activated_metrics=None, thresholds=None, agent_states: int | None = None):
     """A complete *case* (see ``oracle/ref_runner.py`` for the format)."""
@@ -84,6 +167,15 @@ def make_case(n_traj: int, n_agents: int, n_states: int, dt: float = 0.1, seed: 
     return {"dt": dt, "vehicle": {k: float(_f32(v)) for k, v in VEHICLE.items()}, "ego": ego, "agents": agents,
             "activated_metrics": list(ALL_METRICS if activated_metrics is None else activated_metrics),
             "thresholds": dict(DEFAULT_THRESHOLDS if thresholds is None else thresholds)}
+
+
+def make_varied_case(n_traj: int, n_agents: int, n_states: int, dt: float = 0.1, seed: int = SEED,
+                     activated_metrics=None, thresholds=None, *, jitter: bool = False, **agent_kw):
+    """``make_case`` with its trajectories turned by ``rotate_bundle`` and ``varied_agents`` for its agents."""
+    case = make_case(n_traj, 0, n_states, dt, seed, activated_metrics, thresholds)
+    case["ego"] = rotate_bundle(case["ego"], seed)
+    case["agents"] = varied_agents(n_agents, n_states, seed, jitter=jitter, dt=dt, **agent_kw)
+    return case
 
 
 # named BASELINE.json configurations -----------------------------------------------------------

@@ -62,6 +62,8 @@ def check_required_metrics(metric_names):
 
 # --------------------------------------------------------------------------------------------
 def _stack_agents(case):
+    """``var`` [A, Tm, 2] holds (sigma_x^2, sigma_y^2) of every state: the diagonal of the agent's ``cov``
+    (``cov_list``, [T_a, 2, 2]) when it has one, else its scalar ``var`` on both axes."""
     ags = case["agents"]
     A = len(ags)
     Ta = np.array([len(np.asarray(a["yaw"])) for a in ags], dtype=np.int64)
@@ -69,19 +71,28 @@ def _stack_agents(case):
     pos = np.zeros((A, Tm, 2))
     yaw = np.zeros((A, Tm))
     vel = np.zeros((A, Tm))
-    var = np.full((A, Tm), 0.1)
+    var = np.full((A, Tm, 2), 0.1)
     for k, a in enumerate(ags):
         pos[k, :Ta[k]] = np.asarray(a["pos"], dtype=np.float64).reshape(-1, 2)
         yaw[k, :Ta[k]] = a["yaw"]
         vel[k, :Ta[k]] = a["v"]
-        var[k, :Ta[k]] = a["var"]
+        if "cov" in a:
+            c = np.asarray(a["cov"], dtype=np.float64)
+            var[k, :Ta[k]] = np.stack((c[:, 0, 0], c[:, 1, 1]), -1)
+        else:
+            var[k, :Ta[k]] = np.asarray(a["var"], dtype=np.float64)[:, None]
     return A, Ta, Tm, pos, yaw, vel, var
 
 
 def collision_probability(case):
     """CP per step, [N, A, T-1].  collision_probability.py:14-126 (see SURVEY.md appendix A):
     ego state i pairs with agent position i-1, agent yaw i, covariance i-1; 5 m strict gate on the
-    min distance of the three obstacle points to the raw ego point; three axis-aligned ego boxes."""
+    min distance of the three obstacle points to the raw ego point; three axis-aligned ego boxes.
+    sigma_x, sigma_y = sqrt(cov[i-1][0][0]), sqrt(cov[i-1][1][1]) (mvnun with a diagonal covariance factorises
+    per axis); a correlated ``cov`` is ``tests/corr_oracle.py``'s case and raises here."""
+    for k, a in enumerate(case["agents"]):
+        if "cov" in a and np.any(np.asarray(a["cov"])[:, [0, 1], [1, 0]] != 0):
+            raise ValueError(f"agent {k}: correlated covariance (not a diagonal one)")
     ego = np.asarray(case["ego"], dtype=np.float64)
     N, T, _ = ego.shape
     A, Ta, Tm, pos, yaw, vel, var = _stack_agents(case)
@@ -101,8 +112,8 @@ def collision_probability(case):
         e = ego[:, i, 0:2]                                            # [N, n, 2] raw rear-axle point
         d = np.sqrt(((mus[None] - e[:, None]) ** 2).sum(-1))         # [N, 3, n]
         gate = d.min(1) > 5.0                                         # :65-67 strict
-        v = var[a, i - 1].copy()
-        v[v == 0.0] = 0.1                                             # :85-87
+        v = var[a, i - 1].copy()                                      # [n, 2]
+        v[(v == 0.0).all(-1)] = 0.1                                   # :85-87 (an all-zero matrix)
         sig = np.sqrt(v)
         th = ego[:, i, 2]
         off = np.stack((np.cos(th), np.sin(th)), -1) * (L / 3.0)      # r_x*(2/3)*a_x, :160-162
@@ -111,8 +122,8 @@ def collision_probability(case):
         lo = cen - half
         hi = cen + half
         # [N, mu(3), box(3), n, 2]
-        zhi = (hi[:, None] - mus[None, :, None]) / sig[None, None, None, :, None]
-        zlo = (lo[:, None] - mus[None, :, None]) / sig[None, None, None, :, None]
+        zhi = (hi[:, None] - mus[None, :, None]) / sig[None, None, None]
+        zlo = (lo[:, None] - mus[None, :, None]) / sig[None, None, None]
         pr = ndtr(zhi) - ndtr(zlo)
         prob = (pr[..., 0] * pr[..., 1]).sum((1, 2)) / 3.0            # :115-122
         cp[:, a, i - 1] = np.where(gate, 0.0, prob)

@@ -127,13 +127,8 @@ def compare_bundle(out, res, case):
                     rep["fail"].append(f"pair {name} mismatch at {i}: gpu {pair[..., col][i]!r} "
                                        f"oracle {out['hr_pair'][name][i]!r} ({int(bad.sum())})")
             idx_bad = (pair[..., 4].astype(np.int64) != out["hr_pair"]["max_obst_risk_index"]) & ~hr_tie_pair
-            # argmax of a float32 product may tie differently only when two risks are within rounding
             if idx_bad.any():
-                orr = np.nan_to_num(out["obst_risk"], nan=-1.0)
-                gi = pair[..., 4].astype(np.int64)
-                v_g = np.take_along_axis(orr, gi[..., None], -1)[..., 0]
-                v_o = orr.max(-1)
-                real = idx_bad & ~_close(v_g, v_o, 1e-5, 1e-12)
+                real = idx_bad & ~risk_index_tie(out, pair[..., 4].astype(np.int64))
                 rep["ties"]["risk_index"] = int((idx_bad & ~real).sum())
                 if real.any():
                     rep["fail"].append(f"max_obst_risk_index mismatch on {int(real.sum())} pairs")
@@ -191,6 +186,17 @@ def compare_bundle(out, res, case):
         rep["fail"].append(f"validity mask differs on {int(hard.sum())} trajectories, first {int(np.argmax(hard))}")
     rep["n_valid"] = int(out["valid"].sum())
     return rep
+
+
+def risk_index_tie(out, gpu_index):
+    """Risk argmax tie, [...] like ``gpu_index`` (the kernel's max_obst_risk_index per pair): the oracle's obstacle
+    risk at the kernel's index equals its maximum within rounding (1e-5 relative, 1e-12 absolute).  Either two float32
+    risk products are equal within rounding, or all risks of the pair are below 1e-12 -- e.g. exact zeros where the
+    float64 ndtr(hi) - ndtr(lo) of an interval more than ~8 sigma away cancels, while the kernels' erfc of the tails
+    keeps a value of 1e-24, so the first maximum moves from step 0 to that step."""
+    orr = np.nan_to_num(out["obst_risk"], nan=-1.0)
+    v_g = np.take_along_axis(orr, gpu_index[..., None], -1)[..., 0]
+    return _close(v_g, orr.max(-1), 1e-5, 1e-12)
 
 
 def run_gpu(case, want_pair=True, want_step=True, device="cuda:0"):

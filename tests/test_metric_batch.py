@@ -135,8 +135,10 @@ A_SET = [0, 1, 2, 3, 5, 8, 16, 17, 32, 33, 64, 300]
 N_SET = [0, 1, 5, 64, 500]
 
 
-def _problems(seed, T, n_problems=None, a_set=A_SET, n_set=N_SET, metrics=None, thresholds=None):
-    """Seeded problems of synthetic.make_case, each moved to its own place kilometres from the others."""
+def _problems(seed, T, n_problems=None, a_set=A_SET, n_set=N_SET, metrics=None, thresholds=None, varied=False):
+    """Seeded problems of synthetic.make_case, each moved to its own place kilometres from the others.  ``varied``:
+    synthetic.make_varied_case's turned trajectories and agents of every kind that turn, change speed and carry
+    per-axis variances."""
     from frenetix_occlusion_b200 import synthetic as S
     from frenetix_occlusion_b200.engine import AgentSet
     rng = np.random.default_rng(seed)
@@ -144,7 +146,8 @@ def _problems(seed, T, n_problems=None, a_set=A_SET, n_set=N_SET, metrics=None, 
     for p in range(n_problems or len(a_set)):
         A = a_set[p % len(a_set)]
         N = n_set[(p * 3 + seed) % len(n_set)]
-        case = S.make_case(max(N, 1), A, T, seed=seed * 1000 + p, activated_metrics=metrics, thresholds=thresholds)
+        case = (S.make_varied_case if varied else S.make_case)(max(N, 1), A, T, seed=seed * 1000 + p,
+                                                               activated_metrics=metrics, thresholds=thresholds)
         dx, dy = rng.uniform(-5000.0, 5000.0, 2).round(1)
         ego = case["ego"][:N].copy()
         ego[..., 0] += dx
@@ -188,6 +191,13 @@ def _assert_batch_equals_single(problems, monkeypatch, warps):
 @pytest.mark.parametrize("warps", [1, 4])
 def test_batch_equals_single_problem_path(T, warps, cuda_device, monkeypatch):
     _assert_batch_equals_single(_problems(T, T), monkeypatch, warps)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("T", [2, 31, 51, 128])
+@pytest.mark.parametrize("warps", [1, 4])
+def test_batch_equals_single_problem_path_on_varied_agents(T, warps, cuda_device, monkeypatch):
+    _assert_batch_equals_single(_problems(T + 1000, T, varied=True), monkeypatch, warps)
 
 
 @pytest.mark.gpu
@@ -263,11 +273,20 @@ def test_batch_tables_are_byte_identical_to_single_packs(cuda_device):
 
 @pytest.mark.gpu
 def test_every_problem_of_a_mixed_batch_matches_the_oracle(cuda_device, monkeypatch):
+    monkeypatch.setenv("FO_TEAM_WARPS", "1")
+    _assert_every_problem_matches_the_oracle(_problems(23, 31, a_set=[0, 3, 17, 40], n_set=[60, 25, 80, 30]))
+
+
+@pytest.mark.gpu
+def test_every_problem_of_a_mixed_batch_matches_the_oracle_on_varied_agents(cuda_device, monkeypatch):
+    monkeypatch.setenv("FO_TEAM_WARPS", "1")
+    _assert_every_problem_matches_the_oracle(_problems(24, 51, a_set=[0, 5, 17, 40], n_set=[60, 25, 80, 30], varied=True))
+
+
+def _assert_every_problem_matches_the_oracle(probs):
     import parity
     from oracle import metric_oracle as MO
     from test_metric_gpu import _check
-    monkeypatch.setenv("FO_TEAM_WARPS", "1")
-    probs = _problems(23, 31, a_set=[0, 3, 17, 40], n_set=[60, 25, 80, 30])
     eng = _engine(probs[0][3])
     eng.set_agent_batch([p[0] for p in probs], [p[1] for p in probs])
     parts = eng.assess_batch([p[2] for p in probs]).split()

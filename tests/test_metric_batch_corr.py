@@ -205,11 +205,11 @@ def _correlate(problem, seed):
 
 
 def _mixed(seed, T, a_set=(0, 1, 5, 17, 40, 300), n_set=(0, 1, 64, 500), n_problems=16, metrics=None,
-           thresholds=None, every=2):
+           thresholds=None, every=2, varied=False):
     """test_metric_batch._problems with one vehicle each; every `every`-th problem (from the first) correlated, none for
     every = 0."""
     probs = _problems(seed, T, n_problems=n_problems, a_set=list(a_set), n_set=list(n_set), metrics=metrics,
-                      thresholds=thresholds)
+                      thresholds=thresholds, varied=varied)
     probs = [_correlate(p, seed * 100 + i) if every and i % every == 0 else p for i, p in enumerate(probs)]
     return probs, _fleet(len(probs), seed)
 

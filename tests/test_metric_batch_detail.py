@@ -148,10 +148,19 @@ def test_detail_batch_equals_single_problem_path_metrics_and_thresholds(metrics,
 
 @pytest.mark.gpu
 def test_every_problem_of_a_detail_batch_matches_the_oracle(cuda_device):
+    _assert_every_detail_problem_matches_the_oracle(_problems(29, 31, a_set=[0, 3, 17, 40], n_set=[60, 25, 80, 30]))
+
+
+@pytest.mark.gpu
+def test_every_problem_of_a_detail_batch_matches_the_oracle_on_varied_agents(cuda_device):
+    _assert_every_detail_problem_matches_the_oracle(_problems(30, 51, a_set=[0, 5, 17, 40], n_set=[60, 25, 80, 30],
+                                                              varied=True))
+
+
+def _assert_every_detail_problem_matches_the_oracle(probs):
     import parity
     from oracle import metric_oracle as MO
     from test_metric_gpu import _check
-    probs = _problems(29, 31, a_set=[0, 3, 17, 40], n_set=[60, 25, 80, 30])
     eng = _engine(probs[0][3])
     eng.set_agent_batch([p[0] for p in probs], [p[1] for p in probs])
     parts = eng.assess_batch([p[2] for p in probs], want_pair=True, want_step=True).split()

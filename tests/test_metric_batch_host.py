@@ -143,9 +143,9 @@ def _far(probs, seed):
 
 
 def _mix(seed, T, a_set=(0, 1, 3, 16, 17, 33, 300), n_set=(0, 1, 64, 500), n_problems=14, metrics=None,
-         thresholds=None):
+         thresholds=None, varied=False):
     return _far(_problems(seed, T, n_problems=n_problems, a_set=list(a_set), n_set=list(n_set), metrics=metrics,
-                          thresholds=thresholds), seed)
+                          thresholds=thresholds, varied=varied), seed)
 
 
 def _engine(case):
@@ -242,6 +242,12 @@ def test_batch_host_equals_the_engine_batch(T, outputs, fleet, cuda_device):
     assert {p[0].n_agents for p in probs} == {0, 1, 3, 16, 17, 33, 300} and {len(p[2]) for p in probs} == {0, 1, 64, 500}
     vehicles = _fleet(len(probs), T) if fleet else None
     _assert_host_equals_engine(probs, vehicles, outputs in ("pair", "both"), outputs in ("step", "both"))
+
+
+@pytest.mark.gpu
+def test_batch_host_equals_the_engine_batch_on_varied_agents(cuda_device):
+    probs = _mix(451, 51, varied=True)
+    _assert_host_equals_engine(probs, _fleet(len(probs), 51), True, True)
 
 
 @pytest.mark.gpu

@@ -41,11 +41,11 @@ def _fleet(n, seed):
 
 
 def _mixed(seed, T, a_set=(0, 1, 3, 16, 17, 33, 300), n_set=(0, 1, 64, 500), n_problems=14, metrics=None,
-           thresholds=None):
+           thresholds=None, varied=False):
     """Problems of test_metric_batch._problems (every agent count with every trajectory count of its residue) and one
     vehicle each."""
     probs = _problems(seed, T, n_problems=n_problems, a_set=list(a_set), n_set=list(n_set), metrics=metrics,
-                      thresholds=thresholds)
+                      thresholds=thresholds, varied=varied)
     return probs, _fleet(len(probs), seed)
 
 
@@ -261,11 +261,21 @@ def test_the_vehicle_changes_the_result(detail, cuda_device, monkeypatch):
 
 @pytest.mark.gpu
 def test_every_problem_of_a_fleet_batch_matches_the_oracle(cuda_device, monkeypatch):
+    monkeypatch.setenv("FO_TEAM_WARPS", "1")
+    _assert_every_fleet_problem_matches_the_oracle(*_mixed(47, 31, a_set=(0, 3, 17, 40), n_set=(60, 25, 80, 30), n_problems=8))
+
+
+@pytest.mark.gpu
+def test_every_problem_of_a_fleet_batch_matches_the_oracle_on_varied_agents(cuda_device, monkeypatch):
+    monkeypatch.setenv("FO_TEAM_WARPS", "1")
+    _assert_every_fleet_problem_matches_the_oracle(*_mixed(48, 51, a_set=(0, 5, 17, 40), n_set=(60, 25, 80, 30),
+                                                           n_problems=8, varied=True))
+
+
+def _assert_every_fleet_problem_matches_the_oracle(probs, fleet):
     import parity
     from oracle import metric_oracle as MO
     from test_metric_gpu import _check
-    monkeypatch.setenv("FO_TEAM_WARPS", "1")
-    probs, fleet = _mixed(47, 31, a_set=(0, 3, 17, 40), n_set=(60, 25, 80, 30), n_problems=8)
     for detail in (False, True):
         eng = _engine(probs[0][3])
         eng.set_agent_batch([p[0] for p in probs], [p[1] for p in probs], vehicles=fleet)

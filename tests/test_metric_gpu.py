@@ -92,7 +92,10 @@ def test_latency_config_parity(cuda_device):
 def test_summary_kernel_equals_detail_kernel(cuda_device):
     """The summary kernel (bench / planner path) against the detail kernel at a size the CPU
     oracle would need minutes for: identical masks/flags/discrete values, floats to 1e-5."""
-    case = S.make_case(3000, 300, 51, seed=9)       # > 256 agents: exercises agent tiling
+    assert_summary_equals_detail(S.make_case(3000, 300, 51, seed=9))      # > 256 agents: exercises agent tiling
+
+
+def assert_summary_equals_detail(case):
     res_d, _ = parity.run_gpu(case, want_pair=True, want_step=True)
     res_s, _ = parity.run_gpu(case, want_pair=False, want_step=False)
     # FO_F_BE_RANGE is a float32 comparison (re-timed path length vs original path length); the two

@@ -166,6 +166,18 @@ def test_selected_is_the_first_valid_row_of_the_batch_call(T, warps, every, cuda
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("warps", [1, 4])
+@pytest.mark.parametrize("every", [0, 1, 2], ids=["diagonal", "correlated", "mixed"])
+def test_selected_is_the_first_valid_row_of_the_batch_call_on_varied_agents(warps, every, cuda_device, monkeypatch):
+    monkeypatch.setenv("FO_TEAM_WARPS", str(warps))
+    for P in (1, 3, 17):
+        probs, fleet = _mixed(P + every + 900, 51, a_set=(0, 1, 17, 40), n_set=(0, 1, 31, 1000), n_problems=P,
+                              thresholds=ARMED, every=every, varied=True)
+        full, got = _run(_batch_engine_for(probs, fleet), [p[2] for p in probs])
+        _assert_select_matches(full, got)
+
+
+@pytest.mark.gpu
 @pytest.mark.parametrize("metrics", [None, "default"], ids=["all", "default"])
 @pytest.mark.parametrize("armed", [False, True], ids=["null", "armed"])
 def test_selected_with_metric_sets_and_thresholds(metrics, armed, cuda_device, monkeypatch):

@@ -75,3 +75,68 @@ def test_no_agents_is_valid():
     case["agents"] = []
     out = MO.evaluate_bundle(case)
     assert out["valid"].all()                     # metric.py:44-45
+
+
+def test_varied_agents_reach_what_agent_table_does_not():
+    """Every kind of the C ABI, headings outside [-pi, pi], changing heading and speed, var_x != var_y, all-zero
+    covariances and ragged lengths, all float32-representable; a parked vehicle does not move."""
+    from frenetix_occlusion_b200 import _lib as L
+    from frenetix_occlusion_b200 import synthetic as S
+    for jitter in (False, True):
+        ags = S.varied_agents(60, 31, 3, jitter=jitter)
+        assert {a["agent_type"].lower() for a in ags} == set(L.KINDS)
+        assert {len(a["yaw"]) for a in ags} == {1, 2, 8, 9, 31, 51}
+        assert any((np.abs(a["yaw"]) > np.pi).any() for a in ags)
+        moving = [a for a in ags if len(a["yaw"]) > 2 and a["agent_type"] != "ParkedVehicle"]
+        assert all(np.ptp(a["yaw"]) > 0 and np.ptp(a["v"]) > 0 for a in moving)
+        assert all(not a["v"].any() for a in ags if a["agent_type"] == "ParkedVehicle")
+        cov = np.concatenate([a["cov"] for a in ags])
+        assert not cov[:, [0, 1], [1, 0]].any() and (cov[:, 0, 0] != cov[:, 1, 1]).mean() > 0.8
+        zero = (cov == 0).all((1, 2))
+        assert 0.05 < zero.mean() < 0.15 and ((cov[:, 0, 0] == 0) == zero).all() and ((cov[:, 1, 1] == 0) == zero).all()
+        for a in ags:
+            for k in ("pos", "yaw", "v", "var", "cov"):
+                assert np.array_equal(S._f32(a[k]), a[k])
+            assert np.array_equal(a["var"], a["cov"][:, 0, 0])
+            if a["agent_type"] in ("Car", "PriorityVehicle", "ParkedVehicle", "Taxi"):
+                assert MO.obstacle_mass(a["agent_type"], a["buf_length"] * a["buf_width"]) > 0
+
+
+def test_oracle_b_per_axis_covariance():
+    """Oracle B's collision probability with a diagonal ``cov`` (sigma_x = sqrt(cov[i-1][0][0]), sigma_y =
+    sqrt(cov[i-1][1][1])) equals the correlated oracle at rho = 0 (pinned to scipy and quadrature in test_metric_corr)
+    on every step, and the reference's nine mvnun terms (``ref_shims.mvnun``) on gated steps with var_x != var_y.
+    A correlated covariance is refused."""
+    import corr_oracle as CO
+    from frenetix_occlusion_b200 import synthetic as S
+    from oracle.ref_shims import mvnun
+    for jitter in (False, True):
+        case = S.make_varied_case(300, 40, 31, seed=11 + jitter, jitter=jitter)
+        cp, inside, _ = MO.collision_probability(case)
+        cp_c, inside_c, _ = CO.collision_probability(case)
+        assert np.array_equal(inside, inside_c) and inside.mean() > 0.01
+        assert np.abs(cp - cp_c).max() <= 1e-13
+        ego, L, W = case["ego"], case["vehicle"]["length"], case["vehicle"]["width"]
+        rng = np.random.default_rng(3)
+        hits = np.argwhere(inside & (cp > 1e-3))
+        checked = 0
+        for n, a, j in hits[rng.permutation(len(hits))]:
+            ag, i = case["agents"][a], j + 1
+            c = ag["cov"][i - 1]
+            if c[0, 0] == c[1, 1] or c[0, 0] == 0:
+                continue
+            h = np.array([np.cos(ag["yaw"][i]), np.sin(ag["yaw"][i])]) * ag["buf_length"] / 2
+            p = ag["pos"][i - 1]
+            e, th = ego[n, i, :2], ego[n, i, 2]
+            off = np.array([np.cos(th), np.sin(th)]) * L / 3
+            half = np.array([L / 6, W / 2])
+            want = sum(mvnun(b - half, b + half, mu, c)[0] for mu in (p, p + h, p - h) for b in (e, e + off, e - off)) / 3
+            assert abs(cp[n, a, j] - want) <= 1e-13 * max(1.0, want), (n, a, j)
+            checked += 1
+            if checked == 12:
+                break
+        assert checked == 12
+    case["agents"][3]["cov"] = case["agents"][3]["cov"].copy()
+    case["agents"][3]["cov"][5, 0, 1] = case["agents"][3]["cov"][5, 1, 0] = 0.01
+    with pytest.raises(ValueError, match="correlated"):
+        MO.collision_probability(case)

@@ -55,31 +55,9 @@ __host__ __device__ inline size_t detail_warp_bytes(int T) {
 // MUFU forms without the denormal-scaling wrappers nvcc puts around rsqrtf / exp2f when -ftz is off (their arguments
 // here are clamped or far from the denormal range)
 __device__ __forceinline__ float fast_rsqrt(float x) { float r; asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
-__device__ __forceinline__ float fast_ex2(float x) { float r; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
-__device__ __forceinline__ float fast_rcp(float x) { float r; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
 // 1 / (1 + exp(-z))
-__device__ __forceinline__ float dt_sigmoid(float z) { return fast_rcp(1.0f + fast_ex2(-1.4426950408889634f * z)); }
+__device__ __forceinline__ float dt_sigmoid(float z) { return rcp_approx(1.0f + ex2_approx(-1.4426950408889634f * z)); }
 
-// LR4S impact-angle coefficients of ego and obstacle (logistic_regression.py:35-48, harm_model.py:81-105); one copy
-// in the kernel (atan2f is ~100 instructions and the kernel sits next to a 32 kB instruction cache)
-static __device__ __noinline__ float2 dt_lr4s_pair(float dyr, float dxr, float th, float psi, float side, float rear) {
-  const float PI_F = 3.14159265358979323846f;
-  const float rel = atan2f(dyr, dxr);
-  return make_float2(lr4s_coef(rel - th, side, rear), lr4s_coef(PI_F + rel - psi, side, rear));
-}
-
-// per-agent logit coefficients: harm = sigmoid(ks * dv + kc (+ LR4S class coefficient)); harm_model.py:96-105,
-// logistic_regression.py:45-48, 71-73
-struct HarmLin { float kse, kce, kso, kco; };
-__device__ __forceinline__ HarmLin harm_lin(const FoHarmCoeffs& hc, int model, float ke, float ko) {
-  HarmLin h;
-  const bool m0 = model == 0;
-  h.kse = (m0 ? hc.ia_speed : hc.rs_speed) * ke;
-  h.kso = (m0 ? hc.ped_speed : hc.rs_speed) * ko;
-  h.kce = m0 ? hc.ia_const : hc.rs_const;
-  h.kco = m0 ? -hc.ped_const : hc.rs_const;
-  return h;
-}
 // exact harm of one (agent, state): harm_model.py:81-105
 __device__ __forceinline__ void dt_harm(const FoHarmCoeffs& hc, int model, const HarmLin& h, float ve, float va, float c,
                                         float dxr, float dyr, float th, float psi, float& he, float& ho) {
@@ -87,7 +65,7 @@ __device__ __forceinline__ void dt_harm(const FoHarmCoeffs& hc, int model, const
   const float dv = dv2 * fast_rsqrt(dv2);
   float ze = fmaf(h.kse, dv, h.kce), zo = fmaf(h.kso, dv, h.kco);
   if (model == 1) {
-    const float2 cls = dt_lr4s_pair(dyr, dxr, th, psi, hc.rs_side, hc.rs_rear);
+    const float2 cls = lr4s_coefs(dyr, dxr, th, psi, hc.rs_side, hc.rs_rear);
     ze += cls.x;
     zo += cls.y;
   }
@@ -301,9 +279,7 @@ __device__ __forceinline__ void detail_body(const MetricKArgs& k, const DetailVi
           const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + as));
           const float4 EA = egoA[ii];
           const float c = fmaf(EA.z, s0.z, EA.w * s0.w), s = fmaf(s0.w, EA.z, -s0.z * EA.w);
-          const float dx = (s0.x - EA.x) - veh.wb * EA.z, dy = (s0.y - EA.y) - veh.wb * EA.w;
-          const float rx = fmaf(dx, EA.z, dy * EA.w), ry = fmaf(dy, EA.z, -dx * EA.w);
-          const float d = sqrtf(obb_d2(rx, ry, c, s, veh.hEx, veh.hEy, __int_as_float(pa.z), __int_as_float(pa.w)));
+          const float d = ego_box_dist(s0.x - EA.x, s0.y - EA.y, EA, c, s, veh, __int_as_float(pa.z), __int_as_float(pa.w));
           uint32_t r = (uint32_t)__float2int_rn(fminf(d, 8000.0f) * 1000.0f);   // np.round(d, 3), dce.py:79
           // rounding ties: a candidate for the pair's minimum next to a x.xxx5 boundary is queued for a float64
           // re-rounding (the float32 value is off by at most one unit there); until then r + 1 bounds it from above

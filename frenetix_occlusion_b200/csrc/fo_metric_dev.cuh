@@ -10,8 +10,6 @@
 
 namespace fo {
 
-
-constexpr int kWarpsPerCta = 8;
 constexpr unsigned kFull = 0xffffffffu;
 
 // Constants of the ego vehicle in the units the kernels use (fill_ego_const in fo_metric.cu).  A batch of independent
@@ -101,6 +99,16 @@ __device__ __forceinline__ float obb_d2(float rx, float ry, float c, float s, fl
   return d2;
 }
 
+// Exact distance between the ego box and an agent box (half extents hl, hw) of one state (dce.py:75-79): (dxr, dyr) =
+// agent position minus ego reference point, EA = (x, y, cos theta, sin theta) of the ego, (c, s) = cos / sin of the
+// agent's heading relative to the ego's.
+__device__ __forceinline__ float ego_box_dist(float dxr, float dyr, float4 EA, float c, float s, const EgoConst& veh,
+                                              float hl, float hw) {
+  const float dx = dxr - veh.wb * EA.z, dy = dyr - veh.wb * EA.w;
+  const float rx = fmaf(dx, EA.z, dy * EA.w), ry = fmaf(dy, EA.z, -dx * EA.w);
+  return sqrtf(obb_d2(rx, ry, c, s, veh.hEx, veh.hEy, hl, hw));
+}
+
 // ---- rounding-tie refinement of np.round(d, 3) (dce.py:79) ---------------------------------------------------------
 // The float32 distance carries an error of a few 1e-5 m; when d * 1000 lies within kTieBand of a rounding boundary
 // (x.5) the float64 reference may round the other way.  Such candidates are re-evaluated here in double from the
@@ -182,14 +190,6 @@ __device__ __forceinline__ bool obb_hit(float rx, float ry, float c, float s, fl
   bool sep = (fabsf(rx) > hEx + fmaf(hl, ac, hw * as)) | (fabsf(ry) > hEy + fmaf(hl, as, hw * ac)) |
              (fabsf(rox) > hl + fmaf(hEx, ac, hEy * as)) | (fabsf(roy) > hw + fmaf(hEx, as, hEy * ac));
   return !sep;
-}
-
-// 0.5*(erf(b) - erf(a)) for a < b, evaluated on the tails (no cancellation far from the mean).
-__device__ __forceinline__ float half_derf(float a, float b) {
-  float ea = erfcf(fabsf(a)), eb = erfcf(fabsf(b));
-  bool same = (a > 0.0f) == (b > 0.0f);
-  float r = same ? fabsf(ea - eb) : (2.0f - ea - eb);
-  return 0.5f * r;
 }
 
 // Single MUFU forms.  __fdividef / __expf wrap the same MUFU.RCP / MUFU.EX2 in range guards (denormal divisor, result
@@ -408,10 +408,6 @@ __device__ __forceinline__ float cp_bvn_boxes(float mx, float my, float hx, floa
   return (float)(prob > 0.0 ? prob / 3.0 : (prob == prob ? 0.0 : prob));
 }
 
-__device__ __forceinline__ float logistic_neg(float z) {  // 1 / (1 + exp(z))
-  return __fdividef(1.0f, 1.0f + __expf(z));
-}
-
 // LR4S angle coefficient, logistic_regression.py:35-42 (angles are NOT wrapped)
 __device__ __forceinline__ float lr4s_coef(float ang, float side, float rear) {
   const float ta = 0.78539816339744830962f, tb = 2.35619449019234492885f;
@@ -419,6 +415,29 @@ __device__ __forceinline__ float lr4s_coef(float ang, float side, float rear) {
   if ((ang >= ta && ang < tb) || (ang <= -ta && ang > -tb)) c = side;
   if (ang > -ta && ang < ta) c = 0.0f;
   return c;
+}
+
+// LR4S impact-angle coefficients of ego and obstacle (logistic_regression.py:35-48, harm_model.py:81-105); one copy per
+// kernel (atan2f is ~100-150 instructions, the harm logits are needed at several inlined sites, and the kernels sit next
+// to a 32 kB instruction cache: they are instruction-cache-bound, not call-bound).  ptxas lays a kernel's out-of-line
+// helpers out in the order of their mangled names, so a rename can move this one and every call offset with it.
+static __device__ __noinline__ float2 lr4s_coefs(float dyr, float dxr, float th, float psi, float side, float rear) {
+  const float PI_F = 3.14159265358979323846f;
+  const float rel = atan2f(dyr, dxr);
+  return make_float2(lr4s_coef(rel - th, side, rear), lr4s_coef(PI_F + rel - psi, side, rear));
+}
+
+// per-agent logit coefficients: harm = sigmoid(ks * dv + kc (+ LR4S class coefficient)); harm_model.py:96-105,
+// logistic_regression.py:45-48, 71-73
+struct HarmLin { float kse, kce, kso, kco; };
+__device__ __forceinline__ HarmLin harm_lin(const FoHarmCoeffs& hc, int model, float ke, float ko) {
+  HarmLin h;
+  const bool m0 = model == 0;
+  h.kse = (m0 ? hc.ia_speed : hc.rs_speed) * ke;
+  h.kso = (m0 ? hc.ped_speed : hc.rs_speed) * ko;
+  h.kce = m0 ? hc.ia_const : hc.rs_const;
+  h.kco = m0 ? -hc.ped_const : hc.rs_const;
+  return h;
 }
 
 // ---- BE (be.py:66-193) shared by the summary kernels: warp-cooperative bisection on a re-timed ego path -----
@@ -742,11 +761,6 @@ static __device__ __noinline__ BeWalk be_walk(const BeConst k, const AgentParams
   r.rcd = rcd;
   return r;
 }
-
-struct EgoState {
-  float x, y, th, v, c, s;
-};
-
 
 // one zeroed-per-launch device counter (trajectory claims of the persistent kernels), see fo_metric_sweep.cu
 unsigned int* claim_slot(cudaStream_t st);

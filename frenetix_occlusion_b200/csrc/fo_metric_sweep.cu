@@ -135,14 +135,6 @@ __device__ __forceinline__ float nan_maxf(float a, float b) { return __uint_as_f
 
 __device__ __forceinline__ float sw_sigmoid(float z) { return rcp_approx(1.0f + __expf(-z)); }   // 1 + exp >= 1: same bits as __fdividef(1, .)
 
-// impact-angle class coefficients of both parties (one copy in the kernel: atan2f is ~150 instructions and the harm
-// logits are needed at five inlined sites; the kernel is instruction-cache-bound, not call-bound)
-static __device__ __noinline__ float2 sw_lr4s_pair(float dyr, float dxr, float th, float psi, float side, float rear) {
-  const float PI_F = 3.14159265358979323846f;
-  const float rel = atan2f(dyr, dxr);
-  return make_float2(lr4s_coef(rel - th, side, rear), lr4s_coef(PI_F + rel - psi, side, rear));
-}
-
 // exact harm logits for one (agent, state) -- harm_model.py:81-105, logistic_regression.py:35-48,71-73
 __device__ __forceinline__ void sw_harm_logits(const MetricKArgs& k, int model, float ke, float ko, float dv, float dxr,
                                                float dyr, float th, float psi, float& ze, float& zo) {
@@ -150,7 +142,7 @@ __device__ __forceinline__ void sw_harm_logits(const MetricKArgs& k, int model, 
     ze = fmaf(k.hc.ia_speed * ke, dv, k.hc.ia_const);
     zo = fmaf(k.hc.ped_speed * ko, dv, -k.hc.ped_const);
   } else if (model == 1) {
-    const float2 cls = sw_lr4s_pair(dyr, dxr, th, psi, k.hc.rs_side, k.hc.rs_rear);
+    const float2 cls = lr4s_coefs(dyr, dxr, th, psi, k.hc.rs_side, k.hc.rs_rear);
     ze = fmaf(k.hc.rs_speed * ke, dv, k.hc.rs_const) + cls.x;
     zo = fmaf(k.hc.rs_speed * ko, dv, k.hc.rs_const) + cls.y;
   } else {
@@ -420,7 +412,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
       int qn = 0, qc = 0, qt = 0;
       // per-lane bound state of the current lane group (refreshed after every drain)
       float lim0 = 0.0f, lim2 = 0.0f, thr2 = CUDART_INF_F;
-      float kse = 0.0f, kso = 0.0f, kce = 0.0f, kco = 0.0f;
+      HarmLin hl{};
       bool is_m1 = false;
 
       // distance >= |centres| - rE - rO: the exact box distance is needed only while that bound can still lower
@@ -435,8 +427,10 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
         float t2 = CUDART_INF_F;
         if (is_m1) {
           const float ze_m = fmaxf(zb_e, acc_ze), zo_m = fmaxf(zb_o, acc_zo);
-          const float te = (kse > 1e-30f) ? (ze_m - cmax - kce) * rcp_approx(kse) : ((kce + cmax > ze_m) ? -1.0f : CUDART_INF_F);
-          const float to = (kso > 1e-30f) ? (zo_m - cmax - kco) * rcp_approx(kso) : ((kco + cmax > zo_m) ? -1.0f : CUDART_INF_F);
+          const float te = (hl.kse > 1e-30f) ? (ze_m - cmax - hl.kce) * rcp_approx(hl.kse)
+                                             : ((hl.kce + cmax > ze_m) ? -1.0f : CUDART_INF_F);
+          const float to = (hl.kso > 1e-30f) ? (zo_m - cmax - hl.kco) * rcp_approx(hl.kso)
+                                             : ((hl.kco + cmax > zo_m) ? -1.0f : CUDART_INF_F);
           const float tm = fminf(te, to);
           t2 = (tm > 0.0f) ? tm * tm * 0.99999f : -1.0f;
         }
@@ -459,9 +453,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
           const float dxr = s0.x - EA.x, dyr = s0.y - EA.y;
           if (item & 0x40000000u) {            // exact oriented-box distance, np.round(d, 3) (dce.py:75-79)
             const int4 pa = __ldg(reinterpret_cast<const int4*>(tab.prm + a));
-            const float dx = dxr - veh.wb * EA.z, dy = dyr - veh.wb * EA.w;
-            const float rx = fmaf(dx, EA.z, dy * EA.w), ry = fmaf(dy, EA.z, -dx * EA.w);
-            const float d = sqrtf(obb_d2(rx, ry, c, s, veh.hEx, veh.hEy, __int_as_float(pa.z), __int_as_float(pa.w)));
+            const float d = ego_box_dist(dxr, dyr, EA, c, s, veh, __int_as_float(pa.z), __int_as_float(pa.w));
             r = (uint32_t)__float2int_rn(fminf(d, 8000.0f) * 1000.0f);
             // np.round(d, 3) next to a x.xxx5 boundary: a candidate for the minimum is queued for a float64
             // re-rounding (rmin only falls, so "r <= rmin + 2" is a superset of the candidates of the final minimum);
@@ -557,11 +549,7 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
         const int n_it = flush ? 1 : (int)__reduce_max_sync(kFull, (unsigned)max(nS - i_lo, 0));
         const bool is_m0 = P.model == 0;
         is_m1 = P.model == 1;
-        // harm logit = ks * dv + kc (+ LR4S class coefficient for protected agents)
-        kse = (is_m0 ? k.hc.ia_speed : k.hc.rs_speed) * P.ke;
-        kso = (is_m0 ? k.hc.ped_speed : k.hc.rs_speed) * P.ko;
-        kce = is_m0 ? k.hc.ia_const : k.hc.rs_const;
-        kco = is_m0 ? -k.hc.ped_const : k.hc.rs_const;
+        hl = harm_lin(k.hc, P.model, P.ke, P.ko);
         if (do_hr && alive && P.model == 2 && nH > i_lo) { acc_ze = CUDART_INF_F; acc_zo = CUDART_INF_F; }
         lim0 = rE + P.pad;
         upd_lim();
@@ -627,8 +615,8 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
         }
         if (do_hr && is_m0 && acc_dv2 >= 0.0f) {
           const float dvm = acc_dv2 * rsqrtf(fmaxf(acc_dv2, 1e-30f));
-          acc_ze = fmaxf(acc_ze, fmaf(kse, dvm, kce));
-          acc_zo = fmaxf(acc_zo, fmaf(kso, dvm, kco));
+          acc_ze = fmaxf(acc_ze, fmaf(hl.kse, dvm, hl.kce));
+          acc_zo = fmaxf(acc_zo, fmaf(hl.kso, dvm, hl.kco));
         }
         if (do_hr) {
           zb_e = fmaxf(zb_e, warp_max_signed(acc_ze));
@@ -666,15 +654,12 @@ __device__ __forceinline__ void sweep_body(const MetricKArgs& k, const SweepShap
               f_reach2 = reach * reach;
               float t2 = CUDART_INF_F;                      // harm logit <= ks (|v_e| + |v_a|) + kc (+ cmax)
               if (do_hr && P.model != 2) {
-                const bool m0 = P.model == 0;
-                const float cm = m0 ? 0.0f : cmax;
-                const float fse = (m0 ? k.hc.ia_speed : k.hc.rs_speed) * P.ke;
-                const float fso = (m0 ? k.hc.ped_speed : k.hc.rs_speed) * P.ko;
-                const float fce = (m0 ? k.hc.ia_const : k.hc.rs_const) + cm;
-                const float fco = (m0 ? -k.hc.ped_const : k.hc.rs_const) + cm;
+                const float cm = P.model == 0 ? 0.0f : cmax;
+                const HarmLin h = harm_lin(k.hc, P.model, P.ke, P.ko);
+                const float fce = h.kce + cm, fco = h.kco + cm;
                 const float ze_m = fmaxf(zb_e, acc_ze), zo_m = fmaxf(zb_o, acc_zo);
-                const float te = (fse > 1e-30f) ? (ze_m - fce) * rcp_approx(fse) : ((fce > ze_m) ? -1.0f : CUDART_INF_F);
-                const float to = (fso > 1e-30f) ? (zo_m - fco) * rcp_approx(fso) : ((fco > zo_m) ? -1.0f : CUDART_INF_F);
+                const float te = (h.kse > 1e-30f) ? (ze_m - fce) * rcp_approx(h.kse) : ((fce > ze_m) ? -1.0f : CUDART_INF_F);
+                const float to = (h.kso > 1e-30f) ? (zo_m - fco) * rcp_approx(h.kso) : ((fco > zo_m) ? -1.0f : CUDART_INF_F);
                 const float tm = fminf(te, to);
                 t2 = (tm > 0.0f) ? tm * tm * 0.99999f : -1.0f;
               }

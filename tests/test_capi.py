@@ -5,6 +5,7 @@ import os
 import re
 
 from conftest import ROOT
+from kernel_sizes import size_of
 
 
 def _header_functions():
@@ -69,39 +70,10 @@ def test_hot_kernels_stay_inside_the_instruction_cache_budget():
     """The summary and detail kernels are instruction-issue-bound and sit next to the 32 kB L1.5 instruction cache:
     inlined duplicates showed up as stall_no_inst and cost 25 % (summary, 70 kB -> 47 kB) and 2.6x (detail, 111 kB ->
     59 kB) -- DESIGN.md section 6.  Guard the code size of the shapes the benchmark and the planner use."""
-    import shutil
-    import subprocess
-    import pytest
-    from torch.utils.cpp_extension import CUDA_HOME
-    from frenetix_occlusion_b200 import _lib as L
-    # the toolkit that built the library has it, whether or not its bin/ is on PATH
-    cuobjdump = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
-    if not cuobjdump:
-        pytest.skip("cuobjdump not found (no CUDA toolkit)")
-    sass = subprocess.run([cuobjdump, "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
-    sizes, name = {}, None
-    for line in sass.splitlines():
-        m = re.search(r"Function : (\S+)", line)
-        if m:
-            name = m.group(1)
-        elif name and re.match(r"\s+/\*[0-9a-f]+\*/\s+\S", line):
-            sizes[name] = sizes.get(name, 0) + 16
-    # cold helpers that live in the kernel's text section but not in its hot set: the float64 re-rounding of
-    # np.round(d, 3) ties runs for a fraction of a per cent of the exact distance evaluations
-    cold = {}
-    elf = subprocess.run([cuobjdump, "-elf", L.LIB_PATH], capture_output=True, text=True).stdout
-    for line in elf.splitlines():
-        m = re.match(r"\s*0x[0-9a-f]+\s+0x[0-9a-f]+\s+(0x[0-9a-f]+)\s+.*\$(_ZN\S+?)\$(_ZN\S+)", line)
-        if m and ("obb_round_mm_f64" in m.group(3) or "sincos_f64_of_f32" in m.group(3)):
-            cold[m.group(2)] = cold.get(m.group(2), 0) + int(m.group(1), 16)
-    def size_of(*parts):
-        hit = [v - cold.get(k, 0) for k, v in sizes.items() if all(p in k for p in parts)]
-        assert len(hit) == 1, (parts, sorted(sizes))
-        return hit[0]
     # the throughput kernel sits at the edge of the instruction cache: +2-5 kB cost 5-8 % in every experiment (DESIGN.md 5.1)
-    assert size_of("fo_metric_sweep_kernel", "ILj127ELb0ELb1ELb0E") <= 44 * 1024   # all 7 metrics, one-warp window-filter shape
-    assert size_of("fo_metric_sweep_kernel", "ILj127ELb0ELb1ELb1E") <= 52 * 1024   # ... with the float64 tie path (armed dce / ttc / be)
-    assert size_of("fo_metric_sweep_kernel", "ILj111ELb0ELb1ELb0E") <= 34 * 1024   # default metrics (no BE)
-    assert size_of("fo_metric_sweep_kernel", "ILj127ELb0ELb0ELb0E") <= 56 * 1024   # team shape (latency path)
-    assert size_of("fo_metric_detail_kernel", "ILj127E") <= 50 * 1024            # detail kernel (lane = agent), all 7 metrics, incl. BE helpers
-    assert size_of("fo_metric_detail_kernel", "ILj111E") <= 38 * 1024            # default metrics
+    assert size_of("fo_metric_sweep_kernel", "ILj127ELb0ELb1ELb0E", hot=True) <= 44 * 1024   # all 7 metrics, one-warp window-filter shape
+    assert size_of("fo_metric_sweep_kernel", "ILj127ELb0ELb1ELb1E", hot=True) <= 52 * 1024   # ... with the float64 tie path (armed dce / ttc / be)
+    assert size_of("fo_metric_sweep_kernel", "ILj111ELb0ELb1ELb0E", hot=True) <= 34 * 1024   # default metrics (no BE)
+    assert size_of("fo_metric_sweep_kernel", "ILj127ELb0ELb0ELb0E", hot=True) <= 56 * 1024   # team shape (latency path)
+    assert size_of("fo_metric_detail_kernel", "ILj127E", hot=True) <= 50 * 1024            # detail kernel (lane = agent), all 7 metrics, incl. BE helpers
+    assert size_of("fo_metric_detail_kernel", "ILj111E", hot=True) <= 38 * 1024            # default metrics

@@ -5,14 +5,12 @@ batch gets exactly what the single-problem path gives it."""
 import ctypes as C
 import os
 import random
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
 
 from conftest import GOLDEN
+from kernel_sizes import size_of
 
 FO_ERR_INVALID_ARG, FO_ERR_UNSUPPORTED = -1, -2
 
@@ -100,34 +98,10 @@ def test_batch_argument_validation_without_device():
 def test_batched_kernels_stay_inside_the_instruction_cache_budget():
     """The batched kernels share the summary kernel's body (DESIGN.md 5.1 and 5.4): they are held to the budgets of
     their single-problem counterparts in test_capi.py."""
-    from torch.utils.cpp_extension import CUDA_HOME
-    from frenetix_occlusion_b200 import _lib as L
-    cuobjdump = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
-    if not cuobjdump:
-        pytest.skip("cuobjdump not found (no CUDA toolkit)")
-    sass = subprocess.run([cuobjdump, "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
-    sizes, name = {}, None
-    for line in sass.splitlines():
-        m = re.search(r"Function : (\S+)", line)
-        if m:
-            name = m.group(1)
-        elif name and re.match(r"\s+/\*[0-9a-f]+\*/\s+\S", line):
-            sizes[name] = sizes.get(name, 0) + 16
-    cold = {}
-    elf = subprocess.run([cuobjdump, "-elf", L.LIB_PATH], capture_output=True, text=True).stdout
-    for line in elf.splitlines():
-        m = re.match(r"\s*0x[0-9a-f]+\s+0x[0-9a-f]+\s+(0x[0-9a-f]+)\s+.*\$(_ZN\S+?)\$(_ZN\S+)", line)
-        if m and ("obb_round_mm_f64" in m.group(3) or "sincos_f64_of_f32" in m.group(3)):
-            cold[m.group(2)] = cold.get(m.group(2), 0) + int(m.group(1), 16)
-
-    def size_of(*parts):
-        hit = [v - cold.get(k, 0) for k, v in sizes.items() if all(p in k for p in parts)]
-        assert len(hit) == 1, (parts, sorted(sizes))
-        return hit[0]
-    assert size_of("fo_metric_batch_kernel", "ILj127ELb1ELb0E") <= 44 * 1024   # all 7 metrics, one-warp window-filter shape
-    assert size_of("fo_metric_batch_kernel", "ILj127ELb1ELb1E") <= 52 * 1024   # ... with the float64 tie path
-    assert size_of("fo_metric_batch_kernel", "ILj111ELb1ELb0E") <= 34 * 1024   # default metrics
-    assert size_of("fo_metric_batch_kernel", "ILj127ELb0ELb0E") <= 56 * 1024   # team shape
+    assert size_of("fo_metric_batch_kernel", "ILj127ELb1ELb0E", hot=True) <= 44 * 1024   # all 7 metrics, one-warp window-filter shape
+    assert size_of("fo_metric_batch_kernel", "ILj127ELb1ELb1E", hot=True) <= 52 * 1024   # ... with the float64 tie path
+    assert size_of("fo_metric_batch_kernel", "ILj111ELb1ELb0E", hot=True) <= 34 * 1024   # default metrics
+    assert size_of("fo_metric_batch_kernel", "ILj127ELb0ELb0E", hot=True) <= 56 * 1024   # team shape
 
 
 # ---------------------------------------------------------------------------------------------------- GPU

@@ -7,16 +7,13 @@ the single-problem path gives it: fo_agents_pack_corr + fo_metric_bundle_corr wh
 fo_metric_bundle when not."""
 import copy
 import ctypes as C
-import os
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
 
 import corr_oracle as CO
 import parity
+from kernel_sizes import size_of
 from test_metric_batch import _batch_args, _problems
 from test_metric_batch_detail import SCENES, _assert_same_assessments, _trajectories
 from test_metric_batch_vehicles import (_assert_equal, _engine, _fleet, _malformed_detail_cases, _malformed_summary_cases,
@@ -162,24 +159,6 @@ def test_correlated_entry_points_validate_like_their_diagonal_counterparts_witho
 
 def test_batched_correlated_kernels_stay_inside_their_code_size_budgets():
     """Budgets: the sizes measured when the kernels were added (DESIGN.md 5.11) plus 4 kB."""
-    from torch.utils.cpp_extension import CUDA_HOME
-    from frenetix_occlusion_b200 import _lib as L
-    cuobjdump = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
-    if not cuobjdump:
-        pytest.skip("cuobjdump not found (no CUDA toolkit)")
-    sass = subprocess.run([cuobjdump, "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
-    sizes, name = {}, None
-    for line in sass.splitlines():
-        m = re.search(r"Function : (\S+)", line)
-        if m:
-            name = m.group(1)
-        elif name and re.match(r"\s+/\*[0-9a-f]+\*/\s+\S", line):
-            sizes[name] = sizes.get(name, 0) + 16
-
-    def size_of(*parts):
-        hit = [v for k, v in sizes.items() if all(p in k for p in parts)]
-        assert len(hit) == 1, (parts, sorted(sizes))
-        return hit[0]
     budget = {("fo_metric_batch_corr_kernel", "ILb1ELb0E"): 72.25,    # one-warp window-filter shape
               ("fo_metric_batch_corr_kernel", "ILb1ELb1E"): 85.375,   # ... with the float64 tie path
               ("fo_metric_batch_corr_kernel", "ILb0ELb0E"): 83.125,   # team shape

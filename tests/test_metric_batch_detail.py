@@ -4,15 +4,12 @@ batch.prefetch_interfaces).  The CPU part checks the argument validation (before
 batched detail kernel; the GPU part checks that every problem of a batch gets exactly what the single-problem detail path
 gives it, and that a prefetch over many interfaces serves the per-trajectory protocol as each interface's own would."""
 import ctypes as C
-import os
-import re
-import shutil
-import subprocess
 import types
 
 import numpy as np
 import pytest
 
+from kernel_sizes import size_of
 from test_metric_batch import A_SET, N_SET, _batch_args, _engine, _problems, _scene_interface
 
 FO_ERR_INVALID_ARG, FO_ERR_UNSUPPORTED = -1, -2
@@ -72,32 +69,8 @@ def test_batch_detail_argument_validation_without_device():
 
 def test_batched_detail_kernel_stays_inside_the_instruction_cache_budget():
     """The batched detail kernel shares the detail kernel's body: it is held to that kernel's budgets in test_capi.py."""
-    from torch.utils.cpp_extension import CUDA_HOME
-    from frenetix_occlusion_b200 import _lib as L
-    cuobjdump = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
-    if not cuobjdump:
-        pytest.skip("cuobjdump not found (no CUDA toolkit)")
-    sass = subprocess.run([cuobjdump, "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
-    sizes, name = {}, None
-    for line in sass.splitlines():
-        m = re.search(r"Function : (\S+)", line)
-        if m:
-            name = m.group(1)
-        elif name and re.match(r"\s+/\*[0-9a-f]+\*/\s+\S", line):
-            sizes[name] = sizes.get(name, 0) + 16
-    cold = {}
-    elf = subprocess.run([cuobjdump, "-elf", L.LIB_PATH], capture_output=True, text=True).stdout
-    for line in elf.splitlines():
-        m = re.match(r"\s*0x[0-9a-f]+\s+0x[0-9a-f]+\s+(0x[0-9a-f]+)\s+.*\$(_ZN\S+?)\$(_ZN\S+)", line)
-        if m and ("obb_round_mm_f64" in m.group(3) or "sincos_f64_of_f32" in m.group(3)):
-            cold[m.group(2)] = cold.get(m.group(2), 0) + int(m.group(1), 16)
-
-    def size_of(*parts):
-        hit = [v - cold.get(k, 0) for k, v in sizes.items() if all(p in k for p in parts)]
-        assert len(hit) == 1, (parts, sorted(sizes))
-        return hit[0]
-    assert size_of("fo_metric_batch_detail_kernel", "ILj127E") <= 50 * 1024   # all 7 metrics, incl. BE helpers
-    assert size_of("fo_metric_batch_detail_kernel", "ILj111E") <= 38 * 1024   # default metrics
+    assert size_of("fo_metric_batch_detail_kernel", "ILj127E", hot=True) <= 50 * 1024   # all 7 metrics, incl. BE helpers
+    assert size_of("fo_metric_batch_detail_kernel", "ILj111E", hot=True) <= 38 * 1024   # default metrics
 
 
 # ---------------------------------------------------------------------------------------------------- GPU

@@ -6,10 +6,6 @@ code-size budgets of the new kernels.  GPU (-m gpu): parity with the float64 ora
 the drop-in Metric protocol, the correlated table with zero correlation against the diagonal path, CUDA-graph capture
 and NaN for a covariance that is not positive definite."""
 import ctypes as C
-import os
-import re
-import shutil
-import subprocess
 import types
 import warnings
 
@@ -20,6 +16,7 @@ from scipy.special import ndtr
 
 import corr_oracle as CO
 import parity
+from kernel_sizes import size_of
 from frenetix_occlusion_b200 import synthetic as S
 from oracle import metric_oracle as MO
 
@@ -131,24 +128,6 @@ def test_correlated_kernels_stay_inside_their_code_size_budgets():
     """The correlated kernels carry the float64 rectangle mass (bvn_rect and its out-of-line CDF / exp, about 18 kB)
     on top of the runtime-mask kernel they are built from.  Budgets: the sizes measured when they were added (DESIGN.md
     5.10) plus 4 kB."""
-    from torch.utils.cpp_extension import CUDA_HOME
-    from frenetix_occlusion_b200 import _lib as L
-    cuobjdump = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
-    if not cuobjdump:
-        pytest.skip("cuobjdump not found (no CUDA toolkit)")
-    sass = subprocess.run([cuobjdump, "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
-    sizes, name = {}, None
-    for line in sass.splitlines():
-        m = re.search(r"Function : (\S+)", line)
-        if m:
-            name = m.group(1)
-        elif name and re.match(r"\s+/\*[0-9a-f]+\*/\s+\S", line):
-            sizes[name] = sizes.get(name, 0) + 16
-
-    def size_of(*parts):
-        hit = [v for k, v in sizes.items() if all(p in k for p in parts)]
-        assert len(hit) == 1, (parts, sorted(sizes))
-        return hit[0]
     budget = {("fo_metric_sweep_corr_kernel", "ILb1ELb0E"): 71.375,   # one-warp window-filter shape
               ("fo_metric_sweep_corr_kernel", "ILb1ELb1E"): 83.75,  # ... with the float64 tie path
               ("fo_metric_sweep_corr_kernel", "ILb0ELb0E"): 82.0,  # team shape

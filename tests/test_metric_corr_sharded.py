@@ -10,8 +10,6 @@ the counter pass writes the outputs of fo_metric_bundle_corr."""
 import ctypes as C
 import os
 import re
-import shutil
-import subprocess
 import sys
 
 import numpy as np
@@ -21,6 +19,7 @@ import torch.distributed as dist
 import torch.multiprocessing as mp
 
 import corr_oracle as CO
+from kernel_sizes import size_of
 from frenetix_occlusion_b200 import synthetic as S
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -82,27 +81,13 @@ def test_stats_call_checks_its_arguments_without_device():
 def test_correlated_counter_kernels_stay_inside_their_code_size_budgets():
     """The counter kernels are fo_metric_sweep_corr_kernel plus the increments and the epilogue's atomics.  Budgets: the
     sizes measured when they were added (DESIGN.md 5.13) plus 4 kB."""
-    from torch.utils.cpp_extension import CUDA_HOME
-    from frenetix_occlusion_b200 import _lib as L
-    cuobjdump = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
-    if not cuobjdump:
-        pytest.skip("cuobjdump not found (no CUDA toolkit)")
-    sass = subprocess.run([cuobjdump, "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
-    sizes, name = {}, None
-    for line in sass.splitlines():
-        m = re.search(r"Function : (\S+)", line)
-        if m:
-            name = m.group(1)
-        elif name and re.match(r"\s+/\*[0-9a-f]+\*/\s+\S", line):
-            sizes[name] = sizes.get(name, 0) + 16
     budget = {"ILb1ELb0E": 77.375,      # one-warp window-filter shape
               "ILb1ELb1E": 90.0,        # ... with the float64 tie path
               "ILb0ELb0E": 86.625,      # team shape
               "ILb0ELb1E": 102.375}
     for tmpl, kb in budget.items():
-        hit = [v for k, v in sizes.items() if "fo_metric_sweep_corr_stats_kernel" in k and tmpl in k]
-        assert len(hit) == 1, (tmpl, sorted(sizes))
-        assert hit[0] <= (kb + 4) * 1024, (tmpl, hit[0])
+        size = size_of("fo_metric_sweep_corr_stats_kernel", tmpl)
+        assert size <= (kb + 4) * 1024, (tmpl, size)
 
 
 # ---------------------------------------------------------------------------------------------------------------- GPU

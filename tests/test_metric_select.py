@@ -8,12 +8,11 @@ far fewer rows than it has; on the golden scene fans the interface calls equal t
 import ctypes as C
 import os
 import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
 
+from kernel_sizes import size_of
 from test_metric_batch import _batch_args
 from test_metric_batch_corr import _flags, _mixed, _vehicles
 from test_metric_batch_vehicles import _malformed_summary_cases
@@ -71,25 +70,11 @@ def test_select_checks_its_arguments_without_device():
 def test_select_kernels_stay_inside_their_code_size_budgets():
     """fo_metric_batch_select_kernel is fo_metric_batch_kernel<0> / fo_metric_batch_corr_kernel plus the rank-major
     claim map and three early-exit checks.  Budgets: the sizes measured when they were added (DESIGN.md 5.14) + 4 kB."""
-    from torch.utils.cpp_extension import CUDA_HOME
-    from frenetix_occlusion_b200 import _lib as L
-    cuobjdump = shutil.which("cuobjdump") or (CUDA_HOME and shutil.which("cuobjdump", path=os.path.join(CUDA_HOME, "bin")))
-    if not cuobjdump:
-        pytest.skip("cuobjdump not found (no CUDA toolkit)")
-    sass = subprocess.run([cuobjdump, "-sass", L.LIB_PATH], capture_output=True, text=True).stdout
-    sizes, name = {}, None
-    for line in sass.splitlines():
-        m = re.search(r"Function : (\S+)", line)
-        if m:
-            name = m.group(1)
-        elif name and re.match(r"\s+/\*[0-9a-f]+\*/\s+\S", line):
-            sizes[name] = sizes.get(name, 0) + 16
     budget = {"ILb1ELb0ELb0E": 54.0, "ILb1ELb1ELb0E": 67.875, "ILb0ELb0ELb0E": 63.375, "ILb0ELb1ELb0E": 79.625,
               "ILb1ELb0ELb1E": 76.5, "ILb1ELb1ELb1E": 88.875, "ILb0ELb0ELb1E": 86.125, "ILb0ELb1ELb1E": 101.375}
     for tmpl, kb in budget.items():
-        hit = [v for k, v in sizes.items() if "fo_metric_batch_select_kernel" in k and tmpl in k]
-        assert len(hit) == 1, (tmpl, sorted(sizes))
-        assert hit[0] <= (kb + 4) * 1024, (tmpl, hit[0])
+        size = size_of("fo_metric_batch_select_kernel", tmpl)
+        assert size <= (kb + 4) * 1024, (tmpl, size)
 
 
 # ---------------------------------------------------------------------------------------------------- GPU

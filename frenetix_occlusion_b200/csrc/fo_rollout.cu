@@ -11,6 +11,9 @@ namespace fo {
 
 constexpr int kMaxPathPts = 1024;
 constexpr unsigned kFullMask = 0xffffffffu;
+// a vertex closer than this to its predecessor is dropped: the heading of a (near-)zero chord is atan2 of rounding noise,
+// and it would enter the curvature and yaw of the neighbouring samples (route paths end in such chords)
+constexpr double kMinChord = 1e-3;
 
 struct FrenetState { double s, sd, d, dd; };
 
@@ -60,14 +63,34 @@ __global__ void __launch_bounds__(32) fo_rollout_path_kernel(const FoRolloutPath
   __shared__ float2 pts[kMaxPathPts];
   __shared__ double head[kMaxPathPts];     // heading of segment j (vertex j -> j + 1)
   const int job = blockIdx.x, lane = threadIdx.x;
-  const int off = k.path_off[job], np = min(k.path_off[job + 1] - off, kMaxPathPts);
+  const int off = k.path_off[job], n_in = min(k.path_off[job + 1] - off, kMaxPathPts);
   const size_t row = (size_t)job * k.t_stride;
+  int np = 0;
+  {   // stage the polyline without vertices closer than kMinChord to their input predecessor: ballot + prefix per chunk
+    const float2* src = reinterpret_cast<const float2*>(k.path_xy) + off;
+    for (int j0 = 0; j0 < n_in; j0 += 32) {
+      const int j = j0 + lane;
+      bool keep = false;
+      float2 p = make_float2(0.0f, 0.0f);
+      if (j < n_in) {
+        p = src[j];
+        keep = j == 0;
+        if (!keep) {
+          const float2 q = src[j - 1];
+          const double dx = (double)p.x - q.x, dy = (double)p.y - q.y;
+          keep = !(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) < kMinChord * kMinChord);
+        }
+      }
+      const unsigned kept = __ballot_sync(kFullMask, keep);
+      if (keep) pts[np + __popc(kept & ((1u << lane) - 1u))] = p;   // writes only at or below j: reads come from src
+      np += __popc(kept);
+    }
+  }
   if (np < 2) {
     if (lane == 0) k.sample[job] = -1;
     for (int i = lane; i < k.t_stride; i += 32) { k.x[row + i] = 0; k.y[row + i] = 0; k.yaw[row + i] = 0; k.vel[row + i] = 0; k.var_x[row + i] = 0; k.var_y[row + i] = 0; }
     return;
   }
-  for (int j = lane; j < np; j += 32) pts[j] = reinterpret_cast<const float2*>(k.path_xy)[off + j];
   __syncwarp();
   {   // arc length at every vertex: warp scan over chunks of 32 chords (a route path has up to 1024 vertices)
     double carry = 0.0;

@@ -592,7 +592,10 @@ typedef struct FoRolloutPathArgs {
   double dt, t1;               /* t1 = 3.0 (frenetix_handler.py:80) */
   double var0, var_factor;
   const float *path_xy;        /* dev [P_total, 2] reference polylines of all jobs, concatenated */
-  const int32_t *path_off;     /* dev [n_jobs + 1] offsets into path_xy (each path: 2..1024 points) */
+  const int32_t *path_off;     /* dev [n_jobs + 1] offsets into path_xy (each path: 2..1024 points).  A vertex j >= 1
+                                  whose chord to vertex j - 1 (float32 inputs, squared length in float64) is shorter
+                                  than 1 mm is dropped: repeated vertices do not change the rollout.  A path left with
+                                  fewer than 2 vertices gives sample -1 and zero rows */
   const double *x0, *y0, *v0;  /* dev [n_jobs] initial position and speed */
   float *x, *y, *yaw, *vel, *var_x, *var_y;   /* dev [n_jobs, t_stride] */
   int32_t *sample;             /* dev [n_jobs] selected sample 0..8 (speed-major), -1 = no valid projection */

@@ -182,12 +182,24 @@ def rollout_cv(x0, y0, v, phi, dt, horizon, var0=0.1, var_factor=1.05):
             "var": np.repeat((var0 * np.power(var_factor, k))[None], len(v), 0)}
 
 
+MIN_CHORD = 1e-3          # [m] fo_rollout.cu kMinChord
+
+
 def rollout_path(path, x0, y0, v0, dt, horizon, t1=3.0, var0=0.1, var_factor=1.05):
     """float64 restatement of the path-following vehicle rollout for ONE reference polyline
     (agent.py:364-426 + utils/frenetix_handler.py:66-125; the C++ frenetix arithmetic is restated from
     the published Werling quartic/quintic scheme -- PARITY UNPINNED).  ``path`` is rounded to float32
-    like the kernel input.  Returns dict of [T] arrays and the selected sample index."""
+    like the kernel input; vertices closer than ``MIN_CHORD`` to their predecessor are dropped, and a path left
+    with fewer than 2 vertices gives sample -1 and zero rows (as the kernel).  Returns dict of [T] arrays and the
+    selected sample index."""
     pts = np.asarray(path, dtype=np.float64).astype(np.float32).astype(np.float64).reshape(-1, 2)
+    # a vertex closer than MIN_CHORD to its input predecessor is dropped (the heading of a zero chord is atan2(0, 0))
+    dp = np.diff(pts, axis=0)
+    pts = pts[np.concatenate(([True], ~(dp[:, 0] * dp[:, 0] + dp[:, 1] * dp[:, 1] < MIN_CHORD * MIN_CHORD)))[:len(pts)]]
+    if len(pts) < 2:
+        T = int(horizon / dt) + 1
+        z = np.zeros(T)
+        return {"x": z, "y": z.copy(), "yaw": z.copy(), "v": z.copy(), "var": z.copy(), "sample": -1, "s0": 0.0, "d0": 0.0}
     seg = np.diff(pts, axis=0)
     ln = np.hypot(seg[:, 0], seg[:, 1])
     cum = np.concatenate(([0.0], np.cumsum(ln)))
@@ -272,6 +284,44 @@ def points_in_polygon(P, poly):
     with np.errstate(divide="ignore", invalid="ignore"):
         xin = (x1 - x0) * (y - y0) / (y1 - y0) + x0
     return (np.sum(cond & (x < xin), axis=1) % 2).astype(bool)
+
+
+def point_blockers(P, ego_xy, rect, flags, boundary, chunk=2048):
+    """First opaque thing the segment ego -> P meets (float64): the owner (obstacle index or HIT_BOUNDARY) of the
+    crossing with the smallest parameter along the segment (closed edges, first in edge order on ties), otherwise the
+    lowest-index opaque obstacle that contains P (closed), otherwise HIT_NONE.  Returns (blocker [M], t12 [M, 2]): t12
+    holds the segment parameters of the two nearest crossings (inf where there are fewer), so callers can tell
+    near-ties apart."""
+    P = np.asarray(P, dtype=np.float64).reshape(-1, 2) - np.asarray(ego_xy, dtype=np.float64)[:2]
+    segs, owner = _edges(ego_xy, rect, flags, boundary)
+    M = len(P)
+    out = np.full(M, HIT_NONE, dtype=np.int64)
+    t12 = np.full((M, 2), np.inf)
+    if len(segs):
+        ax, ay = segs[None, :, 0], segs[None, :, 1]
+        ex, ey = segs[None, :, 2] - ax, segs[None, :, 3] - ay
+        for c0 in range(0, M, chunk):
+            px, py = P[c0:c0 + chunk, 0:1], P[c0:c0 + chunk, 1:2]
+            D = px * ey - py * ex
+            with np.errstate(divide="ignore", invalid="ignore"):
+                t = (ax * ey - ay * ex) / D
+                u = (ax * py - ay * px) / D
+            t = np.where((D != 0) & (t >= 0) & (t <= 1) & (u >= 0) & (u <= 1), t, np.inf)
+            j = t.argmin(1)
+            hit = np.isfinite(t[np.arange(len(t)), j])
+            out[c0:c0 + chunk] = np.where(hit, owner[j], HIT_NONE)
+            t12[c0:c0 + chunk] = np.sort(t, 1)[:, :2] if t.shape[1] > 1 else np.concatenate((t, np.full_like(t, np.inf)), 1)
+    rect = np.asarray(rect, dtype=np.float64).reshape(-1, 5)
+    flags = np.asarray(flags).reshape(-1)
+    container = np.full(M, HIT_NONE, dtype=np.int64)
+    for o in range(len(rect) - 1, -1, -1):              # descending: the lowest index is written last
+        if not (flags[o] & RECT_EXISTS) or (flags[o] & RECT_TRANSPARENT):
+            continue
+        cs, sn = np.cos(rect[o, 2]), np.sin(rect[o, 2])
+        dx, dy = P[:, 0] - (rect[o, 0] - ego_xy[0]), P[:, 1] - (rect[o, 1] - ego_xy[1])
+        inside = (np.abs(dx * cs + dy * sn) <= rect[o, 3]) & (np.abs(-dx * sn + dy * cs) <= rect[o, 4])
+        container = np.where(inside, o, container)
+    return np.where(out == HIT_NONE, container, out), t12
 
 
 def classify_points(P, ego, rect, flags, boundary, polygons, sensor_radius, fov_deg, occluded_radius, focus=-1,

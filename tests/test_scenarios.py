@@ -198,42 +198,107 @@ def test_cuda_masks_equal_oracle_on_pipeline_predictions(cuda_device):
             assert list(results.keys()) == ["cp", "dce", "ttc", "hr", "be", "ttce", "wttc"]
 
 
+# Jitter radius of the explained-mismatch rule below.  The inputs are float32: coordinates up to 70 m carry half an ulp,
+# 3.8e-6 m; obstacle corners come from sincosf and float32 products at up to 70 m, within ~1e-5 m.  A shadow line
+# extends a corner that lies at least 3.5 m from the ego out to 70 m, 20x further, so its float32 image may sit up to
+# ~2e-4 m from the float64 line.  1 mm is five times that: a point the kernel and the float64 oracle disagree on must
+# have a neighbour within 1 mm on which the oracle gives the kernel's answer.
+PT_EPS = 1e-3
+PT_JITTER = PT_EPS * np.stack((np.cos(np.arange(8) * np.pi / 4), np.sin(np.arange(8) * np.pi / 4)), -1)
+# per-seed variations: 70 lanelet polygons (two with fewer than 3 vertices), the focus obstacle transparent or absent,
+# and point counts around the 256-thread block
+PT_VARIANTS = {27: {"polys": 70}, 28: {"focus": "transparent"}, 29: {"focus": -1}, 30: {"M": 1}, 31: {"M": 255},
+               32: {"M": 257}}
+
+
+def _many_polygons(rng):
+    """70 lanelet polygons: random convex-ish quads and triangles (bits 64..69 only reach ON_ROAD) plus a 2-vertex and a
+    1-vertex ring, which are never inside."""
+    polys = []
+    for k in range(68):
+        c = rng.uniform(-60, 60, 2)
+        ang = np.sort(rng.uniform(0, 2 * np.pi, 3 + k % 2))
+        rad = rng.uniform(4.0, 15.0, len(ang))
+        polys.append(c + np.stack((rad * np.cos(ang), rad * np.sin(ang)), -1))
+    polys.insert(20, np.array([[-30.0, -30.0], [30.0, 30.0]]))
+    polys.insert(66, np.array([[5.0, 5.0]]))
+    return polys
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("seed,n_obst,ring,fov", [(21, 40, True, 360.0), (22, 12, True, 120.0), (23, 200, False, 360.0),
-                                                  (24, 0, True, 360.0)])
+                                                  (24, 0, True, 360.0), (25, 300, True, 360.0), (26, 700, True, 360.0),
+                                                  (27, 40, True, 360.0), (28, 40, True, 200.0), (29, 40, True, 360.0),
+                                                  (30, 40, True, 360.0), (31, 40, True, 360.0), (32, 40, True, 360.0)])
 def test_cuda_point_classification_matches_oracle(seed, n_obst, ring, fov, cuda_device):
+    """fo_visibility_points against the float64 oracle: flags, lanelet bits and the blocker.  The obstacle edges are
+    staged in tiles of 1024 (300 obstacles and the ring: two tiles; 700: three, the last partial).  Every mismatch must
+    be explained: the oracle, evaluated within PT_EPS of the point, gives the kernel's answer."""
     from test_visibility import _frame
     from frenetix_occlusion_b200.visibility import FrameGeometry
     from oracle import visibility_oracle as VO
+    var = PT_VARIANTS.get(seed, {})
     ego, rect, flags, boundary = _frame(seed, n_obst, ring, transparent_every=5)
     rng = np.random.default_rng(seed)
     origin = np.array([103.25, -47.5])
     # three overlapping "lanelet" quads around the ego
     polys = [np.array([[-60, -6], [60, -6], [60, 6], [-60, 6.0]]), np.array([[-5, -60], [7, -60], [7, 60], [-5, 60.0]]),
              np.array([[10, 10], [45, 20], [40, 35], [5, 25.0]])]
-    M = 20000
+    if var.get("polys"):
+        polys = _many_polygons(rng)
+        assert len(polys) == var["polys"]
+    M = var.get("M", 20000)
     P = rng.uniform(-70, 70, (M, 2))
     f32 = lambda a: np.asarray(a, np.float64).astype(np.float32).astype(np.float64)  # noqa: E731
     rect, P, ego = f32(rect), f32(P), f32(ego)
+    polys = [f32(p) for p in polys]
     boundary = None if boundary is None else f32(boundary)
     rect_w = rect.copy()
     rect_w[:, :2] += origin
     frame = FrameGeometry(origin, ego[2], rect_w, flags, None if boundary is None else boundary + np.tile(origin, 2),
                           [p + origin for p in polys], 50.0, fov)
     focus = int(np.argmax(flags == 1)) if n_obst else -1
+    if var.get("focus") == "transparent":
+        focus = int(np.argmax(flags == VO.RECT_EXISTS | VO.RECT_TRANSPARENT))
+        assert flags[focus] & VO.RECT_TRANSPARENT
+    elif "focus" in var:
+        focus = var["focus"]
     gf, gb, gl = frame.classify(P + origin, focus_obstacle=focus, focus_margin=1.0)
-    of, ol = VO.classify_points(P, np.array([0.0, 0.0, ego[2]]), rect, flags, boundary, polys, 50.0, fov, 75.0, focus=focus,
-                                focus_margin=1.0)
-    assert np.array_equal(gl, ol) or (gl != ol).mean() < 1e-3
-    inside = (of & VO.PT_IN_OBSTACLE) != 0
-    for bit, name in ((VO.PT_IN_SENSOR, "in_sensor"), (VO.PT_ON_ROAD, "on_road"), (VO.PT_IN_OBSTACLE, "in_obstacle"),
-                      (VO.PT_VISIBLE, "visible"), (VO.PT_OCCLUDED, "occluded"), (VO.PT_FOCUS_SHADOW, "focus_shadow"),
-                      (VO.PT_FOCUS_NEAR, "focus_near")):
-        bad = ((gf & bit) != 0) != ((of & bit) != 0)
-        assert bad.mean() < 2e-3, (name, int(bad.sum()))          # float32 ties on region borders only
-    bad = (((gf & VO.PT_SHADOWED) != 0) != ((of & VO.PT_SHADOWED) != 0)) & ~inside
-    assert bad.mean() < 2e-3, int(bad.sum())
-    assert ((of & VO.PT_VISIBLE) != 0).sum() > 50 and ((of & VO.PT_OCCLUDED) != 0).sum() > 50
+    e3 = np.array([0.0, 0.0, ego[2]])
+
+    def oracle(Q):
+        f, lan = VO.classify_points(Q, e3, rect, flags, boundary, polys, 50.0, fov, 75.0, focus=focus, focus_margin=1.0)
+        # the segment ego -> point of a point inside an opaque obstacle crosses that obstacle's edge: the kernel calls it
+        # shadowed, where the reference's construction removes the obstacle itself
+        f = np.where((f & VO.PT_IN_OBSTACLE) != 0, f | VO.PT_SHADOWED, f).astype(np.uint32)
+        b, t12 = VO.point_blockers(Q, e3[:2], rect, flags, boundary)
+        return f, lan, b, t12
+
+    of, ol, ob, t12 = oracle(P)
+    gf = gf.astype(np.uint32)
+    fbad, lbad, bbad = gf ^ of, gl ^ ol, gb != ob
+    excused, unexcused = 0, []
+    for m in np.nonzero((fbad != 0) | (lbad != 0) | bbad)[0]:
+        jf, jl, jb, _ = oracle(P[m] + PT_JITTER)
+        ok = all(((jf & np.uint32(bit)) == (gf[m] & np.uint32(bit))).any() for bit in (1 << k for k in range(8)) if fbad[m] & bit)
+        ok &= all(((jl & np.uint64(1 << k)) == (gl[m] & np.uint64(1 << k))).any() for k in range(64) if int(lbad[m]) >> k & 1)
+        if bbad[m]:
+            # the two nearest crossings within PT_EPS of each other along the segment: either owner is right
+            near_tie = (t12[m, 1] - t12[m, 0]) * np.hypot(*P[m]) <= PT_EPS
+            ok &= bool(near_tie or (jb == gb[m]).any())
+        if ok:
+            excused += 1
+        else:
+            unexcused.append((int(m), P[m].tolist(), int(gf[m]), int(of[m]), int(gl[m]), int(ol[m]), int(gb[m]), int(ob[m])))
+    assert not unexcused, unexcused[:5]
+    assert excused <= 1e-3 * M, excused
+    print(f"seed {seed}: {excused} excused mismatches of {M} points (eps {PT_EPS} m)")
+    if M >= 20000 and n_obst <= 200 and not var:
+        assert ((of & VO.PT_VISIBLE) != 0).sum() > 50 and ((of & VO.PT_OCCLUDED) != 0).sum() > 50
+    if n_obst and M >= 20000:
+        assert (ob >= 0).sum() > 100 and (ob == VO.HIT_NONE).sum() > 100
+    if var.get("polys"):
+        assert (ol >> np.uint64(60)).any() and ((of & VO.PT_ON_ROAD) != 0).sum() > (ol != 0).sum()
 
 
 @pytest.mark.gpu

@@ -141,7 +141,9 @@ __global__ void __launch_bounds__(kVisThreads) fo_visibility_kernel(const FoVisi
           ax = b.x - ex0; ay = b.y - ey0; bx = b.z - ex0; by = b.w - ey0;
           own = FO_HIT_BOUNDARY;
           d2 = edge_dist2(ax, ay, bx, by);
-          keep = d2 <= R2;
+          // a border segment whose line passes through the ego (cross(a, e) == 0) could only block at range 0, and
+          // only the half-plane its listed direction faces: dropped, so the result does not depend on that direction
+          keep = d2 <= R2 && ax * (by - ay) - ay * (bx - ax) != 0.0f;
         }
       }
       const unsigned m = __ballot_sync(0xffffffffu, keep);
@@ -156,7 +158,9 @@ __global__ void __launch_bounds__(kVisThreads) fo_visibility_kernel(const FoVisi
           ax = bx; ay = by; exx = -exx; eyy = -eyy; tn = -tn;  // needs cross(d, e) > 0 and the ray test loses its
         }                                                    // sign products and absolute values
         sg[w] = make_float4(ax, ay, exx, eyy);
-        st[w] = make_float2(tn, __int_as_float(own));
+        // +0, never -0 (an edge through the ego): a range of -0 would be the largest key of the cast's unsigned
+        // warp maximum and end the walk of every ray of the warp
+        st[w] = make_float2(fabsf(tn), __int_as_float(own));
         // distance key: squared ego distance of the closest point, shrunk by 0.2 % and truncated to 8 mantissa bits
         // (both conservative); ring = its distance bin
         const int b = min(kVisBins - 1, (int)(sqrtf(d2) * bin_scale));

@@ -392,12 +392,16 @@ enum { FO_RECT_EXISTS = 1u << 0,        /* obstacle has a state at this time ste
 
 typedef struct FoVisibilityArgs {
   int32_t n_frames, n_rays, n_obstacles, n_boundary;
-  const float *ego;            /* dev [F, 3] (x, y, heading) */
+  const float *ego;            /* dev [F, 3] (x, y, heading); tested for headings in [-20 pi, 20 pi] */
   const float *rect;           /* dev [F, O, 5] (cx, cy, yaw, half_length, half_width): corner points as
-                                  helper_functions.py:99-112 */
+                                  helper_functions.py:99-112.  An ego standing exactly on a side is blocked at
+                                  range 0 by the rays that point to the box's side of it (at a corner: of either
+                                  side) and by no other ray; a zero-width box blocks both sides */
   const uint8_t *rect_flags;   /* dev [F, O] FO_RECT_* */
   const float *boundary;       /* dev [B, 4] (x1, y1, x2, y2) opaque road-border segments, world frame,
-                                  shared by all frames; may be NULL when n_boundary == 0 */
+                                  shared by all frames; may be NULL when n_boundary == 0.  A segment whose line
+                                  passes exactly through the ego (float32 cross(a - ego, b - a) == 0) is ignored:
+                                  an ego on a border segment is not blocked by it, whichever way it is listed */
   float sensor_radius;         /* occlusion.yaml:36 */
   float sensor_angle_deg;      /* occlusion.yaml:37 */
   float *range;                /* dev [F, R] first-hit distance, <= sensor_radius */

@@ -3,6 +3,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <vector>
 
@@ -274,18 +275,159 @@ extern "C" int fo_metric_bundle_host(const float* ego_host, int32_t n_traj, int3
   return FO_OK;
 }
 
-// fo_metric_batch_host and fo_metric_batch_host_corr.  corr: NULL = every table diagonal; else corr[p] != 0 = problem
-// p's table is a correlated one, its off-diagonal terms in cov_xy (host, aligned with ag->var_x / var_y).  The pack and
-// metric calls are the *_corr ones either way.
+namespace fo {
+
+// Page-locked host buffers of fo_metric_batch_host_select, per calling thread, grown on demand: `in` holds a round's
+// window table and, for pageable callers, the window rows the device reads; `out` receives a round's results.
+struct PinnedBuf {
+  unsigned char* p = nullptr;
+  size_t bytes = 0;
+};
+static thread_local PinnedBuf g_pin_in, g_pin_out;
+
+static int pin_reserve(PinnedBuf& b, size_t bytes) {
+  if (bytes <= b.bytes) return FO_OK;
+  if (b.p) FO_CUDA_TRY(cudaFreeHost(b.p));
+  b.p = nullptr; b.bytes = 0;
+  const size_t want = bytes + bytes / 4 > 4096 ? bytes + bytes / 4 : 4096;
+  FO_CUDA_TRY(cudaMallocHost(&b.p, want));
+  b.bytes = want;
+  return FO_OK;
+}
+
+// The rounds of fo_metric_batch_host_select (DESIGN.md 5.15), after the agents are packed: b is the whole batch with the
+// library's arena in place (problems pr = b->problems, n_run of them with rows, the fewest agents among those a_min);
+// corr / veh per problem (corr NULL = none correlated); d_e32 room for n_traj float32 rows, d_win for n_run windows,
+// d_res for n_traj result rows and n_run selections.
+static int host_select_rounds(const char* fn, const double* ego_host, const double* origins_host,
+                              const FoMetricBatchArgs* b, int n_run, int a_min, const uint8_t* corr, const FoVehicle* veh,
+                              float* d_e32, IngestWindow* d_win, unsigned char* d_res, int32_t* out_selected,
+                              uint8_t* out_valid, float* out_summary, uint32_t* out_flags) {
+  const FoMetricArgs& c = b->common;
+  const int P = b->n_problems, T = c.n_states;
+  const FoBatchProblem* pr = b->problems;
+  const size_t row_elems = (size_t)T * 5;
+  cudaStream_t st = g_ws.stream;
+  // every round's team size and shape classes are those fo_metric_batch_host_corr picks for the whole batch
+  int W = 1, teams = 1;
+  int rc = batch_team_shape(c.n_traj, T, a_min, &W, &teams);
+  if (rc != FO_OK) return rc;
+  // page-locked or registered rows are read in place; pageable ones are copied window by window into g_pin_in
+  const double* mapped = nullptr;
+  {
+    cudaPointerAttributes at{};
+    if (cudaPointerGetAttributes(&at, ego_host) == cudaSuccess && at.devicePointer)
+      mapped = static_cast<const double*>(at.devicePointer);
+    cudaGetLastError();
+  }
+  // round 0 gives every problem w0 ranks: together at least one per resident team
+  const int w0 = std::max(32, (teams + n_run - 1) / n_run);
+  std::vector<int> active, start(P, 0), next_len(P, w0);
+  for (int p = 0; p < P; ++p) {
+    out_selected[p] = pr[p].n_traj;                  // N_p; 0 for a problem without rows
+    if (pr[p].n_traj > 0) active.push_back(p);
+  }
+  memset(out_valid, FO_VALID_SKIPPED, (size_t)c.n_traj);
+  std::vector<FoBatchProblem> wp;
+  std::vector<uint8_t> wcorr;
+  std::vector<FoVehicle> wveh;
+  const size_t tab_bytes = ((size_t)n_run * sizeof(IngestWindow) + 255) & ~(size_t)255;
+  while (!active.empty()) {
+    const int n_win = (int)active.size();
+    // ---- the window table: problem p's ranks [start, start + len) become compact rows [rows, rows + len)
+    int rows = 0;
+    for (int i = 0; i < n_win; ++i) {
+      const int p = active[i];
+      rows += std::min(next_len[p], pr[p].n_traj - start[p]);
+    }
+    rc = pin_reserve(g_pin_in, tab_bytes + (mapped ? 0 : (size_t)rows * row_elems * sizeof(double)));
+    if (rc != FO_OK) return rc;
+    IngestWindow* win = reinterpret_cast<IngestWindow*>(g_pin_in.p);
+    double* staged = reinterpret_cast<double*>(g_pin_in.p + tab_bytes);
+    wp.assign(n_win, FoBatchProblem{});
+    wcorr.assign(n_win, 0);
+    wveh.assign(n_win, FoVehicle{});
+    for (int i = 0, at = 0; i < n_win; ++i) {
+      const int p = active[i];
+      const int len = std::min(next_len[p], pr[p].n_traj - start[p]);
+      const long long src_row = pr[p].traj_begin + start[p];
+      if (!mapped) memcpy(staged + (size_t)at * row_elems, ego_host + (size_t)src_row * row_elems, (size_t)len * row_elems * 8);
+      win[i] = IngestWindow{mapped ? src_row : at, at, len, make_double2(origins_host[2 * p], origins_host[2 * p + 1])};
+      wp[i] = pr[p];
+      wp[i].traj_begin = at;
+      wp[i].n_traj = len;
+      wcorr[i] = corr ? corr[p] : 0;
+      wveh[i] = veh[p];
+      at += len;
+    }
+    // ---- the window rows in float32, then the select launches over them (one descriptor per window)
+    FO_CUDA_TRY(cudaMemcpyAsync(d_win, win, (size_t)n_win * sizeof(IngestWindow), cudaMemcpyHostToDevice, st));
+    const double* src = mapped;
+    if (!mapped) FO_CUDA_TRY(cudaHostGetDevicePointer((void**)&src, staged, 0));
+    rc = launch_ego_window_ingest(src, d_e32, rows, T, d_win, n_win, st);
+    if (rc != FO_OK) return rc;
+    // results of the round back to back, for one read-back: summary, flags, selections, valid bytes
+    const size_t sum_bytes = out_summary ? (size_t)rows * FO_SUMMARY_K * 4 : 0, flag_bytes = out_flags ? (size_t)rows * 4 : 0;
+    const size_t sel_off = sum_bytes + flag_bytes, valid_off = sel_off + (size_t)n_win * 4, res_bytes = valid_off + rows;
+    FoMetricBatchArgs rb = *b;
+    rb.common.ego = d_e32;
+    rb.common.n_traj = rows;
+    rb.common.summary = out_summary ? reinterpret_cast<float*>(d_res) : nullptr;
+    rb.common.flags = out_flags ? reinterpret_cast<uint32_t*>(d_res + sum_bytes) : nullptr;
+    rb.common.valid = d_res + valid_off;
+    rb.n_problems = n_win;
+    rb.problems = wp.data();
+    rc = metric_batch_select_w(fn, &rb, corr ? wcorr.data() : nullptr, wveh.data(), W,
+                               reinterpret_cast<int32_t*>(d_res + sel_off), st);
+    if (rc != FO_OK) return rc;
+    rc = pin_reserve(g_pin_out, res_bytes);
+    if (rc != FO_OK) return rc;
+    FO_CUDA_TRY(cudaMemcpyAsync(g_pin_out.p, d_res, res_bytes, cudaMemcpyDeviceToHost, st));
+    FO_CUDA_TRY(cudaStreamSynchronize(st));
+    // ---- scatter: an assessed row's results go to its place; a window with a valid row finishes its problem
+    const float* h_sum = reinterpret_cast<const float*>(g_pin_out.p);
+    const uint32_t* h_flags = reinterpret_cast<const uint32_t*>(g_pin_out.p + sum_bytes);
+    const int32_t* h_sel = reinterpret_cast<const int32_t*>(g_pin_out.p + sel_off);
+    const uint8_t* h_valid = g_pin_out.p + valid_off;
+    int kept = 0;
+    for (int i = 0; i < n_win; ++i) {
+      const int p = active[i], at = (int)wp[i].traj_begin, len = wp[i].n_traj;
+      const size_t dst = (size_t)pr[p].traj_begin + start[p];
+      for (int r = 0; r < len; ++r) {
+        const uint8_t v = h_valid[at + r];
+        out_valid[dst + r] = v;
+        if (v == FO_VALID_SKIPPED) continue;
+        if (out_summary) memcpy(out_summary + (dst + r) * FO_SUMMARY_K, h_sum + (size_t)(at + r) * FO_SUMMARY_K, FO_SUMMARY_K * 4);
+        if (out_flags) out_flags[dst + r] = h_flags[at + r];
+      }
+      if (h_sel[i] < len) {
+        out_selected[p] = start[p] + h_sel[i];
+      } else if (start[p] + len < pr[p].n_traj) {      // no valid row in the window: the next, four times longer
+        start[p] += len;
+        next_len[p] = (int)std::min<long long>(4ll * next_len[p], pr[p].n_traj);
+        active[kept++] = p;
+      }
+    }
+    active.resize(kept);
+  }
+  return FO_OK;
+}
+
+}  // namespace fo
+
+// fo_metric_batch_host, fo_metric_batch_host_corr and (select) fo_metric_batch_host_select.  corr: NULL = every table
+// diagonal; else corr[p] != 0 = problem p's table is a correlated one, its off-diagonal terms in cov_xy (host, aligned
+// with ag->var_x / var_y).  The pack and metric calls are the *_corr ones either way.
 static int metric_batch_host_impl(const char* fn, const double* ego_host, int32_t n_traj, int32_t n_states,
                                   const double* origins_host, const FoAgentsRaw* ag, const float* cov_xy, int32_t n_problems,
                                   const FoBatchProblem* problems_host, const uint8_t* corr, const FoVehicle* vehicles_host,
                                   const FoMetricArgs* params, uint8_t* out_valid, float* out_summary, uint32_t* out_flags,
-                                  float* out_pair, float* out_step) {
+                                  float* out_pair, float* out_step, bool select = false, int32_t* out_selected = nullptr) {
   const int P = n_problems;
   // ---- every check before any device work
   if (!params) { fo::set_error("%s: NULL params", fn); return FO_ERR_INVALID_ARG; }
   if (params->n_peers != 0) { fo::set_error("%s: peer stores exist on the device entry points only", fn); return FO_ERR_UNSUPPORTED; }
+  if (select && P > 0 && !out_selected) { fo::set_error("%s: out_selected must not be NULL with %d problems", fn, P); return FO_ERR_INVALID_ARG; }
   if (P > 0 && (!problems_host || !origins_host || !ag)) {
     fo::set_error("%s: NULL problems / origins / agents with %d problems", fn, P);
     return FO_ERR_INVALID_ARG;
@@ -339,24 +481,28 @@ static int metric_batch_host_impl(const char* fn, const double* ego_host, int32_
       }
     }
   }
-  if (n_traj == 0) return FO_OK;
+  if (n_traj == 0) {                             // every N_p is 0
+    for (int q = 0; select && q < P; ++q) out_selected[q] = 0;
+    return FO_OK;
+  }
 
   // ---- workspace: float64 rows, float32 bundle, raw agents (with cov_xy when correlated), arena, per-problem ingest
-  // table, outputs
+  // table, outputs (select: no float64 rows; a window table, and the outputs hold one round's results in one block)
   const size_t N = n_traj, T = n_states, A = ag->n_agents, S = ag->t_stride;
   long long pairs = 0;                           // sum of N_p A_p: the rows of the pair / step blocks
   for (int p = 0; p < P; ++p) pairs += (long long)pr[p].n_traj * pr[p].n_agents;
   // as MetricEngine.assess_batch: with no pair or step left to write the summary path runs
   const bool want_pair = out_pair && pairs > 0, want_step = out_step && pairs > 0 && T > 1;
   auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-  const size_t b_e64 = al(N * T * 5 * 8), b_e32 = al(N * T * 5 * 4), b_f = al(A * S * 4), b_a = al(A * 4 + 4);
+  const size_t b_e64 = select ? 0 : al(N * T * 5 * 8), b_e32 = al(N * T * 5 * 4), b_f = al(A * S * 4), b_a = al(A * 4 + 4);
   const size_t b_first = ((size_t)n_run * 4 + 15) & ~(size_t)15, b_idx = al(b_first + (size_t)n_run * 16);
   const size_t b_arena = al(arena_bytes), b_valid = al(N), b_sum = al(N * FO_SUMMARY_K * 4), b_flags = al(N * 4);
   const size_t b_pair = want_pair ? al((size_t)pairs * FO_PAIR_K * 4) : 0;
   const size_t b_step = want_step ? al((size_t)pairs * (T - 1) * FO_STEP_K * 4) : 0;
   const size_t b_cov = corr ? b_f : 0;
+  const size_t b_win = select ? al((size_t)n_run * sizeof(fo::IngestWindow)) : 0, b_sel = select ? al((size_t)n_run * 4) : 0;
   rc = fo::ws_reserve(b_e64 + b_e32 + 6 * b_f + b_cov + 6 * b_a + b_idx + b_arena + b_valid + b_sum + b_flags + b_pair +
-                      b_step);
+                      b_step + b_win + b_sel);
   if (rc != FO_OK) return rc;
   cudaStream_t st = fo::g_ws.stream;
   char* p = (char*)fo::g_ws.dev;
@@ -407,6 +553,15 @@ static int metric_batch_host_impl(const char* fn, const double* ego_host, int32_
     rc = fo_agents_pack_batch_corr(&d, n_corr ? d_cov : nullptr, P, pr.data(), corr_flags, veh, d_arena, arena_bytes, st);
     if (rc != FO_OK) return fo::ws_fail(rc);
   }
+  b.common.agent_table = arena_bytes ? d_arena : nullptr;
+  if (select) {                                  // rank windows in rounds instead of every row at once
+    fo::IngestWindow* d_win = (fo::IngestWindow*)take(b_win);
+    unsigned char* d_res = (unsigned char*)take(b_valid + b_sum + b_flags + b_sel);
+    rc = fo::host_select_rounds(fn, ego_host, origins_host, &b, n_run, a_min, corr, veh, d_e32, d_win, d_res, out_selected,
+                                out_valid, out_summary, out_flags);
+    if (rc != FO_OK) return fo::ws_fail(rc);
+    return FO_OK;
+  }
 
   // ---- ego: chunk k+1 crosses PCIe on the copy stream while chunk k is converted on the compute stream
   const size_t row_bytes = T * 5 * 8;
@@ -426,7 +581,6 @@ static int metric_batch_host_impl(const char* fn, const double* ego_host, int32_
 
   // ---- the batch call itself, after the last chunk is converted (one W for the whole batch)
   b.common.ego = d_e32;
-  b.common.agent_table = arena_bytes ? d_arena : nullptr;
   b.common.valid = (uint8_t*)take(b_valid);
   b.common.summary = (float*)take(b_sum);
   b.common.flags = (uint32_t*)take(b_flags);
@@ -468,4 +622,14 @@ extern "C" int fo_metric_batch_host_corr(const double* ego_host, int32_t n_traj,
   // (with no problems there is nothing to assess: NULL flags reach no pack or metric call)
   return metric_batch_host_impl(fn, ego_host, n_traj, n_states, origins_host, ag, cov_xy_host, n_problems, problems_host,
                                 corr_host, vehicles_host, params, out_valid, out_summary, out_flags, out_pair, out_step);
+}
+
+extern "C" int fo_metric_batch_host_select(const double* ego_host, int32_t n_traj, int32_t n_states,
+                                           const double* origins_host, const FoAgentsRaw* ag, const float* cov_xy_host,
+                                           int32_t n_problems, const FoBatchProblem* problems_host, const uint8_t* corr_host,
+                                           const FoVehicle* vehicles_host, const FoMetricArgs* params, int32_t* out_selected,
+                                           uint8_t* out_valid, float* out_summary, uint32_t* out_flags) {
+  return metric_batch_host_impl("fo_metric_batch_host_select", ego_host, n_traj, n_states, origins_host, ag, cov_xy_host,
+                                n_problems, problems_host, corr_host, vehicles_host, params, out_valid, out_summary,
+                                out_flags, nullptr, nullptr, true, out_selected);
 }

@@ -26,6 +26,25 @@ int check_pack_batch(const char* fn, const FoAgentsRaw* raw, int32_t n_problems,
 int launch_ego_ingest(const double* src, float* dst, int row0, int n_rows, int T, const int* first_dev,
                       const double2* origin_dev, int n_first, cudaStream_t st);
 
+// fo_metric_batch_host_select's ingest of one round: window w takes the n_rows float64 rows from row src_row of src and
+// writes them as float32 rows from row dst_row of dst, shifted by origin as launch_ego_ingest shifts them.  The windows'
+// dst_row ranges are contiguous and increasing from 0 and together cover [0, n_rows).  One launch (fo_metric.cu).
+struct __align__(16) IngestWindow {
+  long long src_row;
+  int dst_row, n_rows;
+  double2 origin;
+};
+int launch_ego_window_ingest(const double* src, float* dst, int n_rows, int T, const IngestWindow* win_dev, int n_win,
+                             cudaStream_t st);
+
+// The team size W fo_metric_batch[_corr] picks for a batch of n_traj rows of T states whose problems with rows have at
+// least a_min agents, and the number of such teams resident on the current device at once.
+int batch_team_shape(int n_traj, int T, int a_min, int* W, int* resident_teams);
+// fo_metric_batch_select with the team size fixed to W (and the shape classes it implies) instead of the one picked
+// from the batch's own rows; fn names the entry point in the messages.
+int metric_batch_select_w(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles,
+                          int W, int32_t* selected_dev, cudaStream_t st);
+
 #define FO_CUDA_TRY(expr)                                                                      \
   do {                                                                                         \
     cudaError_t _e = (expr);                                                                   \

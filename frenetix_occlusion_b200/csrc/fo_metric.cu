@@ -198,6 +198,19 @@ static void launch_corr(const FoAgentsRaw& raw, const float* cov_xy, const PackP
 // 4-byte stores.
 constexpr int kIngestThreads = 256, kIngestTileRows = 256;
 
+// One element of an ego row: column col of (x, y, theta, v, a); org points at the row's problem origin, read only for x
+// and y.  The one conversion of both ingest kernels.
+__device__ __forceinline__ float ingest_elem(double v, int col, const double2* org) {
+  float o;
+  if (col < 2) {
+    const double2 g = *org;
+    o = __double2float_rn(__dsub_rn(v, col == 0 ? g.x : g.y));
+  } else {
+    o = __double2float_rn(v);
+  }
+  return o;
+}
+
 __global__ void __launch_bounds__(kIngestThreads)
 fo_ego_ingest_kernel(const double* __restrict__ src, float* __restrict__ dst, int row0, int n_rows, int row_elems,
                      int tile_rows, const int* __restrict__ first, const double2* __restrict__ origin, int n_first) {
@@ -213,14 +226,7 @@ fo_ego_ingest_kernel(const double* __restrict__ src, float* __restrict__ dst, in
     for (int j = threadIdx.x; j < m; j += kIngestThreads) {
       const double v = s[j];
       const int col = j % 5;                     // row_elems = 5 T: every row starts at a multiple of 5
-      float o;
-      if (col < 2) {
-        const double2 g = org[j / row_elems];
-        o = __double2float_rn(__dsub_rn(v, col == 0 ? g.x : g.y));
-      } else {
-        o = __double2float_rn(v);
-      }
-      d[j] = o;
+      d[j] = ingest_elem(v, col, org + j / row_elems);
     }
     __syncthreads();
   }
@@ -235,6 +241,58 @@ int launch_ego_ingest(const double* src, float* dst, int row0, int n_rows, int T
   const int n_tiles = (n_rows + tile_rows - 1) / tile_rows;
   fo_ego_ingest_kernel<<<min(n_tiles, 4096), kIngestThreads, 0, st>>>(src, dst, row0, n_rows, row_elems, tile_rows,
                                                                      first_dev, origin_dev, n_first);
+  count_launch();
+  FO_CUDA_TRY(cudaGetLastError());
+  return FO_OK;
+}
+
+// fo_metric_batch_host_select's ingest: the rank windows of one round, each a run of float64 rows (src: host memory
+// through its mapped device address) converted into a run of compact float32 rows.  The arithmetic is ingest_elem's, so
+// a row's float32 values equal fo_ego_ingest_kernel's.  A CTA takes a tile of whole compact rows, finds each row's
+// window and source row once, then streams the tile: coalesced 8-byte loads within each row and 4-byte stores.
+__device__ __forceinline__ int find_window(const IngestWindow* __restrict__ win, int n_win, int row) {
+  int lo = 0, hi = n_win - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (__ldg(&win[mid].dst_row) <= row) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+__global__ void __launch_bounds__(kIngestThreads)
+fo_ego_window_ingest_kernel(const double* __restrict__ src, float* __restrict__ dst, int n_rows, int row_elems,
+                            int tile_rows, const IngestWindow* __restrict__ win, int n_win) {
+  __shared__ double2 org[kIngestTileRows];
+  __shared__ long long base[kIngestTileRows];      // source element of each row's first value
+  const int n_tiles = (n_rows + tile_rows - 1) / tile_rows;
+  for (int t = blockIdx.x; t < n_tiles; t += gridDim.x) {
+    const int r_lo = t * tile_rows, rows = min(tile_rows, n_rows - r_lo);
+    if ((int)threadIdx.x < rows) {
+      const int row = r_lo + threadIdx.x;
+      const IngestWindow* w = win + find_window(win, n_win, row);
+      org[threadIdx.x] = __ldg(&w->origin);
+      base[threadIdx.x] = (__ldg(&w->src_row) + (row - __ldg(&w->dst_row))) * row_elems;
+    }
+    __syncthreads();
+    float* d = dst + (size_t)r_lo * row_elems;
+    const int m = rows * row_elems;
+    for (int j = threadIdx.x; j < m; j += kIngestThreads) {
+      const int r = j / row_elems;
+      const double v = src[base[r] + (j - r * row_elems)];
+      d[j] = ingest_elem(v, j % 5, org + r);     // row_elems = 5 T: every row starts at a multiple of 5
+    }
+    __syncthreads();
+  }
+}
+
+int launch_ego_window_ingest(const double* src, float* dst, int n_rows, int T, const IngestWindow* win_dev, int n_win,
+                             cudaStream_t st) {
+  if (n_rows <= 0) return FO_OK;
+  const int row_elems = 5 * T;
+  const int tile_rows = max(1, min(kIngestTileRows, 2048 / row_elems));   // as launch_ego_ingest
+  const int n_tiles = (n_rows + tile_rows - 1) / tile_rows;
+  fo_ego_window_ingest_kernel<<<min(n_tiles, 4096), kIngestThreads, 0, st>>>(src, dst, n_rows, row_elems, tile_rows,
+                                                                            win_dev, n_win);
   count_launch();
   FO_CUDA_TRY(cudaGetLastError());
   return FO_OK;
@@ -706,12 +764,13 @@ struct BatchStage {
 // vehicles: problem p's ego vehicle is vehicles[p]; NULL = common.vehicle for every problem.  corr: problem p's table is a
 // correlated one when corr[p] != 0; NULL = none is.  by_size: within a class the descriptors are sorted by N_p in
 // descending order (stable), else they are in problem order.  Stages first[] of all classes, then their descriptors
-// (16-byte aligned), class by class, and reserves extra_bytes behind them; the caller uploads.
+// (16-byte aligned), class by class, and reserves extra_bytes behind them; the caller uploads.  team_warps > 0 fixes W
+// (fo_metric_batch_host_select's rounds take the W of the whole batch), else it is picked from this batch.
 static int stage_batch(const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles, int n_run, int a_min,
-                       int num_sms, bool by_size, size_t extra_bytes, BatchStage& s) {
+                       int num_sms, bool by_size, size_t extra_bytes, int team_warps, BatchStage& s) {
   const FoMetricArgs& c = b->common;
   const int P = b->n_problems;
-  s.W = fo::pick_team_warps(c.n_traj, c.n_states, a_min, num_sms);
+  s.W = team_warps > 0 ? team_warps : fo::pick_team_warps(c.n_traj, c.n_states, a_min, num_sms);
   const auto class_of = [&](int p) {
     return (corr && corr[p] ? 2 : 0) + (s.W == 1 && fo::lane_group_log2(b->problems[p].n_agents) == 5 ? 0 : 1);
   };
@@ -763,9 +822,9 @@ static void batch_kargs(const FoMetricArgs& c, fo::MetricKArgs& k) {
 
 // select (fo_metric_batch_select): the descriptors are sorted by N_p within each class, and staged behind them are the
 // rank segments of every class (at most one per descriptor), the problem index of each descriptor and N_p of every
-// problem, which is copied into selected_dev before the launches.
+// problem, which is copied into selected_dev before the launches.  team_warps as in stage_batch.
 static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles,
-                             bool select, int32_t* selected_dev, void* stream) {
+                             bool select, int32_t* selected_dev, void* stream, int team_warps = 0) {
   int n_run = 0, a_min = 0;
   {
     const int rc = fo::check_batch(fn, b, corr, false, &n_run, &a_min);
@@ -787,7 +846,7 @@ static int metric_batch_impl(const char* fn, const FoMetricBatchArgs* b, const u
   const size_t out_bytes = select ? ((size_t)n_run * sizeof(int) + 15) & ~(size_t)15 : 0;
   const size_t init_bytes = select ? (size_t)P * sizeof(int32_t) : 0;
   BatchStage s;
-  int rc = stage_batch(b, corr, vehicles, n_run, a_min, num_sms, select, seg_bytes + out_bytes + init_bytes, s);
+  int rc = stage_batch(b, corr, vehicles, n_run, a_min, num_sms, select, seg_bytes + out_bytes + init_bytes, team_warps, s);
   if (rc != FO_OK) return rc;
   // class cl: descriptors start[cl] .. with N descending; the ranks in [N of descriptor m, N of descriptor m - 1) have
   // the first m descriptors active
@@ -977,4 +1036,18 @@ extern "C" int fo_metric_batch_detail_corr(const FoMetricBatchArgs* b, const uin
 extern "C" int fo_metric_batch_select(const FoMetricBatchArgs* b, const uint8_t* corr_host, const FoVehicle* vehicles_host,
                                       int32_t* selected_dev, void* stream) {
   return metric_batch_impl("fo_metric_batch_select", b, corr_host, vehicles_host, true, selected_dev, stream);
+}
+
+int fo::batch_team_shape(int n_traj, int T, int a_min, int* W, int* resident_teams) {
+  int num_sms = 0;
+  const int rc = num_sms_of_current_device(&num_sms);
+  if (rc != FO_OK) return rc;
+  *W = fo::pick_team_warps(n_traj, T, a_min, num_sms);
+  *resident_teams = fo::resident_teams(*W, num_sms);
+  return FO_OK;
+}
+
+int fo::metric_batch_select_w(const char* fn, const FoMetricBatchArgs* b, const uint8_t* corr, const FoVehicle* vehicles,
+                              int W, int32_t* selected_dev, cudaStream_t st) {
+  return metric_batch_impl(fn, b, corr, vehicles, true, selected_dev, st, W);
 }

@@ -889,5 +889,6 @@ int launch_metric_batch(const MetricKArgs& k, int num_sms, int W, bool uni, cons
                         cudaStream_t st);
 int lane_group_log2(int A);                                  // team shape: a warp holds 1 << lg agents
 int pick_team_warps(int N, int T, int A, int num_sms);       // team size W (FO_TEAM_WARPS overrides)
+int resident_teams(int W, int num_sms);                      // teams of W warps resident on the device at once
 
 }  // namespace fo

@@ -957,6 +957,9 @@ int pick_team_warps(int N, int T, int A, int num_sms) {
   return w;
 }
 
+// Teams of W warps resident at once: the warp slots pick_team_warps shares out.
+int resident_teams(int W, int num_sms) { return num_sms * 8 * FO_SW_MINB / (W > 0 ? W : 1); }
+
 // Claim counters: one 4-byte slot per launch, zeroed in-stream before the kernel.  Eager launches rotate through a ring
 // (a slot is reused kClaimRing launches later); a launch recorded into a CUDA graph keeps a slot of its own for the
 // life of the process, because the graph may be replayed while later eager launches are in flight.  When the graph

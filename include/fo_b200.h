@@ -376,6 +376,33 @@ int fo_metric_batch_host_corr(const double *ego_host, int32_t n_traj, int32_t n_
                               const FoVehicle *vehicles_host, const FoMetricArgs *params, uint8_t *out_valid,
                               float *out_summary, uint32_t *out_flags, float *out_pair, float *out_step);
 
+/* fo_metric_batch_select from HOST buffers: the first valid row of every problem, for a host-memory embedder whose
+ * planner takes the first candidate of a cost-ordered list that passes.  The inputs are fo_metric_batch_host_corr's,
+ * except that corr_host may be NULL (no problem is correlated) and cov_xy_host may be NULL when no flagged problem has
+ * agents.
+ *   out_selected  HOST int32 [n_problems]: what fo_metric_batch_select writes for the same problems on the bundle
+ *                 fo_metric_batch_host's ingest produces -- problem p's smallest rank whose valid byte
+ *                 fo_metric_batch_host_corr writes as 1, or N_p when there is none (0 for N_p = 0; a problem without
+ *                 agents or metrics gets 0)
+ *   out_valid     every byte is written.  A row that is assessed equals fo_metric_batch_host_corr's row bit for bit in
+ *                 valid, summary and flags; every other row gets valid = FO_VALID_SKIPPED and its out_summary /
+ *                 out_flags entries are left unwritten.  out_summary / out_flags may be NULL
+ * Rows cross PCIe only as far as the selection needs them.  The call assesses rank windows in rounds: round 0 ranks
+ * [0, w0) of every problem with rows, and each later round the next window, four times longer than the last, of every
+ * problem whose windows held no valid row yet.  Every round uses the team size and shape classes that
+ * fo_metric_batch_host_corr picks for the whole batch, so its rows are that call's.  Rows of a page-locked ego_host
+ * (cudaMallocHost / cudaHostAlloc, or cudaHostRegister over the whole array) are read by the device in place; pageable
+ * rows are first copied, window by window, into a library-owned page-locked buffer (per calling thread, grown on
+ * demand).  One synchronise per round.
+ * Checks as in fo_metric_batch_host_corr, with its messages, the covariance check included; n_peers != 0 is
+ * FO_ERR_UNSUPPORTED, and a NULL out_selected with n_problems > 0 is FO_ERR_INVALID_ARG.  There are no pair / step
+ * outputs.  All checks run before any device work.  Synchronous; device workspace as fo_metric_batch_host's. */
+int fo_metric_batch_host_select(const double *ego_host, int32_t n_traj, int32_t n_states, const double *origins_host,
+                                const FoAgentsRaw *agents_host, const float *cov_xy_host, int32_t n_problems,
+                                const FoBatchProblem *problems_host, const uint8_t *corr_host,
+                                const FoVehicle *vehicles_host, const FoMetricArgs *params, int32_t *out_selected,
+                                uint8_t *out_valid, float *out_summary, uint32_t *out_flags);
+
 
 /* ---- stage 1: sensor visibility by ray casting ----------------------------------------------------
  * Replaces SensorModel.calc_visible_and_occluded_area (sensor_model.py:41-193): the reference clips
